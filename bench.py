@@ -41,6 +41,8 @@ SEED0 = 1000
 LEVELS = (1, 2)
 METRIC = "xpng encode+decode MPix/s at levels -1/-2 over a 1080p frame batch"
 REF_SAMPLE = 64
+DUMP_FILE_BYTES = 1 << 22      # --dump-outputs: sampled file bytes per level (16 MiB as float32)
+DUMP_PIXEL_BYTES = 1 << 21     # --dump-outputs: sampled decoded bytes per level (8 MiB as float32)
 
 
 def peaks():
@@ -261,7 +263,7 @@ def run_reference(args, rank, world):
     from xpng_b200 import synth
     nf = min(args.frames, REF_SAMPLE)
     frames = synth.sintel_batch(range(SEED0, SEED0 + nf))
-    steps = max(1, min(args.steps, 10))
+    steps = args.steps
     per_step, calls, kind, cores, how = reference_steps(frames, steps, args.warmup)
     npx = nf * FW * FH
     value = 4 * npx / 1e6 / per_step
@@ -275,6 +277,34 @@ def run_reference(args, rank, world):
             "e2e": {"value": round(value, 2), "unit": "MPix/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "breakdown": call_table(calls, npx)}
     print(json.dumps(line), flush=True)
+
+
+def _sample_positions(n, k, seed):
+    """Every position below n when n <= k, else k fixed, seeded positions in increasing order."""
+    return np.arange(n, dtype=np.int64) if n <= k else np.sort(np.random.default_rng(seed).integers(0, n, k, dtype=np.int64))
+
+
+def dump_outputs(out_dir, files, back, offs, sizes, npx_bytes):
+    """Write what a step handed back, per level L, as .npy files under out_dir (about 50 MB in all):
+    L<L>_sizes / L<L>_offsets (float64): every file's size and its offset in the file arena;
+    L<L>_file_bytes (float32): the files of all frames concatenated in frame order, every byte or a fixed seeded sample;
+    L<L>_decoded_pixels (float32): the decoded pixel arena, every byte or a fixed seeded sample.
+    The inputs depend on the arguments only, so two builds run with the same arguments can be compared file for file."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+
+    def take(t, idx):
+        return t[torch.from_numpy(idx).to(t.device)].float().cpu().numpy()
+    for lv in LEVELS:
+        sz, of = np.asarray(sizes[lv], np.int64), np.asarray(offs[lv], np.int64)
+        starts = np.cumsum(sz) - sz                              # where each file begins in the concatenation
+        pos = _sample_positions(int(sz.sum()), DUMP_FILE_BYTES, lv)
+        k = np.searchsorted(starts, pos, side="right") - 1
+        out = {"sizes": sz.astype(np.float64), "offsets": of.astype(np.float64),
+               "file_bytes": take(files[lv], of[k] + (pos - starts[k])),
+               "decoded_pixels": take(back[lv], _sample_positions(npx_bytes, DUMP_PIXEL_BYTES, 100 + lv))}
+        for name, a in out.items():
+            np.save(os.path.join(out_dir, f"L{lv}_{name}.npy"), a)
 
 
 def workload_config(frames, world):
@@ -449,6 +479,8 @@ def run_ours(args, rank, world, local_rank):
     for lv in LEVELS:
         if n:
             assert torch.equal(d_back[lv][:total], d_px[:total]), f"rank {rank} level {lv}: decoded pixels differ after the timed steps"
+    if args.dump_outputs and rank == 0:                       # before the legs below overwrite the arenas
+        dump_outputs(args.dump_outputs, d_files, d_back, state["offs"], state["sizes"], total)
     # the same step with the two level jobs one after the other: per-call device-resident times for the breakdown
     ms_seq, calls_dev = timed(d_px, d_files, d_back, 1, 2, 1, "sequential")
     table_sha = state["table_sha"]
@@ -629,7 +661,14 @@ def main():
                     help="device-resident leg: all jobs at once / each job's encode starts when the previous job has encoded / one job at a time")
     ap.add_argument("--e2e-schedule", default=os.environ.get("XPNG_BENCH_E2E_SCHEDULE", "chained"), choices=["concurrent", "chained", "sequential"],
                     help="host-buffer leg (chained keeps both PCIe directions busy: one job's decode downloads next to the next job's encode uploads)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (per level: file sizes and offsets, a fixed sample of "
+                         "the file bytes and of the decoded pixels; rank 0's shard) as DIR/<name>.npy, float32 / float64, about 50 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this library computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

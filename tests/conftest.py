@@ -58,6 +58,12 @@ def make_case(group, name, entry):
 BIG = {"rgb_4k_s1", "gray_4096_s3000", "rgba_8192_s2"}
 
 
+def reference_pins():
+    """What the reference comparisons of the suite compare against (tools/make_golden_pins.py)."""
+    with open(os.path.join(GOLD, "reference_pins.json")) as f:
+        return json.load(f)
+
+
 def all_cases(groups=("synthetic", "special", "crops"), big=False):
     man = manifest()
     out = []

@@ -31,14 +31,14 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(L, s), s
 
 
-def test_no_cpu_fallback_without_device():
+def test_no_cpu_fallback_without_device(tmp_path):
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present")
     with pytest.raises(RuntimeError):
         xpng_b200.Codec(0)
     # the file API reports failure (returns 1) instead of silently using a CPU path
-    assert xpng_b200.xpng_store(1, synth.rgb(8, 8, 1), "/tmp/_xpng_nogpu.xpng") is True
+    assert xpng_b200.xpng_store(1, synth.rgb(8, 8, 1), str(tmp_path / "nogpu.xpng")) is True
 
 
 def test_seven_container_roundtrip(tmp_path):

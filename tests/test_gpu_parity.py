@@ -7,7 +7,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import ROOT, all_cases, make_case, manifest, sha
+from conftest import ROOT, all_cases, make_case, manifest, reference_pins, sha
 from oracle import pyoracle as po
 from xpng_b200 import synth
 
@@ -114,17 +114,24 @@ def test_device_resident_buffers(codec):
     assert np.array_equal(dback.cpu().numpy(), host)
 
 
+CLI_CASES = {"rgb_333x517_s8": (synth.rgb, 333, 517, 8), "rgba_250x300_s9": (synth.rgba, 250, 300, 9)}
+
+
 def test_file_api_and_cli_against_reference(codec, tmp_path):
-    """xpng_store / xpng_load (xpng.h) and the CLI contract of xpng.c / test.rb: .7 -> .xpng -> .7 + cmp."""
+    """xpng_store / xpng_load (xpng.h) and the CLI contract of xpng.c / test.rb: .7 -> .xpng -> .7 + cmp.  The files must be
+    the reference's (tests/golden/reference_pins.json; the reference binary decodes them too when oracle/_ref is built)."""
     import xpng_b200
     cli = os.path.join(ROOT, "xpng_b200", "bin", "xpng")
-    for px in (synth.rgb(333, 517, 8), synth.rgba(250, 300, 9)):
+    pins = reference_pins()["file_api_cli"]
+    for key, (gen, h, w, seed) in CLI_CASES.items():
+        px = gen(h, w, seed)
         src = str(tmp_path / "src.7"); po.write_7(src, px)
         for lv in (1, 2, 7):
             dst, back = str(tmp_path / "res.xpng"), str(tmp_path / "res.7")
             r = subprocess.run([cli, f"-{lv}", src, dst], capture_output=True, text=True)
             assert r.returncode == 0, r.stderr
             assert open(dst, "rb").read() == po.encode(lv, px)
+            assert sha(open(dst, "rb").read()) == pins[key][str(lv)], (key, lv)
             if lv != 7:
                 assert r.stdout.startswith("encode,") and r.stdout.rstrip().endswith("MPx/s")   # libxpng.c:761
             r = subprocess.run([cli, "-d", dst, back], capture_output=True, text=True)

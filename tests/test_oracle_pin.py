@@ -1,11 +1,12 @@
 """Pins the CPU oracle (oracle/xpng_oracle.c) to the unmodified reference:
  * against the committed golden manifest (sha256 of files the reference produced, tools/make_golden.py),
- * and, when oracle/_ref is present, directly against the reference binary on fresh random inputs.
+ * against the stored results of the reference on random inputs (tests/golden/reference_pins.json),
+ * and, when oracle/_ref is present, directly against the reference binary on those inputs.
 CPU only."""
 import numpy as np
 import pytest
 
-from conftest import all_cases, make_case, sha
+from conftest import all_cases, make_case, reference_pins, sha
 from oracle import pyoracle as po
 from xpng_b200 import synth
 
@@ -36,17 +37,29 @@ def test_oracle_matches_golden_full_size(name):
     test_oracle_matches_golden("synthetic", name, e)
 
 
-@pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("seed", range(6))
-def test_oracle_matches_reference_binary(seed):
+def random_case(seed):
+    """Input of test_oracle_matches_reference_binary for one seed (also read by tools/make_golden_pins.py)."""
     rng = np.random.default_rng(100 + seed)
     h, w = int(rng.integers(5, 700)), int(rng.integers(5, 900))
     gen = [synth.rgb, synth.rgba, synth.gray_as_rgb][seed % 3]
-    px = gen(h, w, 500 + seed)
+    return gen(h, w, 500 + seed)
+
+
+@pytest.mark.parametrize("seed", range(6))
+def test_oracle_matches_reference_binary(seed):
+    """The oracle against the reference encoder and decoder on random shapes: against what the reference produced for these
+    inputs (tests/golden/reference_pins.json) always, and against the reference binary itself when oracle/_ref is built."""
+    px = random_case(seed)
+    pin = reference_pins()["oracle_vs_reference"][str(seed)]
+    assert list(px.shape) == pin["shape"]
     for lv in (1, 2, 7):
-        a, b = po.encode(lv, px), po.ref_encode(lv, px)
-        assert a == b
-        assert np.array_equal(po.decode(a), po.ref_decode(a))
+        a = po.encode(lv, px)
+        back = po.decode(a)
+        assert len(a) == pin[str(lv)]["size"] and sha(a) == pin[str(lv)]["sha256"], lv
+        assert list(back.shape) == pin["decoded_shape"] and sha(back.tobytes()) == pin[str(lv)]["decoded_sha256"], lv
+        if po.ref_available():
+            assert a == po.ref_encode(lv, px)
+            assert np.array_equal(back, po.ref_decode(a))
 
 
 def test_tile_grid_baseline_shapes():

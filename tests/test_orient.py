@@ -1,6 +1,6 @@
 """Traversal-order operations (SURVEY §8 f3; reference Mirroring_and_Rotating/tool.c).
-CPU: the numpy restatement in oracle/pyoracle.py against the unmodified reference tool (oracle/_ref/tool) and the
-reference's own reversibility.rb properties.  GPU: k_orient through the C ABI against the restatement, the encoder's
+CPU: the numpy restatement in oracle/pyoracle.py against the unmodified reference tool (its stored outputs, and
+oracle/_ref/tool when built) and the reference's own reversibility.rb properties.  GPU: k_orient through the C ABI against the restatement, the encoder's
 orientation option against "tool then xpng" of the oracle, and the `tool` command line."""
 import os
 import subprocess
@@ -8,7 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import ROOT
+from conftest import ROOT, reference_pins, sha
 from oracle import pyoracle as po
 from xpng_b200 import synth
 
@@ -20,12 +20,18 @@ def _px(shape, seed=5):
     return np.random.default_rng(seed).integers(0, 256, shape, dtype=np.uint8)
 
 
-@pytest.mark.skipif(not os.path.exists(po.REF_TOOL), reason="oracle/_ref/tool not built")
 @pytest.mark.parametrize("op", po.TOOL_OPS)
 def test_restatement_matches_reference_tool(op):
+    """Against what the reference tool wrote for these inputs (tests/golden/reference_pins.json) always, and against the tool
+    itself when oracle/_ref is built."""
+    pins = reference_pins()["orient"][op]
     for shape in SHAPES:
         px = _px(shape)
-        assert np.array_equal(po.orient(op, px), po.ref_orient(op, px)), (op, shape)
+        got = po.orient(op, px)
+        want_shape, want_sha = pins["x".join(map(str, shape))]
+        assert list(got.shape) == want_shape and sha(got.tobytes()) == want_sha, (op, shape)
+        if os.path.exists(po.REF_TOOL):
+            assert np.array_equal(got, po.ref_orient(op, px)), (op, shape)
 
 
 def test_restatement_reversibility():
