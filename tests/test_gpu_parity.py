@@ -176,8 +176,9 @@ def test_ycocg_r_side_kernel(codec):
 
 
 def test_throughput_kernel_family(monkeypatch):
-    """Large batches switch from the warp-per-block (latency) entropy kernels to the lane-per-block ones
-    (XPNGB_LAT_MAX_BLOCKS, read when the context is created): both families must produce the same bytes."""
+    """Large batches decode with the pair-lane rANS decoders, the three-tiles-per-warp context walk and the row-pitched
+    un-predict instead of the warp-per-block (latency) kernels; XPNGB_LAT_MAX_BLOCKS=0 (read when the context is created)
+    selects them for small inputs: both families must produce the same bytes and pixels."""
     import xpng_b200
     monkeypatch.setenv("XPNGB_LAT_MAX_BLOCKS", "0")
     cd = xpng_b200.Codec(0)

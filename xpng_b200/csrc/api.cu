@@ -44,12 +44,8 @@ struct xpngb_ctx {
     cudaStream_t stream = nullptr, side[NSIDE] = {}, cur = nullptr;   // main stream, side streams for independent chains, stream of the next launch
     cudaStream_t hi = nullptr;                 // high-priority twin of the main stream: serial-chain kernels (LAUNCH_HI)
     cudaEvent_t ev_hi = nullptr;
-    bool enc_sorted = true;                    // root: XPNGB_ENC_SORT=0: pair encoders take blocks in tile order (A/B)
-    bool use_prio = true;                      // root: XPNGB_PRIO=0 switches the priorities off (A/B)
     cudaEvent_t ev_fork = nullptr, ev_join[NSIDE] = {};
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, pe0 = nullptr, pe1 = nullptr, ev_done = nullptr;
-    cudaEvent_t ev_stage = nullptr;            // decode: this lane's chunk has finished its context-decode (or walk) phase (staggered waves)
-    uint32_t dec_stagger1 = 0, dec_stagger2 = 0, dec_stagger_at = 0;   // root: XPNGB_DEC_STAGGER1/2 = S: chunk k of a level-1/2 batch decode starts when chunk k - S has passed its stage (0: all at once); XPNGB_DEC_STAGGER_AT: 0 contexts decoded, 1 walked
     int profile = 0;   // 1: per-kernel CUDA-event timing accumulated (serialises the launches); 2: also print to stderr;
                        // 3: timeline — start/end of every launch relative to the call's start, launches NOT serialised (stderr)
     int lane_id = 0;
@@ -63,14 +59,12 @@ struct xpngb_ctx {
     uint64_t max_chunk_px = 1ull << 30;       // XPNGB_CHUNK_MPIX: upper bound of a chunk (bounds the scratch of a lane)
     uint32_t pipe_lanes = 8;                  // XPNGB_PIPE_LANES: chunks in flight per call
     uint64_t pipe_min_px = 32ull << 20;       // XPNGB_PIPE_MIN_MPIX: no chunk smaller than this
-    bool front_v1 = false;                    // XPNGB_FRONT=1: first-generation front end for RGB tiles too (A/B, tests)
-    bool walk_global = false, walk_ring = false;   // XPNGB_WALK=global | ring: force a walk variant (tests, A/B)
+    bool walk_ring = false;                   // XPNGB_WALK=ring: force the ring walk (tests)
     uint32_t direct_max_tiles = 148;  // level-2 decode: tiles per call up to which the 64 KiB direct tables are used (3 chains per SM stay resident)
     uint32_t v2_direct_max_tiles = ~0u;  // level-1 decode: same trade for the 16 KiB context tables
-    uint32_t unr_multi_max_tiles = 592, unr_force = 0;   // un-predict: tiles per call up to which a tile gets 8 warps; XPNGB_UNR_NW forces a variant (A/B)
+    uint32_t unr_multi_max_tiles = 592;  // un-predict: tiles per call up to which a tile gets 8 warps
     uint32_t s16_lat_max_tiles = 1776;  // level-2 decode, pair family: calls up to this many tiles decode the 16-symbol value stream (the longest chain) warp-per-block
     uint32_t lat_max_blocks = 12000;  // decode: entropy blocks per call up to which the warp-per-block (latency) kernels are used (measured crossover, profiles/)
-    uint32_t enc_lat_max_blocks = ~0u; // encode: the pair-lane encoders serve every batch size (chunks in flight keep their launches resident)
     // device scratch
     DevBuf pixels, norm, files, arena, tiles, imgs, seg_tile, costs, hist, seginfo, place, vplace, vcnt, sym_area,
         bits_area, alpha, streams, blocks, state, outs, flags, skip, dimgs, dtiles, plane, nlseq, rowcnt, rowbits, eord,
@@ -118,7 +112,7 @@ struct xpngb_ctx {
 static cudaStream_t prio_stream(const xpngb_ctx* ctx, int level) {
     cudaStream_t s = nullptr;
     int lo = 0, hi = 0;   // numerically lower = served first
-    if (ctx->root->use_prio && cudaDeviceGetStreamPriorityRange(&lo, &hi) == cudaSuccess && hi != lo)
+    if (cudaDeviceGetStreamPriorityRange(&lo, &hi) == cudaSuccess && hi != lo)
         cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, (hi + level < lo) ? hi + level : hi);
     else cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
     return s;
@@ -130,7 +124,7 @@ static cudaStream_t side_of(xpngb_ctx* ctx, int k) {
 #define LAUNCH_HI(kernel, grid, block, smem, ...)                                                   \
     do {                                                                                            \
         cudaStream_t base_ = ctx->cur;                                                              \
-        const bool tw_ = base_ == ctx->stream && ctx->root->use_prio && (ctx->root->profile == 0 || ctx->root->profile == 3);       \
+        const bool tw_ = base_ == ctx->stream && (ctx->root->profile == 0 || ctx->root->profile == 3);       \
         if (tw_) {                                                                                  \
             if (!ctx->hi) ctx->hi = prio_stream(ctx, 1);                                               \
             CK(cudaEventRecord(ctx->ev_hi, base_)); CK(cudaStreamWaitEvent(ctx->hi, ctx->ev_hi, 0)); ctx->cur = ctx->hi; \
@@ -270,13 +264,8 @@ static int upload_plan(xpngb_ctx* ctx, const Plan& P) {
 constexpr uint32_t lat_smem(uint32_t lut_bytes) { return LAT_CUM_WORDS * 4 + lut_bytes + LAT_RING_WORDS * 4; }
 constexpr uint32_t LUT_ONE_12 = 4u << 12, LUT_ONE_14 = 4u << 14, LUT_TWO_12 = 1024 + (1u << 12), LUT_TWO_14 = 1024 + (1u << 14), LUT_TWO_15 = 1024 + (1u << 15);
 
-static void m2_set_attributes() {
-    auto k_big = k_rans_v1<256, 32>;
-    cudaFuncSetAttribute(k_big, cudaFuncAttributeMaxDynamicSharedMemorySize, 256 * 32 * 16);
-}
-
 // classification, RGB front end (contexts + value streams), grey candidates, backward rANS, size decisions
-static int m2_encode_tiles(xpngb_ctx* ctx, const Plan& P, uint32_t ntiles, uint32_t nseg, bool lat) {
+static int m2_encode_tiles(xpngb_ctx* ctx, const Plan& P, uint32_t ntiles, uint32_t nseg) {
     const TileDesc* d_tiles = (const TileDesc*)ctx->tiles.p;
     const uint32_t* d_seg_tile = (const uint32_t*)ctx->seg_tile.p;
     ENSURE(tclass, ntiles); ENSURE(skip, ntiles); ENSURE(tabs, (size_t)ntiles * 17 * TAB_WORDS * 4);
@@ -286,12 +275,9 @@ static int m2_encode_tiles(xpngb_ctx* ctx, const Plan& P, uint32_t ntiles, uint3
     LAUNCH(k_m2_skipmask, (ntiles + 255) / 256, 256, 0, (const uint8_t*)ctx->tclass.p, (uint8_t*)ctx->skip.p, ntiles);
     FrontArgs fa{ d_tiles, d_seg_tile, nullptr, (const uint32_t*)ctx->costs.p, (const uint8_t*)ctx->skip.p, (SegInfo*)ctx->seginfo.p,
                   (uint8_t*)ctx->sym_area.p, (uint8_t*)ctx->bits_area.p, nullptr, (uint32_t*)ctx->hist.p, (uint16_t*)ctx->vcnt.p, 0u };
-    if (ctx->root->front_v1) LAUNCH(k_front<2>, nseg, FRONT_THREADS, 0, fa);
-    else {                                                     // level 2 codes RGB tiles only
-        LAUNCH(k_front2<2>, nseg, FRONT_THREADS, 0, fa);
-        fa.rgba_only = 1;
-        if (P.any_wide) LAUNCH(k_front<2>, nseg, FRONT_THREADS, 0, fa);
-    }
+    LAUNCH(k_front2<2>, nseg, FRONT_THREADS, 0, fa);           // level 2 codes RGB tiles only
+    fa.rgba_only = 1;
+    if (P.any_wide) LAUNCH(k_front<2>, nseg, FRONT_THREADS, 0, fa);
     TileScanArgs ta{ d_tiles, (const SegInfo*)ctx->seginfo.p, (const uint32_t*)ctx->costs.p, (const uint16_t*)ctx->vcnt.p,
                      (SegPlace*)ctx->place.p, (SegPlace*)ctx->vplace.p, (uint32_t*)ctx->hist.p, (TileState*)ctx->state.p,
                      (const uint8_t*)ctx->skip.p, ntiles };
@@ -303,36 +289,26 @@ static int m2_encode_tiles(xpngb_ctx* ctx, const Plan& P, uint32_t ntiles, uint3
     LAUNCH(k_m2_grey_front, nseg, 256, 0, d_tiles, d_seg_tile, (const uint8_t*)ctx->tclass.p, (uint8_t*)ctx->streams.p, (uint32_t*)ctx->hist.p);
     RansV1Args ra{ d_tiles, (TileState*)ctx->state.p, (const uint32_t*)ctx->hist.p, (const uint8_t*)ctx->tclass.p,
                    (const uint8_t*)ctx->streams.p, (uint8_t*)ctx->blocks.p, (uint32_t*)ctx->tabs.p, ntiles, 0, 17, 0, 0 };
-    if (lat) {
-        auto k_rans_v1_pair_16 = k_rans_v1_pair<16>; auto k_rans_v1_pair_256 = k_rans_v1_pair<256>;
-        const uint32_t ecap = 17u * ntiles;
-        if (ctx->root->enc_sorted) {                   // blocks by decreasing length, one list per table size (enc_order.cuh)
-            ENSURE(eord, (size_t)(2 * ecap + 2) * 4);
-            uint32_t* eo = (uint32_t*)ctx->eord.p;
-            LAUNCH_HI(k_enc_order, 1, 1024, 0, EncOrderArgs{ d_tiles, (const TileState*)ctx->state.p, (const uint8_t*)ctx->tclass.p, ntiles, 2u, eo + 2, eo, ecap });
-            ra.order = eo + 2; ra.total = eo;
-        }
-        // alphabets above 16 symbols and the grey candidates go to a side stream that forks BEFORE the main launch but is
-        // fed AFTER it: the small-alphabet kernel holds the longest chains, and in a batch its CTAs must be placed first
-        // (the 98 KiB CTAs of the other kernel would otherwise take the shared memory and delay them)
-        FORK_SIDE(0);
-        BACK_TO_MAIN();
-        LAUNCH_HI(k_rans_v1_pair_16, (17 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 17 * PAIR_BLK * 24, ra);
-        ctx->cur = ctx->side[0];
-        RansV1Args rb = ra; rb.c0 = 9; rb.nc = 8; rb.nmin = 16;
-        if (ra.order) { rb.order = ra.order + ecap; rb.total = ra.total + 1; }
-        LAUNCH_HI(k_rans_v1_pair_256, (8 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 257 * PAIR_BLK * 24, rb);
-        rb.c0 = 0; rb.nc = 4; rb.nmin = 0; rb.grey = 1; rb.order = nullptr; rb.total = nullptr;
-        LAUNCH_HI(k_rans_v1_pair_256, (4 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 257 * PAIR_BLK * 24, rb);
-        JOIN_SIDE(0);
-    } else {
-    auto k_rans_v1_lane_16 = k_rans_v1<16, 128>; auto k_rans_v1_lane_256 = k_rans_v1<256, 32>;
-    LAUNCH(k_rans_v1_lane_16, (17 * ntiles + 127) / 128, 128, 16 * 128 * 16, ra);
-    ra.c0 = 9; ra.nc = 8; ra.nmin = 16;
-    LAUNCH(k_rans_v1_lane_256, (8 * ntiles + 31) / 32, 32, 256 * 32 * 16, ra);
-    ra.c0 = 0; ra.nc = 4; ra.nmin = 0; ra.grey = 1;
-    LAUNCH(k_rans_v1_lane_256, (4 * ntiles + 31) / 32, 32, 256 * 32 * 16, ra);
-    }
+    auto k_rans_v1_pair_16 = k_rans_v1_pair<16>; auto k_rans_v1_pair_256 = k_rans_v1_pair<256>;
+    const uint32_t ecap = 17u * ntiles;
+    // blocks by decreasing length, one list per table size (enc_order.cuh)
+    ENSURE(eord, (size_t)(2 * ecap + 2) * 4);
+    uint32_t* eo = (uint32_t*)ctx->eord.p;
+    LAUNCH_HI(k_enc_order, 1, 1024, 0, EncOrderArgs{ d_tiles, (const TileState*)ctx->state.p, (const uint8_t*)ctx->tclass.p, ntiles, 2u, eo + 2, eo, ecap });
+    ra.order = eo + 2; ra.total = eo;
+    // alphabets above 16 symbols and the grey candidates go to a side stream that forks BEFORE the main launch but is
+    // fed AFTER it: the small-alphabet kernel holds the longest chains, and in a batch its CTAs must be placed first
+    // (the 98 KiB CTAs of the other kernel would otherwise take the shared memory and delay them)
+    FORK_SIDE(0);
+    BACK_TO_MAIN();
+    LAUNCH_HI(k_rans_v1_pair_16, (17 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 17 * PAIR_BLK * 24, ra);
+    ctx->cur = ctx->side[0];
+    RansV1Args rb = ra; rb.c0 = 9; rb.nc = 8; rb.nmin = 16;
+    rb.order = ra.order + ecap; rb.total = ra.total + 1;
+    LAUNCH_HI(k_rans_v1_pair_256, (8 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 257 * PAIR_BLK * 24, rb);
+    rb.c0 = 0; rb.nc = 4; rb.nmin = 0; rb.grey = 1; rb.order = nullptr; rb.total = nullptr;
+    LAUNCH_HI(k_rans_v1_pair_256, (4 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 257 * PAIR_BLK * 24, rb);
+    JOIN_SIDE(0);
     LAUNCH_HI(k_m2_finish, (ntiles + 127) / 128, 128, 0, d_tiles, (const uint8_t*)ctx->tclass.p, (TileState*)ctx->state.p, ntiles);
     return 0;
 }
@@ -363,7 +339,7 @@ static void lane_free(xpngb_ctx* ctx) {
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
     if (ctx->pin_o.p) cudaFreeHost(ctx->pin_o.p);
     if (ctx->hi) { cudaStreamSynchronize(ctx->hi); cudaStreamDestroy(ctx->hi); }
-    cudaEvent_t evs[] = { ctx->ev0, ctx->ev1, ctx->ev_fork, ctx->pe0, ctx->pe1, ctx->ev_done, ctx->ev_hi, ctx->ev_stage };
+    cudaEvent_t evs[] = { ctx->ev0, ctx->ev1, ctx->ev_fork, ctx->pe0, ctx->pe1, ctx->ev_done, ctx->ev_hi };
     for (cudaEvent_t e : evs) if (e) cudaEventDestroy(e);
     for (int k = 0; k < xpngb_ctx::NSIDE; k++) { if (ctx->ev_join[k]) cudaEventDestroy(ctx->ev_join[k]); if (ctx->side[k]) cudaStreamDestroy(ctx->side[k]); }
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -377,7 +353,6 @@ static xpngb_ctx* lane_new(int device, xpngb_ctx* root) {
     bool ok = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) == cudaSuccess &&
               cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) == cudaSuccess &&
               cudaEventCreateWithFlags(&ctx->ev_done, cudaEventDisableTiming) == cudaSuccess &&
-              cudaEventCreateWithFlags(&ctx->ev_stage, cudaEventDisableTiming) == cudaSuccess &&
               cudaEventCreateWithFlags(&ctx->ev_hi, cudaEventDisableTiming) == cudaSuccess &&
               cudaEventCreate(&ctx->ev0) == cudaSuccess && cudaEventCreate(&ctx->ev1) == cudaSuccess &&
               cudaEventCreate(&ctx->pe0) == cudaSuccess && cudaEventCreate(&ctx->pe1) == cudaSuccess;
@@ -415,21 +390,11 @@ extern "C" int xpngb_create(xpngb_ctx** out, int device) {
     if (const char* e = getenv("XPNGB_CHUNK_MPIX")) { const long v = atol(e); if (v > 0) ctx->max_chunk_px = (uint64_t)v << 20; }
     if (const char* e = getenv("XPNGB_PIPE_LANES")) { const long v = atol(e); if (v > 0 && v <= 64) ctx->pipe_lanes = (uint32_t)v; }
     if (const char* e = getenv("XPNGB_PIPE_MIN_MPIX")) { const long v = atol(e); if (v > 0) ctx->pipe_min_px = (uint64_t)v << 20; }
-    { auto k_big = k_rans_v2<256, 32>; cudaFuncSetAttribute(k_big, cudaFuncAttributeMaxDynamicSharedMemorySize, 256 * 32 * 16); }
-    m2_set_attributes();
     if (const char* e = getenv("XPNGB_LAT_MAX_BLOCKS")) ctx->lat_max_blocks = (uint32_t)atol(e);
     if (const char* e = getenv("XPNGB_S16_LAT_MAX_TILES")) ctx->s16_lat_max_tiles = (uint32_t)atol(e);
-    if (const char* e = getenv("XPNGB_DEC_STAGGER1")) ctx->dec_stagger1 = (uint32_t)atol(e);
-    if (const char* e = getenv("XPNGB_DEC_STAGGER2")) ctx->dec_stagger2 = (uint32_t)atol(e);
-    if (const char* e = getenv("XPNGB_DEC_STAGGER_AT")) ctx->dec_stagger_at = (uint32_t)atol(e);
-    if (const char* e = getenv("XPNGB_ENC_LAT_MAX_BLOCKS")) ctx->enc_lat_max_blocks = (uint32_t)atol(e);
     if (const char* e = getenv("XPNGB_V2_DIRECT_MAX_TILES")) ctx->v2_direct_max_tiles = (uint32_t)atol(e);
-    if (const char* e = getenv("XPNGB_WALK")) { ctx->walk_global = !strcmp(e, "global"); ctx->walk_ring = !strcmp(e, "ring"); }
+    if (const char* e = getenv("XPNGB_WALK")) ctx->walk_ring = !strcmp(e, "ring");
     if (const char* e = getenv("XPNGB_DIRECT_MAX_TILES")) ctx->direct_max_tiles = (uint32_t)atol(e);
-    if (const char* e = getenv("XPNGB_UNR_NW")) ctx->unr_force = (uint32_t)atol(e);
-    if (const char* e = getenv("XPNGB_FRONT")) ctx->front_v1 = atoi(e) == 1;
-    if (const char* e = getenv("XPNGB_PRIO")) ctx->use_prio = atoi(e) != 0;
-    if (const char* e = getenv("XPNGB_ENC_SORT")) ctx->enc_sorted = atoi(e) != 0;
     { auto p = k_rans_v2_pair<256>; cudaFuncSetAttribute(p, cudaFuncAttributeMaxDynamicSharedMemorySize, 257 * PAIR_BLK * 24); }
     { auto p = k_rans_v1_pair<256>; cudaFuncSetAttribute(p, cudaFuncAttributeMaxDynamicSharedMemorySize, 257 * PAIR_BLK * 24); }
     cudaFuncSetAttribute(k_dec_unpredict_rows<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16 * 2 * 32 * UNR_PITCH);
@@ -532,7 +497,7 @@ static int encode_finish(xpngb_ctx* ctx, EncChunk& C);
 
 // Launch everything for one chunk on lane `ctx`; nothing here waits for the device unless the chunk holds RGBA images
 // (alpha normalisation changes the pixel size, which the tile plan depends on).
-static int encode_issue(xpngb_ctx* ctx, int level, bool lat, const uint8_t* dpix, uint8_t* dout, EncChunk& C) {
+static int encode_issue(xpngb_ctx* ctx, int level, const uint8_t* dpix, uint8_t* dout, EncChunk& C) {
     xpngb_image* imgs = C.imgs; const uint32_t n = C.n;
     ctx->cur = ctx->stream;
     bool any_rgba = false;
@@ -606,7 +571,7 @@ static int encode_issue(xpngb_ctx* ctx, int level, bool lat, const uint8_t* dpix
             for (size_t k = 0; k < idx.size(); k++) sub[k] = imgs[idx[k]];
             EncChunk S; S.lane = ctx; S.imgs = sub.data(); S.n = (uint32_t)idx.size(); S.out_offsets = so.data(); S.out_sizes = ss.data();
             S.out_base = base; S.out_end = C.out_end;
-            if (encode_issue(ctx, fam == 0 ? 1 : 2, lat, dpix, dout, S) || encode_finish(ctx, S)) return 1;
+            if (encode_issue(ctx, fam == 0 ? 1 : 2, dpix, dout, S) || encode_finish(ctx, S)) return 1;
             base = S.used_end;
             for (size_t k = 0; k < idx.size(); k++) { imgs[idx[k]] = sub[k]; C.out_offsets[idx[k]] = so[k]; C.out_sizes[idx[k]] = ss[k]; }
         }
@@ -646,14 +611,11 @@ static int encode_issue(xpngb_ctx* ctx, int level, bool lat, const uint8_t* dpix
     if (any1) {
         FrontArgs fa{ d_tiles, d_seg_tile, nullptr, (const uint32_t*)ctx->costs.p, nullptr, (SegInfo*)ctx->seginfo.p,
                       (uint8_t*)ctx->sym_area.p, (uint8_t*)ctx->bits_area.p, (uint8_t*)ctx->alpha.p, (uint32_t*)ctx->hist.p, nullptr, 0u };
-        if (ctx->root->front_v1) LAUNCH(k_front<1>, nseg, FRONT_THREADS, 0, fa);
-        else {
-            bool any_rgb = false;
-            for (uint32_t i = 0; i < n; i++) any_rgb |= pxsz[i] == 3 && mode[i] == 1;
-            if (any_rgb) LAUNCH(k_front2<1>, nseg, FRONT_THREADS, 0, fa);
-            fa.rgba_only = 1;
-            if (P.any_rgba || P.any_wide) LAUNCH(k_front<1>, nseg, FRONT_THREADS, 0, fa);
-        }
+        bool any_rgb = false;
+        for (uint32_t i = 0; i < n; i++) any_rgb |= pxsz[i] == 3 && mode[i] == 1;
+        if (any_rgb) LAUNCH(k_front2<1>, nseg, FRONT_THREADS, 0, fa);
+        fa.rgba_only = 1;
+        if (P.any_rgba || P.any_wide) LAUNCH(k_front<1>, nseg, FRONT_THREADS, 0, fa);
         TileScanArgs ta{ d_tiles, (const SegInfo*)ctx->seginfo.p, (const uint32_t*)ctx->costs.p, nullptr, (SegPlace*)ctx->place.p, nullptr,
                          (uint32_t*)ctx->hist.p, (TileState*)ctx->state.p, nullptr, ntiles };
         LAUNCH_HI(k_tile_scan<1>, (ntiles + 3) / 4, 128, 0, ta);
@@ -663,38 +625,28 @@ static int encode_issue(xpngb_ctx* ctx, int level, bool lat, const uint8_t* dpix
         LAUNCH(k_compact<1>, nseg, 256, 0, ca);
         RansV2Args ra{ d_tiles, (TileState*)ctx->state.p, (uint32_t*)ctx->hist.p, (const uint8_t*)ctx->streams.p,
                        (const uint8_t*)ctx->alpha.p, (uint8_t*)ctx->blocks.p, ntiles, 0, 9 };
-        if (lat) {
-            auto k_rans_v2_pair_16 = k_rans_v2_pair<16>; auto k_rans_v2_pair_256 = k_rans_v2_pair<256>;
-            const uint32_t ecap = 10u * ntiles;
-            if (ctx->root->enc_sorted) {               // blocks by decreasing length (enc_order.cuh)
-                ENSURE(eord, (size_t)(2 * ecap + 2) * 4);
-                uint32_t* eo = (uint32_t*)ctx->eord.p;
-                LAUNCH_HI(k_enc_order, 1, 1024, 0, EncOrderArgs{ d_tiles, (const TileState*)ctx->state.p, nullptr, ntiles, 1u, eo + 2, eo, ecap });
-                ra.order = eo + 2; ra.total = eo;
-            }
-            if (P.any_rgba) {                          // the alpha blocks are independent of the context blocks: side stream
-                FORK_SIDE(0);                          // forks before, is fed after the main launch (see m2_encode_tiles)
-                BACK_TO_MAIN();
-            }
-            LAUNCH_HI(k_rans_v2_pair_16, (9 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 17 * PAIR_BLK * 24, ra);
-            if (P.any_rgba) {
-                RansV2Args rb = ra; rb.c0 = 9; rb.nc = 1;
-                if (ra.order) { rb.order = ra.order + ecap; rb.total = ra.total + 1; }
-                ctx->cur = ctx->side[0];
-                LAUNCH_HI(k_rans_v2_pair_256, (ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 257 * PAIR_BLK * 24, rb);
-                JOIN_SIDE(0);
-            }
-        } else {
-            auto k_rans_v2_lane_9 = k_rans_v2<9, 128>; auto k_rans_v2_lane_256 = k_rans_v2<256, 32>;
-            LAUNCH(k_rans_v2_lane_9, (9 * ntiles + 127) / 128, 128, 9 * 128 * 16, ra);
-            if (P.any_rgba) {
-                ra.c0 = 9; ra.nc = 1;
-                LAUNCH(k_rans_v2_lane_256, (ntiles + 31) / 32, 32, 256 * 32 * 16, ra);
-            }
+        auto k_rans_v2_pair_16 = k_rans_v2_pair<16>; auto k_rans_v2_pair_256 = k_rans_v2_pair<256>;
+        const uint32_t ecap = 10u * ntiles;
+        // blocks by decreasing length (enc_order.cuh)
+        ENSURE(eord, (size_t)(2 * ecap + 2) * 4);
+        uint32_t* eo = (uint32_t*)ctx->eord.p;
+        LAUNCH_HI(k_enc_order, 1, 1024, 0, EncOrderArgs{ d_tiles, (const TileState*)ctx->state.p, nullptr, ntiles, 1u, eo + 2, eo, ecap });
+        ra.order = eo + 2; ra.total = eo;
+        if (P.any_rgba) {                          // the alpha blocks are independent of the context blocks: side stream
+            FORK_SIDE(0);                          // forks before, is fed after the main launch (see m2_encode_tiles)
+            BACK_TO_MAIN();
+        }
+        LAUNCH_HI(k_rans_v2_pair_16, (9 * ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 17 * PAIR_BLK * 24, ra);
+        if (P.any_rgba) {
+            RansV2Args rb = ra; rb.c0 = 9; rb.nc = 1;
+            rb.order = ra.order + ecap; rb.total = ra.total + 1;
+            ctx->cur = ctx->side[0];
+            LAUNCH_HI(k_rans_v2_pair_256, (ntiles + PAIR_BLK - 1) / PAIR_BLK, 32, 257 * PAIR_BLK * 24, rb);
+            JOIN_SIDE(0);
         }
     }
     if (any2) {
-        if (m2_encode_tiles(ctx, P, ntiles, nseg, lat)) return 1;
+        if (m2_encode_tiles(ctx, P, ntiles, nseg)) return 1;
     }
     LAUNCH_HI(k_image_sizes, (n + 127) / 128, 128, 0, d_imgs, d_tiles, (TileState*)ctx->state.p, (ImageOut*)ctx->outs.p, n);
     LAUNCH_HI(k_image_offsets, 1, 1, 0, (ImageOut*)ctx->outs.p, n, C.out_base);
@@ -780,10 +732,6 @@ extern "C" int xpngb_encode(xpngb_ctx* ctx, int level, xpngb_image* imgs, uint32
     // ---- chunks on lanes
     const std::vector<uint32_t> cuts = cut_chunks(ctx, imgs, n);
     const uint32_t nchunks = (uint32_t)cuts.size() - 1;
-    uint64_t tiles_est = 0;
-    for (uint32_t i = 0; i < n; i++) tiles_est += (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
-    // kernel family by the size of the CALL (what is in flight at once), not of a chunk
-    const bool lat = (level == 2 ? 17 * tiles_est <= (uint64_t)ctx->enc_lat_max_blocks * 5 / 2 : 9 * tiles_est <= ctx->enc_lat_max_blocks);
     std::vector<EncChunk> chunks(nchunks);
     uint64_t host_packed = 0;   // host output: files are packed across chunks
     int rc = 0;
@@ -823,7 +771,7 @@ extern "C" int xpngb_encode(xpngb_ctx* ctx, int level, xpngb_image* imgs, uint32
                 snprintf(ctx->err, sizeof ctx->err, "host to device copy failed"); rc = 1; break;
             }
         }
-        rc = encode_issue(lane, level, lat, dpix, dout, C);
+        rc = encode_issue(lane, level, dpix, dout, C);
     }
     while (!rc && harvested < nchunks) rc = harvest(harvested++);
     // join: the root stream waits for every lane, so that ev1 closes the whole call
@@ -1018,19 +966,14 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, xpngb_image* imgs, uint32_t n,
     PdWork Wl[3] = {};                              // work lists of the pair decoders / the batch walk, per level family
     auto launch_walk = [&](uint32_t mode) -> int {
         WalkArgs wa{ d_tiles, d_imgs, d_dt, (const uint8_t*)ctx->streams.p, (uint8_t*)ctx->nlseq.p, ntiles, mode };
-        if (!lat && !ctx->root->walk_ring && !ctx->root->walk_global) {   // batches: three tiles per warp, longest tiles first
+        if (!lat && !ctx->root->walk_ring) {   // batches: three tiles per warp, longest tiles first
             const PdWork& W = Wl[mode];
             LAUNCH_HI(k_dec_walk3<2>, (ntiles + 5) / 6, 64, 0, wa, (const uint32_t*)(W.order + (size_t)PD_WALK * W.cap), (const uint32_t*)(W.total + PD_WALK));
             return 0;
         }
         // the shared-memory walk only pays when every tile's CTA of the CALL is resident at once (no waves): 227 KB per SM, 148 SMs
         const uint32_t resident = 148u * ((227u * 1024u) / (wsm + 1024u));
-        xpngb_ctx* r = ctx->root;
-        if (call_tiles <= resident && maxpx <= WALK_SMEM_MAX_SYMS && !r->walk_ring && !r->walk_global) LAUNCH_HI(k_dec_walk_smem<0>, ntiles, 32, wsm, wa);
-        else if (r->walk_global) {                     // XPNGB_WALK=global: the older variant with refills straight from global memory
-            if (ntiles <= 592) LAUNCH_HI(k_dec_walk_lat<1>, ntiles, 32, 0, wa);
-            else LAUNCH_HI(k_dec_walk_lat<4>, (ntiles + 3) / 4, 128, 0, wa);
-        }
+        if (call_tiles <= resident && maxpx <= WALK_SMEM_MAX_SYMS && !ctx->root->walk_ring) LAUNCH_HI(k_dec_walk_smem<0>, ntiles, 32, wsm, wa);
         else if (call_tiles <= 592) LAUNCH_HI(k_dec_walk_ring<1>, ntiles, 32, 0, wa);
         else LAUNCH_HI(k_dec_walk_ring<4>, (ntiles + 3) / 4, 128, 0, wa);
         return 0;
@@ -1083,7 +1026,6 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, xpngb_image* imgs, uint32_t n,
             auto k_dec_rans_pair_v2_ctx = k_dec_rans_pair<2, 8>;
             LAUNCH_HI(k_dec_rans_pair_v2_ctx, pd_grid(9), PD_WARPS * 32, 0, pd_args(W, PD_S8));
         }
-        if (!ctx->root->dec_stagger_at && !own_stream) CK(cudaEventRecord(ctx->ev_stage, ctx->stream));
         if (launch_walk(1)) return 1;
         BACK_TO_MAIN();
     }
@@ -1142,12 +1084,10 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, xpngb_image* imgs, uint32_t n,
             LAUNCH_HI(k_pd_fill_blocks, (17u * ntiles + 3) / 4, 128, 0, fa);   // run / raw blocks (contexts among them: before the walk)
             LAUNCH_HI(k_dec_rans_pair_v1_s8, pd_grid(11), PD_WARPS * 32, 0, pd_args(W, PD_S8));
         }
-        if (!ctx->root->dec_stagger_at) CK(cudaEventRecord(ctx->ev_stage, ctx->stream));
         if (launch_walk(2)) return 1;
     }
-    if (ctx->root->dec_stagger_at || !(any1 || any2)) CK(cudaEventRecord(ctx->ev_stage, ctx->stream));
     // batches: RGB tiles with word-aligned rows get the row-pitched residual plane and k_dec_unpredict_rgb
-    const uint32_t pitched = ((!lat || call_tiles > ctx->root->unr_multi_max_tiles) && !ctx->root->unr_force) ? 1u : 0u;
+    const uint32_t pitched = (!lat || call_tiles > ctx->root->unr_multi_max_tiles) ? 1u : 0u;
     bool all_pitched = true;
     for (const TileDesc& t : P.tiles) all_pitched &= tile_pitched(t);
     if (any1 || any2) {
@@ -1167,7 +1107,6 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, xpngb_image* imgs, uint32_t n,
         // that one warp per tile: bands of a tile depend on each other, so extra warps only wait on the band above, and
         // with thousands of tiles the tiles themselves are the parallelism
         uint32_t nw = call_tiles <= 148 ? 16u : (call_tiles <= ctx->root->unr_multi_max_tiles ? 8u : 1u);
-        if (ctx->root->unr_force) nw = ctx->root->unr_force;
         if (pitched) {   // batches: one warp per RGB tile on the row-pitched residual plane; whatever it cannot take goes on below
             LAUNCH(k_dec_unpredict_rgb, ntiles, 32, 0, ua);
             if (all_pitched) nw = 0;
@@ -1175,8 +1114,6 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, xpngb_image* imgs, uint32_t n,
         if (nw == 0) { }
         else if (nw == 16) LAUNCH(k_dec_unpredict_rows<16>, ntiles, 16 * 32, 16 * 2 * 32 * UNR_PITCH, ua);
         else if (nw == 8) LAUNCH(k_dec_unpredict_rows<8>, ntiles, 8 * 32, 8 * 2 * 32 * UNR_PITCH, ua);
-        else if (nw == 4) LAUNCH(k_dec_unpredict_rows<4>, ntiles, 4 * 32, 4 * 2 * 32 * UNR_PITCH, ua);
-        else if (nw == 2) LAUNCH(k_dec_unpredict_rows<2>, ntiles, 2 * 32, 2 * 2 * 32 * UNR_PITCH, ua);
         else LAUNCH(k_dec_unpredict_rows<1>, ntiles, 32, 2 * 32 * UNR_PITCH, ua);
         ua.min_w = UNR_MAXW;
         if (maxw > UNR_MAXW) LAUNCH(k_dec_unpredict, ntiles, UNP_THREADS, 0, ua);   // very wide, flat tiles only
@@ -1235,9 +1172,6 @@ extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const
     int rc = 0;
     std::vector<xpngb_ctx*> used(nchunks, nullptr);
     std::vector<uint32_t> cn(nchunks, 0);
-    // staggered waves (batches only): the latency-bound context decode of one wave runs under the issue-bound walk of the wave before
-    uint32_t stagger = lat ? 0u : (l2 ? ctx->dec_stagger2 : ctx->dec_stagger1);
-    if (stagger >= ctx->pipe_lanes) stagger = 0;
     auto chunk_done = [&](uint32_t ci) -> int {   // wait for chunk ci, read its error flag
         xpngb_ctx* lane = used[ci];
         CK(cudaStreamSynchronize(lane->stream));
@@ -1262,7 +1196,6 @@ extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const
                 snprintf(ctx->err, sizeof ctx->err, "host to device copy failed"); rc = 1; break;
             }
         }
-        if (stagger && ci >= stagger && cudaStreamWaitEvent(lane->stream, used[ci - stagger]->ev_stage, 0) != cudaSuccess) { snprintf(ctx->err, sizeof ctx->err, "cudaStreamWaitEvent failed"); rc = 1; break; }
         rc = decode_issue(lane, lat, imgs + i0, m, hdr.data() + 2 * i0, din, file_offsets + i0, file_sizes + i0, dpx, pixels_cap, (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;

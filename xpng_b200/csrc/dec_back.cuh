@@ -1,5 +1,5 @@
-// dec_back.cuh — decode back end shared by levels 1 and 2, plus the level-2 front (tile parse, v1
-// rANS decode, libxpng.c:262-301, :868-961).
+// dec_back.cuh — decode back end shared by levels 1 and 2, plus the level-2 tile parse (libxpng.c:868-961;
+// the v1 rANS decoders, libxpng.c:262-301, are in dec_rans_lat.cuh and dec_rans_pair.cuh).
 //   nl sequence  ->  per-chunk counts  ->  per-tile scan (bit / value offsets)  ->  residual plane
 //   (one packed zig-zag triple per coded pixel)  ->  wavefront un-predict.
 // Everything except the per-tile chunk scan and the wavefront itself is data-parallel.
@@ -69,148 +69,6 @@ __global__ void k_dec_parse_m2(const TileDesc* tiles, const DecImage* imgs, cons
         d->bsz = bsz; d->nsym = grey ? t.npx - 1 : nsym;
     } else bad = true;
     if (bad) { dec_fail(err, DEC_BAD_BLOCK); d->m = 0xFE; }
-}
-
-// ------------------------------------------------------------------------------------------------
-// v1 block decoder (forward, libxpng.c:262-301): one lane per block.  The frequency table (or the
-// raw symbols of a type-2 block) is read from the tile's shared side stream at bitpos[c].
-// ------------------------------------------------------------------------------------------------
-struct RansV1DecArgs {
-    const TileDesc* tiles;
-    const DecImage* imgs;
-    const DecTile* dt;
-    const uint8_t* in;
-    uint8_t* streams;
-    uint32_t ntiles;
-    uint32_t c0, nc;
-    uint32_t nmin, nmax;   // alphabet sizes handled by this launch: nmin < N <= nmax
-};
-
-#define XPB_RENORM_FWD(x)                                                              \
-    if ((x) < (1ull << 31)) { (x) = ((x) << 32) | wa; wa = wb; if (rp < rend) rp += 4;  \
-        wb = (rp + 8 <= rend) ? ld32u(rp + 4) : 0u; }
-
-// Returns false when the lane has nothing to do; otherwise fills the per-block geometry.
-struct V1Block { const uint8_t* blob; const uint8_t* blk; uint8_t* out; uint32_t n, type, N, bitpos, bsz, bsize; int pb; };
-
-__device__ __forceinline__ bool v1_block_setup(const RansV1DecArgs& A, uint32_t id, V1Block& B) {
-    if (id >= A.nc * A.ntiles) return false;
-    const uint32_t c = A.c0 + id / A.ntiles, tile = id % A.ntiles;
-    const TileDesc t = A.tiles[tile];
-    if (A.imgs[t.img].mode != 2) return false;
-    const DecTile* d = A.dt + tile;
-    const uint32_t kind = d->m >> 4;
-    if (d->m == 0xFE || d->m == 0xFF || d->m == 0 || (kind == 2 && (d->m & 8))) return false;
-    const bool grey = kind == 2;
-    if (grey && c != 0) return false;
-    B.N = grey ? 256u : (uint32_t)DEC_M2_NSYM[c]; B.pb = grey ? 15 : 14;
-    if (B.N <= A.nmin || B.N > A.nmax) return false;
-    const DecBlock b = d->blk[c];
-    B.blob = A.in + d->blob_off; B.blk = B.blob + b.off; B.out = A.streams + t.str_off + b.soff;
-    B.n = b.n; B.type = b.type; B.bitpos = d->bitpos[c]; B.bsz = d->bsz; B.bsize = ld32u(B.blk) & 0xFFFFFFu;
-    if (B.type == 0 || B.n == 0) return false;
-    const bool ctx = !grey && c < 9;   // context streams: symbols above 8 (corrupt data) are stored as 0, the walk indexes lanes by them
-    if (B.type == 1) {
-        const uint32_t v1 = ld32u(B.blk + 4) >> 24, v4 = (ctx && v1 > 8u ? 0u : v1) * 0x01010101u;
-        for (uint32_t k = 0; k < (B.n + 3) / 4; k++) reinterpret_cast<uint32_t*>(B.out)[k] = v4;
-        return false;
-    }
-    if (B.type == 2) {
-        BitR r{ B.blob + 8, B.blob + 4 + B.bsz, B.bitpos };
-        const uint32_t nbit = bitlen32(B.N - 1);
-        for (uint32_t k = 0; k < B.n; k++) { const uint32_t v = r.get(nbit); B.out[k] = (uint8_t)(ctx && v > 8u ? 0u : v); }
-        return false;
-    }
-    return true;
-}
-
-template <int NTH, int LANES>
-__global__ void __launch_bounds__(LANES) k_dec_rans_v1_small(RansV1DecArgs A) {
-    __shared__ uint32_t fs[(NTH + 1) * LANES];   // [sym][lane]: start | freq << 16
-    V1Block B;
-    if (!v1_block_setup(A, blockIdx.x * LANES + threadIdx.x, B)) return;
-    const int pb = B.pb;
-    uint32_t th[NTH];
-    {
-        BitR r{ B.blob + 8, B.blob + 4 + B.bsz, B.bitpos };
-        uint32_t acc = 0;
-#pragma unroll
-        for (int i = 0; i <= NTH; i++) {
-            uint32_t f = 0;
-            if ((uint32_t)i < B.N) f = B.type == 3 ? r.get((uint32_t)pb) : (r.get(1) ? r.get((uint32_t)pb) : 0u);
-            fs[i * LANES + threadIdx.x] = (acc & 0xFFFFu) | (f << 16);
-            acc += f;
-            if (i < NTH) th[i] = (uint32_t)(i + 1) < B.N ? acc : 0xFFFFFFFFu;
-        }
-    }
-    const uint32_t mask = (1u << pb) - 1u;
-    const uint8_t* rend = B.blk + B.bsize; const uint8_t* rp = B.blk + 24;
-    uint64_t x0 = ld64u(B.blk + 8), x1 = ld64u(B.blk + 16);
-    uint32_t wa = (rp + 4 <= rend) ? ld32u(rp) : 0u, wb = (rp + 8 <= rend) ? ld32u(rp + 4) : 0u;
-    auto sym_of = [&](uint64_t x) -> uint32_t {
-        const uint32_t slot = (uint32_t)x & mask; uint32_t s = 0;
-#pragma unroll
-        for (int i = 0; i < NTH; i++) s += slot >= th[i];
-        return s;
-    };
-    auto step = [&](uint64_t& x) -> uint32_t {
-        const uint32_t s = sym_of(x), slot = (uint32_t)x & mask, e = fs[s * LANES + threadIdx.x];
-        x = (uint64_t)(e >> 16) * (x >> pb) + slot - (e & 0xFFFFu);
-        XPB_RENORM_FWD(x)
-        return s;
-    };
-    const uint32_t n = B.n; uint32_t i = 0;
-    for (; i + 4 <= n; i += 4) {
-        const uint32_t s0 = step(x0), s1 = step(x1), s2 = step(x0), s3 = step(x1);
-        *reinterpret_cast<uint32_t*>(B.out + i) = s0 | (s1 << 8) | (s2 << 16) | (s3 << 24);
-    }
-    for (; i < n; i++) B.out[i] = (uint8_t)((i & 1) ? step(x1) : step(x0));
-}
-
-template <int LANES>
-__global__ void __launch_bounds__(LANES) k_dec_rans_v1_big(RansV1DecArgs A) {
-    extern __shared__ __align__(16) uint8_t smem_big[];
-    uint16_t* cumS = reinterpret_cast<uint16_t*>(smem_big) + threadIdx.x * 258;
-    uint8_t* coarse = smem_big + LANES * 258 * 2 + threadIdx.x * 260;
-    V1Block B;
-    if (!v1_block_setup(A, blockIdx.x * LANES + threadIdx.x, B)) return;
-    const int pb = B.pb;
-    {
-        BitR r{ B.blob + 8, B.blob + 4 + B.bsz, B.bitpos };
-        uint32_t acc = 0;
-        for (uint32_t i = 0; i < 256; i++) {
-            cumS[i] = (uint16_t)acc;
-            uint32_t f = 0;
-            if (i < B.N) f = B.type == 3 ? r.get((uint32_t)pb) : (r.get(1) ? r.get((uint32_t)pb) : 0u);
-            acc += f; if (acc > (1u << pb)) acc = 1u << pb;
-        }
-        cumS[256] = (uint16_t)acc;
-        uint32_t s = 0;
-        for (uint32_t k = 0; k < 256; k++) {
-            const uint32_t slot = k << (pb - 8);
-            while (s < 255 && (uint32_t)cumS[s + 1] <= slot) s++;
-            coarse[k] = (uint8_t)s;
-        }
-    }
-    const uint32_t mask = (1u << pb) - 1u;
-    const uint8_t* rend = B.blk + B.bsize; const uint8_t* rp = B.blk + 24;
-    uint64_t x0 = ld64u(B.blk + 8), x1 = ld64u(B.blk + 16);
-    uint32_t wa = (rp + 4 <= rend) ? ld32u(rp) : 0u, wb = (rp + 8 <= rend) ? ld32u(rp + 4) : 0u;
-    auto step = [&](uint64_t& x) -> uint32_t {
-        const uint32_t slot = (uint32_t)x & mask;
-        uint32_t s = coarse[slot >> (pb - 8)];
-        while (s < 255 && (uint32_t)cumS[s + 1] <= slot) s++;
-        const uint32_t start = cumS[s], f = (uint32_t)cumS[s + 1] - start;
-        x = (uint64_t)f * (x >> pb) + slot - start;
-        XPB_RENORM_FWD(x)
-        return s;
-    };
-    const uint32_t n = B.n; uint32_t i = 0;
-    for (; i + 4 <= n; i += 4) {
-        const uint32_t s0 = step(x0), s1 = step(x1), s2 = step(x0), s3 = step(x1);
-        *reinterpret_cast<uint32_t*>(B.out + i) = s0 | (s1 << 8) | (s2 << 16) | (s3 << 24);
-    }
-    for (; i < n; i++) B.out[i] = (uint8_t)((i & 1) ? step(x1) : step(x0));
 }
 
 // ------------------------------------------------------------------------------------------------

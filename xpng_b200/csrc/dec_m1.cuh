@@ -91,9 +91,8 @@ __global__ void k_dec_parse_m1(const TileDesc* tiles, const DecImage* imgs, cons
 }
 
 // ------------------------------------------------------------------------------------------------
-// v2 block decoder: one lane per block.  Small alphabets (<= 16 symbols) search the cumulative
-// table held in registers; the 256-symbol alpha alphabet uses a coarse 256-entry start table plus a
-// short linear scan over cum[] in shared memory.
+// Entropy blocks: the bit reader of block headers and frequency tables, and the argument block of
+// the level-1 rANS decoder (k_dec_rans_v2_lat, dec_rans_lat.cuh).
 // ------------------------------------------------------------------------------------------------
 struct BitR {   // MSB-first reader over unaligned LE words; zero past `end` (libxpng.c:12)
     const uint8_t* base; const uint8_t* end; uint32_t pos;
@@ -123,152 +122,9 @@ struct RansDecArgs {
     int* err;
 };
 
-// decode step shared by all variants: x' = f*(x>>pb) + slot - start, then renormalise from *rp backwards
-#define XPB_RENORM_BACK(x)                                                                 \
-    if ((x) < (1ull << 31)) { const uint32_t wv = wa; wa = wb; if (rp > lo) rp -= 4; \
-        wb = (rp - 8 >= lo) ? ld32u(rp - 8) : 0u; (x) = ((x) << 32) | wv; }
-
-template <int LANES>
-__global__ void __launch_bounds__(LANES) k_dec_rans_v2_small(RansDecArgs A) {
-    __shared__ uint32_t fs[16 * LANES];   // [sym][lane]: start | freq << 16
-    const uint32_t id = blockIdx.x * LANES + threadIdx.x;
-    if (id >= A.nc * A.ntiles) return;
-    const uint32_t c = A.c0 + id / A.ntiles, tile = id % A.ntiles;
-    const TileDesc t = A.tiles[tile];
-    if (A.imgs[t.img].mode != 1) return;
-    const DecTile* d = A.dt + tile;
-    if (d->m == 0 || d->m == 0xFE) return;
-    const DecBlock b = d->blk[c];
-    const uint8_t* blk = A.in + d->blob_off + b.off;
-    uint8_t* out = A.streams + t.str_off + b.soff;
-    const uint32_t n = b.n;
-    if (b.type == 0 || n == 0) return;
-    const uint32_t w1 = ld32u(blk + 4), v2 = w1 >> 24;
-    const uint32_t csz = ld32u(blk) & 0xFFFFFFu;
-    // this kernel only decodes context streams (c < 9): symbols above 8 can only come from corrupt data and are
-    // stored as 0, because the context walk uses them as lane indices
-    if (b.type == 1) {   // run of one symbol
-        const uint32_t v4 = (v2 > 8u ? 0u : v2) * 0x01010101u;
-        for (uint32_t k = 0; k < (n + 3) / 4; k++) reinterpret_cast<uint32_t*>(out)[k] = v4;
-        return;
-    }
-    if (b.type == 2) {   // plain v2-bit symbols
-        BitR r{ blk + 8, blk + csz, 0 };
-        for (uint32_t k = 0; k < n; k++) { const uint32_t v = r.get(v2); out[k] = (uint8_t)(v > 8u ? 0u : v); }
-        return;
-    }
-    const uint32_t N = v2 + 2, w2 = ld32u(blk + 8); const int pb = (int)(w2 >> 24);
-    const uint32_t tabw = w2 & 0xFFFFFFu;
-    if (N > 16 || pb < 10 || pb > 15 || 8 + 4ull * tabw > csz || tabw < 5) { for (uint32_t k = 0; k < n; k++) out[k] = 0; return; }
-    const uint8_t* tab = blk + 8 + 4ull * tabw; const uint8_t* lo = blk + 12;
-    uint32_t cum[17];
-    {
-        BitR r{ tab, blk + csz, 0 };
-        cum[0] = 0;
-        for (uint32_t i = 0; i < 16; i++) {
-            uint32_t f = 0;
-            if (i < N) f = b.type == 3 ? r.get((uint32_t)pb) : (r.get(1) ? r.get((uint32_t)pb) : 0u);
-            cum[i + 1] = cum[i] + f;
-            fs[i * LANES + threadIdx.x] = (cum[i] & 0xFFFFu) | (f << 16);
-        }
-    }
-    // thresholds: symbol s = #{ i in 1..15 : slot >= cum[i] } restricted to symbols with freq > 0.
-    // cum is non-decreasing, zero-width symbols share a threshold with their successor, so the count of
-    // thresholds <= slot lands on the last symbol whose start <= slot, i.e. the one with non-zero width.
-    uint32_t th[15];
-#pragma unroll
-    for (int i = 0; i < 15; i++) th[i] = (uint32_t)(i + 1) < N ? cum[i + 1] : 0xFFFFFFFFu;
-    const uint32_t mask = (1u << pb) - 1u;
-    const uint8_t* rp = tab - 16;
-    uint64_t x0 = ld64u(rp), x1 = ld64u(rp + 8);
-    uint32_t wa = (rp - 4 >= lo) ? ld32u(rp - 4) : 0u, wb = (rp - 8 >= lo) ? ld32u(rp - 8) : 0u;
-    // note: XPB_RENORM_BACK consumes wa (= word at rp-4), then moves rp down by one word.
-    auto step = [&](uint64_t& x) -> uint32_t {
-        const uint32_t slot = (uint32_t)x & mask;
-        uint32_t s = 0;
-#pragma unroll
-        for (int i = 0; i < 15; i++) s += slot >= th[i];
-        const uint32_t e = fs[s * LANES + threadIdx.x];
-        x = (uint64_t)(e >> 16) * (x >> pb) + slot - (e & 0xFFFFu);
-        XPB_RENORM_BACK(x)
-        return s > 8u ? 0u : s;
-    };
-    int64_t i = (int64_t)n - 1;
-    // head: until (i + 1) is a multiple of 4
-    for (; i >= 0 && ((i + 1) & 3); i--) out[i] = (uint8_t)((i & 1) ? step(x1) : step(x0));
-    for (; i >= 3; i -= 4) {
-        const uint32_t s3 = step(x1), s2 = step(x0), s1 = step(x1), s0 = step(x0);
-        *reinterpret_cast<uint32_t*>(out + i - 3) = s0 | (s1 << 8) | (s2 << 16) | (s3 << 24);
-    }
-}
-
-// 256-symbol alphabets (alpha plane, PB = 15): one warp-lane per block, tables in shared memory.
-template <int LANES>
-__global__ void __launch_bounds__(LANES) k_dec_rans_v2_big(RansDecArgs A) {
-    extern __shared__ __align__(16) uint8_t smem_big[];
-    // per lane: cum[257] as u16 (pitch 258 -> odd word pitch 129, conflict-free) + coarse[256] u8
-    uint16_t* cumS = reinterpret_cast<uint16_t*>(smem_big) + threadIdx.x * 258;
-    uint8_t* coarse = smem_big + LANES * 258 * 2 + threadIdx.x * 260;
-    const uint32_t tile = blockIdx.x * LANES + threadIdx.x;
-    if (tile >= A.ntiles) return;
-    const TileDesc t = A.tiles[tile];
-    if (A.imgs[t.img].mode != 1 || t.pxsz != 4) return;
-    const DecTile* d = A.dt + tile;
-    if (d->m == 0 || d->m == 0xFE) return;
-    const DecBlock b = d->blk[9];
-    const uint8_t* blk = A.in + d->blob_off + b.off;
-    uint8_t* out = A.alpha + t.px_off;
-    const uint32_t n = b.n;
-    if (b.type == 0 || n == 0) return;
-    const uint32_t w1 = ld32u(blk + 4), v2 = w1 >> 24, csz = ld32u(blk) & 0xFFFFFFu;
-    if (b.type == 1) { const uint32_t v4 = v2 * 0x01010101u; for (uint32_t k = 0; k < (n + 3) / 4; k++) reinterpret_cast<uint32_t*>(out)[k] = v4; return; }
-    if (b.type == 2) { BitR r{ blk + 8, blk + csz, 0 }; for (uint32_t k = 0; k < n; k++) out[k] = (uint8_t)r.get(v2); return; }
-    const uint32_t N = v2 + 2, w2 = ld32u(blk + 8); const int pb = (int)(w2 >> 24);
-    const uint32_t tabw = w2 & 0xFFFFFFu;
-    if (N > 256 || pb < 10 || pb > 15 || 8 + 4ull * tabw > csz || tabw < 5) { for (uint32_t k = 0; k < n; k++) out[k] = 0; return; }
-    const uint8_t* tab = blk + 8 + 4ull * tabw; const uint8_t* lo = blk + 12;
-    {
-        BitR r{ tab, blk + csz, 0 };
-        uint32_t acc = 0;
-        for (uint32_t i = 0; i < 256; i++) {
-            cumS[i] = (uint16_t)acc;
-            uint32_t f = 0;
-            if (i < N) f = b.type == 3 ? r.get((uint32_t)pb) : (r.get(1) ? r.get((uint32_t)pb) : 0u);
-            acc += f; if (acc > (1u << pb)) acc = 1u << pb;
-        }
-        cumS[256] = (uint16_t)(acc >= 65536u ? 65535u : acc);   // 2^15 at most (pb <= 15)
-        // coarse[k] = symbol containing slot k << (pb-8)
-        uint32_t s = 0;
-        for (uint32_t k = 0; k < 256; k++) {
-            const uint32_t slot = k << (pb - 8);
-            while (s < 255 && (uint32_t)cumS[s + 1] <= slot) s++;
-            coarse[k] = (uint8_t)s;
-        }
-    }
-    const uint32_t mask = (1u << pb) - 1u;
-    const uint8_t* rp = tab - 16;
-    uint64_t x0 = ld64u(rp), x1 = ld64u(rp + 8);
-    uint32_t wa = (rp - 4 >= lo) ? ld32u(rp - 4) : 0u, wb = (rp - 8 >= lo) ? ld32u(rp - 8) : 0u;
-    auto step = [&](uint64_t& x) -> uint32_t {
-        const uint32_t slot = (uint32_t)x & mask;
-        uint32_t s = coarse[slot >> (pb - 8)];
-        while (s < 255 && (uint32_t)cumS[s + 1] <= slot) s++;
-        const uint32_t start = cumS[s], f = (uint32_t)cumS[s + 1] - start;
-        x = (uint64_t)f * (x >> pb) + slot - start;
-        XPB_RENORM_BACK(x)
-        return s;
-    };
-    int64_t i = (int64_t)n - 1;
-    for (; i >= 0 && ((i + 1) & 3); i--) out[i] = (uint8_t)((i & 1) ? step(x1) : step(x0));
-    for (; i >= 3; i -= 4) {
-        const uint32_t s3 = step(x1), s2 = step(x0), s1 = step(x1), s0 = step(x0);
-        *reinterpret_cast<uint32_t*>(out + i - 3) = s0 | (s1 << 8) | (s2 << 16) | (s3 << 24);
-    }
-}
-
 // ------------------------------------------------------------------------------------------------
 // Context walk: nl_{i+1} = next unread symbol of stream nl_i.  Inherently serial per tile; the kernels
-// (k_dec_walk_smem, k_dec_walk_lat) live in dec_rans_lat.cuh, this is their argument block.
+// (k_dec_walk_smem, k_dec_walk_ring in dec_rans_lat.cuh, k_dec_walk3 in dec_walk3.cuh) take this argument block.
 // ------------------------------------------------------------------------------------------------
 struct WalkArgs {
     const TileDesc* tiles;

@@ -12,7 +12,7 @@
 // cooperate on everything that is parallel: table construction, run (type 1) and raw (type 2) blocks.
 // Alphabets above 16 symbols (or PROB_BITS 15) use a byte table slot -> symbol plus a 256-entry
 // (freq, start) table: two dependent shared loads per symbol.
-// The lane-per-block kernels in dec_m1.cuh / dec_back.cuh remain the throughput variant for large batches.
+// Large batches decode with the pair decoders of dec_rans_pair.cuh.
 #pragma once
 #include "common.cuh"
 #include "dec_m1.cuh"
@@ -221,15 +221,14 @@ __global__ void __launch_bounds__(32) k_dec_rans_v2_lat(RansDecArgs A, uint32_t 
     const uint32_t N = v2 + 2, w2 = ld32u(blk + 8); const int pb = (int)(w2 >> 24);
     const uint32_t tabw = w2 & 0xFFFFFFu;
     const bool two = N > 16 || (4u << pb) > lut_bytes;
-    // a context stream never has more than 9 symbols: a larger alphabet is corrupt data and is refused here exactly as in
-    // the lane-per-block kernel (k_dec_rans_v2_small), so both families agree on corrupt input
+    // a context stream never has more than 9 symbols: a table of more than 16 is corrupt data, and the block decodes as zeros
     if (N > 256 || (ctx && N > 16) || pb < 10 || pb > 15 || 8 + 4ull * tabw > csz || tabw < 5 || (two && (1u << pb) + 1024u > lut_bytes)) {
         for (uint32_t k = lane; k < n; k += 32) out[k] = 0;
         return;
     }
     const uint8_t* tab = blk + 8 + 4ull * tabw;
     lat_read_table(cum, tab, blk + csz, 0, N, pb, b.type == 4, lane);
-    if (cum[N] != (1u << pb)) {   // a valid table sums to 2^PROB_BITS exactly (libxpng.c:316-329); refused in both kernel families
+    if (cum[N] != (1u << pb)) {   // a valid table sums to 2^PROB_BITS exactly (libxpng.c:316-329); any other sum fails the call
         if (lane == 0) dec_fail(A.err, DEC_BAD_BLOCK);
         for (uint32_t k = lane; k < n; k += 32) out[k] = 0;
         return;
@@ -309,12 +308,13 @@ __global__ void __launch_bounds__(32) k_dec_rans_v1_lat(RansV1LatArgs A) {
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Context walk, latency variant (nl_{i+1} = next unread symbol of stream nl_i, libxpng.c:803).
-// One warp per tile, lane c < 9 owns stream c (64-bit register window of eight byte symbols, the next
-// eight prefetched).  Every lane publishes the head of its stream in `info`; the whole dependent chain
-// is ONE shuffle per symbol: got = shfl(info, cur) with cur = the previous got.  The owner pops its
-// window while the shuffle is in flight (the pop depends on cur only), so self-transitions cost nothing
-// extra.  Lane j of each group of 32 steps keeps symbol j; one coalesced store per 32 symbols.
+// Context walk (nl_{i+1} = next unread symbol of stream nl_i, libxpng.c:803).  One warp per tile, lane
+// c < 9 owns stream c (64-bit register window of up to 16 nibble symbols, the next eight packed behind
+// it).  Every lane publishes the head of its stream in `info`; the whole dependent chain is ONE shuffle
+// per symbol: got = shfl(info, cur) with cur = the previous got.  The owner pops its window while the
+// shuffle is in flight (the pop depends on cur only), so self-transitions cost nothing extra.  Lane j
+// of each group of 32 steps keeps symbol j; one coalesced store per 32 symbols.  The walks below differ
+// in where a window refill comes from; k_dec_walk3 (dec_walk3.cuh) walks three tiles per warp.
 // ---------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t walk_pack8(uint2 q) {   // eight byte symbols (<= 15) -> eight nibbles, first symbol lowest
     uint32_t a = (q.x | (q.x >> 4)) & 0x00FF00FFu; a = (a | (a >> 8)) & 0xFFFFu;
@@ -322,74 +322,9 @@ __device__ __forceinline__ uint32_t walk_pack8(uint2 q) {   // eight byte symbol
     return a | (b << 16);
 }
 
-template <int WARPS>
-__global__ void __launch_bounds__(WARPS * 32) k_dec_walk_lat(WalkArgs A) {
-    const uint32_t tile = blockIdx.x * WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (tile >= A.ntiles) return;
-    const TileDesc t = A.tiles[tile];
-    if (A.imgs[t.img].mode != A.mode) return;
-    const DecTile* d = A.dt + tile;
-    if (d->m == 0 || d->m >= 0x20) return;   // raw / grey / single colour / failed
-    uint8_t* out = A.nlseq + t.px_off;
-    const uint32_t m = d->nsym;
-    const uint32_t c = lane < 9 ? lane : 0;
-    const uint32_t nch = lane < 9 ? (d->blk[c].n + 7) / 8 : 0;   // 8-symbol chunks of my stream (symbols are <= 8 by construction)
-    const uint2* src = reinterpret_cast<const uint2*>(A.streams + t.str_off + d->blk[c].soff);
-    auto chunk = [&](uint32_t k) -> uint2 { return k < nch ? __ldg(src + k) : make_uint2(0u, 0u); };
-    // window: 64 bits = up to 16 nibble symbols (cnt valid); nbuf: the next 8, packed; raw: the 8 after those, as loaded
-    uint32_t wlo = walk_pack8(chunk(0)), whi = walk_pack8(chunk(1)), cnt = 16;
-    uint32_t nbuf = walk_pack8(chunk(2));
-    uint2 raw = chunk(3);
-    uint32_t ch = 4;
-    uint32_t info = wlo & 0xFu, cur = 0;
-    uint32_t mk[32];
-#pragma unroll
-    for (int j = 0; j < 32; j++) mk[j] = lane == (uint32_t)j ? 0xFFFFFFFFu : 0u;
-    for (uint32_t pos = 0; pos < m; pos += 32) {
-        uint32_t keep = 0;
-#pragma unroll
-        for (int j = 0; j < 32; j++) {
-            const uint32_t got = __shfl_sync(0xffffffffu, info, cur);   // the chain: one shuffle per symbol
-            // the owner pops while the shuffle is in flight (depends on cur only)
-            const bool own = lane == cur;
-            const uint32_t plo = __funnelshift_r(wlo, whi, 4), phi = whi >> 4;
-            wlo = own ? plo : wlo; whi = own ? phi : whi; cnt -= own ? 1u : 0u;
-            info = wlo & 0xFu;
-            keep |= got & mk[j];
-            cur = got;
-            if ((j & 7) == 7) {
-                // every 8 steps, branch-free: windows that dropped to <= 8 symbols take the next 8 (so a window
-                // never runs dry within the following 8 steps), and the prefetch moves on
-                const bool need = cnt <= 8u;
-                const unsigned long long add = (unsigned long long)nbuf << (4u * min(cnt, 8u));
-                wlo |= need ? (uint32_t)add : 0u; whi |= need ? (uint32_t)(add >> 32) : 0u;
-                info = wlo & 0xFu;
-                cnt += need ? 8u : 0u;
-                nbuf = need ? walk_pack8(raw) : nbuf;
-                const uint32_t doload = (need && ch < nch) ? 1u : 0u;
-                raw.x = need ? 0u : raw.x; raw.y = need ? 0u : raw.y;
-#ifndef XPB_WALK_PF
-#define XPB_WALK_PF 16
-#endif
-                // the load is consumed 8 steps (~400 cycles) later: enough for an L1 hit, not for a miss, and a miss stalls
-                // the whole in-order chain.  So the line after next is requested from L2 now (a line = 16 chunks).
-#if XPB_WALK_PF > 0
-                asm volatile("{\n .reg .pred q;\n setp.ne.u32 q, %3, 0;\n @q ld.global.nc.v2.u32 {%0, %1}, [%2];\n @q prefetch.global.L1 [%4];\n}"
-                             : "+r"(raw.x), "+r"(raw.y) : "l"(src + ch), "r"(doload), "l"(src + min(ch + XPB_WALK_PF, nch - 1)));
-#else
-                asm volatile("{\n .reg .pred q;\n setp.ne.u32 q, %3, 0;\n @q ld.global.nc.v2.u32 {%0, %1}, [%2];\n}"
-                             : "+r"(raw.x), "+r"(raw.y) : "l"(src + ch), "r"(doload));
-#endif
-                ch += need ? 1u : 0u;
-            }
-        }
-        if (pos + lane < m) out[pos + lane] = (uint8_t)keep;
-    }
-}
-
 // Shared-memory variant (the tile's streams fit): the warp first packs the nine streams to nibbles in
 // shared memory (coalesced), then walks; a window refill is one shared load of eight symbols, so no
-// global-memory latency remains inside the walk.  ~31 cycles per symbol against ~40 for the variant above.
+// global-memory latency remains inside the walk.  ~31 cycles per symbol.
 constexpr uint32_t WALK_SMEM_MAX_SYMS = 400000;   // 200 KB of nibbles (+ 9 pad words) per tile
 
 template <int DUMMY>

@@ -1,6 +1,6 @@
 // enc_back.cuh — encode back end for level 1: per-tile segment scan, stream compaction, frequency
-// normalisation + 2-state rANS (v2 blocks, libxpng.c:307-427), size decisions and final assembly
-// (libxpng.c:534-571, :723-789).
+// normalisation and rANS encoder symbols (the v2 block encoder, libxpng.c:307-427, is k_rans_v2_pair in
+// enc_rans_lat.cuh), size decisions and final assembly (libxpng.c:534-571, :723-789).
 #pragma once
 #include "common.cuh"
 #include "enc_front.cuh"
@@ -203,15 +203,6 @@ __device__ __forceinline__ uint4 make_encsym(uint32_t freq, uint32_t start, int 
     return make_uint4((uint32_t)rcp, (uint32_t)(rcp >> 32), bias | (cmpl << 16), freq | (shift << 16));
 }
 
-// One rANS step (libxpng.c:370-376): optional 32-bit renormalisation word, then the state update.
-__device__ __forceinline__ void rans_enc_step(uint64_t& x, const uint4 e, int pb, uint32_t*& wp) {
-    const uint64_t xmax = (uint64_t)(e.w & 0xFFFFu) << (63 - pb);
-    if (x >= xmax) { *wp++ = (uint32_t)x; x >>= 32; }
-    const uint64_t rcp = (uint64_t)e.x | ((uint64_t)e.y << 32);
-    const uint64_t q = __umul64hi(x, rcp) >> (e.w >> 16);
-    x += (e.z & 0xFFFFu) + q * (e.z >> 16);
-}
-
 // MSB-first bit writer over 32-bit words (libxpng.c:8-11).
 struct BitW {
     uint64_t acc; uint32_t n; uint32_t* out;
@@ -223,9 +214,7 @@ struct BitW {
 };
 
 // ------------------------------------------------------------------------------------------------
-// v2 block encoder: one lane per stream, LANES lanes per CTA, symbol table in shared memory laid out
-// [symbol][lane] so that lanes indexing different symbols never bank-conflict.
-// Stream ids are context-major (id = c * ntiles + tile) so that a warp holds streams of similar length.
+// v2 block encoder arguments (k_rans_v2_pair, enc_rans_lat.cuh).
 // ------------------------------------------------------------------------------------------------
 struct RansV2Args {
     const TileDesc* tiles;
@@ -238,86 +227,6 @@ struct RansV2Args {
     uint32_t c0, nc;          // stream index range handled by this launch [c0, c0+nc)
     const uint32_t* order = nullptr; const uint32_t* total = nullptr;   // pair encoders: sorted work list instead of the id range
 };
-
-template <int NSYM, int LANES>
-__global__ void __launch_bounds__(LANES) k_rans_v2(RansV2Args A) {
-    extern __shared__ __align__(16) uint4 etab[];   // [NSYM][LANES]
-    const uint32_t id = blockIdx.x * LANES + threadIdx.x;
-    if (id >= A.nc * A.ntiles) return;
-    const uint32_t c = A.c0 + id / A.ntiles, tile = id % A.ntiles;
-    const TileDesc t = A.tiles[tile];
-    TileState* st = A.state + tile;
-    const uint32_t n = st->len[c];
-    if (c == 9 && t.pxsz != 4) { st->bsize[9] = 0; return; }
-    const int pb = c == 9 ? 15 : 12;
-    uint32_t* F = A.hist + (uint64_t)tile * HIST_STRIDE_M1 + (c == 9 ? HIST_ALPHA : HIST_CTX + c * 16);
-    const uint8_t* in = c == 9 ? A.alpha + t.px_off : A.streams + stream_slice(t) + st->soff[c];
-    uint8_t* out = A.blocks + block_slice(t, tile) + st->boff[c];
-    uint32_t* o = reinterpret_cast<uint32_t*>(out);
-    if (n == 0) { o[0] = 4; st->bsize[c] = 4; return; }                       // libxpng.c:313
-    int top = (c == 9 ? 256 : 9); while (F[--top] == 0) {}
-    const uint32_t N = (uint32_t)top + 1, nbit = bitlen32((uint32_t)top);
-    uint32_t used = 0;
-    for (uint32_t i = 0; i < N; i++) used += F[i] != 0;
-    if (used == 1) { o[0] = 8u | (1u << 24); o[1] = n | ((uint32_t)in[0] << 24); st->bsize[c] = 8; return; }   // :318
-
-    uint32_t cum[NSYM + 1];
-    normalise_freqs(F, cum, N, n, pb);
-    uint4* E = etab + threadIdx.x;
-    for (uint32_t i = 0; i < N; i++) E[i * LANES] = make_encsym(cum[i + 1] - cum[i], cum[i], pb);
-
-    uint32_t* wp = o + 3;
-    uint64_t x0 = 1ull << 31, x1 = 1ull << 31;
-    uint32_t i = 0;
-    const uint4* in16 = reinterpret_cast<const uint4*>(in);
-    if (n >= 16) {
-        uint4 nxt = in16[0];
-        for (; i + 16 <= n; i += 16) {
-            const uint4 v = nxt;
-            if (i + 32 <= n) nxt = in16[(i >> 4) + 1];
-            const uint32_t w[4] = { v.x, v.y, v.z, v.w };
-#pragma unroll
-            for (int k = 0; k < 16; k += 2) {
-                const uint32_t s0 = (w[k >> 2] >> (8 * (k & 3))) & 0xFFu, s1 = (w[(k + 1) >> 2] >> (8 * ((k + 1) & 3))) & 0xFFu;
-                const uint4 e0 = E[s0 * LANES], e1 = E[s1 * LANES];
-                rans_enc_step(x0, e0, pb, wp);
-                rans_enc_step(x1, e1, pb, wp);
-            }
-        }
-    }
-    for (; i + 2 <= n; i += 2) {
-        const uint4 e0 = E[(uint32_t)in[i] * LANES], e1 = E[(uint32_t)in[i + 1] * LANES];
-        rans_enc_step(x0, e0, pb, wp);
-        rans_enc_step(x1, e1, pb, wp);
-    }
-    if (n & 1) { const uint4 e0 = E[(uint32_t)in[i] * LANES]; rans_enc_step(x0, e0, pb, wp); }                 // :382-392
-    wp[0] = (uint32_t)x0; wp[1] = (uint32_t)(x0 >> 32); wp[2] = (uint32_t)x1; wp[3] = (uint32_t)(x1 >> 32); wp += 4;   // :394
-
-    const bool sparse = (N + used * (uint32_t)pb) < N * (uint32_t)pb;                                         // :396-397
-    o[1] = n | ((N - 2) << 24);
-    o[2] = (uint32_t)(wp - (o + 2)) | ((uint32_t)pb << 24);                                                   // :400
-    BitW b{ 0, 0, wp };
-    for (uint32_t k = 0; k < N; k++) {
-        const uint32_t f = cum[k + 1] - cum[k];
-        if (!sparse) b.put((uint32_t)pb, f);
-        else if (f) b.put((uint32_t)pb + 1, f + (1u << pb));
-        else b.put(1, 0);
-    }
-    b.end();
-    uint32_t csz = (uint32_t)((uint8_t*)b.out - out);
-    o[0] = csz | ((3u + (uint32_t)sparse) << 24);
-    const uint64_t rawbits = (uint64_t)nbit * n;
-    const uint32_t rawsz = 8 + (uint32_t)(rawbits / 32) * 4 + ((rawbits % 32) ? 4 : 0);
-    if (csz >= rawsz) {                                                                                      // :417-424
-        o[1] = n | (nbit << 24);
-        BitW r{ 0, 0, o + 2 };
-        for (uint32_t k = 0; k < n; k++) r.put(nbit, in[k]);
-        r.end();
-        csz = (uint32_t)((uint8_t*)r.out - out);
-        o[0] = csz | (2u << 24);
-    }
-    st->bsize[c] = csz;
-}
 
 // ------------------------------------------------------------------------------------------------
 // Sizes: per image, serial over its tiles (tile blob sizes, raw-tile and whole-file fallbacks,

@@ -88,8 +88,8 @@ __global__ void __launch_bounds__(256) k_m2_grey_front(const TileDesc* __restric
 }
 
 // ------------------------------------------------------------------------------------------------
-// v1 block encoder (libxpng.c:160-260): symbols are consumed from the END of the stream, the
-// renormalisation words are stored at descending addresses, so the finished block
+// v1 blocks (libxpng.c:160-260; encoder k_rans_v1_pair, enc_rans_lat.cuh): symbols are consumed from the
+// END of the stream, the renormalisation words are stored at descending addresses, so the finished block
 // [hdr][n][state0][state1][words] sits at the end of the stream's scratch region.  The frequency
 // table (or the raw symbols of a type-2 block) is a separate bit-string "piece" that k_assemble_m2
 // splices into the tile's shared side stream.
@@ -114,105 +114,6 @@ struct RansV1Args {
 };
 
 __device__ __constant__ const uint16_t M2_NSYM[17] = { 9, 9, 9, 9, 9, 9, 9, 9, 9, 8, 64, 8, 16, 32, 64, 128, 256 };
-
-template <int NSYM, int LANES>
-__global__ void __launch_bounds__(LANES) k_rans_v1(RansV1Args A) {
-    extern __shared__ __align__(16) uint4 etab[];   // [NSYM][LANES]
-    const uint32_t id = blockIdx.x * LANES + threadIdx.x;
-    if (id >= A.nc * A.ntiles) return;
-    const uint32_t c = A.c0 + id / A.ntiles, tile = id % A.ntiles;
-    const uint8_t cls = A.tclass[tile];
-    if (cls != (A.grey ? TC_GREY : TC_RGB)) return;
-    const TileDesc t = A.tiles[tile];
-    TileState* st = A.state + tile;
-    uint32_t N, n, rsize; int pb; const uint32_t* F; const uint8_t* in; uint8_t* region;
-    if (A.grey) {
-        N = 256; pb = 15; n = t.npx - 1;
-        F = A.hist + (uint64_t)tile * HIST_STRIDE_M2 + c * 256;
-        in = A.streams + t.str_off + (uint64_t)c * grey_plane_pitch(t.npx);
-        rsize = align16u(2 * n + 1024);
-        region = A.blocks + t.blk_off + (uint64_t)c * rsize;
-        st->breg[c] = c * rsize;
-    } else {
-        N = M2_NSYM[c]; pb = 14; n = st->len[c];
-        F = A.hist + (uint64_t)tile * HIST_STRIDE_M2 + (c < 9 ? HIST_CTX + c * 16 : HIST_VAL + VAL_OFF[c - 8]);
-        in = A.streams + t.str_off + st->soff[c];
-        rsize = align16u(2 * n + 256);
-        region = A.blocks + t.blk_off + st->breg[c];
-    }
-    if (N > (uint32_t)NSYM || N <= A.nmin) return;   // handled by the launch with the other table size
-    uint32_t* rend = reinterpret_cast<uint32_t*>(region + rsize);
-    uint32_t* tab = A.tabs + ((uint64_t)tile * 17 + c) * TAB_WORDS;
-    const uint32_t nbit = bitlen32(N - 1);
-    auto finish = [&](uint32_t* start, uint32_t type, uint32_t pbits) {
-        st->boff[c] = st->breg[c] + (uint32_t)((uint8_t*)start - region);
-        st->bsize[c] = (uint32_t)((uint8_t*)rend - (uint8_t*)start);
-        st->btype[c] = type; st->pbits[c] = pbits;
-    };
-    if (n == 0) { rend[-1] = 4; finish(rend - 1, 0, 0); return; }                         // libxpng.c:167
-    uint32_t used = 0;
-    for (uint32_t i = 0; i < N; i++) used += F[i] != 0;
-    if (used == 1) {                                                                     // libxpng.c:169-172
-        rend[-2] = 8u | (1u << 24); rend[-1] = n | ((uint32_t)in[n - 1] << 24);
-        finish(rend - 2, 1, 0); return;
-    }
-    uint32_t cum[NSYM + 1];
-    normalise_freqs(F, cum, N, n, pb);
-    uint4* E = etab + threadIdx.x;
-    for (uint32_t i = 0; i < N; i++) E[i * LANES] = make_encsym(cum[i + 1] - cum[i], cum[i], pb);
-
-    // backward pass; renormalisation words go down from the region end (libxpng.c:215-245)
-    uint32_t* wp = rend;
-    uint64_t x0 = 1ull << 31, x1 = 1ull << 31;
-    auto step = [&](uint64_t& x, uint32_t sym) {
-        const uint4 e = E[sym * LANES];
-        const uint64_t xmax = (uint64_t)(e.w & 0xFFFFu) << (63 - pb);
-        if (x >= xmax) { *--wp = (uint32_t)x; x >>= 32; }
-        const uint64_t rcp = (uint64_t)e.x | ((uint64_t)e.y << 32);
-        const uint64_t q = __umul64hi(x, rcp) >> (e.w >> 16);
-        x += (e.z & 0xFFFFu) + q * (e.z >> 16);
-    };
-    int64_t i = (int64_t)n - 1;
-    for (; i >= 0 && ((i + 1) & 15); i--) { if (i & 1) step(x1, in[i]); else step(x0, in[i]); }
-    if (i >= 15) {
-        const uint4* in16 = reinterpret_cast<const uint4*>(in);
-        uint4 nxt = in16[i >> 4];
-        for (; i >= 15; i -= 16) {
-            const uint4 v = nxt;
-            if (i >= 31) nxt = in16[(i >> 4) - 1];
-            const uint32_t w[4] = { v.x, v.y, v.z, v.w };
-#pragma unroll
-            for (int k = 15; k >= 1; k -= 2) {
-                const uint32_t s1 = (w[k >> 2] >> (8 * (k & 3))) & 0xFFu, s0 = (w[(k - 1) >> 2] >> (8 * ((k - 1) & 3))) & 0xFFu;
-                step(x1, s1);
-                step(x0, s0);
-            }
-        }
-    }
-    wp -= 4; wp[0] = (uint32_t)x0; wp[1] = (uint32_t)(x0 >> 32); wp[2] = (uint32_t)x1; wp[3] = (uint32_t)(x1 >> 32);   // :245
-    const uint32_t payload = (uint32_t)((uint8_t*)rend - (uint8_t*)wp);
-    uint32_t tab_bits = (N - used) + used * ((uint32_t)pb + 1);
-    const bool sparse = tab_bits < N * (uint32_t)pb;
-    if (!sparse) tab_bits = N * (uint32_t)pb;
-    if ((uint64_t)tab_bits + 8ull * payload >= (uint64_t)nbit * n) {                      // :250-254 raw symbols
-        BitW r{ 0, 0, reinterpret_cast<uint32_t*>(region) };
-        for (uint32_t k = 0; k < n; k++) r.put(nbit, in[k]);
-        r.end();
-        rend[-2] = 8u | (2u << 24); rend[-1] = n;
-        finish(rend - 2, 2, nbit * n);
-        return;
-    }
-    BitW b{ 0, 0, tab };                                                                 // :256-257
-    for (uint32_t k = 0; k < N; k++) {
-        const uint32_t f = cum[k + 1] - cum[k];
-        if (!sparse) b.put((uint32_t)pb, f);
-        else if (f) b.put((uint32_t)pb + 1, f + (1u << pb));
-        else b.put(1, 0);
-    }
-    b.end();
-    wp -= 2; wp[0] = (payload + 8) | ((3u + (uint32_t)sparse) << 24); wp[1] = n;          // :258-259
-    finish(wp, 3 + sparse, tab_bits);
-}
 
 // ------------------------------------------------------------------------------------------------
 // Per-tile size decisions (libxpng.c:606-626, :672-678).  One thread per tile.

@@ -8,8 +8,7 @@
 // count plus the partner's bit when the partner emits first (v2: state 0 first, ascending addresses;
 // v1: state 1 first, descending addresses).  The store of step t is issued in step t + 1, so the ballot
 // latency never stalls the recurrence.  16 blocks per warp; everything that is not the recurrence
-// (normalisation, tables, headers, raw fallback) is the even lane's job, exactly as in the lane-per-block
-// kernels of enc_back.cuh / enc_m2.cuh, which stay as the throughput variant for large batches.
+// (normalisation, tables, headers, raw fallback) is the even lane's job.
 #pragma once
 #include "common.cuh"
 #include "enc_back.cuh"
@@ -185,7 +184,7 @@ __global__ void __launch_bounds__(32) k_rans_v2_pair(RansV2Args A) {
 }
 
 // ---------------------------------------------------------------------------------------------------
-// v1 blocks (level 2).  Same block numbering and scratch layout as k_rans_v1 (enc_m2.cuh).
+// v1 blocks (level 2).  Block numbering and scratch layout: see RansV1Args (enc_m2.cuh).
 // ---------------------------------------------------------------------------------------------------
 template <int NSYM>
 __global__ void __launch_bounds__(32) k_rans_v1_pair(RansV1Args A) {
