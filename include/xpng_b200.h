@@ -61,6 +61,28 @@ int xpngb_decode(xpngb_ctx *ctx, xpngb_image *imgs, uint32_t n,
                  const uint64_t *file_offsets, const uint64_t *file_sizes,
                  void *pixels, uint64_t pixels_cap, int pixels_on_device);
 
+/* ---- Region decode.  A coded (level 1 / 2) image is cut into independent tiles of at most 666 x 666 pixels, so a
+ * rectangle of it can be decoded by decoding only the tiles it touches. */
+typedef struct xpngb_rect { uint64_t x, y, w, h; } xpngb_rect;   /* pixels; x, y = top-left corner */
+
+/* Tiles that a region decode of `r` inside a w x h coded (level 1 / 2) image decodes; 0 when r is empty or not inside
+ * the image (or w, h exceed the format's 2^24).  *cover (may be NULL) receives their union: a rectangle of whole tiles,
+ * in image pixels.  Host only. */
+uint32_t xpngb_region_tiles(uint64_t w, uint64_t h, const xpngb_rect *r, xpngb_rect *cover);
+
+/* xpngb_decode of rectangle rects[i] of file i only.  Crop i is written as rects[i].h packed rows of
+ * rects[i].w * (3 + A) bytes at pixels + imgs[i].offset (a multiple of 16).  imgs[i] in/out exactly as for xpngb_decode
+ * (w, h, A from xpngb_peek: the FULL image; mode out).  The same file may appear in several entries.
+ * Every entry is checked before anything is decoded: an empty rectangle, one not inside its image, a crop past
+ * pixels_cap or a misaligned offset fails the call (xpngb_last_error names the entry), as do the header checks of
+ * xpngb_decode.  Corrupt data in a decoded tile fails the call as in a full decode.  Of the tiles a rectangle does not
+ * touch only the 4-byte size words up to the last touched tile row are read: their payload is not checked.
+ * Level-7 (stored) rectangles are copied straight out of the file.  With host buffers the whole files still cross PCIe. */
+int xpngb_decode_region(xpngb_ctx *ctx, xpngb_image *imgs, const xpngb_rect *rects, uint32_t n,
+                        const void *files, uint64_t files_size, int files_on_device,
+                        const uint64_t *file_offsets, const uint64_t *file_sizes,
+                        void *pixels, uint64_t pixels_cap, int pixels_on_device);
+
 /* Traversal-order operations of the exchange scheme (Mirroring_and_Rotating/tool.c:3-127; op codes in the order of
  * its option table, tool.c:133).  TL and TR are empty functions in the reference and therefore plain copies. */
 enum { XPNGB_OP_R90 = 0, XPNGB_OP_R270 = 1, XPNGB_OP_MV = 2, XPNGB_OP_MH = 3, XPNGB_OP_MVH = 4, XPNGB_OP_TL = 5, XPNGB_OP_TR = 6 };

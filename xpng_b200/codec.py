@@ -25,6 +25,10 @@ class _Image(C.Structure):
     _fields_ = [("w", C.c_uint64), ("h", C.c_uint64), ("offset", C.c_uint64), ("A", C.c_uint32), ("mode", C.c_uint32)]
 
 
+class _Rect(C.Structure):  # xpngb_rect: pixels, (x, y) = top-left corner
+    _fields_ = [("x", C.c_uint64), ("y", C.c_uint64), ("w", C.c_uint64), ("h", C.c_uint64)]
+
+
 class _Xpng(C.Structure):  # xpng_t, xpng.h:10
     _fields_ = [("p", C.c_void_p), ("w", C.c_uint64), ("h", C.c_uint64), ("s", C.c_uint64), ("A", C.c_bool)]
 
@@ -56,6 +60,10 @@ def lib():
         L.xpngb_peek.restype = C.c_int; L.xpngb_peek.argtypes = [vp, u64, C.POINTER(_Image)]
         L.xpngb_decode.restype = C.c_int
         L.xpngb_decode.argtypes = [vp, C.POINTER(_Image), u32, vp, u64, C.c_int, C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_region_tiles.restype = u32; L.xpngb_region_tiles.argtypes = [u64, u64, C.POINTER(_Rect), C.POINTER(_Rect)]
+        L.xpngb_decode_region.restype = C.c_int
+        L.xpngb_decode_region.argtypes = [vp, C.POINTER(_Image), C.POINTER(_Rect), u32, vp, u64, C.c_int, C.POINTER(u64), C.POINTER(u64),
+                                          vp, u64, C.c_int]
         L.xpngb_last_kernel_ms.restype = C.c_float; L.xpngb_last_kernel_ms.argtypes = [vp]
         L.xpngb_last_launches.restype = u32; L.xpngb_last_launches.argtypes = [vp]
         L.xpngb_stream.restype = vp; L.xpngb_stream.argtypes = [vp]
@@ -97,6 +105,22 @@ OPS = {"r90": 0, "r270": 1, "mv": 2, "mh": 3, "mvh": 4, "tl": 5, "tr": 6}   # in
 
 def _align16(v):
     return (v + 15) & ~15
+
+
+def rects(boxes):
+    """[(x, y, w, h)] -> ctypes array of xpngb_rect."""
+    arr = (_Rect * len(boxes))()
+    for i, (x, y, w, h) in enumerate(boxes):
+        arr[i].x, arr[i].y, arr[i].w, arr[i].h = int(x), int(y), int(w), int(h)
+    return arr
+
+
+def region_tiles(w, h, rect):
+    """Tiles a region decode of rect = (x, y, w, h) inside a w x h coded image decodes, and their union (x, y, w, h):
+    (0, None) when rect is empty or not inside the image.  Host only."""
+    r, cover = rects([rect])[0], _Rect()
+    n = int(lib().xpngb_region_tiles(int(w), int(h), C.byref(r), C.byref(cover)))
+    return n, ((cover.x, cover.y, cover.w, cover.h) if n else None)
 
 
 class Codec:
@@ -175,6 +199,12 @@ class Codec:
                               C.c_void_p(pix_ptr), pix_cap, int(pix_dev)):
             raise RuntimeError("xpngb_decode: " + self._err())
 
+    def decode_region_raw(self, descs, rect_arr, n, files_ptr, files_size, files_dev, offs, sizes, pix_ptr, pix_cap, pix_dev):
+        """decode_raw of rectangle rect_arr[i] (see rects()) of file i: crop i is written packed at pix_ptr + descs[i].offset."""
+        if lib().xpngb_decode_region(self._h, descs, rect_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev), offs, sizes,
+                                     C.c_void_p(pix_ptr), pix_cap, int(pix_dev)):
+            raise RuntimeError("xpngb_decode_region: " + self._err())
+
     # ---------------------------------------------------------------- numpy convenience (host buffers)
     def encode(self, level, images):
         """list of (h,w,3|4) uint8 arrays -> list of .xpng byte strings."""
@@ -211,6 +241,35 @@ class Codec:
         for d in descs:
             c = 3 + d.A
             out.append(px[d.offset: d.offset + d.w * d.h * c].reshape(d.h, d.w, c).copy())
+        return out
+
+    def decode_region(self, files, boxes):
+        """list of .xpng byte strings and one (x, y, w, h) rectangle per file -> list of (h, w, 3|4) uint8 crops.  Only the
+        tiles a rectangle touches are decoded; the same file may appear several times."""
+        n = len(files)
+        if len(boxes) != n:
+            raise ValueError("one rectangle per file")
+        descs, ra = (_Image * n)(), rects(boxes)
+        foffs, fsizes = (C.c_uint64 * n)(), (C.c_uint64 * n)()
+        off = poff = 0
+        for i, f in enumerate(files):
+            b = np.frombuffer(f, dtype=np.uint8)
+            if lib().xpngb_peek(b.ctypes.data, len(f), C.byref(descs[i])):
+                raise ValueError(f"file {i}: not an .xpng header")
+            foffs[i], fsizes[i] = off, len(f)
+            off = _align16(off + len(f))
+            descs[i].offset = poff
+            if ra[i].w <= descs[i].w and ra[i].h <= descs[i].h:     # other rectangles are refused by the library, naming the entry
+                poff = _align16(poff + ra[i].w * ra[i].h * (3 + descs[i].A))
+        fb = np.zeros(off + 16, dtype=np.uint8)
+        for i, f in enumerate(files):
+            fb[foffs[i]: foffs[i] + len(f)] = np.frombuffer(f, dtype=np.uint8)
+        px = np.empty(poff + 16, dtype=np.uint8)
+        self.decode_region_raw(descs, ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        out = []
+        for d, r in zip(descs, ra):
+            c = 3 + d.A
+            out.append(px[d.offset: d.offset + r.w * r.h * c].reshape(r.h, r.w, c).copy())
         return out
 
     # ---------------------------------------------------------------- traversal-order operations (Mirroring_and_Rotating/tool.c)

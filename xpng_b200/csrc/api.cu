@@ -30,6 +30,7 @@
 #include "dec_walk3.cuh"
 #include "misc.cuh"
 #include "orient.cuh"
+#include "region.cuh"
 
 using namespace xpb;
 
@@ -68,7 +69,8 @@ struct xpngb_ctx {
     // device scratch
     DevBuf pixels, norm, files, arena, tiles, imgs, seg_tile, costs, hist, seginfo, place, vplace, vcnt, sym_area,
         bits_area, alpha, streams, blocks, state, outs, flags, skip, dimgs, dtiles, plane, nlseq, rowcnt, rowbits, eord,
-        rows, edge, errflag, hdr, offs, m2a, m2b, tclass, tabs, ccnt, cbit, resv, oriented, odesc, pdw;
+        rows, edge, errflag, hdr, offs, m2a, m2b, tclass, tabs, ccnt, cbit, resv, oriented, odesc, pdw,
+        region, crops;   // region decode: window of the selected tiles, crop descriptors
     PinBuf pin_a, pin_b, pin_o;   // pin_o: orientation descriptors (their upload may still be in flight when an encode reuses pin_a)
 };
 
@@ -185,12 +187,65 @@ static int ensure_pin(xpngb_ctx* ctx, PinBuf& b, size_t n) {
 // ------------------------------------------------------------------------------------------------
 // Tile grid (libxpng.c:51-83): base tile 444x444 (or full width/height when the image is thinner),
 // the remainder of each axis goes to the first tile, or to the first two when it exceeds half a tile.
+// The grid is part of the format: the encoder, the decoder and region selection all take it from tile_grid.
 // ------------------------------------------------------------------------------------------------
 static uint64_t axis_cut(uint64_t extent, uint64_t base, uint64_t* first, uint64_t* second) {
     uint64_t n = extent / base, rem = extent % base;
     *first = base + rem; *second = base;
     if (rem > base / 2) { n++; *second = (base + rem) / 2; *first = *second + ((base + rem) & 1); }
     return n;
+}
+
+struct TileGrid {
+    uint64_t nw = 1, nh = 1, w0, w1, wb, h0, h1, hb;   // tiles per row / column; sizes of the first, second and other tiles
+    // start / size of tile k along an axis whose first two tiles are a and b long and the others base long
+    static uint64_t start(uint64_t k, uint64_t a, uint64_t b, uint64_t base) { return k == 0 ? 0 : (k == 1 ? a : a + b + (k - 2) * base); }
+    static uint64_t size(uint64_t k, uint64_t a, uint64_t b, uint64_t base) { return k == 0 ? a : (k == 1 ? b : base); }
+    static uint64_t at(uint64_t v, uint64_t n, uint64_t a, uint64_t b, uint64_t base) {   // the tile that holds pixel v
+        const uint64_t k = v < a ? 0 : (v - a < b ? 1 : 2 + (v - a - b) / base);
+        return k < n ? k : n - 1;
+    }
+    uint64_t x_of(uint64_t j) const { return start(j, w0, w1, wb); }
+    uint64_t y_of(uint64_t i) const { return start(i, h0, h1, hb); }
+    uint64_t w_of(uint64_t j) const { return size(j, w0, w1, wb); }
+    uint64_t h_of(uint64_t i) const { return size(i, h0, h1, hb); }
+    uint64_t col_at(uint64_t x) const { return at(x, nw, w0, w1, wb); }
+    uint64_t row_at(uint64_t y) const { return at(y, nh, h0, h1, hb); }
+};
+
+static TileGrid tile_grid(uint64_t W, uint64_t H) {
+    TileGrid g;
+    g.w0 = g.w1 = g.wb = W; g.h0 = g.h1 = g.hb = H;
+    if (W * H > TILE_AREA) {
+        if (W < 444) { g.wb = W; g.hb = TILE_AREA / W; }
+        else if (H < 444) { g.hb = H; g.wb = TILE_AREA / H; }
+        else g.wb = g.hb = 444;
+        g.nw = axis_cut(W, g.wb, &g.w0, &g.w1);
+        g.nh = axis_cut(H, g.hb, &g.h0, &g.h1);
+    }
+    return g;
+}
+
+struct TileSel { uint64_t r0, r1, c0, c1; };   // tile rows [r0, r1] and tile columns [c0, c1] of a grid
+static TileSel all_tiles(const TileGrid& g) { return TileSel{ 0, g.nh - 1, 0, g.nw - 1 }; }
+
+// The tiles a region decode of r (inside a W x H image) decodes, and their union `cover` (whole tiles, image pixels).
+// False when r is empty or not inside the image; x + w > W is tested without overflow.
+static bool region_select(uint64_t W, uint64_t H, const xpngb_rect& r, TileGrid& g, TileSel& s, xpngb_rect& cover) {
+    if (!W || !H || W > (1u << 24) || H > (1u << 24)) return false;
+    if (!r.w || !r.h || r.x >= W || r.w > W - r.x || r.y >= H || r.h > H - r.y) return false;
+    g = tile_grid(W, H);
+    s = TileSel{ g.row_at(r.y), g.row_at(r.y + r.h - 1), g.col_at(r.x), g.col_at(r.x + r.w - 1) };
+    cover.x = g.x_of(s.c0); cover.y = g.y_of(s.r0);
+    cover.w = g.x_of(s.c1) + g.w_of(s.c1) - cover.x; cover.h = g.y_of(s.r1) + g.h_of(s.r1) - cover.y;
+    return true;
+}
+
+extern "C" uint32_t xpngb_region_tiles(uint64_t w, uint64_t h, const xpngb_rect* r, xpngb_rect* cover) {
+    TileGrid g; TileSel s; xpngb_rect c{};
+    if (!r || !region_select(w, h, *r, g, s, c)) return 0;
+    if (cover) *cover = c;
+    return (uint32_t)((s.r1 - s.r0 + 1) * (s.c1 - s.c0 + 1));
 }
 
 struct Plan {
@@ -202,37 +257,32 @@ struct Plan {
     bool any_wide = false;     // a tile wider than the staged front end takes (one-tile images up to 197136 x 1)
 };
 
-// Appends the tiles of one image.  base = absolute device address of its pixels.
-static void plan_image(Plan& P, uint64_t base, uint64_t W, uint64_t H, uint32_t pxsz, uint32_t mode, int sfac, int bfac) {
+// Appends the selected tiles of one W x H image.  Tile (x0, y0) is read (encode) or written (decode) at
+// D + (y0 - oy) * Pd + (x0 - ox) * pxsz: the image itself (D = its pixels, Pd = W * pxsz, origin 0), or for a region
+// decode a window of row pitch Pd whose first pixel is image pixel (ox, oy).
+static void plan_image(Plan& P, const TileGrid& g, const TileSel& s, uint64_t D, uint64_t Pd, uint64_t ox, uint64_t oy,
+                       uint64_t W, uint64_t H, uint32_t pxsz, uint32_t mode, int sfac, int bfac) {
     ImageDesc I{};
-    I.px_off = base; I.raw_size = W * H * pxsz; I.w = (uint32_t)W; I.h = (uint32_t)H; I.pxsz = pxsz;
+    I.px_off = D; I.raw_size = W * H * pxsz; I.w = (uint32_t)W; I.h = (uint32_t)H; I.pxsz = pxsz;
     I.tile0 = (uint32_t)P.tiles.size(); I.mode = mode;
-    uint64_t nw = 1, nh = 1, w0 = W, w1 = W, wb = W, h0 = H, h1 = H, hb = H;
-    if (W * H > TILE_AREA) {
-        if (W < 444) { wb = W; hb = TILE_AREA / W; }
-        else if (H < 444) { hb = H; wb = TILE_AREA / H; }
-        else wb = hb = 444;
-        nw = axis_cut(W, wb, &w0, &w1);
-        nh = axis_cut(H, hb, &h0, &h1);
-    }
     const uint32_t img = (uint32_t)P.imgs.size();
-    uint64_t y = 0; uint32_t tix = 0;
-    for (uint64_t i = 0; i < nh; i++) {
-        const uint64_t th = i == 0 ? h0 : (i == 1 ? h1 : hb);
-        uint64_t x = 0;
-        for (uint64_t j = 0; j < nw; j++) {
-            const uint64_t tw = j == 0 ? w0 : (j == 1 ? w1 : wb);
+    uint64_t y = g.y_of(s.r0);
+    for (uint64_t i = s.r0; i <= s.r1; i++) {
+        const uint64_t th = g.h_of(i);
+        uint64_t x = g.x_of(s.c0);
+        for (uint64_t j = s.c0; j <= s.c1; j++) {
+            const uint64_t tw = g.w_of(j);
             TileDesc t{};
-            t.src_off = base + (y * W + x) * pxsz;
+            t.src_off = D + (y - oy) * Pd + (x - ox) * pxsz;
             t.px_off = P.px_total; t.row_off = P.row_total;
-            t.w = (uint32_t)tw; t.h = (uint32_t)th; t.bpr = (uint32_t)(W * pxsz); t.npx = (uint32_t)(tw * th);
+            t.w = (uint32_t)tw; t.h = (uint32_t)th; t.bpr = (uint32_t)Pd; t.npx = (uint32_t)(tw * th);
             t.img = img; t.seg0 = (uint32_t)P.seg_tile.size(); t.nseg = (t.npx + SEG - 1) / SEG; t.pxsz = pxsz;
-            t.x0 = (uint32_t)x; t.y0 = (uint32_t)y; t.tix = tix++;
+            t.x0 = (uint32_t)x; t.y0 = (uint32_t)y; t.tix = (uint32_t)(i * g.nw + j);
             const uint64_t slice = ((uint64_t)t.npx + 15) / 16 * 16 + 256;
             t.str_off = P.str_total; t.blk_off = P.blk_total;
             P.px_total += slice; P.row_total += th;
             P.str_total += slice * sfac; P.blk_total += slice * bfac + 8192;
-            for (uint32_t s = 0; s < t.nseg; s++) P.seg_tile.push_back((uint32_t)P.tiles.size());
+            for (uint32_t k = 0; k < t.nseg; k++) P.seg_tile.push_back((uint32_t)P.tiles.size());
             if (t.w > FRONT2_MAXW) P.any_wide = true;
             P.tiles.push_back(t);
             x += tw;
@@ -242,6 +292,12 @@ static void plan_image(Plan& P, uint64_t base, uint64_t W, uint64_t H, uint32_t 
     I.ntiles = (uint32_t)P.tiles.size() - I.tile0;
     if (pxsz == 4) P.any_rgba = true;
     P.imgs.push_back(I);
+}
+
+// Every tile of an image, in place.  base = absolute device address of its pixels.
+static void plan_image(Plan& P, uint64_t base, uint64_t W, uint64_t H, uint32_t pxsz, uint32_t mode, int sfac, int bfac) {
+    const TileGrid g = tile_grid(W, H);
+    plan_image(P, g, all_tiles(g), base, W * pxsz, 0, 0, W, H, pxsz, mode, sfac, bfac);
 }
 
 static int upload_plan(xpngb_ctx* ctx, const Plan& P) {
@@ -333,7 +389,7 @@ static void lane_free(xpngb_ctx* ctx) {
                       &ctx->streams, &ctx->blocks, &ctx->state, &ctx->outs, &ctx->flags, &ctx->skip, &ctx->dimgs, &ctx->dtiles,
                       &ctx->plane, &ctx->nlseq, &ctx->rowcnt, &ctx->rowbits, &ctx->rows, &ctx->edge, &ctx->errflag, &ctx->hdr,
                       &ctx->offs, &ctx->m2a, &ctx->m2b, &ctx->tclass, &ctx->tabs, &ctx->ccnt, &ctx->cbit, &ctx->resv, &ctx->oriented,
-                      &ctx->odesc, &ctx->pdw, &ctx->eord };
+                      &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops };
     for (DevBuf* b : all) if (b->p) cudaFree(b->p);
     if (ctx->pin_a.p) cudaFreeHost(ctx->pin_a.p);
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
@@ -890,54 +946,112 @@ static PdWork pdw_at(void* base, uint32_t cap) {
     return W;
 }
 
-// Launch the decode of one chunk on lane `ctx`.  hdr: the two header words of each file.  `lat`: warp-per-block chain
-// kernels (few blocks in the whole call) instead of the pair decoders.  Never waits for the device.
-static int decode_issue(xpngb_ctx* ctx, bool lat, xpngb_image* imgs, uint32_t n, const uint32_t* hdr, const uint8_t* din,
-                        const uint64_t* file_offsets, const uint64_t* file_sizes, uint8_t* dpx, uint64_t pixels_cap, uint32_t call_tiles) {
+// Header checks of file i (libxpng.c:969-976) and of where its pixels go: fills imgs[i] (w, h, A, mode) and D (file,
+// geometry, effective mode).  A region decode (r != nullptr) writes the r->w x r->h crop at imgs[i].offset instead of
+// the whole image.  Runs for every entry of a call before anything is launched.
+static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint32_t* hdr, uint64_t file_off, uint64_t file_size,
+                        const xpngb_rect* r, uint64_t pixels_cap, DecImage& D) {
+    const uint64_t w = (hdr[0] & 0xFFFFFFu) + 1, h = (hdr[1] & 0xFFFFFFu) + 1;
+    const uint32_t A = (hdr[1] >> 24) & 1, mode = hdr[0] >> 24, pxsz = 3 + A;
+    if (!(mode == 1 || mode == 2 || mode == 7)) FAIL("file %u: unknown mode %u", i, mode);   // libxpng.c:972
+    if (img.w && (img.w != w || img.h != h)) FAIL("file %u: header %llux%llu does not match the descriptor", i,
+                                                  (unsigned long long)w, (unsigned long long)h);
+    img.w = w; img.h = h; img.A = A; img.mode = mode;
+    if (r && (!r->w || !r->h)) FAIL("entry %u: empty rectangle", i);
+    if (r && (r->x >= w || r->w > w - r->x || r->y >= h || r->h > h - r->y))
+        FAIL("entry %u: rectangle (%llu, %llu) %llux%llu is not inside the %llux%llu image", i, (unsigned long long)r->x,
+             (unsigned long long)r->y, (unsigned long long)r->w, (unsigned long long)r->h, (unsigned long long)w, (unsigned long long)h);
+    const uint64_t s = w * h * pxsz, out = r ? r->w * r->h * pxsz : s;   // at most 2^24 x 2^24 pixels: no overflow
+    if (img.offset & 15) FAIL("file %u: pixel offset must be a multiple of 16", i);
+    if (out > pixels_cap || img.offset > pixels_cap - out) FAIL("file %u: pixels exceed the output buffer", i);
+    uint32_t m = mode;
+    if (mode == 7) { if (file_size < 8 + s) FAIL("file %u: truncated stored image", i); }
+    else if (file_size == 11 + A && ((hdr[1] >> 24) & 2)) m = mode | 0x100;      // libxpng.c:976
+    // dimensions come from an untrusted header and size every scratch buffer below: a tile is at most 666 x 666 pixels and
+    // its blob at least 8 bytes, so a coded file shorter than that cannot hold the image it claims
+    else if (file_size < 8 + 8 * (w * h / (666ull * 666ull))) FAIL("file %u: %llu bytes cannot hold a %llux%llu image", i,
+                                                                   (unsigned long long)file_size, (unsigned long long)w, (unsigned long long)h);
+    D = DecImage{};
+    D.file_off = file_off; D.file_size = file_size; D.px_off = img.offset; D.w = (uint32_t)w; D.h = (uint32_t)h;
+    D.pxsz = pxsz; D.mode = m;
+    return 0;
+}
+
+// One entry of a region decode: the rectangle, the tiles that hold it and their union.
+struct RegionSel { xpngb_rect rect, cover; TileGrid g; TileSel s; };
+static bool whole_tiles(const RegionSel& R) {
+    return R.rect.x == R.cover.x && R.rect.y == R.cover.y && R.rect.w == R.cover.w && R.rect.h == R.cover.h;
+}
+static uint64_t window_pitch(const RegionSel& R, uint32_t pxsz) { return (R.cover.w * pxsz + 15) & ~15ull; }   // keeps RGB rows word-aligned (tile_pitched)
+
+// Launch the decode of one chunk on lane `ctx`.  DI: the checked images of the chunk.  `lat`: warp-per-block chain
+// kernels (few blocks in the whole call) instead of the pair decoders.  sel == nullptr: every tile of every image, in
+// place.  Otherwise a region decode: only the tiles of sel[i].s, written in place when the rectangle is made of whole
+// tiles, else into a window of the lane's region scratch from which k_crop_rows copies the rectangle; stored images
+// are cropped straight out of their files.  Never waits for the device.
+static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, uint32_t n,
+                        const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
-    std::vector<DecImage> DI(n);
-    bool any1 = false, any2 = false;
-    for (uint32_t i = 0; i < n; i++) {
-        const uint64_t w = (hdr[2 * i] & 0xFFFFFFu) + 1, h = (hdr[2 * i + 1] & 0xFFFFFFu) + 1;
-        const uint32_t A = (hdr[2 * i + 1] >> 24) & 1, mode = hdr[2 * i] >> 24, pxsz = 3 + A;
-        if (!(mode == 1 || mode == 2 || mode == 7)) FAIL("file: unknown mode %u", mode);   // libxpng.c:972
-        if (imgs[i].w && (imgs[i].w != w || imgs[i].h != h)) FAIL("file: header %llux%llu does not match the descriptor",
-                                                                   (unsigned long long)w, (unsigned long long)h);
-        imgs[i].w = w; imgs[i].h = h; imgs[i].A = A; imgs[i].mode = mode;
-        const uint64_t s = w * h * pxsz;
-        if (imgs[i].offset & 15) FAIL("file: pixel offset must be a multiple of 16");
-        if (s > pixels_cap || imgs[i].offset > pixels_cap - s) FAIL("file: pixels exceed the output buffer");
-        uint32_t m = mode;
-        if (mode == 7) { if (file_sizes[i] < 8 + s) FAIL("file: truncated stored image"); }
-        else if (file_sizes[i] == 11 + A && ((hdr[2 * i + 1] >> 24) & 2)) m = mode | 0x100;      // libxpng.c:976
-        // dimensions come from an untrusted header and size every scratch buffer below: a tile is at most 666 x 666 pixels and
-        // its blob at least 8 bytes, so a coded file shorter than that cannot hold the image it claims
-        else if (file_sizes[i] < 8 + 8 * (w * h / (666ull * 666ull))) FAIL("file: %llu bytes cannot hold a %llux%llu image",
-                                                                           (unsigned long long)file_sizes[i], (unsigned long long)w, (unsigned long long)h);
-        any1 |= m == 1; any2 |= m == 2;
-        DecImage& D = DI[i];
-        D.file_off = file_offsets[i]; D.file_size = file_sizes[i]; D.px_off = imgs[i].offset; D.w = (uint32_t)w; D.h = (uint32_t)h;
-        D.pxsz = pxsz; D.mode = m;
+    std::vector<DecImage> DI(DI_in, DI_in + n);
+    std::vector<CropDesc> crops;
+    bool any1 = false, any2 = false, any7 = false;
+    for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
+    if (sel) {   // windows for the rectangles that are not made of whole tiles
+        uint64_t need = 0;
+        for (uint32_t i = 0; i < n; i++) if (DI[i].mode != 7 && !whole_tiles(sel[i])) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
+        if (need) ENSURE(region, need);
     }
+    uint64_t wpos = 0;
     for (uint32_t i = 0; i < n; i++) {
-        plan_image(P, (uint64_t)(dpx + imgs[i].offset), DI[i].w, DI[i].h, DI[i].pxsz, DI[i].mode, any2 ? 4 : 1, 0);
-        DI[i].tile0 = P.imgs[i].tile0; DI[i].ntiles = P.imgs[i].ntiles;
+        DecImage& D = DI[i];
+        uint8_t* out = dpx + imgs[i].offset;
+        const int sfac = any2 ? 4 : 1;
+        if (!sel) {
+            const TileGrid g = tile_grid(D.w, D.h);
+            plan_image(P, g, all_tiles(g), (uint64_t)out, (uint64_t)D.w * D.pxsz, 0, 0, D.w, D.h, D.pxsz, D.mode, sfac, 0);
+            D.gcols = (uint32_t)g.nw; D.r0 = 0; D.c0 = 0; D.nrows = (uint32_t)g.nh; D.ncols = (uint32_t)g.nw;
+        } else if (D.mode == 7) {   // no tiles: the rectangle's rows are read from the file
+            const xpngb_rect& r = sel[i].rect;
+            ImageDesc I{}; I.tile0 = (uint32_t)P.tiles.size(); I.mode = 7; I.w = D.w; I.h = D.h; I.pxsz = D.pxsz;
+            P.imgs.push_back(I);
+            crops.push_back(CropDesc{ (uint64_t)(din + D.file_off + 8 + (r.y * D.w + r.x) * D.pxsz), (uint64_t)out, (uint64_t)D.w * D.pxsz,
+                                      (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+        } else {
+            const RegionSel& R = sel[i];
+            const xpngb_rect &r = R.rect, &c = R.cover;
+            if (whole_tiles(R)) plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
+            else {
+                const uint64_t pitch = window_pitch(R, D.pxsz), win = (uint64_t)ctx->region.p + wpos;
+                plan_image(P, R.g, R.s, win, pitch, c.x, c.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
+                crops.push_back(CropDesc{ win + (r.y - c.y) * pitch + (r.x - c.x) * D.pxsz, (uint64_t)out, pitch,
+                                          (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+                wpos += c.h * pitch;
+            }
+            D.gcols = (uint32_t)R.g.nw; D.r0 = (uint32_t)R.s.r0; D.c0 = (uint32_t)R.s.c0;
+            D.nrows = (uint32_t)(R.s.r1 - R.s.r0 + 1); D.ncols = (uint32_t)(R.s.c1 - R.s.c0 + 1);
+        }
+        D.tile0 = P.imgs[i].tile0; D.ntiles = P.imgs[i].ntiles;
     }
     if (P.tiles.size() > (1u << 24) || P.seg_tile.size() > (1u << 28)) FAIL("too many tiles for one chunk (%zu)", P.tiles.size());
     const uint32_t ntiles = (uint32_t)P.tiles.size();
     if (upload_plan(ctx, P)) return 1;
     ENSURE(dimgs, n * sizeof(DecImage)); ENSURE(dtiles, ntiles * sizeof(DecTile)); ENSURE(errflag, 4);
-    if (ensure_pin(ctx, ctx->pin_b, n * (sizeof(DecImage) + 8) + 64)) return 1;
+    // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop descriptors
+    const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64;
+    if (ensure_pin(ctx, ctx->pin_b, pin_crops + crops.size() * sizeof(CropDesc))) return 1;
     memcpy(ctx->pin_b.p, DI.data(), n * sizeof(DecImage));
     CK(cudaMemcpyAsync(ctx->dimgs.p, ctx->pin_b.p, n * sizeof(DecImage), cudaMemcpyHostToDevice, ctx->stream));
-    bool any7 = false;
-    for (uint32_t i = 0; i < n; i++) any7 |= DI[i].mode == 7;
-    if (any7) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
+    if (any7 && !sel) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
         uint64_t* cf = (uint64_t*)((uint8_t*)ctx->pin_b.p + n * sizeof(DecImage));
         for (uint32_t i = 0; i < n; i++) cf[i] = DI[i].mode == 7 ? DI[i].file_off : ~0ull;
         ENSURE(offs, n * 8);
         CK(cudaMemcpyAsync(ctx->offs.p, cf, n * 8, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (!crops.empty()) {
+        ENSURE(crops, crops.size() * sizeof(CropDesc));
+        memcpy((uint8_t*)ctx->pin_b.p + pin_crops, crops.data(), crops.size() * sizeof(CropDesc));
+        CK(cudaMemcpyAsync(ctx->crops.p, (uint8_t*)ctx->pin_b.p + pin_crops, crops.size() * sizeof(CropDesc), cudaMemcpyHostToDevice, ctx->stream));
     }
     CK(cudaMemsetAsync(ctx->errflag.p, 0, 4, ctx->stream));
     CK(cudaMemsetAsync(ctx->dtiles.p, 0, ntiles * sizeof(DecTile), ctx->stream));
@@ -1119,16 +1233,26 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, xpngb_image* imgs, uint32_t n,
         if (maxw > UNR_MAXW) LAUNCH(k_dec_unpredict, ntiles, UNP_THREADS, 0, ua);   // very wide, flat tiles only
         if (any2) LAUNCH(k_dec_grey_raw, ntiles, 256, 0, d_tiles, d_imgs, (const DecTile*)d_dt, din);
     }
-    if (any7) LAUNCH(k_load7, dim3(296, n), 256, 0, (const ImageDesc*)ctx->imgs.p, (const uint64_t*)ctx->offs.p, din);   // stored images: flat copies
-    LAUNCH(k_dec_copy, ntiles, 256, 0, d_tiles, d_imgs, (const DecTile*)d_dt, din, (uint8_t*)nullptr);
+    if (any7 && !sel) LAUNCH(k_load7, dim3(296, n), 256, 0, (const ImageDesc*)ctx->imgs.p, (const uint64_t*)ctx->offs.p, din);   // stored images: flat copies
+    if (ntiles) LAUNCH(k_dec_copy, ntiles, 256, 0, d_tiles, d_imgs, (const DecTile*)d_dt, din, (uint8_t*)nullptr);
+    if (!crops.empty()) {   // one warp per row; enough row blocks that a single large crop fills the machine
+        uint32_t maxrows = 0;
+        for (const CropDesc& c : crops) if (c.rows > maxrows) maxrows = c.rows;
+        const unsigned gx = (maxrows + 7) / 8 < 296 ? (maxrows + 7) / 8 : 296;
+        for (size_t c0 = 0; c0 < crops.size(); c0 += 65535) {   // grid y limit
+            const unsigned m = (unsigned)(crops.size() - c0 < 65535 ? crops.size() - c0 : 65535);
+            LAUNCH(k_crop_rows, dim3(gx, m), 256, 0, (const CropDesc*)ctx->crops.p + c0);
+        }
+    }
     // the error flag travels to pinned memory behind the DecImage table
     CK(cudaMemcpyAsync((uint8_t*)ctx->pin_b.p + n * (sizeof(DecImage) + 8), d_err, 4, cudaMemcpyDeviceToHost, ctx->stream));
     return 0;
 }
 
-extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
-                            const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
-                            int pixels_on_device) {
+// xpngb_decode (rects == nullptr) and xpngb_decode_region.
+static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, uint32_t n, const void* files, uint64_t files_size,
+                       int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
+                       int pixels_on_device) {
     if (!ctx) return 1;
     ctx->err[0] = 0; ctx->launches = 0; ctx->last_ms = 0.f; ctx->cur = ctx->stream;
     if (!imgs || !files || !file_offsets || !file_sizes || !pixels) FAIL("null argument");
@@ -1152,17 +1276,27 @@ extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const
         CK(cudaMemcpyAsync(hdr.data(), ctx->hdr.p, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
     }
+    // ---- every entry is checked before anything is decoded
+    std::vector<DecImage> DI(n);
+    std::vector<RegionSel> sel(rects ? n : 0);
+    for (uint32_t i = 0; i < n; i++) {
+        if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, pixels_cap, DI[i])) return 1;
+        if (rects) { sel[i].rect = rects[i]; region_select(imgs[i].w, imgs[i].h, rects[i], sel[i].g, sel[i].s, sel[i].cover); }
+    }
     uint8_t* dpx = (uint8_t*)pixels;
     if (!pixels_on_device) { ENSURE(pixels, pixels_cap); dpx = (uint8_t*)ctx->pixels.p; }
-    // chunks are cut by the header dimensions (validated per chunk in decode_issue)
+    // chunks are cut by the pixels each entry decodes: the whole image, or the cover of its rectangle (stored: the rectangle)
     std::vector<xpngb_image> dims(n);
     uint64_t tiles_est = 0; bool l2 = false;
     for (uint32_t i = 0; i < n; i++) {
-        dims[i].w = (hdr[2 * i] & 0xFFFFFFu) + 1; dims[i].h = (hdr[2 * i + 1] & 0xFFFFFFu) + 1;
-        const uint32_t mode = hdr[2 * i] >> 24;
-        if (mode == 1 || mode == 2) tiles_est += (dims[i].w * dims[i].h + TILE_AREA - 1) / TILE_AREA;
+        const uint32_t mode = imgs[i].mode;
+        const xpngb_rect* wh = !rects ? nullptr : (mode == 7 ? &sel[i].rect : &sel[i].cover);
+        dims[i].w = wh ? wh->w : imgs[i].w; dims[i].h = wh ? wh->h : imgs[i].h;
+        if (mode == 1 || mode == 2) tiles_est += rects ? (sel[i].s.r1 - sel[i].s.r0 + 1) * (sel[i].s.c1 - sel[i].s.c0 + 1)
+                                                       : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
         l2 |= mode == 2;
     }
+    auto out_bytes = [&](uint32_t i) { return (rects ? rects[i].w * rects[i].h : imgs[i].w * imgs[i].h) * (3 + imgs[i].A); };
     // level 2: above ~600 tiles the pair family wins, with the 16-symbol value streams warp-per-block while they all fit
     // (s16_lat_max_tiles); level 1: the warp-per-block family up to ~1300 tiles (measured at 125 / 250 / 500 frames, profiles/)
     const bool lat = l2 ? 17 * tiles_est <= (uint64_t)ctx->lat_max_blocks * 5 / 6 : 9 * tiles_est <= ctx->lat_max_blocks;
@@ -1196,11 +1330,12 @@ extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const
                 snprintf(ctx->err, sizeof ctx->err, "host to device copy failed"); rc = 1; break;
             }
         }
-        rc = decode_issue(lane, lat, imgs + i0, m, hdr.data() + 2 * i0, din, file_offsets + i0, file_sizes + i0, dpx, pixels_cap, (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
+        rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, rects ? sel.data() + i0 : nullptr, m, din, dpx,
+                          (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
             for (uint32_t i = i0; i < i0 + m; i++) {
-                const uint64_t a = imgs[i].offset, b = a + imgs[i].w * imgs[i].h * (3 + imgs[i].A);
+                const uint64_t a = imgs[i].offset, b = a + out_bytes(i);
                 if (a < lo) lo = a; if (b > hi) hi = b;
             }
             if (cudaMemcpyAsync((uint8_t*)pixels + lo, dpx + lo, hi - lo, cudaMemcpyDeviceToHost, lane->stream) != cudaSuccess) {
@@ -1225,6 +1360,20 @@ extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const
     CK(cudaEventElapsedTime(&ctx->last_ms, ctx->ev0, ctx->ev1));
     tl_dump(ctx, "dec");
     return 0;
+}
+
+extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
+                            const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
+                            int pixels_on_device) {
+    return decode_call(ctx, imgs, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap, pixels_on_device);
+}
+
+extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, uint32_t n, const void* files,
+                                   uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes,
+                                   void* pixels, uint64_t pixels_cap, int pixels_on_device) {
+    if (!ctx) return 1;
+    if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
+    return decode_call(ctx, imgs, rects, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap, pixels_on_device);
 }
 
 // ------------------------------------------------------------------------------------------------

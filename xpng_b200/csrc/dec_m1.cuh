@@ -12,8 +12,10 @@ struct DecImage {
     uint64_t file_off, file_size;   // inside the input buffer
     uint64_t px_off;                // output pixel offset
     uint32_t w, h, pxsz, mode;      // mode: 1, 2, 7; 0x100 = whole-image single colour
-    uint32_t tile0, ntiles;
-    uint32_t pad[2];
+    uint32_t tile0, ntiles;         // planned (selected) tiles: DecTile tile0 + (row - r0) * ncols + (col - c0)
+    uint32_t gcols;                 // tile columns of the image's grid
+    uint32_t r0, c0, nrows, ncols;  // selected tile rows [r0, r0 + nrows) and columns [c0, c0 + ncols): the whole grid for a full decode
+    uint32_t pad;
 };
 
 struct DecBlock { uint32_t off; uint32_t n; uint32_t type; uint32_t soff; };   // off: from blob start; soff: in stream slice
@@ -32,7 +34,9 @@ __device__ __forceinline__ void dec_fail(int* err, int code) { atomicCAS(err, 0,
 __host__ __device__ __forceinline__ uint32_t align16u_dec(uint32_t v) { return (v + 15u) & ~15u; }
 
 // ------------------------------------------------------------------------------------------------
-// Tile offsets: serial chain over the 24-bit tile sizes of one image (libxpng.c:982).
+// Tile offsets: serial chain over the 24-bit tile sizes of one image (libxpng.c:982).  The chain is walked from the
+// first tile with the same checks for every tile; only the selected tiles get a DecTile, and the walk ends after the
+// last selected row (a region decode reads nothing of the tiles it skips but their size words).
 // ------------------------------------------------------------------------------------------------
 __global__ void k_dec_tile_offsets(const DecImage* imgs, const uint8_t* in, DecTile* dt, uint32_t nimg, int* err) {
     const uint32_t im = blockIdx.x * blockDim.x + threadIdx.x;
@@ -40,13 +44,16 @@ __global__ void k_dec_tile_offsets(const DecImage* imgs, const uint8_t* in, DecT
     const DecImage I = imgs[im];
     if ((I.mode & 0xFF) == 7 || (I.mode & 0x100)) return;
     uint64_t off = 8;
-    for (uint32_t k = 0; k < I.ntiles; k++) {
-        DecTile* d = dt + I.tile0 + k;
-        if (off + 4 > I.file_size) { dec_fail(err, DEC_BAD_TILE_CHAIN); d->size = 0; d->m = 0xFE; d->blob_off = I.file_off; continue; }
+    const uint32_t rend = I.r0 + I.nrows;
+    for (uint32_t row = 0, col = 0; row < rend;) {
+        DecTile* d = (row >= I.r0 && col - I.c0 < I.ncols) ? dt + I.tile0 + (row - I.r0) * I.ncols + (col - I.c0) : nullptr;
+        if (++col == I.gcols) { col = 0; row++; }
+        if (off + 4 > I.file_size) { dec_fail(err, DEC_BAD_TILE_CHAIN); if (d) { d->size = 0; d->m = 0xFE; d->blob_off = I.file_off; } continue; }
         const uint32_t w0 = ld32u(in + I.file_off + off);
         const uint32_t size = w0 & 0xFFFFFFu;
-        d->blob_off = I.file_off + off; d->size = size; d->m = w0 >> 24;
-        if (size < 4 || off + size > I.file_size) { dec_fail(err, DEC_BAD_TILE_CHAIN); d->m = 0xFE; }
+        const bool bad = size < 4 || off + size > I.file_size;
+        if (bad) dec_fail(err, DEC_BAD_TILE_CHAIN);
+        if (d) { d->blob_off = I.file_off + off; d->size = size; d->m = bad ? 0xFE : w0 >> 24; }
         off += size < 4 ? 4 : size;
     }
 }
