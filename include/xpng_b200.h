@@ -101,6 +101,25 @@ int xpngb_encode_oriented(xpngb_ctx *ctx, int level, int op, xpngb_image *imgs, 
                           void *out, uint64_t out_cap, int out_on_device,
                           uint64_t *out_offsets, uint64_t *out_sizes);
 
+/* xpngb_decode (rects == NULL) or xpngb_decode_region (rects != NULL), with entry i written as `tool --<ops[i]>` would
+ * leave what those calls write for it: one op per entry, in the same call.
+ *   ops     : non-NULL, ops[i] one of XPNGB_OP_*.  An unknown op fails the call before anything is launched
+ *             (xpngb_last_error names the entry).  XPNGB_OP_TL and XPNGB_OP_TR are copies in the reference: those
+ *             entries are byte-identical to the unoriented call.
+ *   rects   : in the file's coordinates, as stored; the op is applied to the crop afterwards.  NULL: whole images.
+ *   output  : packed rows at pixels + imgs[i].offset, the same byte count as the unoriented call.  For R90 and R270 the
+ *             width and height are swapped: rects[i].w rows of rects[i].h pixels (whole image: w rows of h pixels).
+ *   imgs[i] : in/out exactly as for xpngb_decode (the file's w, h, A; mode out).  Not swapped, so the array can be reused.
+ * Every other check is that of xpngb_decode / xpngb_decode_region.  Turned entries are decoded into a scratch window and
+ * then written turned (stored level-7 entries are read straight from the file), so they cost one more read and write of
+ * their pixels in device memory; with host buffers nothing more crosses PCIe.
+ * Files written by xpngb_encode_oriented(op) are restored by the inverse op: XPNGB_OP_R270 for XPNGB_OP_R90,
+ * XPNGB_OP_R90 for XPNGB_OP_R270, and `op` itself for every other op. */
+int xpngb_decode_oriented(xpngb_ctx *ctx, const int *ops, xpngb_image *imgs, const xpngb_rect *rects, uint32_t n,
+                          const void *files, uint64_t files_size, int files_on_device,
+                          const uint64_t *file_offsets, const uint64_t *file_sizes,
+                          void *pixels, uint64_t pixels_cap, int pixels_on_device);
+
 /* Device time of the kernels of the last encode/decode call on this context, in milliseconds
  * (CUDA events on the context's stream; excludes host<->device copies). */
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);

@@ -15,4 +15,4 @@ import os as _os
 CONNECTIONS_SET_HERE = "CUDA_DEVICE_MAX_CONNECTIONS" not in _os.environ
 _os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
-from .codec import Codec, LibraryMissing, lib, lib_path, region_tiles, xpng_store, xpng_load, load_7, store_7  # noqa: F401
+from .codec import Codec, LibraryMissing, inverse_op, lib, lib_path, region_tiles, xpng_store, xpng_load, load_7, store_7  # noqa: F401

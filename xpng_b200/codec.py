@@ -64,6 +64,9 @@ def lib():
         L.xpngb_decode_region.restype = C.c_int
         L.xpngb_decode_region.argtypes = [vp, C.POINTER(_Image), C.POINTER(_Rect), u32, vp, u64, C.c_int, C.POINTER(u64), C.POINTER(u64),
                                           vp, u64, C.c_int]
+        L.xpngb_decode_oriented.restype = C.c_int
+        L.xpngb_decode_oriented.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect), u32, vp, u64, C.c_int,
+                                            C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
         L.xpngb_last_kernel_ms.restype = C.c_float; L.xpngb_last_kernel_ms.argtypes = [vp]
         L.xpngb_last_launches.restype = u32; L.xpngb_last_launches.argtypes = [vp]
         L.xpngb_stream.restype = vp; L.xpngb_stream.argtypes = [vp]
@@ -101,6 +104,23 @@ def lib():
 
 
 OPS = {"r90": 0, "r270": 1, "mv": 2, "mh": 3, "mvh": 4, "tl": 5, "tr": 6}   # include/xpng_b200.h, order of tool.c:133
+QUARTER_TURNS = ("r90", "r270")
+
+
+def inverse_op(name):
+    """The op that undoes `name`: decoding a file written by encode_oriented(level, name, ...) with it gives the original
+    orientation back.  r90 and r270 undo each other; every other op undoes itself."""
+    if name not in OPS:
+        raise ValueError(f"unknown op {name!r}")
+    return {"r90": "r270", "r270": "r90"}.get(name, name)
+
+
+def op_codes(names):
+    """[op name] -> ctypes array of XPNGB_OP_* codes."""
+    bad = [o for o in names if o not in OPS]
+    if bad:
+        raise ValueError(f"unknown op {bad[0]!r}")
+    return (C.c_int * len(names))(*(OPS[o] for o in names))
 
 
 def _align16(v):
@@ -205,6 +225,13 @@ class Codec:
                                      C.c_void_p(pix_ptr), pix_cap, int(pix_dev)):
             raise RuntimeError("xpngb_decode_region: " + self._err())
 
+    def decode_oriented_raw(self, descs, ops_arr, rect_arr, n, files_ptr, files_size, files_dev, offs, sizes, pix_ptr, pix_cap, pix_dev):
+        """decode_raw (rect_arr None) or decode_region_raw with entry i turned by ops_arr[i] (see op_codes()): written packed at
+        pix_ptr + descs[i].offset, with width and height swapped for the quarter turns.  descs are not swapped."""
+        if lib().xpngb_decode_oriented(self._h, ops_arr, descs, rect_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev), offs,
+                                       sizes, C.c_void_p(pix_ptr), pix_cap, int(pix_dev)):
+            raise RuntimeError("xpngb_decode_oriented: " + self._err())
+
     # ---------------------------------------------------------------- numpy convenience (host buffers)
     def encode(self, level, images):
         """list of (h,w,3|4) uint8 arrays -> list of .xpng byte strings."""
@@ -218,8 +245,8 @@ class Codec:
         offs, sizes = self.encode_raw(level, descs, len(images), buf.ctypes.data, total, 0, out.ctypes.data, cap, 0)
         return [out[offs[i]: offs[i] + sizes[i]].tobytes() for i in range(len(images))]
 
-    def decode(self, files):
-        """list of .xpng byte strings -> list of (h,w,3|4) uint8 arrays."""
+    def _pack_files(self, files, ra=None):
+        """Files packed at 16-byte offsets and a host output buffer: one whole image, or crop ra[i], per entry."""
         n = len(files)
         descs = (_Image * n)()
         foffs, fsizes = (C.c_uint64 * n)(), (C.c_uint64 * n)()
@@ -231,46 +258,56 @@ class Codec:
             foffs[i], fsizes[i] = off, len(f)
             off = _align16(off + len(f))
             descs[i].offset = poff
-            poff = _align16(poff + descs[i].w * descs[i].h * (3 + descs[i].A))
-        fb = np.zeros(off + 16, dtype=np.uint8)
-        for i, f in enumerate(files):
-            fb[foffs[i]: foffs[i] + len(f)] = np.frombuffer(f, dtype=np.uint8)
-        px = np.empty(poff + 16, dtype=np.uint8)
-        self.decode_raw(descs, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
-        out = []
-        for d in descs:
-            c = 3 + d.A
-            out.append(px[d.offset: d.offset + d.w * d.h * c].reshape(d.h, d.w, c).copy())
-        return out
-
-    def decode_region(self, files, boxes):
-        """list of .xpng byte strings and one (x, y, w, h) rectangle per file -> list of (h, w, 3|4) uint8 crops.  Only the
-        tiles a rectangle touches are decoded; the same file may appear several times."""
-        n = len(files)
-        if len(boxes) != n:
-            raise ValueError("one rectangle per file")
-        descs, ra = (_Image * n)(), rects(boxes)
-        foffs, fsizes = (C.c_uint64 * n)(), (C.c_uint64 * n)()
-        off = poff = 0
-        for i, f in enumerate(files):
-            b = np.frombuffer(f, dtype=np.uint8)
-            if lib().xpngb_peek(b.ctypes.data, len(f), C.byref(descs[i])):
-                raise ValueError(f"file {i}: not an .xpng header")
-            foffs[i], fsizes[i] = off, len(f)
-            off = _align16(off + len(f))
-            descs[i].offset = poff
-            if ra[i].w <= descs[i].w and ra[i].h <= descs[i].h:     # other rectangles are refused by the library, naming the entry
+            if ra is None:
+                poff = _align16(poff + descs[i].w * descs[i].h * (3 + descs[i].A))
+            elif ra[i].w <= descs[i].w and ra[i].h <= descs[i].h:     # other rectangles are refused by the library, naming the entry
                 poff = _align16(poff + ra[i].w * ra[i].h * (3 + descs[i].A))
         fb = np.zeros(off + 16, dtype=np.uint8)
         for i, f in enumerate(files):
             fb[foffs[i]: foffs[i] + len(f)] = np.frombuffer(f, dtype=np.uint8)
         px = np.empty(poff + 16, dtype=np.uint8)
-        self.decode_region_raw(descs, ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        return descs, foffs, fsizes, fb, off, px, poff
+
+    @staticmethod
+    def _unpack(px, descs, sizes, ops):
+        """Entry i of px as an (h, w, c) array, w x h = sizes[i]; (w, h, c) for the quarter turns of ops."""
         out = []
-        for d, r in zip(descs, ra):
+        for i, (d, (w, h)) in enumerate(zip(descs, sizes)):
             c = 3 + d.A
-            out.append(px[d.offset: d.offset + r.w * r.h * c].reshape(r.h, r.w, c).copy())
+            if ops is not None and ops[i] in QUARTER_TURNS:
+                w, h = h, w
+            out.append(px[d.offset: d.offset + w * h * c].reshape(h, w, c).copy())
         return out
+
+    def decode(self, files, ops=None):
+        """list of .xpng byte strings -> list of (h,w,3|4) uint8 arrays.  ops: one OPS name per file, each image written as
+        that op leaves it ((w,h,3|4) for 'r90' and 'r270'); inverse_op(op) restores files written by encode_oriented(op)."""
+        n = len(files)
+        if ops is not None and len(ops) != n:
+            raise ValueError("one op per file")
+        descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files)
+        if ops is None:
+            self.decode_raw(descs, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        else:
+            self.decode_oriented_raw(descs, op_codes(ops), None, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        return self._unpack(px, descs, [(d.w, d.h) for d in descs], ops)
+
+    def decode_region(self, files, boxes, ops=None):
+        """list of .xpng byte strings and one (x, y, w, h) rectangle per file -> list of (h, w, 3|4) uint8 crops.  Only the
+        tiles a rectangle touches are decoded; the same file may appear several times.  ops: one OPS name per entry, applied
+        to the crop (rectangles are in the file's coordinates); 'r90' and 'r270' crops come back as (w, h, 3|4)."""
+        n = len(files)
+        if len(boxes) != n:
+            raise ValueError("one rectangle per file")
+        if ops is not None and len(ops) != n:
+            raise ValueError("one op per file")
+        ra = rects(boxes)
+        descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files, ra)
+        if ops is None:
+            self.decode_region_raw(descs, ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        else:
+            self.decode_oriented_raw(descs, op_codes(ops), ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        return self._unpack(px, descs, [(r.w, r.h) for r in ra], ops)
 
     # ---------------------------------------------------------------- traversal-order operations (Mirroring_and_Rotating/tool.c)
     def _pack(self, images):

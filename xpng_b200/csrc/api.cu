@@ -70,7 +70,8 @@ struct xpngb_ctx {
     DevBuf pixels, norm, files, arena, tiles, imgs, seg_tile, costs, hist, seginfo, place, vplace, vcnt, sym_area,
         bits_area, alpha, streams, blocks, state, outs, flags, skip, dimgs, dtiles, plane, nlseq, rowcnt, rowbits, eord,
         rows, edge, errflag, hdr, offs, m2a, m2b, tclass, tabs, ccnt, cbit, resv, oriented, odesc, pdw,
-        region, crops;   // region decode: window of the selected tiles, crop descriptors
+        region, crops,   // region decode: window of the selected tiles, crop descriptors
+        orients;         // oriented decode: OrientDesc of the lane's chunk (odesc belongs to xpngb_transform / encode_oriented)
     PinBuf pin_a, pin_b, pin_o;   // pin_o: orientation descriptors (their upload may still be in flight when an encode reuses pin_a)
 };
 
@@ -389,7 +390,7 @@ static void lane_free(xpngb_ctx* ctx) {
                       &ctx->streams, &ctx->blocks, &ctx->state, &ctx->outs, &ctx->flags, &ctx->skip, &ctx->dimgs, &ctx->dtiles,
                       &ctx->plane, &ctx->nlseq, &ctx->rowcnt, &ctx->rowbits, &ctx->rows, &ctx->edge, &ctx->errflag, &ctx->hdr,
                       &ctx->offs, &ctx->m2a, &ctx->m2b, &ctx->tclass, &ctx->tabs, &ctx->ccnt, &ctx->cbit, &ctx->resv, &ctx->oriented,
-                      &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops };
+                      &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops, &ctx->orients };
     for (DevBuf* b : all) if (b->p) cudaFree(b->p);
     if (ctx->pin_a.p) cudaFreeHost(ctx->pin_a.p);
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
@@ -847,16 +848,25 @@ extern "C" int xpngb_encode(xpngb_ctx* ctx, int level, xpngb_image* imgs, uint32
 // ------------------------------------------------------------------------------------------------
 // Traversal-order operations (Mirroring_and_Rotating/tool.c): mirror / quarter-turn n pixmaps
 // ------------------------------------------------------------------------------------------------
+// The w x h source rectangle at src (rows src_pitch bytes apart) turned by op into packed rows at dst; *ctas: CTAs of the
+// launch so far (k_orient runs one per 64 x 64 patch).  False when the launch would exceed the grid limit.
+static bool orient_desc(OrientDesc& d, uint64_t src, uint64_t src_pitch, uint64_t dst, uint64_t w, uint64_t h, uint32_t pxsz,
+                        int op, uint64_t* ctas) {
+    d.src = src; d.dst = dst; d.src_pitch = src_pitch;
+    d.w = (uint32_t)w; d.h = (uint32_t)h; d.pxsz = pxsz; d.op = (uint32_t)op;
+    d.tiles_x = (d.w + ORI_T - 1) / ORI_T; d.first_cta = (uint32_t)*ctas;
+    *ctas += (uint64_t)d.tiles_x * ((d.h + ORI_T - 1) / ORI_T);
+    return *ctas <= 0x7FFFFFFFull;
+}
+
 static int orient_launch(xpngb_ctx* ctx, int op, xpngb_image* imgs, uint32_t n, const uint8_t* dsrc, uint8_t* ddst) {
     std::vector<OrientDesc> D(n);
     uint64_t ctas = 0;
     for (uint32_t i = 0; i < n; i++) {
-        OrientDesc& d = D[i];
-        d.src = (uint64_t)(dsrc + imgs[i].offset); d.dst = (uint64_t)(ddst + imgs[i].offset);
-        d.w = (uint32_t)imgs[i].w; d.h = (uint32_t)imgs[i].h; d.pxsz = imgs[i].A ? 4 : 3; d.op = (uint32_t)op;
-        d.tiles_x = (d.w + ORI_T - 1) / ORI_T; d.first_cta = (uint32_t)ctas;
-        ctas += (uint64_t)d.tiles_x * ((d.h + ORI_T - 1) / ORI_T);
-        if (ctas > 0x7FFFFFFFull) FAIL("too many pixels for one orientation launch");
+        const uint32_t pxsz = imgs[i].A ? 4 : 3;
+        if (!orient_desc(D[i], (uint64_t)(dsrc + imgs[i].offset), imgs[i].w * pxsz, (uint64_t)(ddst + imgs[i].offset), imgs[i].w,
+                         imgs[i].h, pxsz, op, &ctas))
+            FAIL("too many pixels for one orientation launch");
     }
     const size_t nb = n * sizeof(OrientDesc);
     ENSURE(odesc, nb);
@@ -983,23 +993,31 @@ static bool whole_tiles(const RegionSel& R) {
     return R.rect.x == R.cover.x && R.rect.y == R.cover.y && R.rect.w == R.cover.w && R.rect.h == R.cover.h;
 }
 static uint64_t window_pitch(const RegionSel& R, uint32_t pxsz) { return (R.cover.w * pxsz + 15) & ~15ull; }   // keeps RGB rows word-aligned (tile_pitched)
+// Entry i of an oriented decode is written turned or mirrored.  TL and TR are copies in the reference: those entries are
+// decoded exactly as without an op.
+static bool turned(const int* ops, uint32_t i) { return ops && ops[i] != OP_TL && ops[i] != OP_TR; }
 
 // Launch the decode of one chunk on lane `ctx`.  DI: the checked images of the chunk.  `lat`: warp-per-block chain
 // kernels (few blocks in the whole call) instead of the pair decoders.  sel == nullptr: every tile of every image, in
 // place.  Otherwise a region decode: only the tiles of sel[i].s, written in place when the rectangle is made of whole
 // tiles, else into a window of the lane's region scratch from which k_crop_rows copies the rectangle; stored images
-// are cropped straight out of their files.  Never waits for the device.
-static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, uint32_t n,
-                        const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
+// are cropped straight out of their files.  ops (only with sel): an entry that is turned (turned()) always goes through a
+// window, or for a stored image straight out of its file, and one k_orient launch writes all of them.  Never waits for
+// the device.
+static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
+                        uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
     std::vector<CropDesc> crops;
+    std::vector<OrientDesc> odescs;
+    uint64_t octas = 0;
     bool any1 = false, any2 = false, any7 = false;
     for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
-    if (sel) {   // windows for the rectangles that are not made of whole tiles
+    if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned entry
         uint64_t need = 0;
-        for (uint32_t i = 0; i < n; i++) if (DI[i].mode != 7 && !whole_tiles(sel[i])) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
+        for (uint32_t i = 0; i < n; i++)
+            if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i))) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
         if (need) ENSURE(region, need);
     }
     uint64_t wpos = 0;
@@ -1015,17 +1033,21 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             const xpngb_rect& r = sel[i].rect;
             ImageDesc I{}; I.tile0 = (uint32_t)P.tiles.size(); I.mode = 7; I.w = D.w; I.h = D.h; I.pxsz = D.pxsz;
             P.imgs.push_back(I);
-            crops.push_back(CropDesc{ (uint64_t)(din + D.file_off + 8 + (r.y * D.w + r.x) * D.pxsz), (uint64_t)out, (uint64_t)D.w * D.pxsz,
-                                      (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+            const uint64_t src = (uint64_t)(din + D.file_off + 8 + (r.y * D.w + r.x) * D.pxsz);   // any byte alignment
+            if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, (uint64_t)D.w * D.pxsz, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+            else if (!orient_desc(odescs.emplace_back(), src, (uint64_t)D.w * D.pxsz, (uint64_t)out, r.w, r.h, D.pxsz, ops[i], &octas))
+                FAIL("too many pixels for one orientation launch");
         } else {
             const RegionSel& R = sel[i];
             const xpngb_rect &r = R.rect, &c = R.cover;
-            if (whole_tiles(R)) plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
-            else {
+            if (whole_tiles(R) && !turned(ops, i)) plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
+            else {   // a turned rectangle cannot be decoded in place, even when it is made of whole tiles
                 const uint64_t pitch = window_pitch(R, D.pxsz), win = (uint64_t)ctx->region.p + wpos;
                 plan_image(P, R.g, R.s, win, pitch, c.x, c.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
-                crops.push_back(CropDesc{ win + (r.y - c.y) * pitch + (r.x - c.x) * D.pxsz, (uint64_t)out, pitch,
-                                          (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+                const uint64_t src = win + (r.y - c.y) * pitch + (r.x - c.x) * D.pxsz;
+                if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, pitch, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+                else if (!orient_desc(odescs.emplace_back(), src, pitch, (uint64_t)out, r.w, r.h, D.pxsz, ops[i], &octas))
+                    FAIL("too many pixels for one orientation launch");
                 wpos += c.h * pitch;
             }
             D.gcols = (uint32_t)R.g.nw; D.r0 = (uint32_t)R.s.r0; D.c0 = (uint32_t)R.s.c0;
@@ -1037,9 +1059,9 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     const uint32_t ntiles = (uint32_t)P.tiles.size();
     if (upload_plan(ctx, P)) return 1;
     ENSURE(dimgs, n * sizeof(DecImage)); ENSURE(dtiles, ntiles * sizeof(DecTile)); ENSURE(errflag, 4);
-    // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop descriptors
-    const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64;
-    if (ensure_pin(ctx, ctx->pin_b, pin_crops + crops.size() * sizeof(CropDesc))) return 1;
+    // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop descriptors, orientation descriptors
+    const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64, pin_orients = pin_crops + crops.size() * sizeof(CropDesc);
+    if (ensure_pin(ctx, ctx->pin_b, pin_orients + odescs.size() * sizeof(OrientDesc))) return 1;
     memcpy(ctx->pin_b.p, DI.data(), n * sizeof(DecImage));
     CK(cudaMemcpyAsync(ctx->dimgs.p, ctx->pin_b.p, n * sizeof(DecImage), cudaMemcpyHostToDevice, ctx->stream));
     if (any7 && !sel) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
@@ -1052,6 +1074,12 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         ENSURE(crops, crops.size() * sizeof(CropDesc));
         memcpy((uint8_t*)ctx->pin_b.p + pin_crops, crops.data(), crops.size() * sizeof(CropDesc));
         CK(cudaMemcpyAsync(ctx->crops.p, (uint8_t*)ctx->pin_b.p + pin_crops, crops.size() * sizeof(CropDesc), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (!odescs.empty()) {   // this lane's staging and descriptor buffer: the lanes of a call run concurrently
+        const size_t nb = odescs.size() * sizeof(OrientDesc);
+        ENSURE(orients, nb);
+        memcpy((uint8_t*)ctx->pin_b.p + pin_orients, odescs.data(), nb);
+        CK(cudaMemcpyAsync(ctx->orients.p, (uint8_t*)ctx->pin_b.p + pin_orients, nb, cudaMemcpyHostToDevice, ctx->stream));
     }
     CK(cudaMemsetAsync(ctx->errflag.p, 0, 4, ctx->stream));
     CK(cudaMemsetAsync(ctx->dtiles.p, 0, ntiles * sizeof(DecTile), ctx->stream));
@@ -1244,15 +1272,17 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             LAUNCH(k_crop_rows, dim3(gx, m), 256, 0, (const CropDesc*)ctx->crops.p + c0);
         }
     }
+    if (!odescs.empty()) LAUNCH(k_orient, (unsigned)octas, 256, 0, (const OrientDesc*)ctx->orients.p, (uint32_t)odescs.size());
     // the error flag travels to pinned memory behind the DecImage table
     CK(cudaMemcpyAsync((uint8_t*)ctx->pin_b.p + n * (sizeof(DecImage) + 8), d_err, 4, cudaMemcpyDeviceToHost, ctx->stream));
     return 0;
 }
 
-// xpngb_decode (rects == nullptr) and xpngb_decode_region.
-static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, uint32_t n, const void* files, uint64_t files_size,
-                       int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
-                       int pixels_on_device) {
+// xpngb_decode (rects == nullptr), xpngb_decode_region and, with ops, xpngb_decode_oriented.  An oriented call always
+// selects tiles per entry: without rects every entry's rectangle is its whole image.
+static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, uint32_t n, const void* files,
+                       uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
+                       uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     ctx->err[0] = 0; ctx->launches = 0; ctx->last_ms = 0.f; ctx->cur = ctx->stream;
     if (!imgs || !files || !file_offsets || !file_sizes || !pixels) FAIL("null argument");
@@ -1260,6 +1290,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     CK(cudaSetDevice(ctx->device));
     for (uint32_t i = 0; i < n; i++) {
         if (file_sizes[i] < 11 || file_sizes[i] > files_size || file_offsets[i] > files_size - file_sizes[i]) FAIL("file %u: bad offset/size", i);
+        if (ops && (ops[i] < OP_R90 || ops[i] > OP_TR)) FAIL("entry %u: unknown orientation op %d", i, ops[i]);
     }
     const uint8_t* din = (const uint8_t*)files;
     if (!files_on_device) { ENSURE(files, files_size); din = (const uint8_t*)ctx->files.p; }
@@ -1278,10 +1309,14 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     }
     // ---- every entry is checked before anything is decoded
     std::vector<DecImage> DI(n);
-    std::vector<RegionSel> sel(rects ? n : 0);
+    const bool use_sel = rects || ops;
+    std::vector<RegionSel> sel(use_sel ? n : 0);
     for (uint32_t i = 0; i < n; i++) {
         if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, pixels_cap, DI[i])) return 1;
-        if (rects) { sel[i].rect = rects[i]; region_select(imgs[i].w, imgs[i].h, rects[i], sel[i].g, sel[i].s, sel[i].cover); }
+        if (use_sel) {
+            sel[i].rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
+            region_select(imgs[i].w, imgs[i].h, sel[i].rect, sel[i].g, sel[i].s, sel[i].cover);
+        }
     }
     uint8_t* dpx = (uint8_t*)pixels;
     if (!pixels_on_device) { ENSURE(pixels, pixels_cap); dpx = (uint8_t*)ctx->pixels.p; }
@@ -1290,13 +1325,13 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     uint64_t tiles_est = 0; bool l2 = false;
     for (uint32_t i = 0; i < n; i++) {
         const uint32_t mode = imgs[i].mode;
-        const xpngb_rect* wh = !rects ? nullptr : (mode == 7 ? &sel[i].rect : &sel[i].cover);
+        const xpngb_rect* wh = !use_sel ? nullptr : (mode == 7 ? &sel[i].rect : &sel[i].cover);
         dims[i].w = wh ? wh->w : imgs[i].w; dims[i].h = wh ? wh->h : imgs[i].h;
-        if (mode == 1 || mode == 2) tiles_est += rects ? (sel[i].s.r1 - sel[i].s.r0 + 1) * (sel[i].s.c1 - sel[i].s.c0 + 1)
-                                                       : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
+        if (mode == 1 || mode == 2) tiles_est += use_sel ? (sel[i].s.r1 - sel[i].s.r0 + 1) * (sel[i].s.c1 - sel[i].s.c0 + 1)
+                                                         : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
         l2 |= mode == 2;
     }
-    auto out_bytes = [&](uint32_t i) { return (rects ? rects[i].w * rects[i].h : imgs[i].w * imgs[i].h) * (3 + imgs[i].A); };
+    auto out_bytes = [&](uint32_t i) { return (use_sel ? sel[i].rect.w * sel[i].rect.h : imgs[i].w * imgs[i].h) * (3 + imgs[i].A); };
     // level 2: above ~600 tiles the pair family wins, with the 16-symbol value streams warp-per-block while they all fit
     // (s16_lat_max_tiles); level 1: the warp-per-block family up to ~1300 tiles (measured at 125 / 250 / 500 frames, profiles/)
     const bool lat = l2 ? 17 * tiles_est <= (uint64_t)ctx->lat_max_blocks * 5 / 6 : 9 * tiles_est <= ctx->lat_max_blocks;
@@ -1330,7 +1365,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
                 snprintf(ctx->err, sizeof ctx->err, "host to device copy failed"); rc = 1; break;
             }
         }
-        rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, rects ? sel.data() + i0 : nullptr, m, din, dpx,
+        rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr, m, din, dpx,
                           (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
@@ -1365,7 +1400,8 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
 extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
                             const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
                             int pixels_on_device) {
-    return decode_call(ctx, imgs, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap, pixels_on_device);
+    return decode_call(ctx, imgs, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+                       pixels_on_device);
 }
 
 extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, uint32_t n, const void* files,
@@ -1373,7 +1409,17 @@ extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpng
                                    void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap, pixels_on_device);
+    return decode_call(ctx, imgs, rects, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+                       pixels_on_device);
+}
+
+extern "C" int xpngb_decode_oriented(xpngb_ctx* ctx, const int* ops, xpngb_image* imgs, const xpngb_rect* rects, uint32_t n,
+                                     const void* files, uint64_t files_size, int files_on_device, const uint64_t* file_offsets,
+                                     const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
+    if (!ctx) return 1;
+    if (!ops) { ctx->err[0] = 0; FAIL("null argument"); }
+    return decode_call(ctx, imgs, rects, ops, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+                       pixels_on_device);
 }
 
 // ------------------------------------------------------------------------------------------------
