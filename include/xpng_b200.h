@@ -120,6 +120,30 @@ int xpngb_decode_oriented(xpngb_ctx *ctx, const int *ops, xpngb_image *imgs, con
                           const uint64_t *file_offsets, const uint64_t *file_sizes,
                           void *pixels, uint64_t pixels_cap, int pixels_on_device);
 
+/* ---- Resized decode: each image or crop resampled to a requested size in the same call, for fixed-size batches. */
+typedef struct xpngb_size { uint32_t w, h; } xpngb_size;
+
+/* Entry i is orient(ops[i], resize(crop_i, sizes[i].w, sizes[i].h)), where crop_i is rects[i] in the stored file's
+ * coordinates (rects == NULL: the whole image), and ops == NULL means no op (otherwise as for xpngb_decode_oriented).
+ *   resize  : byte-identical to Pillow's Image.resize((w, h), Image.BILINEAR) of the crop (8-bit path: horizontal pass
+ *             first, rounded to bytes, then vertical; 22-bit fixed-point weights).  Alpha is resampled as a fourth
+ *             independent channel, NOT premultiplied: it equals PIL's resize of each channel as an "L" image, and differs
+ *             from PIL's own RGBA resize, which premultiplies.
+ *   output  : sizes[i].h packed rows of sizes[i].w * (3 + A) bytes at pixels + imgs[i].offset (a multiple of 16).  The op
+ *             is applied after the resize, so R90 and R270 write sizes[i].w rows of sizes[i].h pixels.
+ *   imgs[i] : in/out exactly as for xpngb_decode (the file's w, h, A; mode out).
+ * Every entry is checked before anything is decoded, and the error (xpngb_last_error) names the entry: every check of
+ * xpngb_decode_region and xpngb_decode_oriented, sizes == NULL, a zero w or h or one above 2^24, an output past
+ * pixels_cap, and a resampled crop side above 2^23 pixels (the 32-bit accumulator of the passes is exact up to there).
+ * An entry whose size equals its crop is byte-identical to xpngb_decode_oriented / xpngb_decode_region and takes their
+ * path.  Resized entries are decoded into a scratch window (stored level-7 entries are read straight from the file) and
+ * resampled in device memory: with host buffers only the resized outputs cross PCIe back. */
+int xpngb_decode_resized(xpngb_ctx *ctx, const int *ops, xpngb_image *imgs, const xpngb_rect *rects,
+                         const xpngb_size *sizes, uint32_t n,
+                         const void *files, uint64_t files_size, int files_on_device,
+                         const uint64_t *file_offsets, const uint64_t *file_sizes,
+                         void *pixels, uint64_t pixels_cap, int pixels_on_device);
+
 /* Device time of the kernels of the last encode/decode call on this context, in milliseconds
  * (CUDA events on the context's stream; excludes host<->device copies). */
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);

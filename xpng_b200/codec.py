@@ -29,6 +29,10 @@ class _Rect(C.Structure):  # xpngb_rect: pixels, (x, y) = top-left corner
     _fields_ = [("x", C.c_uint64), ("y", C.c_uint64), ("w", C.c_uint64), ("h", C.c_uint64)]
 
 
+class _Size(C.Structure):  # xpngb_size: output pixels of a resized decode
+    _fields_ = [("w", C.c_uint32), ("h", C.c_uint32)]
+
+
 class _Xpng(C.Structure):  # xpng_t, xpng.h:10
     _fields_ = [("p", C.c_void_p), ("w", C.c_uint64), ("h", C.c_uint64), ("s", C.c_uint64), ("A", C.c_bool)]
 
@@ -67,6 +71,9 @@ def lib():
         L.xpngb_decode_oriented.restype = C.c_int
         L.xpngb_decode_oriented.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect), u32, vp, u64, C.c_int,
                                             C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_decode_resized.restype = C.c_int
+        L.xpngb_decode_resized.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect), C.POINTER(_Size), u32, vp, u64,
+                                           C.c_int, C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
         L.xpngb_last_kernel_ms.restype = C.c_float; L.xpngb_last_kernel_ms.argtypes = [vp]
         L.xpngb_last_launches.restype = u32; L.xpngb_last_launches.argtypes = [vp]
         L.xpngb_stream.restype = vp; L.xpngb_stream.argtypes = [vp]
@@ -133,6 +140,17 @@ def rects(boxes):
     for i, (x, y, w, h) in enumerate(boxes):
         arr[i].x, arr[i].y, arr[i].w, arr[i].h = int(x), int(y), int(w), int(h)
     return arr
+
+
+def sizes(whs):
+    """[(w, h)] -> ctypes array of xpngb_size."""
+    arr = (_Size * len(whs))()
+    for i, (w, h) in enumerate(whs):
+        arr[i].w, arr[i].h = int(w), int(h)
+    return arr
+
+
+_sizes = sizes   # Codec.decode_resized's argument of the same name hides it
 
 
 def region_tiles(w, h, rect):
@@ -232,6 +250,15 @@ class Codec:
                                        sizes, C.c_void_p(pix_ptr), pix_cap, int(pix_dev)):
             raise RuntimeError("xpngb_decode_oriented: " + self._err())
 
+    def decode_resized_raw(self, descs, ops_arr, rect_arr, size_arr, n, files_ptr, files_size, files_dev, offs, sizes, pix_ptr, pix_cap,
+                           pix_dev):
+        """decode_oriented_raw with entry i resampled to size_arr[i] (see sizes()) before its op: Pillow's bilinear resize of the
+        crop rect_arr[i] (None: whole images), ops_arr None for no op.  Written packed at pix_ptr + descs[i].offset as
+        size_arr[i].h rows of size_arr[i].w pixels, swapped for the quarter turns."""
+        if lib().xpngb_decode_resized(self._h, ops_arr, descs, rect_arr, size_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev),
+                                      offs, sizes, C.c_void_p(pix_ptr), pix_cap, int(pix_dev)):
+            raise RuntimeError("xpngb_decode_resized: " + self._err())
+
     # ---------------------------------------------------------------- numpy convenience (host buffers)
     def encode(self, level, images):
         """list of (h,w,3|4) uint8 arrays -> list of .xpng byte strings."""
@@ -245,8 +272,8 @@ class Codec:
         offs, sizes = self.encode_raw(level, descs, len(images), buf.ctypes.data, total, 0, out.ctypes.data, cap, 0)
         return [out[offs[i]: offs[i] + sizes[i]].tobytes() for i in range(len(images))]
 
-    def _pack_files(self, files, ra=None):
-        """Files packed at 16-byte offsets and a host output buffer: one whole image, or crop ra[i], per entry."""
+    def _pack_files(self, files, ra=None, sa=None):
+        """Files packed at 16-byte offsets and a host output buffer: one whole image, crop ra[i] or size sa[i] per entry."""
         n = len(files)
         descs = (_Image * n)()
         foffs, fsizes = (C.c_uint64 * n)(), (C.c_uint64 * n)()
@@ -258,7 +285,10 @@ class Codec:
             foffs[i], fsizes[i] = off, len(f)
             off = _align16(off + len(f))
             descs[i].offset = poff
-            if ra is None:
+            if sa is not None:
+                if 0 < sa[i].w <= 1 << 24 and 0 < sa[i].h <= 1 << 24:   # other sizes are refused by the library, naming the entry
+                    poff = _align16(poff + sa[i].w * sa[i].h * (3 + descs[i].A))
+            elif ra is None:
                 poff = _align16(poff + descs[i].w * descs[i].h * (3 + descs[i].A))
             elif ra[i].w <= descs[i].w and ra[i].h <= descs[i].h:     # other rectangles are refused by the library, naming the entry
                 poff = _align16(poff + ra[i].w * ra[i].h * (3 + descs[i].A))
@@ -308,6 +338,25 @@ class Codec:
         else:
             self.decode_oriented_raw(descs, op_codes(ops), ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         return self._unpack(px, descs, [(r.w, r.h) for r in ra], ops)
+
+    def decode_resized(self, files, sizes, boxes=None, ops=None):
+        """list of .xpng byte strings and one (w, h) output size per file -> list of (h, w, 3|4) uint8 arrays: each whole image,
+        or rectangle boxes[i] = (x, y, w, h) of it, resampled as Pillow's Image.resize((w, h), Image.BILINEAR) does, every
+        channel on its own (alpha is not premultiplied).  ops: one OPS name per entry, applied after the resize; 'r90' and
+        'r270' entries come back as (w, h, 3|4).  An entry whose size equals its crop is the crop itself."""
+        n = len(files)
+        if len(sizes) != n:
+            raise ValueError("one size per file")
+        if boxes is not None and len(boxes) != n:
+            raise ValueError("one rectangle per file")
+        if ops is not None and len(ops) != n:
+            raise ValueError("one op per file")
+        ra = None if boxes is None else rects(boxes)
+        sa = _sizes(sizes)
+        descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files, ra, sa)
+        self.decode_resized_raw(descs, None if ops is None else op_codes(ops), ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes,
+                                px.ctypes.data, poff, 0)
+        return self._unpack(px, descs, [(z.w, z.h) for z in sa], ops)
 
     # ---------------------------------------------------------------- traversal-order operations (Mirroring_and_Rotating/tool.c)
     def _pack(self, images):

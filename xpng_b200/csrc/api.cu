@@ -31,6 +31,7 @@
 #include "misc.cuh"
 #include "orient.cuh"
 #include "region.cuh"
+#include "resize.cuh"
 
 using namespace xpb;
 
@@ -71,7 +72,8 @@ struct xpngb_ctx {
         bits_area, alpha, streams, blocks, state, outs, flags, skip, dimgs, dtiles, plane, nlseq, rowcnt, rowbits, eord,
         rows, edge, errflag, hdr, offs, m2a, m2b, tclass, tabs, ccnt, cbit, resv, oriented, odesc, pdw,
         region, crops,   // region decode: window of the selected tiles, crop descriptors
-        orients;         // oriented decode: OrientDesc of the lane's chunk (odesc belongs to xpngb_transform / encode_oriented)
+        orients,         // oriented decode: OrientDesc of the lane's chunk (odesc belongs to xpngb_transform / encode_oriented)
+        rdescs, rtab, rtmp;   // resized decode: ResizeDesc of the lane's chunk, windows and weights, the first pass's rows
     PinBuf pin_a, pin_b, pin_o;   // pin_o: orientation descriptors (their upload may still be in flight when an encode reuses pin_a)
 };
 
@@ -390,7 +392,8 @@ static void lane_free(xpngb_ctx* ctx) {
                       &ctx->streams, &ctx->blocks, &ctx->state, &ctx->outs, &ctx->flags, &ctx->skip, &ctx->dimgs, &ctx->dtiles,
                       &ctx->plane, &ctx->nlseq, &ctx->rowcnt, &ctx->rowbits, &ctx->rows, &ctx->edge, &ctx->errflag, &ctx->hdr,
                       &ctx->offs, &ctx->m2a, &ctx->m2b, &ctx->tclass, &ctx->tabs, &ctx->ccnt, &ctx->cbit, &ctx->resv, &ctx->oriented,
-                      &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops, &ctx->orients };
+                      &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops, &ctx->orients,
+                      &ctx->rdescs, &ctx->rtab, &ctx->rtmp };
     for (DevBuf* b : all) if (b->p) cudaFree(b->p);
     if (ctx->pin_a.p) cudaFreeHost(ctx->pin_a.p);
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
@@ -958,9 +961,10 @@ static PdWork pdw_at(void* base, uint32_t cap) {
 
 // Header checks of file i (libxpng.c:969-976) and of where its pixels go: fills imgs[i] (w, h, A, mode) and D (file,
 // geometry, effective mode).  A region decode (r != nullptr) writes the r->w x r->h crop at imgs[i].offset instead of
-// the whole image.  Runs for every entry of a call before anything is launched.
+// the whole image, and a resized decode (sz != nullptr) an sz->w x sz->h image.  Runs for every entry of a call before
+// anything is launched.
 static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint32_t* hdr, uint64_t file_off, uint64_t file_size,
-                        const xpngb_rect* r, uint64_t pixels_cap, DecImage& D) {
+                        const xpngb_rect* r, const xpngb_size* sz, uint64_t pixels_cap, DecImage& D) {
     const uint64_t w = (hdr[0] & 0xFFFFFFu) + 1, h = (hdr[1] & 0xFFFFFFu) + 1;
     const uint32_t A = (hdr[1] >> 24) & 1, mode = hdr[0] >> 24, pxsz = 3 + A;
     if (!(mode == 1 || mode == 2 || mode == 7)) FAIL("file %u: unknown mode %u", i, mode);   // libxpng.c:972
@@ -971,7 +975,7 @@ static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint
     if (r && (r->x >= w || r->w > w - r->x || r->y >= h || r->h > h - r->y))
         FAIL("entry %u: rectangle (%llu, %llu) %llux%llu is not inside the %llux%llu image", i, (unsigned long long)r->x,
              (unsigned long long)r->y, (unsigned long long)r->w, (unsigned long long)r->h, (unsigned long long)w, (unsigned long long)h);
-    const uint64_t s = w * h * pxsz, out = r ? r->w * r->h * pxsz : s;   // at most 2^24 x 2^24 pixels: no overflow
+    const uint64_t s = w * h * pxsz, out = sz ? (uint64_t)sz->w * sz->h * pxsz : r ? r->w * r->h * pxsz : s;   // at most 2^24 x 2^24 pixels: no overflow
     if (img.offset & 15) FAIL("file %u: pixel offset must be a multiple of 16", i);
     if (out > pixels_cap || img.offset > pixels_cap - out) FAIL("file %u: pixels exceed the output buffer", i);
     uint32_t m = mode;
@@ -996,30 +1000,89 @@ static uint64_t window_pitch(const RegionSel& R, uint32_t pxsz) { return (R.cove
 // Entry i of an oriented decode is written turned or mirrored.  TL and TR are copies in the reference: those entries are
 // decoded exactly as without an op.
 static bool turned(const int* ops, uint32_t i) { return ops && ops[i] != OP_TL && ops[i] != OP_TR; }
+// Entry i of a resized decode is resampled: its size differs from its rectangle's.  Other entries are decoded exactly as
+// by an oriented or region decode.
+static bool resized(const xpngb_size* sizes, const RegionSel* sel, uint32_t i) {
+    return sizes && (sizes[i].w != sel[i].rect.w || sizes[i].h != sel[i].rect.h);
+}
+// Pillow's number of weights per output coordinate of one axis (0: the axis is not resampled).
+static uint32_t resize_ksize(uint64_t in, uint64_t out) {
+    if (in == out) return 0;
+    const double scale = (double)in / (double)out;
+    return 2 * (uint32_t)ceil(scale < 1.0 ? 1.0 : scale) + 1;
+}
+static uint64_t resize_tab_bytes(const RegionSel& R, const xpngb_size& z) {
+    return resize_table_bytes((uint32_t)R.rect.w, z.w, resize_ksize(R.rect.w, z.w)) +
+           resize_table_bytes((uint32_t)R.rect.h, z.h, resize_ksize(R.rect.h, z.h));
+}
+// Scratch of resized entry i: tables (a multiple of 8 bytes) and the first pass's rows (16-byte aligned) when both axes are
+// resampled: in_h rows of out_w pixels, or out_h rows of in_w pixels when the vertical pass runs first.
+static uint64_t resize_tmp_bytes(const RegionSel& R, const xpngb_size& z, uint32_t pxsz) {
+    if (R.rect.w == z.w || R.rect.h == z.h) return 0;
+    const uint64_t px = resize_vfirst(R.rect.w, R.rect.h, z.w, z.h) ? z.h * R.rect.w : R.rect.h * z.w;
+    return (px * pxsz + 15) & ~15ull;
+}
 
 // Launch the decode of one chunk on lane `ctx`.  DI: the checked images of the chunk.  `lat`: warp-per-block chain
 // kernels (few blocks in the whole call) instead of the pair decoders.  sel == nullptr: every tile of every image, in
 // place.  Otherwise a region decode: only the tiles of sel[i].s, written in place when the rectangle is made of whole
 // tiles, else into a window of the lane's region scratch from which k_crop_rows copies the rectangle; stored images
 // are cropped straight out of their files.  ops (only with sel): an entry that is turned (turned()) always goes through a
-// window, or for a stored image straight out of its file, and one k_orient launch writes all of them.  Never waits for
-// the device.
+// window, or for a stored image straight out of its file, and one k_orient launch writes all of them.  sizes (only with
+// sel): a resized entry (resized()) also always goes through a window or its file, and is resampled and written through
+// its op by one launch of each resize kernel for the chunk.  Never waits for the device.
 static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
-                        uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
+                        const xpngb_size* sizes, uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
     std::vector<CropDesc> crops;
     std::vector<OrientDesc> odescs;
-    uint64_t octas = 0;
+    std::vector<ResizeDesc> rdescs;
+    uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0;
     bool any1 = false, any2 = false, any7 = false;
     for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
-    if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned entry
-        uint64_t need = 0;
-        for (uint32_t i = 0; i < n; i++)
-            if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i))) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
+    if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned or resized entry
+        uint64_t need = 0, tab = 0, tmp = 0;
+        for (uint32_t i = 0; i < n; i++) {
+            const bool rs = resized(sizes, sel, i);
+            if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
+            if (rs) { tab += resize_tab_bytes(sel[i], sizes[i]); tmp += resize_tmp_bytes(sel[i], sizes[i], DI[i].pxsz); }
+        }
         if (need) ENSURE(region, need);
+        if (tab) ENSURE(rtab, tab);
+        if (tmp) ENSURE(rtmp, tmp);
     }
+    // resized entry i: its crop at src (rows `pitch` bytes apart) resampled into out through its op, each pass reading the
+    // previous one's packed rows
+    uint64_t tpos = 0, mpos = 0;
+    auto resize_desc = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out) -> int {
+        const xpngb_rect& r = sel[i].rect;
+        const xpngb_size& z = sizes[i];
+        ResizeDesc d{};
+        d.coef = (uint64_t)ctx->rtab.p + tpos; tpos += resize_tab_bytes(sel[i], z);
+        const uint64_t tmp = (uint64_t)ctx->rtmp.p + mpos; mpos += resize_tmp_bytes(sel[i], z, DI[i].pxsz);
+        d.in_w = (uint32_t)r.w; d.in_h = (uint32_t)r.h; d.out_w = z.w; d.out_h = z.h;
+        d.pxsz = DI[i].pxsz; d.op = ops ? (uint32_t)ops[i] : (uint32_t)OP_TL;
+        d.kx = resize_ksize(r.w, z.w); d.ky = resize_ksize(r.h, z.h);
+        if (!d.kx) d.v = ResizePass{ src, pitch, (uint64_t)out, z.w, 1 };
+        else if (!d.ky) d.h = ResizePass{ src, pitch, (uint64_t)out, z.h, 1 };
+        else if (resize_vfirst(r.w, r.h, z.w, z.h)) {
+            d.v = ResizePass{ src, pitch, tmp, (uint32_t)r.w, 0 };
+            d.h = ResizePass{ tmp, r.w * DI[i].pxsz, (uint64_t)out, z.h, 1 };
+        } else {
+            d.h = ResizePass{ src, pitch, tmp, (uint32_t)r.h, 0 };
+            d.v = ResizePass{ tmp, (uint64_t)z.w * DI[i].pxsz, (uint64_t)out, z.w, 1 };
+        }
+        d.first_coef = (uint32_t)rcoef; d.first_h = (uint32_t)rh; d.first_v = (uint32_t)rv;
+        d.h_tiles_x = (z.w + RH_X - 1) / RH_X;
+        rcoef += (d.kx ? z.w : 0) + (d.ky ? z.h : 0);
+        if (d.kx) rh += (uint64_t)d.h_tiles_x * ((d.h.n + RH_ROWS - 1) / RH_ROWS);
+        if (d.ky) rv += ((uint64_t)d.v.n * d.pxsz + RV_X - 1) / RV_X * ((z.h + RV_ROWS - 1) / RV_ROWS);
+        if (rcoef > 0xFFFFFFFFull || rh > 0x7FFFFFFFull || rv > 0x7FFFFFFFull) FAIL("too many pixels for one resize launch");
+        rdescs.push_back(d);
+        return 0;
+    };
     uint64_t wpos = 0;
     for (uint32_t i = 0; i < n; i++) {
         DecImage& D = DI[i];
@@ -1034,18 +1097,21 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             ImageDesc I{}; I.tile0 = (uint32_t)P.tiles.size(); I.mode = 7; I.w = D.w; I.h = D.h; I.pxsz = D.pxsz;
             P.imgs.push_back(I);
             const uint64_t src = (uint64_t)(din + D.file_off + 8 + (r.y * D.w + r.x) * D.pxsz);   // any byte alignment
-            if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, (uint64_t)D.w * D.pxsz, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+            if (resized(sizes, sel, i)) { if (resize_desc(i, src, (uint64_t)D.w * D.pxsz, out)) return 1; }
+            else if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, (uint64_t)D.w * D.pxsz, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
             else if (!orient_desc(odescs.emplace_back(), src, (uint64_t)D.w * D.pxsz, (uint64_t)out, r.w, r.h, D.pxsz, ops[i], &octas))
                 FAIL("too many pixels for one orientation launch");
         } else {
             const RegionSel& R = sel[i];
             const xpngb_rect &r = R.rect, &c = R.cover;
-            if (whole_tiles(R) && !turned(ops, i)) plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
-            else {   // a turned rectangle cannot be decoded in place, even when it is made of whole tiles
+            const bool rs = resized(sizes, sel, i);
+            if (whole_tiles(R) && !turned(ops, i) && !rs) plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
+            else {   // a turned or resized rectangle cannot be decoded in place, even when it is made of whole tiles
                 const uint64_t pitch = window_pitch(R, D.pxsz), win = (uint64_t)ctx->region.p + wpos;
                 plan_image(P, R.g, R.s, win, pitch, c.x, c.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
                 const uint64_t src = win + (r.y - c.y) * pitch + (r.x - c.x) * D.pxsz;
-                if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, pitch, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
+                if (rs) { if (resize_desc(i, src, pitch, out)) return 1; }
+                else if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, pitch, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
                 else if (!orient_desc(odescs.emplace_back(), src, pitch, (uint64_t)out, r.w, r.h, D.pxsz, ops[i], &octas))
                     FAIL("too many pixels for one orientation launch");
                 wpos += c.h * pitch;
@@ -1059,9 +1125,10 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     const uint32_t ntiles = (uint32_t)P.tiles.size();
     if (upload_plan(ctx, P)) return 1;
     ENSURE(dimgs, n * sizeof(DecImage)); ENSURE(dtiles, ntiles * sizeof(DecTile)); ENSURE(errflag, 4);
-    // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop descriptors, orientation descriptors
+    // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop, orientation and resize descriptors
     const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64, pin_orients = pin_crops + crops.size() * sizeof(CropDesc);
-    if (ensure_pin(ctx, ctx->pin_b, pin_orients + odescs.size() * sizeof(OrientDesc))) return 1;
+    const size_t pin_resize = pin_orients + odescs.size() * sizeof(OrientDesc);
+    if (ensure_pin(ctx, ctx->pin_b, pin_resize + rdescs.size() * sizeof(ResizeDesc))) return 1;
     memcpy(ctx->pin_b.p, DI.data(), n * sizeof(DecImage));
     CK(cudaMemcpyAsync(ctx->dimgs.p, ctx->pin_b.p, n * sizeof(DecImage), cudaMemcpyHostToDevice, ctx->stream));
     if (any7 && !sel) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
@@ -1080,6 +1147,12 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         ENSURE(orients, nb);
         memcpy((uint8_t*)ctx->pin_b.p + pin_orients, odescs.data(), nb);
         CK(cudaMemcpyAsync(ctx->orients.p, (uint8_t*)ctx->pin_b.p + pin_orients, nb, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (!rdescs.empty()) {
+        const size_t nb = rdescs.size() * sizeof(ResizeDesc);
+        ENSURE(rdescs, nb);
+        memcpy((uint8_t*)ctx->pin_b.p + pin_resize, rdescs.data(), nb);
+        CK(cudaMemcpyAsync(ctx->rdescs.p, (uint8_t*)ctx->pin_b.p + pin_resize, nb, cudaMemcpyHostToDevice, ctx->stream));
     }
     CK(cudaMemsetAsync(ctx->errflag.p, 0, 4, ctx->stream));
     CK(cudaMemsetAsync(ctx->dtiles.p, 0, ntiles * sizeof(DecTile), ctx->stream));
@@ -1273,6 +1346,16 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         }
     }
     if (!odescs.empty()) LAUNCH(k_orient, (unsigned)octas, 256, 0, (const OrientDesc*)ctx->orients.p, (uint32_t)odescs.size());
+    if (!rdescs.empty()) {   // windows and weights, then the two passes, in Pillow's order for most entries
+        const ResizeDesc* d_rd = (const ResizeDesc*)ctx->rdescs.p;
+        const uint32_t nr = (uint32_t)rdescs.size();
+        bool vfirst = false;   // a chunk with a vertical-first entry gets a vertical launch before the horizontal one too
+        for (const ResizeDesc& d : rdescs) vfirst |= d.kx && d.ky && d.h.last;
+        LAUNCH(k_resize_coeffs, (unsigned)((rcoef + 255) / 256), 256, 0, d_rd, nr, (uint32_t)rcoef);
+        if (vfirst && rv) LAUNCH(k_resize_v, (unsigned)rv, RV_X, 0, d_rd, nr, 1u);
+        if (rh) LAUNCH(k_resize_h, (unsigned)rh, RH_X, 0, d_rd, nr);
+        if (rv) LAUNCH(k_resize_v, (unsigned)rv, RV_X, 0, d_rd, nr, vfirst ? 2u : 3u);
+    }
     // the error flag travels to pinned memory behind the DecImage table
     CK(cudaMemcpyAsync((uint8_t*)ctx->pin_b.p + n * (sizeof(DecImage) + 8), d_err, 4, cudaMemcpyDeviceToHost, ctx->stream));
     return 0;
@@ -1280,7 +1363,7 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
 
 // xpngb_decode (rects == nullptr), xpngb_decode_region and, with ops, xpngb_decode_oriented.  An oriented call always
 // selects tiles per entry: without rects every entry's rectangle is its whole image.
-static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, uint32_t n, const void* files,
+static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, const xpngb_size* sizes, uint32_t n, const void* files,
                        uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
                        uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
@@ -1291,6 +1374,8 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     for (uint32_t i = 0; i < n; i++) {
         if (file_sizes[i] < 11 || file_sizes[i] > files_size || file_offsets[i] > files_size - file_sizes[i]) FAIL("file %u: bad offset/size", i);
         if (ops && (ops[i] < OP_R90 || ops[i] > OP_TR)) FAIL("entry %u: unknown orientation op %d", i, ops[i]);
+        if (sizes && (!sizes[i].w || !sizes[i].h || sizes[i].w > (1u << 24) || sizes[i].h > (1u << 24)))
+            FAIL("entry %u: output size %ux%u is not in 1..2^24 on each side", i, sizes[i].w, sizes[i].h);
     }
     const uint8_t* din = (const uint8_t*)files;
     if (!files_on_device) { ENSURE(files, files_size); din = (const uint8_t*)ctx->files.p; }
@@ -1309,13 +1394,17 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     }
     // ---- every entry is checked before anything is decoded
     std::vector<DecImage> DI(n);
-    const bool use_sel = rects || ops;
+    const bool use_sel = rects || ops || sizes;
     std::vector<RegionSel> sel(use_sel ? n : 0);
     for (uint32_t i = 0; i < n; i++) {
-        if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, pixels_cap, DI[i])) return 1;
+        if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr,
+                         pixels_cap, DI[i])) return 1;
         if (use_sel) {
             sel[i].rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
             region_select(imgs[i].w, imgs[i].h, sel[i].rect, sel[i].g, sel[i].s, sel[i].cover);
+            // a 32-bit accumulator holds 2^21 + 255 * (sum of the weights) exactly for windows of up to 2^23 taps
+            if (sizes && ((sizes[i].w != sel[i].rect.w && sel[i].rect.w > (1u << 23)) || (sizes[i].h != sel[i].rect.h && sel[i].rect.h > (1u << 23))))
+                FAIL("entry %u: a crop side above 2^23 pixels cannot be resized", i);
         }
     }
     uint8_t* dpx = (uint8_t*)pixels;
@@ -1331,7 +1420,9 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
                                                          : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
         l2 |= mode == 2;
     }
-    auto out_bytes = [&](uint32_t i) { return (use_sel ? sel[i].rect.w * sel[i].rect.h : imgs[i].w * imgs[i].h) * (3 + imgs[i].A); };
+    auto out_bytes = [&](uint32_t i) {
+        return (sizes ? (uint64_t)sizes[i].w * sizes[i].h : use_sel ? sel[i].rect.w * sel[i].rect.h : imgs[i].w * imgs[i].h) * (3 + imgs[i].A);
+    };
     // level 2: above ~600 tiles the pair family wins, with the 16-symbol value streams warp-per-block while they all fit
     // (s16_lat_max_tiles); level 1: the warp-per-block family up to ~1300 tiles (measured at 125 / 250 / 500 frames, profiles/)
     const bool lat = l2 ? 17 * tiles_est <= (uint64_t)ctx->lat_max_blocks * 5 / 6 : 9 * tiles_est <= ctx->lat_max_blocks;
@@ -1365,7 +1456,8 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
                 snprintf(ctx->err, sizeof ctx->err, "host to device copy failed"); rc = 1; break;
             }
         }
-        rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr, m, din, dpx,
+        rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr,
+                          sizes ? sizes + i0 : nullptr, m, din, dpx,
                           (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
@@ -1400,7 +1492,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
 extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
                             const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
                             int pixels_on_device) {
-    return decode_call(ctx, imgs, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1409,7 +1501,7 @@ extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpng
                                    void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1418,7 +1510,16 @@ extern "C" int xpngb_decode_oriented(xpngb_ctx* ctx, const int* ops, xpngb_image
                                      const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!ops) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+                       pixels_on_device);
+}
+
+extern "C" int xpngb_decode_resized(xpngb_ctx* ctx, const int* ops, xpngb_image* imgs, const xpngb_rect* rects, const xpngb_size* sizes,
+                                    uint32_t n, const void* files, uint64_t files_size, int files_on_device, const uint64_t* file_offsets,
+                                    const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
+    if (!ctx) return 1;
+    if (!sizes) { ctx->err[0] = 0; FAIL("null argument"); }
+    return decode_call(ctx, imgs, rects, ops, sizes, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
