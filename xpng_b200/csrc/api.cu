@@ -1223,8 +1223,9 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
                 LAUNCH(k_dec_rows_rgba, ntiles, 32, 0, d_tiles, d_imgs, (const DecTile*)d_dt, (const uint32_t*)ctx->rowcnt.p, (RowInfo*)ctx->rows.p);
             }
             ctx->cur = f1;
-            const uint32_t lut12 = call_tiles <= ctx->root->v2_direct_max_tiles ? LUT_ONE_12 : LUT_TWO_12;
-            LAUNCH_HI(k_dec_rans_v2_lat, 9 * ntiles, 32, lat_smem(lut12), ra, lut12);
+            auto k_dec_rans_v2_lat_two = k_dec_rans_v2_lat;   // the two-level table's name in the profile report
+            if (call_tiles <= ctx->root->v2_direct_max_tiles) LAUNCH_HI(k_dec_rans_v2_lat, 9 * ntiles, 32, lat_smem(LUT_ONE_12), ra, LUT_ONE_12);
+            else LAUNCH_HI(k_dec_rans_v2_lat_two, 9 * ntiles, 32, lat_smem(LUT_TWO_12), ra, LUT_TWO_12);
         } else {
             PdWork& W = Wl[1];
             if (pd_lists(1, W)) return 1;
@@ -1256,9 +1257,10 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             RansV1LatArgs la{ d_tiles, d_imgs, d_dt, din, (uint8_t*)ctx->streams.p, ntiles, 0, 3, lut16, 0u, ~0u, d_err };
             auto k_dec_rans_v1_lat_values16 = k_dec_rans_v1_lat; auto k_dec_rans_v1_lat_values256 = k_dec_rans_v1_lat;
             auto k_dec_rans_v1_lat_grey = k_dec_rans_v1_lat; auto k_dec_rans_v1_lat_ctx = k_dec_rans_v1_lat;   // names for the profile report
-            auto k_dec_rans_v1_lat_ctx_short = k_dec_rans_v1_lat;
+            auto k_dec_rans_v1_lat_ctx_short = k_dec_rans_v1_lat; auto k_dec_rans_v1_lat_values16_two = k_dec_rans_v1_lat;
             FORK_SIDE(0); side_busy[0] = true;
-            LAUNCH_HI(k_dec_rans_v1_lat_values16, 3 * ntiles, 32, lat_smem(lut16), la);
+            if (direct) LAUNCH_HI(k_dec_rans_v1_lat_values16, 3 * ntiles, 32, lat_smem(lut16), la);
+            else LAUNCH_HI(k_dec_rans_v1_lat_values16_two, 3 * ntiles, 32, lat_smem(lut16), la);
             FORK_SIDE(1); side_busy[1] = true;
             la.j0 = 3; la.nj = 5; la.lut_bytes = LUT_TWO_14;
             LAUNCH_HI(k_dec_rans_v1_lat_values256, 5 * ntiles, 32, lat_smem(LUT_TWO_14), la);
