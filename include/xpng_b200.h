@@ -144,6 +144,44 @@ int xpngb_decode_resized(xpngb_ctx *ctx, const int *ops, xpngb_image *imgs, cons
                          const uint64_t *file_offsets, const uint64_t *file_sizes,
                          void *pixels, uint64_t pixels_cap, int pixels_on_device);
 
+/* ---- Tensor decode: each entry written as the normalised tensor a network takes, in the same call. */
+enum { XPNGB_DT_U8 = 0, XPNGB_DT_F32 = 1, XPNGB_DT_F16 = 2, XPNGB_DT_BF16 = 3 };
+enum { XPNGB_CHW = 0, XPNGB_HWC = 1 };
+enum { XPNGB_SCALE_DIV = 0, XPNGB_SCALE_MUL = 1 };   /* torchvision v1 to_tensor / v2 ToDtype(scale=True) */
+typedef struct xpngb_tensor {
+    uint32_t dtype, layout, scale;
+    uint32_t channels;          /* 3: RGB only (alpha dropped); 0: as stored, 3 + A */
+    float mean[4], std[4];      /* per output channel; only the first C are used */
+} xpngb_tensor;
+
+/* Entry i's pixels P_i are what xpngb_decode_resized writes for it (sizes == NULL: no resize, as xpngb_decode_oriented /
+ * xpngb_decode_region; rects == NULL: whole images; ops == NULL: no op).  They are written as a tensor of C channels:
+ * C = 3 when fmt->channels == 3 (alpha dropped, as PIL's convert("RGB")), else 3 + A.  H and W are the output's dimensions
+ * after the op.  For each byte b of channel c, every float operation in IEEE float32, round-to-nearest-even, each rounded
+ * on its own:
+ *   XPNGB_DT_U8   : b (scale, mean and std unused)
+ *   XPNGB_DT_F32  : v = b / 255.0f (XPNGB_SCALE_DIV) or v = b * (float)(1.0 / 255) (XPNGB_SCALE_MUL); y = (v - mean[c]) / std[c]
+ *   XPNGB_DT_F16, XPNGB_DT_BF16 : that float32 y rounded to nearest-even into the 16-bit type
+ *   layout        : XPNGB_CHW puts element (c, y, x) at c*H*W + y*W + x; XPNGB_HWC at (y*W + x)*C + c.
+ * DIV + F32 is torchvision's F.normalize(F.to_tensor(pil), mean, std); MUL + F32 is v2.Normalize(mean, std) after
+ * v2.ToDtype(torch.float32, scale=True); F16 / BF16 are those passed through .to(dtype); U8 + CHW is F.pil_to_tensor.
+ * mean 0, std 1 gives either pipeline without Normalize, bit for bit.
+ *   out     : entry i's C*H*W elements at out + imgs[i].offset (a multiple of 16).  A (N, 3, 224, 224) float32 batch uses
+ *             offset i * 602112.
+ *   imgs[i] : in/out exactly as for xpngb_decode (the file's w, h, A; mode out).
+ * Every check runs before anything is decoded, and xpngb_last_error names the entry or the field: every check of
+ * xpngb_decode_resized (without sizes: of xpngb_decode_oriented / xpngb_decode_region), fmt == NULL, an unknown dtype,
+ * layout or scale, channels other than 0 or 3, for a float dtype a std[c] that is zero or not finite or a mean[c] that is
+ * not finite for c < C (all 4 channels when channels == 0), and an output past out_cap.
+ * Every entry goes through a scratch window (stored level-7 entries are read straight from their files), and resized
+ * entries through a scratch copy of their resized pixels, before one launch per chunk writes the tensors.  Device output
+ * is the intended use: with host output a float32 tensor is 4 times the uint8 bytes over PCIe (float16 / bfloat16: 2). */
+int xpngb_decode_tensor(xpngb_ctx *ctx, const xpngb_tensor *fmt, const int *ops, xpngb_image *imgs,
+                        const xpngb_rect *rects, const xpngb_size *sizes, uint32_t n,
+                        const void *files, uint64_t files_size, int files_on_device,
+                        const uint64_t *file_offsets, const uint64_t *file_sizes,
+                        void *out, uint64_t out_cap, int out_on_device);
+
 /* Device time of the kernels of the last encode/decode call on this context, in milliseconds
  * (CUDA events on the context's stream; excludes host<->device copies). */
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);

@@ -33,6 +33,11 @@ class _Size(C.Structure):  # xpngb_size: output pixels of a resized decode
     _fields_ = [("w", C.c_uint32), ("h", C.c_uint32)]
 
 
+class _Tensor(C.Structure):  # xpngb_tensor: the format of a tensor decode (see tensor_format)
+    _fields_ = [("dtype", C.c_uint32), ("layout", C.c_uint32), ("scale", C.c_uint32), ("channels", C.c_uint32),
+                ("mean", C.c_float * 4), ("std", C.c_float * 4)]
+
+
 class _Xpng(C.Structure):  # xpng_t, xpng.h:10
     _fields_ = [("p", C.c_void_p), ("w", C.c_uint64), ("h", C.c_uint64), ("s", C.c_uint64), ("A", C.c_bool)]
 
@@ -74,6 +79,9 @@ def lib():
         L.xpngb_decode_resized.restype = C.c_int
         L.xpngb_decode_resized.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect), C.POINTER(_Size), u32, vp, u64,
                                            C.c_int, C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_decode_tensor.restype = C.c_int
+        L.xpngb_decode_tensor.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect), C.POINTER(_Size),
+                                          u32, vp, u64, C.c_int, C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
         L.xpngb_last_kernel_ms.restype = C.c_float; L.xpngb_last_kernel_ms.argtypes = [vp]
         L.xpngb_last_launches.restype = u32; L.xpngb_last_launches.argtypes = [vp]
         L.xpngb_stream.restype = vp; L.xpngb_stream.argtypes = [vp]
@@ -152,6 +160,37 @@ def sizes(whs):
 
 _sizes = sizes   # Codec.decode_resized's argument of the same name hides it
 
+DTYPES = {"uint8": 0, "float32": 1, "float16": 2, "bfloat16": 3}   # XPNGB_DT_*
+DTYPE_BYTES = {"uint8": 1, "float32": 4, "float16": 2, "bfloat16": 2}
+LAYOUTS = {"chw": 0, "hwc": 1}
+SCALES = {"div": 0, "mul": 1}   # torchvision v1 to_tensor (x / 255), v2 ToDtype(scale=True) (x * (1 / 255))
+
+
+def _dtype_name(dtype):
+    """torch.float32 or "float32" -> "float32"."""
+    name = dtype if isinstance(dtype, str) else str(dtype).removeprefix("torch.")
+    if name not in DTYPES:
+        raise ValueError(f"unsupported tensor dtype {dtype!r}: one of {sorted(DTYPES)}")
+    return name
+
+
+def tensor_format(dtype, layout="chw", scale="div", mean=(0, 0, 0, 0), std=(1, 1, 1, 1), drop_alpha=False):
+    """The xpngb_tensor of a tensor decode.  dtype: torch.uint8 / float32 / float16 / bfloat16 (or its name); layout "chw" or
+    "hwc"; scale "div" (torchvision's to_tensor) or "mul" (v2 ToDtype(scale=True)); mean and std per output channel (missing
+    channels get mean 0, std 1); drop_alpha: 3 channels for RGBA files too, as PIL's convert("RGB")."""
+    if layout not in LAYOUTS:
+        raise ValueError(f"unknown layout {layout!r}")
+    if scale not in SCALES:
+        raise ValueError(f"unknown scale {scale!r}")
+    mean, std = list(mean), list(std)
+    if len(mean) > 4 or len(std) > 4:
+        raise ValueError("at most 4 channels of mean and std")
+    f = _Tensor()
+    f.dtype, f.layout, f.scale, f.channels = DTYPES[_dtype_name(dtype)], LAYOUTS[layout], SCALES[scale], 3 if drop_alpha else 0
+    f.mean[:] = [float(v) for v in mean + [0.0] * (4 - len(mean))]
+    f.std[:] = [float(v) for v in std + [1.0] * (4 - len(std))]
+    return f
+
 
 def region_tiles(w, h, rect):
     """Tiles a region decode of rect = (x, y, w, h) inside a w x h coded image decodes, and their union (x, y, w, h):
@@ -166,6 +205,7 @@ class Codec:
 
     def __init__(self, device=0):
         self._h = C.c_void_p()
+        self.device = int(device)
         if lib().xpngb_create(C.byref(self._h), int(device)):
             raise RuntimeError("xpngb_create failed: no usable CUDA device (there is no CPU fallback)")
         # CUDA is initialised now: the queue count asked for in __init__.py has been read, children need not inherit it
@@ -258,6 +298,59 @@ class Codec:
         if lib().xpngb_decode_resized(self._h, ops_arr, descs, rect_arr, size_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev),
                                       offs, sizes, C.c_void_p(pix_ptr), pix_cap, int(pix_dev)):
             raise RuntimeError("xpngb_decode_resized: " + self._err())
+
+    def decode_tensor_raw(self, fmt, descs, ops_arr, rect_arr, size_arr, n, files_ptr, files_size, files_dev, offs, sizes, out_ptr,
+                          out_cap, out_dev):
+        """decode_resized_raw (size_arr None: no resize, as decode_oriented_raw) with entry i written as a tensor of format fmt
+        (see tensor_format()) at out_ptr + descs[i].offset: C * H * W elements, H and W after the op."""
+        if lib().xpngb_decode_tensor(self._h, C.byref(fmt), ops_arr, descs, rect_arr, size_arr, n, C.c_void_p(files_ptr), files_size,
+                                     int(files_dev), offs, sizes, C.c_void_p(out_ptr), out_cap, int(out_dev)):
+            raise RuntimeError("xpngb_decode_tensor: " + self._err())
+
+    def decode_tensor(self, files, sizes=None, boxes=None, ops=None, dtype=None, layout="chw", scale="div", mean=None, std=None,
+                      drop_alpha=False):
+        """list of .xpng byte strings -> one torch tensor on this codec's device, (N, C, H, W) for layout "chw" or (N, H, W, C)
+        for "hwc": each whole image, or rectangle boxes[i] = (x, y, w, h) of it, resized to sizes[i] = (w, h) as decode_resized
+        does (None: not resized), turned by ops[i] (None: no op), then scaled and normalised as torchvision does, bit for bit:
+        scale "div" is F.normalize(F.to_tensor(pil), mean, std), "mul" is v2.Normalize after v2.ToDtype(float32, scale=True);
+        float16 / bfloat16 are those results rounded by .to(dtype).  dtype: torch.float32 (default), float16, bfloat16 or
+        uint8 (the bytes themselves, as F.pil_to_tensor).  mean / std None: 0 and 1 (no Normalize).  C is 3 + A, or 3 with
+        drop_alpha.  Every entry must have the same output shape (ValueError otherwise); ragged batches use
+        decode_tensor_raw."""
+        import torch
+        n = len(files)
+        if n == 0:
+            raise ValueError("decode_tensor needs at least one file")
+        for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops)):
+            if arg is not None and len(arg) != n:
+                raise ValueError(f"one {name} per file")
+        dname = _dtype_name(torch.float32 if dtype is None else dtype)
+        fmt = tensor_format(dname, layout, scale, (0, 0, 0, 0) if mean is None else mean, (1, 1, 1, 1) if std is None else std, drop_alpha)
+        ra = None if boxes is None else rects(boxes)
+        sa = None if sizes is None else _sizes(sizes)
+        descs, foffs, fsizes, fb, off, _, _ = self._pack_files(files, ra, sa)
+        shapes = set()
+        for i, d in enumerate(descs):
+            w, h = (sa[i].w, sa[i].h) if sa is not None else (ra[i].w, ra[i].h) if ra is not None else (d.w, d.h)
+            if ops is not None and ops[i] in QUARTER_TURNS:
+                w, h = h, w
+            shapes.add((3 if drop_alpha else 3 + d.A, h, w))
+        if len(shapes) != 1:
+            raise ValueError(f"entries have different output shapes {sorted(shapes)}: use decode_tensor_raw for ragged batches")
+        c, h, w = shapes.pop()
+        per = c * h * w
+        stride = _align16(per * DTYPE_BYTES[dname]) // DTYPE_BYTES[dname]   # entry offsets are multiples of 16 bytes
+        for i in range(n):
+            descs[i].offset = i * stride * DTYPE_BYTES[dname]
+        dev = torch.device("cuda", self.device)
+        flat = torch.empty(n * stride, dtype=getattr(torch, dname), device=dev)
+        # the library writes on its own stream: memory fresh from the caching allocator may still be in use by queued work
+        torch.cuda.current_stream(dev).synchronize()
+        self.decode_tensor_raw(fmt, descs, None if ops is None else op_codes(ops), ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes,
+                               flat.data_ptr(), n * stride * DTYPE_BYTES[dname], 1)
+        out = flat.view(n, stride)[:, :per]
+        out = out.reshape(n, c, h, w) if layout == "chw" else out.reshape(n, h, w, c)
+        return out.contiguous()
 
     # ---------------------------------------------------------------- numpy convenience (host buffers)
     def encode(self, level, images):

@@ -32,6 +32,7 @@
 #include "orient.cuh"
 #include "region.cuh"
 #include "resize.cuh"
+#include "tensor.cuh"
 
 using namespace xpb;
 
@@ -73,7 +74,8 @@ struct xpngb_ctx {
         rows, edge, errflag, hdr, offs, m2a, m2b, tclass, tabs, ccnt, cbit, resv, oriented, odesc, pdw,
         region, crops,   // region decode: window of the selected tiles, crop descriptors
         orients,         // oriented decode: OrientDesc of the lane's chunk (odesc belongs to xpngb_transform / encode_oriented)
-        rdescs, rtab, rtmp;   // resized decode: ResizeDesc of the lane's chunk, windows and weights, the first pass's rows
+        rdescs, rtab, rtmp,   // resized decode: ResizeDesc of the lane's chunk, windows and weights, the first pass's rows
+        tdescs, tsrc;         // tensor decode: TensorDesc of the lane's chunk, the resized entries' pixels
     PinBuf pin_a, pin_b, pin_o;   // pin_o: orientation descriptors (their upload may still be in flight when an encode reuses pin_a)
 };
 
@@ -393,7 +395,7 @@ static void lane_free(xpngb_ctx* ctx) {
                       &ctx->plane, &ctx->nlseq, &ctx->rowcnt, &ctx->rowbits, &ctx->rows, &ctx->edge, &ctx->errflag, &ctx->hdr,
                       &ctx->offs, &ctx->m2a, &ctx->m2b, &ctx->tclass, &ctx->tabs, &ctx->ccnt, &ctx->cbit, &ctx->resv, &ctx->oriented,
                       &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops, &ctx->orients,
-                      &ctx->rdescs, &ctx->rtab, &ctx->rtmp };
+                      &ctx->rdescs, &ctx->rtab, &ctx->rtmp, &ctx->tdescs, &ctx->tsrc };
     for (DevBuf* b : all) if (b->p) cudaFree(b->p);
     if (ctx->pin_a.p) cudaFreeHost(ctx->pin_a.p);
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
@@ -959,12 +961,22 @@ static PdWork pdw_at(void* base, uint32_t cap) {
     return W;
 }
 
+// Bytes an entry writes at its offset: the whole image (img: w, h, A), the r->w x r->h crop or the sz->w x sz->h image, as
+// 3 + A bytes per pixel, or with a tensor format as C elements of its dtype.  The bounds check and the device-to-host copy
+// both take it from here.
+static uint64_t entry_out_bytes(const xpngb_image& img, const xpngb_rect* r, const xpngb_size* sz, const xpngb_tensor* fmt) {
+    const uint64_t px = sz ? (uint64_t)sz->w * sz->h : r ? r->w * r->h : img.w * img.h;   // at most 2^24 x 2^24: no overflow
+    if (!fmt) return px * (3 + img.A);
+    static const uint32_t elem_bytes[4] = { 1, 4, 2, 2 };   // XPNGB_DT_*
+    return px * (fmt->channels == 3 ? 3 : 3 + img.A) * elem_bytes[fmt->dtype];
+}
+
 // Header checks of file i (libxpng.c:969-976) and of where its pixels go: fills imgs[i] (w, h, A, mode) and D (file,
 // geometry, effective mode).  A region decode (r != nullptr) writes the r->w x r->h crop at imgs[i].offset instead of
-// the whole image, and a resized decode (sz != nullptr) an sz->w x sz->h image.  Runs for every entry of a call before
-// anything is launched.
+// the whole image, a resized decode (sz != nullptr) an sz->w x sz->h image, and a tensor decode (fmt != nullptr) that
+// as a tensor.  Runs for every entry of a call before anything is launched.
 static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint32_t* hdr, uint64_t file_off, uint64_t file_size,
-                        const xpngb_rect* r, const xpngb_size* sz, uint64_t pixels_cap, DecImage& D) {
+                        const xpngb_rect* r, const xpngb_size* sz, const xpngb_tensor* fmt, uint64_t pixels_cap, DecImage& D) {
     const uint64_t w = (hdr[0] & 0xFFFFFFu) + 1, h = (hdr[1] & 0xFFFFFFu) + 1;
     const uint32_t A = (hdr[1] >> 24) & 1, mode = hdr[0] >> 24, pxsz = 3 + A;
     if (!(mode == 1 || mode == 2 || mode == 7)) FAIL("file %u: unknown mode %u", i, mode);   // libxpng.c:972
@@ -975,7 +987,7 @@ static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint
     if (r && (r->x >= w || r->w > w - r->x || r->y >= h || r->h > h - r->y))
         FAIL("entry %u: rectangle (%llu, %llu) %llux%llu is not inside the %llux%llu image", i, (unsigned long long)r->x,
              (unsigned long long)r->y, (unsigned long long)r->w, (unsigned long long)r->h, (unsigned long long)w, (unsigned long long)h);
-    const uint64_t s = w * h * pxsz, out = sz ? (uint64_t)sz->w * sz->h * pxsz : r ? r->w * r->h * pxsz : s;   // at most 2^24 x 2^24 pixels: no overflow
+    const uint64_t s = w * h * pxsz, out = entry_out_bytes(img, r, sz, fmt);
     if (img.offset & 15) FAIL("file %u: pixel offset must be a multiple of 16", i);
     if (out > pixels_cap || img.offset > pixels_cap - out) FAIL("file %u: pixels exceed the output buffer", i);
     uint32_t m = mode;
@@ -1030,40 +1042,47 @@ static uint64_t resize_tmp_bytes(const RegionSel& R, const xpngb_size& z, uint32
 // are cropped straight out of their files.  ops (only with sel): an entry that is turned (turned()) always goes through a
 // window, or for a stored image straight out of its file, and one k_orient launch writes all of them.  sizes (only with
 // sel): a resized entry (resized()) also always goes through a window or its file, and is resampled and written through
-// its op by one launch of each resize kernel for the chunk.  Never waits for the device.
+// its op by one launch of each resize kernel for the chunk.  fmt (only with sel): every entry goes through a window or its
+// file, a resized one is resampled without its op into the lane's tsrc scratch, and one k_to_tensor launch writes every
+// entry's tensor through its op.  Never waits for the device.
 static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
-                        const xpngb_size* sizes, uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
+                        const xpngb_size* sizes, const xpngb_tensor* fmt, uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
     std::vector<CropDesc> crops;
     std::vector<OrientDesc> odescs;
     std::vector<ResizeDesc> rdescs;
-    uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0;
+    std::vector<TensorDesc> tdescs;
+    uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0, tctas = 0;
     bool any1 = false, any2 = false, any7 = false;
     for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
-    if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned or resized entry
-        uint64_t need = 0, tab = 0, tmp = 0;
+    // resized pixels of a tensor entry (16-byte aligned)
+    auto tsrc_bytes = [&](uint32_t i) -> uint64_t { return ((uint64_t)sizes[i].w * sizes[i].h * DI[i].pxsz + 15) & ~15ull; };
+    if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned, resized or tensor entry
+        uint64_t need = 0, tab = 0, tmp = 0, tsz = 0;
         for (uint32_t i = 0; i < n; i++) {
             const bool rs = resized(sizes, sel, i);
-            if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
+            if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs || fmt)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
             if (rs) { tab += resize_tab_bytes(sel[i], sizes[i]); tmp += resize_tmp_bytes(sel[i], sizes[i], DI[i].pxsz); }
+            if (rs && fmt) tsz += tsrc_bytes(i);
         }
         if (need) ENSURE(region, need);
         if (tab) ENSURE(rtab, tab);
         if (tmp) ENSURE(rtmp, tmp);
+        if (tsz) ENSURE(tsrc, tsz);
     }
     // resized entry i: its crop at src (rows `pitch` bytes apart) resampled into out through its op, each pass reading the
     // previous one's packed rows
     uint64_t tpos = 0, mpos = 0;
-    auto resize_desc = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out) -> int {
+    auto resize_desc = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out, uint32_t op) -> int {
         const xpngb_rect& r = sel[i].rect;
         const xpngb_size& z = sizes[i];
         ResizeDesc d{};
         d.coef = (uint64_t)ctx->rtab.p + tpos; tpos += resize_tab_bytes(sel[i], z);
         const uint64_t tmp = (uint64_t)ctx->rtmp.p + mpos; mpos += resize_tmp_bytes(sel[i], z, DI[i].pxsz);
         d.in_w = (uint32_t)r.w; d.in_h = (uint32_t)r.h; d.out_w = z.w; d.out_h = z.h;
-        d.pxsz = DI[i].pxsz; d.op = ops ? (uint32_t)ops[i] : (uint32_t)OP_TL;
+        d.pxsz = DI[i].pxsz; d.op = op;
         d.kx = resize_ksize(r.w, z.w); d.ky = resize_ksize(r.h, z.h);
         if (!d.kx) d.v = ResizePass{ src, pitch, (uint64_t)out, z.w, 1 };
         else if (!d.ky) d.h = ResizePass{ src, pitch, (uint64_t)out, z.h, 1 };
@@ -1083,6 +1102,35 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         rdescs.push_back(d);
         return 0;
     };
+    // tensor entry i: its w x h pixels at src (rows `pitch` bytes apart) written as its tensor at out through its op
+    auto tensor_desc = [&](uint32_t i, uint64_t src, uint64_t pitch, uint64_t w, uint64_t h, uint8_t* out) -> int {
+        TensorDesc d{};
+        d.src = src; d.src_pitch = pitch; d.dst = (uint64_t)out; d.w = (uint32_t)w; d.h = (uint32_t)h;
+        d.pxsz = DI[i].pxsz; d.c = fmt->channels == 3 ? 3 : DI[i].pxsz; d.op = ops ? (uint32_t)ops[i] : (uint32_t)OP_TL;
+        d.tiles_x = (d.w + TT - 1) / TT; d.first_cta = (uint32_t)tctas;
+        tctas += (uint64_t)d.tiles_x * ((d.h + TT - 1) / TT);
+        if (tctas > 0x7FFFFFFFull) FAIL("too many pixels for one tensor launch");
+        tdescs.push_back(d);
+        return 0;
+    };
+    // entry i of a region call: its rectangle at src (rows `pitch` bytes apart) cropped, turned, resized or made a tensor
+    uint64_t spos = 0;
+    auto region_out = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out) -> int {
+        const xpngb_rect& r = sel[i].rect;
+        const uint32_t pxsz = DI[i].pxsz;
+        if (fmt && resized(sizes, sel, i)) {   // resampled without the op; k_to_tensor applies it
+            uint8_t* t = (uint8_t*)ctx->tsrc.p + spos;
+            spos += tsrc_bytes(i);
+            if (resize_desc(i, src, pitch, t, OP_TL)) return 1;
+            return tensor_desc(i, (uint64_t)t, (uint64_t)sizes[i].w * pxsz, sizes[i].w, sizes[i].h, out);
+        }
+        if (fmt) return tensor_desc(i, src, pitch, r.w, r.h, out);
+        if (resized(sizes, sel, i)) return resize_desc(i, src, pitch, out, ops ? (uint32_t)ops[i] : (uint32_t)OP_TL);
+        if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, pitch, (uint32_t)(r.w * pxsz), (uint32_t)r.h });
+        else if (!orient_desc(odescs.emplace_back(), src, pitch, (uint64_t)out, r.w, r.h, pxsz, ops[i], &octas))
+            FAIL("too many pixels for one orientation launch");
+        return 0;
+    };
     uint64_t wpos = 0;
     for (uint32_t i = 0; i < n; i++) {
         DecImage& D = DI[i];
@@ -1097,23 +1145,16 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             ImageDesc I{}; I.tile0 = (uint32_t)P.tiles.size(); I.mode = 7; I.w = D.w; I.h = D.h; I.pxsz = D.pxsz;
             P.imgs.push_back(I);
             const uint64_t src = (uint64_t)(din + D.file_off + 8 + (r.y * D.w + r.x) * D.pxsz);   // any byte alignment
-            if (resized(sizes, sel, i)) { if (resize_desc(i, src, (uint64_t)D.w * D.pxsz, out)) return 1; }
-            else if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, (uint64_t)D.w * D.pxsz, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
-            else if (!orient_desc(odescs.emplace_back(), src, (uint64_t)D.w * D.pxsz, (uint64_t)out, r.w, r.h, D.pxsz, ops[i], &octas))
-                FAIL("too many pixels for one orientation launch");
+            if (region_out(i, src, (uint64_t)D.w * D.pxsz, out)) return 1;
         } else {
             const RegionSel& R = sel[i];
             const xpngb_rect &r = R.rect, &c = R.cover;
-            const bool rs = resized(sizes, sel, i);
-            if (whole_tiles(R) && !turned(ops, i) && !rs) plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
-            else {   // a turned or resized rectangle cannot be decoded in place, even when it is made of whole tiles
+            if (whole_tiles(R) && !turned(ops, i) && !resized(sizes, sel, i) && !fmt)
+                plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
+            else {   // a turned, resized or tensor rectangle cannot be decoded in place, even when it is made of whole tiles
                 const uint64_t pitch = window_pitch(R, D.pxsz), win = (uint64_t)ctx->region.p + wpos;
                 plan_image(P, R.g, R.s, win, pitch, c.x, c.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
-                const uint64_t src = win + (r.y - c.y) * pitch + (r.x - c.x) * D.pxsz;
-                if (rs) { if (resize_desc(i, src, pitch, out)) return 1; }
-                else if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, pitch, (uint32_t)(r.w * D.pxsz), (uint32_t)r.h });
-                else if (!orient_desc(odescs.emplace_back(), src, pitch, (uint64_t)out, r.w, r.h, D.pxsz, ops[i], &octas))
-                    FAIL("too many pixels for one orientation launch");
+                if (region_out(i, win + (r.y - c.y) * pitch + (r.x - c.x) * D.pxsz, pitch, out)) return 1;
                 wpos += c.h * pitch;
             }
             D.gcols = (uint32_t)R.g.nw; D.r0 = (uint32_t)R.s.r0; D.c0 = (uint32_t)R.s.c0;
@@ -1125,10 +1166,10 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     const uint32_t ntiles = (uint32_t)P.tiles.size();
     if (upload_plan(ctx, P)) return 1;
     ENSURE(dimgs, n * sizeof(DecImage)); ENSURE(dtiles, ntiles * sizeof(DecTile)); ENSURE(errflag, 4);
-    // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop, orientation and resize descriptors
+    // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop, orientation, resize and tensor descriptors
     const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64, pin_orients = pin_crops + crops.size() * sizeof(CropDesc);
-    const size_t pin_resize = pin_orients + odescs.size() * sizeof(OrientDesc);
-    if (ensure_pin(ctx, ctx->pin_b, pin_resize + rdescs.size() * sizeof(ResizeDesc))) return 1;
+    const size_t pin_resize = pin_orients + odescs.size() * sizeof(OrientDesc), pin_tensor = pin_resize + rdescs.size() * sizeof(ResizeDesc);
+    if (ensure_pin(ctx, ctx->pin_b, pin_tensor + tdescs.size() * sizeof(TensorDesc))) return 1;
     memcpy(ctx->pin_b.p, DI.data(), n * sizeof(DecImage));
     CK(cudaMemcpyAsync(ctx->dimgs.p, ctx->pin_b.p, n * sizeof(DecImage), cudaMemcpyHostToDevice, ctx->stream));
     if (any7 && !sel) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
@@ -1153,6 +1194,12 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         ENSURE(rdescs, nb);
         memcpy((uint8_t*)ctx->pin_b.p + pin_resize, rdescs.data(), nb);
         CK(cudaMemcpyAsync(ctx->rdescs.p, (uint8_t*)ctx->pin_b.p + pin_resize, nb, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (!tdescs.empty()) {
+        const size_t nb = tdescs.size() * sizeof(TensorDesc);
+        ENSURE(tdescs, nb);
+        memcpy((uint8_t*)ctx->pin_b.p + pin_tensor, tdescs.data(), nb);
+        CK(cudaMemcpyAsync(ctx->tdescs.p, (uint8_t*)ctx->pin_b.p + pin_tensor, nb, cudaMemcpyHostToDevice, ctx->stream));
     }
     CK(cudaMemsetAsync(ctx->errflag.p, 0, 4, ctx->stream));
     CK(cudaMemsetAsync(ctx->dtiles.p, 0, ntiles * sizeof(DecTile), ctx->stream));
@@ -1358,14 +1405,17 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         if (rh) LAUNCH(k_resize_h, (unsigned)rh, RH_X, 0, d_rd, nr);
         if (rv) LAUNCH(k_resize_v, (unsigned)rv, RV_X, 0, d_rd, nr, vfirst ? 2u : 3u);
     }
+    if (!tdescs.empty()) LAUNCH(k_to_tensor, (unsigned)tctas, 256, 0, (const TensorDesc*)ctx->tdescs.p, (uint32_t)tdescs.size(), *fmt);
     // the error flag travels to pinned memory behind the DecImage table
     CK(cudaMemcpyAsync((uint8_t*)ctx->pin_b.p + n * (sizeof(DecImage) + 8), d_err, 4, cudaMemcpyDeviceToHost, ctx->stream));
     return 0;
 }
 
-// xpngb_decode (rects == nullptr), xpngb_decode_region and, with ops, xpngb_decode_oriented.  An oriented call always
-// selects tiles per entry: without rects every entry's rectangle is its whole image.
-static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, const xpngb_size* sizes, uint32_t n, const void* files,
+// xpngb_decode (rects == nullptr), xpngb_decode_region and, with ops, xpngb_decode_oriented; with sizes
+// xpngb_decode_resized, with fmt xpngb_decode_tensor.  An oriented, resized or tensor call always selects tiles per entry:
+// without rects every entry's rectangle is its whole image.
+static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, const xpngb_size* sizes,
+                       const xpngb_tensor* fmt, uint32_t n, const void* files,
                        uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
                        uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
@@ -1396,11 +1446,11 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     }
     // ---- every entry is checked before anything is decoded
     std::vector<DecImage> DI(n);
-    const bool use_sel = rects || ops || sizes;
+    const bool use_sel = rects || ops || sizes || fmt;
     std::vector<RegionSel> sel(use_sel ? n : 0);
     for (uint32_t i = 0; i < n; i++) {
         if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr,
-                         pixels_cap, DI[i])) return 1;
+                         fmt, pixels_cap, DI[i])) return 1;
         if (use_sel) {
             sel[i].rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
             region_select(imgs[i].w, imgs[i].h, sel[i].rect, sel[i].g, sel[i].s, sel[i].cover);
@@ -1422,9 +1472,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
                                                          : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
         l2 |= mode == 2;
     }
-    auto out_bytes = [&](uint32_t i) {
-        return (sizes ? (uint64_t)sizes[i].w * sizes[i].h : use_sel ? sel[i].rect.w * sel[i].rect.h : imgs[i].w * imgs[i].h) * (3 + imgs[i].A);
-    };
+    auto out_bytes = [&](uint32_t i) { return entry_out_bytes(imgs[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr, fmt); };
     // level 2: above ~600 tiles the pair family wins, with the 16-symbol value streams warp-per-block while they all fit
     // (s16_lat_max_tiles); level 1: the warp-per-block family up to ~1300 tiles (measured at 125 / 250 / 500 frames, profiles/)
     const bool lat = l2 ? 17 * tiles_est <= (uint64_t)ctx->lat_max_blocks * 5 / 6 : 9 * tiles_est <= ctx->lat_max_blocks;
@@ -1459,7 +1507,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             }
         }
         rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr,
-                          sizes ? sizes + i0 : nullptr, m, din, dpx,
+                          sizes ? sizes + i0 : nullptr, fmt, m, din, dpx,
                           (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
@@ -1494,7 +1542,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
 extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
                             const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
                             int pixels_on_device) {
-    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1503,7 +1551,7 @@ extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpng
                                    void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1512,7 +1560,7 @@ extern "C" int xpngb_decode_oriented(xpngb_ctx* ctx, const int* ops, xpngb_image
                                      const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!ops) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1521,8 +1569,34 @@ extern "C" int xpngb_decode_resized(xpngb_ctx* ctx, const int* ops, xpngb_image*
                                     const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!sizes) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, sizes, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
+}
+
+// The format of a tensor decode, checked before anything else.  A float dtype normalises every channel it may write: the
+// first 3, or all 4 when alpha is kept (a batch may hold RGBA files).
+static int tensor_check(xpngb_ctx* ctx, const xpngb_tensor* f) {
+    if (!f) FAIL("null argument (fmt)");
+    if (f->dtype > XPNGB_DT_BF16) FAIL("tensor format: unknown dtype %u", f->dtype);
+    if (f->layout > XPNGB_HWC) FAIL("tensor format: unknown layout %u", f->layout);
+    if (f->scale > XPNGB_SCALE_MUL) FAIL("tensor format: unknown scale %u", f->scale);
+    if (f->channels != 0 && f->channels != 3) FAIL("tensor format: channels %u is neither 0 (as stored) nor 3 (RGB)", f->channels);
+    if (f->dtype != XPNGB_DT_U8)
+        for (uint32_t c = 0; c < (f->channels == 3 ? 3u : 4u); c++) {
+            if (!isfinite(f->mean[c])) FAIL("tensor format: mean[%u] is not finite", c);
+            if (!isfinite(f->std[c]) || f->std[c] == 0.f) FAIL("tensor format: std[%u] is zero or not finite", c);
+        }
+    return 0;
+}
+
+extern "C" int xpngb_decode_tensor(xpngb_ctx* ctx, const xpngb_tensor* fmt, const int* ops, xpngb_image* imgs, const xpngb_rect* rects,
+                                   const xpngb_size* sizes, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
+                                   const uint64_t* file_offsets, const uint64_t* file_sizes, void* out, uint64_t out_cap, int out_on_device) {
+    if (!ctx) return 1;
+    ctx->err[0] = 0;
+    if (tensor_check(ctx, fmt)) return 1;
+    return decode_call(ctx, imgs, rects, ops, sizes, fmt, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
+                       out_on_device);
 }
 
 // ------------------------------------------------------------------------------------------------
