@@ -182,6 +182,32 @@ int xpngb_decode_tensor(xpngb_ctx *ctx, const xpngb_tensor *fmt, const int *ops,
                         const uint64_t *file_offsets, const uint64_t *file_sizes,
                         void *out, uint64_t out_cap, int out_on_device);
 
+/* ---- Resampled decode: Pillow's five convolution filters per entry, and a window of the resized image.
+ * Entry i is orient(ops[i], window_i(resize_f(crop_i, sizes[i]))): crop_i is rects[i] (NULL: whole images); resize_f is
+ * Pillow's Image.resize(sizes[i], filters[i]) of the crop, byte-identical (Resample.c, 8-bit path), every channel on its
+ * own (alpha not premultiplied); window_i keeps windows[i] = (x, y, w, h) in the coordinates of the sizes[i] image (NULL:
+ * all of it); the op comes last.  fmt == NULL writes uint8 pixels as xpngb_decode_resized, else a tensor as
+ * xpngb_decode_tensor.  filters == NULL and windows == NULL give exactly what xpngb_decode_resized / xpngb_decode_tensor
+ * give.  An entry writes windows[i].w * windows[i].h pixels (or tensor elements).  Only the tiles under the support of its
+ * window are decoded.  Every check of those calls runs before anything is launched, plus, naming the entry: an unknown
+ * filter (NEAREST included: Pillow does not resize with it by convolution), sizes == NULL, an empty window or one not
+ * inside sizes[i], and a resampled crop side above the filter's accumulator limit (2^23 box, bilinear and hamming; 2^22
+ * bicubic; 2^21 lanczos). */
+enum { XPNGB_LANCZOS = 1, XPNGB_BILINEAR = 2, XPNGB_BICUBIC = 3, XPNGB_BOX = 4, XPNGB_HAMMING = 5 };   /* PIL.Image.Resampling */
+int xpngb_decode_resampled(xpngb_ctx *ctx, const xpngb_tensor *fmt /* NULL: uint8 pixels, as xpngb_decode_resized */,
+                           const int *filters /* NULL: all bilinear */, const int *ops, xpngb_image *imgs,
+                           const xpngb_rect *rects, const xpngb_size *sizes /* required */,
+                           const xpngb_rect *windows /* NULL: whole resized image */, uint32_t n,
+                           const void *files, uint64_t files_size, int files_on_device,
+                           const uint64_t *file_offsets, const uint64_t *file_sizes,
+                           void *out, uint64_t out_cap, int out_on_device);
+/* Diagnostics of the weight tables: Pillow's number of weights per output coordinate of an in -> out axis (0 for in == out
+ * or an unknown filter), and the device's tables for output coordinates first .. first + count - 1: xmin_n gets 2 * count
+ * int32 (xmin, n), k count * ksize int32 22-bit weights, zero past each window. */
+uint32_t xpngb_resize_ksize(int filter, uint32_t in, uint32_t out);
+int xpngb_resize_coeffs(xpngb_ctx *ctx, int filter, uint32_t in, uint32_t out, uint32_t first, uint32_t count,
+                        int32_t *xmin_n, int32_t *k);
+
 /* Device time of the kernels of the last encode/decode call on this context, in milliseconds
  * (CUDA events on the context's stream; excludes host<->device copies). */
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);

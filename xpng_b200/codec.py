@@ -82,6 +82,13 @@ def lib():
         L.xpngb_decode_tensor.restype = C.c_int
         L.xpngb_decode_tensor.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect), C.POINTER(_Size),
                                           u32, vp, u64, C.c_int, C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_decode_resampled.restype = C.c_int
+        L.xpngb_decode_resampled.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_Image),
+                                             C.POINTER(_Rect), C.POINTER(_Size), C.POINTER(_Rect), u32, vp, u64, C.c_int, C.POINTER(u64),
+                                             C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_resize_ksize.restype = u32; L.xpngb_resize_ksize.argtypes = [C.c_int, u32, u32]
+        L.xpngb_resize_coeffs.restype = C.c_int
+        L.xpngb_resize_coeffs.argtypes = [vp, C.c_int, u32, u32, u32, u32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.xpngb_last_kernel_ms.restype = C.c_float; L.xpngb_last_kernel_ms.argtypes = [vp]
         L.xpngb_last_launches.restype = u32; L.xpngb_last_launches.argtypes = [vp]
         L.xpngb_stream.restype = vp; L.xpngb_stream.argtypes = [vp]
@@ -159,6 +166,58 @@ def sizes(whs):
 
 
 _sizes = sizes   # Codec.decode_resized's argument of the same name hides it
+
+FILTERS = {"lanczos": 1, "bilinear": 2, "bicubic": 3, "box": 4, "hamming": 5}   # XPNGB_LANCZOS .. = PIL.Image.Resampling
+
+
+def filter_code(f):
+    """A resampling filter as Pillow numbers it: a name ("bicubic"), a PIL.Image.Resampling value or a torchvision
+    InterpolationMode (whose .value is the name).  NEAREST is refused: Pillow does not resize with it by convolution."""
+    if not isinstance(f, int):
+        name = getattr(f, "value", f)
+        if isinstance(name, str) and name.lower() in FILTERS:
+            return FILTERS[name.lower()]
+        raise ValueError(f"unknown resampling filter {f!r}: one of {sorted(FILTERS)}")
+    if int(f) not in FILTERS.values():
+        raise ValueError(f"unknown resampling filter {f!r}: one of {sorted(FILTERS)} (PIL.Image.Resampling numbers)")
+    return int(f)
+
+
+def filter_codes(filters, n):
+    """None, one filter for all n entries, or a list of n -> ctypes array of filter codes (None for None)."""
+    if filters is None:
+        return None
+    if isinstance(filters, (list, tuple)):
+        if len(filters) != n:
+            raise ValueError("one filter per file")
+        return (C.c_int * n)(*(filter_code(f) for f in filters))
+    return (C.c_int * n)(*([filter_code(filters)] * n))
+
+
+def resize_center_crop(w, h, resize, crop, max_size=None):
+    """torchvision's Resize(resize, max_size=max_size) followed by CenterCrop(crop) of a w x h PIL image, as the codec's
+    resized size (W, H) and window (x, y, cw, ch).  resize: an int (the shorter side; the longer one is
+    int(resize * long / short), capped by max_size) or torchvision's (h, w) sequence.  crop: an int or (h, w).  A crop larger
+    than the resized image raises ValueError (torchvision pads it)."""
+    if isinstance(resize, int) or len(resize) == 1:
+        r = resize if isinstance(resize, int) else resize[0]
+        short, long = (w, h) if w <= h else (h, w)
+        new_short, new_long = r, int(r * long / short)
+        if max_size is not None:
+            if max_size <= r:
+                raise ValueError(f"max_size = {max_size} must be strictly greater than the requested size {r}")
+            if new_long > max_size:
+                new_short, new_long = int(max_size * new_short / new_long), max_size
+        W, H = (new_short, new_long) if w <= h else (new_long, new_short)
+    else:
+        if max_size is not None:
+            raise ValueError("max_size applies only to an int resize")
+        H, W = resize
+    ch, cw = (crop, crop) if isinstance(crop, int) else (crop[0], crop[0]) if len(crop) == 1 else crop
+    if cw > W or ch > H:
+        raise ValueError(f"crop {cw}x{ch} is larger than the resized {W}x{H} image (torchvision would pad it)")
+    return (W, H), (int(round((W - cw) / 2.0)), int(round((H - ch) / 2.0)), cw, ch)
+
 
 DTYPES = {"uint8": 0, "float32": 1, "float16": 2, "bfloat16": 3}   # XPNGB_DT_*
 DTYPE_BYTES = {"uint8": 1, "float32": 4, "float16": 2, "bfloat16": 2}
@@ -307,31 +366,59 @@ class Codec:
                                      int(files_dev), offs, sizes, C.c_void_p(out_ptr), out_cap, int(out_dev)):
             raise RuntimeError("xpngb_decode_tensor: " + self._err())
 
+    def decode_resampled_raw(self, fmt, descs, filt_arr, ops_arr, rect_arr, size_arr, win_arr, n, files_ptr, files_size, files_dev,
+                             offs, sizes, out_ptr, out_cap, out_dev):
+        """decode_resized_raw (fmt None) or decode_tensor_raw with entry i resampled by filt_arr[i] (see filter_codes(); None:
+        bilinear) and only window win_arr[i] (see rects(), in size_arr[i]'s coordinates; None: all of it) written, as
+        win_arr[i].h rows of win_arr[i].w pixels (or tensor elements), swapped for the quarter turns."""
+        if lib().xpngb_decode_resampled(self._h, None if fmt is None else C.byref(fmt), filt_arr, ops_arr, descs, rect_arr, size_arr,
+                                        win_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev), offs, sizes, C.c_void_p(out_ptr),
+                                        out_cap, int(out_dev)):
+            raise RuntimeError("xpngb_decode_resampled: " + self._err())
+
+    def resize_coeffs(self, filt, inn, out, first=0, count=None):
+        """The device's weight tables of an inn -> out axis for output coordinates first .. first + count - 1: (xmin, n) as
+        an (count, 2) int32 array and the (count, ksize) int32 weights, zero past each window."""
+        f = filter_code(filt)
+        count = out - first if count is None else count
+        ksize = int(lib().xpngb_resize_ksize(f, inn, out))
+        xn = np.zeros((max(count, 1), 2), np.int32)
+        k = np.zeros((max(count, 1), max(ksize, 1)), np.int32)
+        if lib().xpngb_resize_coeffs(self._h, f, inn, out, first, count, xn.ctypes.data_as(C.POINTER(C.c_int32)),
+                                     k.ctypes.data_as(C.POINTER(C.c_int32))):
+            raise RuntimeError("xpngb_resize_coeffs: " + self._err())
+        return xn[:count], k[:count, :ksize]
+
     def decode_tensor(self, files, sizes=None, boxes=None, ops=None, dtype=None, layout="chw", scale="div", mean=None, std=None,
-                      drop_alpha=False):
+                      drop_alpha=False, filters=None, windows=None):
         """list of .xpng byte strings -> one torch tensor on this codec's device, (N, C, H, W) for layout "chw" or (N, H, W, C)
         for "hwc": each whole image, or rectangle boxes[i] = (x, y, w, h) of it, resized to sizes[i] = (w, h) as decode_resized
         does (None: not resized), turned by ops[i] (None: no op), then scaled and normalised as torchvision does, bit for bit:
         scale "div" is F.normalize(F.to_tensor(pil), mean, std), "mul" is v2.Normalize after v2.ToDtype(float32, scale=True);
         float16 / bfloat16 are those results rounded by .to(dtype).  dtype: torch.float32 (default), float16, bfloat16 or
         uint8 (the bytes themselves, as F.pil_to_tensor).  mean / std None: 0 and 1 (no Normalize).  C is 3 + A, or 3 with
-        drop_alpha.  Every entry must have the same output shape (ValueError otherwise); ragged batches use
-        decode_tensor_raw."""
+        drop_alpha.  filters and windows (only with sizes) as decode_resized: torchvision's Resize(256) + CenterCrop(224) of
+        each image is sizes[i], windows[i] = resize_center_crop(w, h, 256, 224).  Every entry must have the same output shape
+        (ValueError otherwise); ragged batches use decode_tensor_raw or decode_resampled_raw."""
         import torch
         n = len(files)
         if n == 0:
             raise ValueError("decode_tensor needs at least one file")
-        for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops)):
+        for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops), ("window", windows)):
             if arg is not None and len(arg) != n:
                 raise ValueError(f"one {name} per file")
+        if sizes is None and (filters is not None or windows is not None):
+            raise ValueError("filters and windows need sizes")
         dname = _dtype_name(torch.float32 if dtype is None else dtype)
         fmt = tensor_format(dname, layout, scale, (0, 0, 0, 0) if mean is None else mean, (1, 1, 1, 1) if std is None else std, drop_alpha)
         ra = None if boxes is None else rects(boxes)
         sa = None if sizes is None else _sizes(sizes)
+        wa = None if windows is None else rects(windows)
+        fa = filter_codes(filters, n)
         descs, foffs, fsizes, fb, off, _, _ = self._pack_files(files, ra, sa)
         shapes = set()
         for i, d in enumerate(descs):
-            w, h = (sa[i].w, sa[i].h) if sa is not None else (ra[i].w, ra[i].h) if ra is not None else (d.w, d.h)
+            w, h = (wa[i].w, wa[i].h) if wa is not None else (sa[i].w, sa[i].h) if sa is not None else (ra[i].w, ra[i].h) if ra is not None else (d.w, d.h)
             if ops is not None and ops[i] in QUARTER_TURNS:
                 w, h = h, w
             shapes.add((3 if drop_alpha else 3 + d.A, h, w))
@@ -346,8 +433,13 @@ class Codec:
         flat = torch.empty(n * stride, dtype=getattr(torch, dname), device=dev)
         # the library writes on its own stream: memory fresh from the caching allocator may still be in use by queued work
         torch.cuda.current_stream(dev).synchronize()
-        self.decode_tensor_raw(fmt, descs, None if ops is None else op_codes(ops), ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes,
-                               flat.data_ptr(), n * stride * DTYPE_BYTES[dname], 1)
+        oa = None if ops is None else op_codes(ops)
+        if fa is None and wa is None:
+            self.decode_tensor_raw(fmt, descs, oa, ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes, flat.data_ptr(),
+                                   n * stride * DTYPE_BYTES[dname], 1)
+        else:
+            self.decode_resampled_raw(fmt, descs, fa, oa, ra, sa, wa, n, fb.ctypes.data, off, 0, foffs, fsizes, flat.data_ptr(),
+                                      n * stride * DTYPE_BYTES[dname], 1)
         out = flat.view(n, stride)[:, :per]
         out = out.reshape(n, c, h, w) if layout == "chw" else out.reshape(n, h, w, c)
         return out.contiguous()
@@ -365,8 +457,9 @@ class Codec:
         offs, sizes = self.encode_raw(level, descs, len(images), buf.ctypes.data, total, 0, out.ctypes.data, cap, 0)
         return [out[offs[i]: offs[i] + sizes[i]].tobytes() for i in range(len(images))]
 
-    def _pack_files(self, files, ra=None, sa=None):
-        """Files packed at 16-byte offsets and a host output buffer: one whole image, crop ra[i] or size sa[i] per entry."""
+    def _pack_files(self, files, ra=None, sa=None, wa=None):
+        """Files packed at 16-byte offsets and a host output buffer: one whole image, crop ra[i], size sa[i] or window wa[i]
+        per entry."""
         n = len(files)
         descs = (_Image * n)()
         foffs, fsizes = (C.c_uint64 * n)(), (C.c_uint64 * n)()
@@ -378,7 +471,10 @@ class Codec:
             foffs[i], fsizes[i] = off, len(f)
             off = _align16(off + len(f))
             descs[i].offset = poff
-            if sa is not None:
+            if wa is not None:
+                if 0 < wa[i].w <= 1 << 24 and 0 < wa[i].h <= 1 << 24:   # other windows are refused by the library, naming the entry
+                    poff = _align16(poff + wa[i].w * wa[i].h * (3 + descs[i].A))
+            elif sa is not None:
                 if 0 < sa[i].w <= 1 << 24 and 0 < sa[i].h <= 1 << 24:   # other sizes are refused by the library, naming the entry
                     poff = _align16(poff + sa[i].w * sa[i].h * (3 + descs[i].A))
             elif ra is None:
@@ -432,11 +528,14 @@ class Codec:
             self.decode_oriented_raw(descs, op_codes(ops), ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         return self._unpack(px, descs, [(r.w, r.h) for r in ra], ops)
 
-    def decode_resized(self, files, sizes, boxes=None, ops=None):
+    def decode_resized(self, files, sizes, boxes=None, ops=None, filters=None, windows=None):
         """list of .xpng byte strings and one (w, h) output size per file -> list of (h, w, 3|4) uint8 arrays: each whole image,
-        or rectangle boxes[i] = (x, y, w, h) of it, resampled as Pillow's Image.resize((w, h), Image.BILINEAR) does, every
-        channel on its own (alpha is not premultiplied).  ops: one OPS name per entry, applied after the resize; 'r90' and
-        'r270' entries come back as (w, h, 3|4).  An entry whose size equals its crop is the crop itself."""
+        or rectangle boxes[i] = (x, y, w, h) of it, resampled as Pillow's Image.resize((w, h), filter) does, every channel on
+        its own (alpha is not premultiplied).  filters: None (bilinear), one filter for all entries or one per entry, each a
+        name ("bicubic", ...), a PIL.Image.Resampling value or a torchvision InterpolationMode.  windows: one (x, y, w, h) per
+        entry in the resized image's coordinates, the part of it that is returned (None: all of it).  ops: one OPS name per
+        entry, applied last; 'r90' and 'r270' entries come back as (w, h, 3|4).  An entry whose size equals its crop is the
+        crop itself."""
         n = len(files)
         if len(sizes) != n:
             raise ValueError("one size per file")
@@ -444,12 +543,19 @@ class Codec:
             raise ValueError("one rectangle per file")
         if ops is not None and len(ops) != n:
             raise ValueError("one op per file")
+        if windows is not None and len(windows) != n:
+            raise ValueError("one window per file")
         ra = None if boxes is None else rects(boxes)
         sa = _sizes(sizes)
-        descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files, ra, sa)
-        self.decode_resized_raw(descs, None if ops is None else op_codes(ops), ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes,
-                                px.ctypes.data, poff, 0)
-        return self._unpack(px, descs, [(z.w, z.h) for z in sa], ops)
+        wa = None if windows is None else rects(windows)
+        fa = filter_codes(filters, n)
+        oa = None if ops is None else op_codes(ops)
+        descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files, ra, sa, wa)
+        if fa is None and wa is None:
+            self.decode_resized_raw(descs, oa, ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        else:
+            self.decode_resampled_raw(None, descs, fa, oa, ra, sa, wa, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        return self._unpack(px, descs, [(z.w, z.h) for z in (sa if wa is None else wa)], ops)
 
     # ---------------------------------------------------------------- traversal-order operations (Mirroring_and_Rotating/tool.c)
     def _pack(self, images):

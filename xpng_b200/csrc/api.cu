@@ -961,11 +961,13 @@ static PdWork pdw_at(void* base, uint32_t cap) {
     return W;
 }
 
-// Bytes an entry writes at its offset: the whole image (img: w, h, A), the r->w x r->h crop or the sz->w x sz->h image, as
-// 3 + A bytes per pixel, or with a tensor format as C elements of its dtype.  The bounds check and the device-to-host copy
-// both take it from here.
-static uint64_t entry_out_bytes(const xpngb_image& img, const xpngb_rect* r, const xpngb_size* sz, const xpngb_tensor* fmt) {
-    const uint64_t px = sz ? (uint64_t)sz->w * sz->h : r ? r->w * r->h : img.w * img.h;   // at most 2^24 x 2^24: no overflow
+// Bytes an entry writes at its offset: the whole image (img: w, h, A), the r->w x r->h crop, the sz->w x sz->h image or
+// its win->w x win->h window, as 3 + A bytes per pixel, or with a tensor format as C elements of its dtype.  The bounds
+// check and the device-to-host copy both take it from here.
+static uint64_t entry_out_bytes(const xpngb_image& img, const xpngb_rect* r, const xpngb_size* sz, const xpngb_rect* win,
+                                const xpngb_tensor* fmt) {
+    // at most 2^24 x 2^24 (a window lies inside its size): no overflow
+    const uint64_t px = win ? win->w * win->h : sz ? (uint64_t)sz->w * sz->h : r ? r->w * r->h : img.w * img.h;
     if (!fmt) return px * (3 + img.A);
     static const uint32_t elem_bytes[4] = { 1, 4, 2, 2 };   // XPNGB_DT_*
     return px * (fmt->channels == 3 ? 3 : 3 + img.A) * elem_bytes[fmt->dtype];
@@ -973,10 +975,11 @@ static uint64_t entry_out_bytes(const xpngb_image& img, const xpngb_rect* r, con
 
 // Header checks of file i (libxpng.c:969-976) and of where its pixels go: fills imgs[i] (w, h, A, mode) and D (file,
 // geometry, effective mode).  A region decode (r != nullptr) writes the r->w x r->h crop at imgs[i].offset instead of
-// the whole image, a resized decode (sz != nullptr) an sz->w x sz->h image, and a tensor decode (fmt != nullptr) that
-// as a tensor.  Runs for every entry of a call before anything is launched.
+// the whole image, a resized decode (sz != nullptr) an sz->w x sz->h image or its window win, and a tensor decode
+// (fmt != nullptr) that as a tensor.  Runs for every entry of a call before anything is launched.
 static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint32_t* hdr, uint64_t file_off, uint64_t file_size,
-                        const xpngb_rect* r, const xpngb_size* sz, const xpngb_tensor* fmt, uint64_t pixels_cap, DecImage& D) {
+                        const xpngb_rect* r, const xpngb_size* sz, const xpngb_rect* win, const xpngb_tensor* fmt, uint64_t pixels_cap,
+                        DecImage& D) {
     const uint64_t w = (hdr[0] & 0xFFFFFFu) + 1, h = (hdr[1] & 0xFFFFFFu) + 1;
     const uint32_t A = (hdr[1] >> 24) & 1, mode = hdr[0] >> 24, pxsz = 3 + A;
     if (!(mode == 1 || mode == 2 || mode == 7)) FAIL("file %u: unknown mode %u", i, mode);   // libxpng.c:972
@@ -987,7 +990,7 @@ static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint
     if (r && (r->x >= w || r->w > w - r->x || r->y >= h || r->h > h - r->y))
         FAIL("entry %u: rectangle (%llu, %llu) %llux%llu is not inside the %llux%llu image", i, (unsigned long long)r->x,
              (unsigned long long)r->y, (unsigned long long)r->w, (unsigned long long)r->h, (unsigned long long)w, (unsigned long long)h);
-    const uint64_t s = w * h * pxsz, out = entry_out_bytes(img, r, sz, fmt);
+    const uint64_t s = w * h * pxsz, out = entry_out_bytes(img, r, sz, win, fmt);
     if (img.offset & 15) FAIL("file %u: pixel offset must be a multiple of 16", i);
     if (out > pixels_cap || img.offset > pixels_cap - out) FAIL("file %u: pixels exceed the output buffer", i);
     uint32_t m = mode;
@@ -1003,8 +1006,13 @@ static int decode_check(xpngb_ctx* ctx, uint32_t i, xpngb_image& img, const uint
     return 0;
 }
 
-// One entry of a region decode: the rectangle, the tiles that hold it and their union.
-struct RegionSel { xpngb_rect rect, cover; TileGrid g; TileSel s; };
+// One entry of a region decode: the rectangle, the tiles that hold it and their union.  A resampled entry (rs) of a resized
+// decode resamples its crop to `full` with `filter` and keeps the window `win` (in full's coordinates); its rectangle is
+// then the span of the crop that the window's support reaches.
+struct RegionSel {
+    xpngb_rect rect, cover; TileGrid g; TileSel s;
+    bool rs; uint32_t filter; xpngb_rect crop, win; xpngb_size full;
+};
 static bool whole_tiles(const RegionSel& R) {
     return R.rect.x == R.cover.x && R.rect.y == R.cover.y && R.rect.w == R.cover.w && R.rect.h == R.cover.h;
 }
@@ -1012,41 +1020,55 @@ static uint64_t window_pitch(const RegionSel& R, uint32_t pxsz) { return (R.cove
 // Entry i of an oriented decode is written turned or mirrored.  TL and TR are copies in the reference: those entries are
 // decoded exactly as without an op.
 static bool turned(const int* ops, uint32_t i) { return ops && ops[i] != OP_TL && ops[i] != OP_TR; }
-// Entry i of a resized decode is resampled: its size differs from its rectangle's.  Other entries are decoded exactly as
-// by an oriented or region decode.
-static bool resized(const xpngb_size* sizes, const RegionSel* sel, uint32_t i) {
-    return sizes && (sizes[i].w != sel[i].rect.w || sizes[i].h != sel[i].rect.h);
-}
-// Pillow's number of weights per output coordinate of one axis (0: the axis is not resampled).
-static uint32_t resize_ksize(uint64_t in, uint64_t out) {
-    if (in == out) return 0;
+// Pillow's number of weights per output coordinate of one axis (0: the axis is not resampled, or not a filter).
+static uint32_t resize_ksize(uint32_t filter, uint64_t in, uint64_t out) {
+    if (in == out || resize_support(filter) == 0.0) return 0;
     const double scale = (double)in / (double)out;
-    return 2 * (uint32_t)ceil(scale < 1.0 ? 1.0 : scale) + 1;
+    return 2 * (uint32_t)ceil(resize_support(filter) * (scale < 1.0 ? 1.0 : scale)) + 1;
 }
-static uint64_t resize_tab_bytes(const RegionSel& R, const xpngb_size& z) {
-    return resize_table_bytes((uint32_t)R.rect.w, z.w, resize_ksize(R.rect.w, z.w)) +
-           resize_table_bytes((uint32_t)R.rect.h, z.h, resize_ksize(R.rect.h, z.h));
+static uint32_t resize_kx(const RegionSel& R) { return resize_ksize(R.filter, R.crop.w, R.full.w); }
+static uint32_t resize_ky(const RegionSel& R) { return resize_ksize(R.filter, R.crop.h, R.full.h); }
+static uint64_t resize_tab_bytes(const RegionSel& R) {
+    return resize_table_bytes((uint32_t)R.win.w, resize_kx(R)) + resize_table_bytes((uint32_t)R.win.h, resize_ky(R));
 }
-// Scratch of resized entry i: tables (a multiple of 8 bytes) and the first pass's rows (16-byte aligned) when both axes are
-// resampled: in_h rows of out_w pixels, or out_h rows of in_w pixels when the vertical pass runs first.
-static uint64_t resize_tmp_bytes(const RegionSel& R, const xpngb_size& z, uint32_t pxsz) {
-    if (R.rect.w == z.w || R.rect.h == z.h) return 0;
-    const uint64_t px = resize_vfirst(R.rect.w, R.rect.h, z.w, z.h) ? z.h * R.rect.w : R.rect.h * z.w;
+// Scratch of resampled entry R: tables (a multiple of 8 bytes) and the first pass's rows (16-byte aligned) when both axes
+// are resampled: the span's rows of window-wide pixels, or window rows of span-wide pixels when the vertical pass runs first.
+static uint64_t resize_tmp_bytes(const RegionSel& R, uint32_t pxsz) {
+    if (!resize_kx(R) || !resize_ky(R)) return 0;
+    const uint64_t px = resize_vfirst(R.crop.w, R.crop.h, R.full.w, R.full.h) ? R.win.h * R.rect.w : R.rect.h * R.win.w;
     return (px * pxsz + 15) & ~15ull;
 }
+// [lo, hi): the input coordinates that the windows of output coordinates o0 .. o1 - 1 of one axis read, widened by one
+// pixel on each side and clipped to [0, in), so that this plain host arithmetic needs no bit-exact agreement with the
+// device's tables (windows are monotone in the output coordinate for every filter).
+static void resize_span(uint32_t filter, uint64_t in, uint64_t out, uint64_t o0, uint64_t o1, uint64_t& lo, uint64_t& hi) {
+    const double scale = (double)in / (double)out, support = resize_support(filter) * (scale < 1.0 ? 1.0 : scale);
+    const int64_t a = (int64_t)((o0 + 0.5) * scale - support + 0.5) - 1, b = (int64_t)((o1 - 0.5) * scale + support + 0.5) + 1;
+    lo = a < 0 ? 0 : (uint64_t)a;
+    hi = b > (int64_t)in ? in : (uint64_t)b;
+}
+// The longest crop side a filter may resample.  The accumulator starts at 2^21 and adds src * k over an axis's n <= in
+// taps, src in 0..255, in any order of signs; every partial sum lies within 2^21 +- 255 * sum |k|.  Each integer weight is
+// its normalised weight w times 2^22, rounded by at most 1/2, so sum |k| <= 2^22 * (1 + 2 * N) + n / 2, N being the sum of
+// the negative normalised weights of one output coordinate.  That stays below 2^31 while 1 + 2 * N + n / 2^23 <= 2.0058
+// (2^31 is 2.0078 * 255 * 2^22, less the 2^21 start).  Box, bilinear and hamming have no negative weights (N = 0):
+// n <= 2^23.  Over every in, out <= 256, where clipped windows make it largest, N is at most 0.134 for bicubic (208 -> 193)
+// and 0.286 for lanczos (4 -> 5; tests/test_resampled_decode.py measures both).  So bicubic gets 2^22 (room for N up to
+// 0.25) and lanczos 2^21 (room for N up to 0.375).
+static uint64_t resize_side_max(uint32_t filter) { return filter == RF_LANCZOS ? 1ull << 21 : filter == RF_BICUBIC ? 1ull << 22 : 1ull << 23; }
 
 // Launch the decode of one chunk on lane `ctx`.  DI: the checked images of the chunk.  `lat`: warp-per-block chain
 // kernels (few blocks in the whole call) instead of the pair decoders.  sel == nullptr: every tile of every image, in
 // place.  Otherwise a region decode: only the tiles of sel[i].s, written in place when the rectangle is made of whole
 // tiles, else into a window of the lane's region scratch from which k_crop_rows copies the rectangle; stored images
 // are cropped straight out of their files.  ops (only with sel): an entry that is turned (turned()) always goes through a
-// window, or for a stored image straight out of its file, and one k_orient launch writes all of them.  sizes (only with
-// sel): a resized entry (resized()) also always goes through a window or its file, and is resampled and written through
-// its op by one launch of each resize kernel for the chunk.  fmt (only with sel): every entry goes through a window or its
+// window, or for a stored image straight out of its file, and one k_orient launch writes all of them.  A resampled entry
+// (sel[i].rs) also always goes through a window or its file, and is resampled and written through its op by one launch
+// of each resize kernel for the chunk.  fmt (only with sel): every entry goes through a window or its
 // file, a resized one is resampled without its op into the lane's tsrc scratch, and one k_to_tensor launch writes every
 // entry's tensor through its op.  Never waits for the device.
 static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
-                        const xpngb_size* sizes, const xpngb_tensor* fmt, uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
+                        const xpngb_tensor* fmt, uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
@@ -1057,14 +1079,14 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0, tctas = 0;
     bool any1 = false, any2 = false, any7 = false;
     for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
-    // resized pixels of a tensor entry (16-byte aligned)
-    auto tsrc_bytes = [&](uint32_t i) -> uint64_t { return ((uint64_t)sizes[i].w * sizes[i].h * DI[i].pxsz + 15) & ~15ull; };
+    // resampled window of a tensor entry (16-byte aligned)
+    auto tsrc_bytes = [&](uint32_t i) -> uint64_t { return (sel[i].win.w * sel[i].win.h * DI[i].pxsz + 15) & ~15ull; };
     if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned, resized or tensor entry
         uint64_t need = 0, tab = 0, tmp = 0, tsz = 0;
         for (uint32_t i = 0; i < n; i++) {
-            const bool rs = resized(sizes, sel, i);
+            const bool rs = sel[i].rs;
             if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs || fmt)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
-            if (rs) { tab += resize_tab_bytes(sel[i], sizes[i]); tmp += resize_tmp_bytes(sel[i], sizes[i], DI[i].pxsz); }
+            if (rs) { tab += resize_tab_bytes(sel[i]); tmp += resize_tmp_bytes(sel[i], DI[i].pxsz); }
             if (rs && fmt) tsz += tsrc_bytes(i);
         }
         if (need) ENSURE(region, need);
@@ -1072,32 +1094,34 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         if (tmp) ENSURE(rtmp, tmp);
         if (tsz) ENSURE(tsrc, tsz);
     }
-    // resized entry i: its crop at src (rows `pitch` bytes apart) resampled into out through its op, each pass reading the
-    // previous one's packed rows
+    // resampled entry i: the span of its crop at src (rows `pitch` bytes apart) resampled, and its window written into out
+    // through its op, each pass reading the previous one's packed rows
     uint64_t tpos = 0, mpos = 0;
     auto resize_desc = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out, uint32_t op) -> int {
-        const xpngb_rect& r = sel[i].rect;
-        const xpngb_size& z = sizes[i];
+        const RegionSel& R = sel[i];
+        const xpngb_rect &r = R.rect, &c = R.crop, &win = R.win;
         ResizeDesc d{};
-        d.coef = (uint64_t)ctx->rtab.p + tpos; tpos += resize_tab_bytes(sel[i], z);
-        const uint64_t tmp = (uint64_t)ctx->rtmp.p + mpos; mpos += resize_tmp_bytes(sel[i], z, DI[i].pxsz);
-        d.in_w = (uint32_t)r.w; d.in_h = (uint32_t)r.h; d.out_w = z.w; d.out_h = z.h;
-        d.pxsz = DI[i].pxsz; d.op = op;
-        d.kx = resize_ksize(r.w, z.w); d.ky = resize_ksize(r.h, z.h);
-        if (!d.kx) d.v = ResizePass{ src, pitch, (uint64_t)out, z.w, 1 };
-        else if (!d.ky) d.h = ResizePass{ src, pitch, (uint64_t)out, z.h, 1 };
-        else if (resize_vfirst(r.w, r.h, z.w, z.h)) {
+        d.coef = (uint64_t)ctx->rtab.p + tpos; tpos += resize_tab_bytes(R);
+        const uint64_t tmp = (uint64_t)ctx->rtmp.p + mpos; mpos += resize_tmp_bytes(R, DI[i].pxsz);
+        d.in_w = (uint32_t)c.w; d.in_h = (uint32_t)c.h; d.out_w = (uint32_t)win.w; d.out_h = (uint32_t)win.h;
+        d.full_w = R.full.w; d.full_h = R.full.h; d.wx = (uint32_t)win.x; d.wy = (uint32_t)win.y;
+        d.bx = (uint32_t)(r.x - c.x); d.by = (uint32_t)(r.y - c.y);
+        d.filter = R.filter; d.pxsz = DI[i].pxsz; d.op = op;
+        d.kx = resize_kx(R); d.ky = resize_ky(R);
+        if (!d.kx) d.v = ResizePass{ src, pitch, (uint64_t)out, d.out_w, 1 };
+        else if (!d.ky) d.h = ResizePass{ src, pitch, (uint64_t)out, d.out_h, 1 };
+        else if (resize_vfirst(c.w, c.h, R.full.w, R.full.h)) {
             d.v = ResizePass{ src, pitch, tmp, (uint32_t)r.w, 0 };
-            d.h = ResizePass{ tmp, r.w * DI[i].pxsz, (uint64_t)out, z.h, 1 };
+            d.h = ResizePass{ tmp, r.w * DI[i].pxsz, (uint64_t)out, d.out_h, 1 };
         } else {
             d.h = ResizePass{ src, pitch, tmp, (uint32_t)r.h, 0 };
-            d.v = ResizePass{ tmp, (uint64_t)z.w * DI[i].pxsz, (uint64_t)out, z.w, 1 };
+            d.v = ResizePass{ tmp, (uint64_t)d.out_w * DI[i].pxsz, (uint64_t)out, d.out_w, 1 };
         }
         d.first_coef = (uint32_t)rcoef; d.first_h = (uint32_t)rh; d.first_v = (uint32_t)rv;
-        d.h_tiles_x = (z.w + RH_X - 1) / RH_X;
-        rcoef += (d.kx ? z.w : 0) + (d.ky ? z.h : 0);
+        d.h_tiles_x = (d.out_w + RH_X - 1) / RH_X;
+        rcoef += (d.kx ? d.out_w : 0) + (d.ky ? d.out_h : 0);
         if (d.kx) rh += (uint64_t)d.h_tiles_x * ((d.h.n + RH_ROWS - 1) / RH_ROWS);
-        if (d.ky) rv += ((uint64_t)d.v.n * d.pxsz + RV_X - 1) / RV_X * ((z.h + RV_ROWS - 1) / RV_ROWS);
+        if (d.ky) rv += ((uint64_t)d.v.n * d.pxsz + RV_X - 1) / RV_X * ((d.out_h + RV_ROWS - 1) / RV_ROWS);
         if (rcoef > 0xFFFFFFFFull || rh > 0x7FFFFFFFull || rv > 0x7FFFFFFFull) FAIL("too many pixels for one resize launch");
         rdescs.push_back(d);
         return 0;
@@ -1118,14 +1142,14 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     auto region_out = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out) -> int {
         const xpngb_rect& r = sel[i].rect;
         const uint32_t pxsz = DI[i].pxsz;
-        if (fmt && resized(sizes, sel, i)) {   // resampled without the op; k_to_tensor applies it
+        if (fmt && sel[i].rs) {   // resampled without the op; k_to_tensor applies it
             uint8_t* t = (uint8_t*)ctx->tsrc.p + spos;
             spos += tsrc_bytes(i);
             if (resize_desc(i, src, pitch, t, OP_TL)) return 1;
-            return tensor_desc(i, (uint64_t)t, (uint64_t)sizes[i].w * pxsz, sizes[i].w, sizes[i].h, out);
+            return tensor_desc(i, (uint64_t)t, sel[i].win.w * pxsz, sel[i].win.w, sel[i].win.h, out);
         }
         if (fmt) return tensor_desc(i, src, pitch, r.w, r.h, out);
-        if (resized(sizes, sel, i)) return resize_desc(i, src, pitch, out, ops ? (uint32_t)ops[i] : (uint32_t)OP_TL);
+        if (sel[i].rs) return resize_desc(i, src, pitch, out, ops ? (uint32_t)ops[i] : (uint32_t)OP_TL);
         if (!turned(ops, i)) crops.push_back(CropDesc{ src, (uint64_t)out, pitch, (uint32_t)(r.w * pxsz), (uint32_t)r.h });
         else if (!orient_desc(odescs.emplace_back(), src, pitch, (uint64_t)out, r.w, r.h, pxsz, ops[i], &octas))
             FAIL("too many pixels for one orientation launch");
@@ -1149,7 +1173,7 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         } else {
             const RegionSel& R = sel[i];
             const xpngb_rect &r = R.rect, &c = R.cover;
-            if (whole_tiles(R) && !turned(ops, i) && !resized(sizes, sel, i) && !fmt)
+            if (whole_tiles(R) && !turned(ops, i) && !R.rs && !fmt)
                 plan_image(P, R.g, R.s, (uint64_t)out, r.w * D.pxsz, r.x, r.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
             else {   // a turned, resized or tensor rectangle cannot be decoded in place, even when it is made of whole tiles
                 const uint64_t pitch = window_pitch(R, D.pxsz), win = (uint64_t)ctx->region.p + wpos;
@@ -1412,10 +1436,11 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
 }
 
 // xpngb_decode (rects == nullptr), xpngb_decode_region and, with ops, xpngb_decode_oriented; with sizes
-// xpngb_decode_resized, with fmt xpngb_decode_tensor.  An oriented, resized or tensor call always selects tiles per entry:
-// without rects every entry's rectangle is its whole image.
+// xpngb_decode_resized, with fmt xpngb_decode_tensor, with filters or windows (only with sizes) xpngb_decode_resampled.
+// An oriented, resized or tensor call always selects tiles per entry: without rects every entry's rectangle is its whole
+// image.
 static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, const xpngb_size* sizes,
-                       const xpngb_tensor* fmt, uint32_t n, const void* files,
+                       const int* filters, const xpngb_rect* windows, const xpngb_tensor* fmt, uint32_t n, const void* files,
                        uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
                        uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
@@ -1428,6 +1453,12 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
         if (ops && (ops[i] < OP_R90 || ops[i] > OP_TR)) FAIL("entry %u: unknown orientation op %d", i, ops[i]);
         if (sizes && (!sizes[i].w || !sizes[i].h || sizes[i].w > (1u << 24) || sizes[i].h > (1u << 24)))
             FAIL("entry %u: output size %ux%u is not in 1..2^24 on each side", i, sizes[i].w, sizes[i].h);
+        if (filters && resize_support((uint32_t)filters[i]) == 0.0)
+            FAIL("entry %u: unknown resampling filter %d (LANCZOS 1, BILINEAR 2, BICUBIC 3, BOX 4, HAMMING 5; NEAREST is not one)", i, filters[i]);
+        const xpngb_rect* wr = windows ? windows + i : nullptr;
+        if (wr && (!wr->w || !wr->h || wr->x >= sizes[i].w || wr->w > sizes[i].w - wr->x || wr->y >= sizes[i].h || wr->h > sizes[i].h - wr->y))
+            FAIL("entry %u: window (%llu, %llu) %llux%llu is empty or not inside the %ux%u resized image", i, (unsigned long long)wr->x,
+                 (unsigned long long)wr->y, (unsigned long long)wr->w, (unsigned long long)wr->h, sizes[i].w, sizes[i].h);
     }
     const uint8_t* din = (const uint8_t*)files;
     if (!files_on_device) { ENSURE(files, files_size); din = (const uint8_t*)ctx->files.p; }
@@ -1450,13 +1481,27 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     std::vector<RegionSel> sel(use_sel ? n : 0);
     for (uint32_t i = 0; i < n; i++) {
         if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr,
-                         fmt, pixels_cap, DI[i])) return 1;
+                         windows ? windows + i : nullptr, fmt, pixels_cap, DI[i])) return 1;
         if (use_sel) {
-            sel[i].rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
-            region_select(imgs[i].w, imgs[i].h, sel[i].rect, sel[i].g, sel[i].s, sel[i].cover);
-            // a 32-bit accumulator holds 2^21 + 255 * (sum of the weights) exactly for windows of up to 2^23 taps
-            if (sizes && ((sizes[i].w != sel[i].rect.w && sel[i].rect.w > (1u << 23)) || (sizes[i].h != sel[i].rect.h && sel[i].rect.h > (1u << 23))))
-                FAIL("entry %u: a crop side above 2^23 pixels cannot be resized", i);
+            RegionSel& R = sel[i];
+            R.rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
+            if (sizes) {
+                R.crop = R.rect; R.full = sizes[i];
+                R.win = windows ? windows[i] : xpngb_rect{ 0, 0, sizes[i].w, sizes[i].h };
+                R.filter = filters ? (uint32_t)filters[i] : (uint32_t)RF_BILINEAR;
+                const bool rx = R.crop.w != R.full.w, ry = R.crop.h != R.full.h;
+                R.rs = rx || ry;
+                const uint64_t side_max = resize_side_max(R.filter);
+                if ((rx && R.crop.w > side_max) || (ry && R.crop.h > side_max))
+                    FAIL("entry %u: a crop side above %llu pixels cannot be resized with filter %u", i, (unsigned long long)side_max, R.filter);
+                // the decoded rectangle: the span the window's support reaches on a resampled axis, the window itself on
+                // an identity axis (an entry with no resampled axis is a plain crop of the window)
+                uint64_t x0 = R.win.x, x1 = R.win.x + R.win.w, y0 = R.win.y, y1 = R.win.y + R.win.h;
+                if (rx) resize_span(R.filter, R.crop.w, R.full.w, R.win.x, R.win.x + R.win.w, x0, x1);
+                if (ry) resize_span(R.filter, R.crop.h, R.full.h, R.win.y, R.win.y + R.win.h, y0, y1);
+                R.rect = xpngb_rect{ R.crop.x + x0, R.crop.y + y0, x1 - x0, y1 - y0 };
+            }
+            region_select(imgs[i].w, imgs[i].h, R.rect, R.g, R.s, R.cover);
         }
     }
     uint8_t* dpx = (uint8_t*)pixels;
@@ -1472,7 +1517,9 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
                                                          : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
         l2 |= mode == 2;
     }
-    auto out_bytes = [&](uint32_t i) { return entry_out_bytes(imgs[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr, fmt); };
+    auto out_bytes = [&](uint32_t i) {
+        return entry_out_bytes(imgs[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr, windows ? windows + i : nullptr, fmt);
+    };
     // level 2: above ~600 tiles the pair family wins, with the 16-symbol value streams warp-per-block while they all fit
     // (s16_lat_max_tiles); level 1: the warp-per-block family up to ~1300 tiles (measured at 125 / 250 / 500 frames, profiles/)
     const bool lat = l2 ? 17 * tiles_est <= (uint64_t)ctx->lat_max_blocks * 5 / 6 : 9 * tiles_est <= ctx->lat_max_blocks;
@@ -1507,7 +1554,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             }
         }
         rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr,
-                          sizes ? sizes + i0 : nullptr, fmt, m, din, dpx,
+                          fmt, m, din, dpx,
                           (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
@@ -1542,7 +1589,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
 extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
                             const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
                             int pixels_on_device) {
-    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1551,7 +1598,7 @@ extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpng
                                    void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1560,7 +1607,7 @@ extern "C" int xpngb_decode_oriented(xpngb_ctx* ctx, const int* ops, xpngb_image
                                      const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!ops) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1569,7 +1616,7 @@ extern "C" int xpngb_decode_resized(xpngb_ctx* ctx, const int* ops, xpngb_image*
                                     const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!sizes) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1595,8 +1642,50 @@ extern "C" int xpngb_decode_tensor(xpngb_ctx* ctx, const xpngb_tensor* fmt, cons
     if (!ctx) return 1;
     ctx->err[0] = 0;
     if (tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, fmt, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, fmt, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
                        out_on_device);
+}
+
+extern "C" int xpngb_decode_resampled(xpngb_ctx* ctx, const xpngb_tensor* fmt, const int* filters, const int* ops, xpngb_image* imgs,
+                                      const xpngb_rect* rects, const xpngb_size* sizes, const xpngb_rect* windows, uint32_t n,
+                                      const void* files, uint64_t files_size, int files_on_device, const uint64_t* file_offsets,
+                                      const uint64_t* file_sizes, void* out, uint64_t out_cap, int out_on_device) {
+    if (!ctx) return 1;
+    ctx->err[0] = 0;
+    if (!sizes) FAIL("null argument (sizes)");
+    if (fmt && tensor_check(ctx, fmt)) return 1;
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, n, files, files_size, files_on_device, file_offsets, file_sizes,
+                       out, out_cap, out_on_device);
+}
+
+extern "C" uint32_t xpngb_resize_ksize(int filter, uint32_t in, uint32_t out) {
+    return in && out ? resize_ksize((uint32_t)filter, in, out) : 0;
+}
+
+// The tables k_resize_coeffs computes for output coordinates first .. first + count - 1 of one axis, copied back:
+// (xmin, n) pairs and count rows of ksize weights, zero past each window.
+extern "C" int xpngb_resize_coeffs(xpngb_ctx* ctx, int filter, uint32_t in, uint32_t out, uint32_t first, uint32_t count,
+                                   int32_t* xmin_n, int32_t* k) {
+    if (!ctx) return 1;
+    ctx->err[0] = 0; ctx->launches = 0; ctx->cur = ctx->stream;
+    if (!xmin_n || !k) FAIL("null argument");
+    if (resize_support((uint32_t)filter) == 0.0) FAIL("unknown resampling filter %d", filter);
+    if (!in || !out || in > (1u << 24) || out > (1u << 24) || in == out) FAIL("in %u, out %u: not a resampled axis", in, out);
+    if (!count || first >= out || count > out - first) FAIL("coordinates %u + %u are not inside 0..%u", first, count, out);
+    CK(cudaSetDevice(ctx->device));
+    ResizeDesc d{};
+    d.in_w = in; d.full_w = out; d.out_w = count; d.wx = first; d.filter = (uint32_t)filter;
+    d.kx = resize_ksize((uint32_t)filter, in, out);
+    const uint64_t tab = resize_table_bytes(count, d.kx);
+    ENSURE(rtab, tab); ENSURE(rdescs, sizeof(ResizeDesc));
+    d.coef = (uint64_t)ctx->rtab.p;
+    CK(cudaMemsetAsync(ctx->rtab.p, 0, tab, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->rdescs.p, &d, sizeof d, cudaMemcpyHostToDevice, ctx->stream));
+    LAUNCH(k_resize_coeffs, (count + 255) / 256, 256, 0, (const ResizeDesc*)ctx->rdescs.p, 1u, count);
+    CK(cudaMemcpyAsync(xmin_n, ctx->rtab.p, (uint64_t)count * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(k, (uint8_t*)ctx->rtab.p + (uint64_t)count * 8, (uint64_t)count * d.kx * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------
