@@ -208,6 +208,42 @@ uint32_t xpngb_resize_ksize(int filter, uint32_t in, uint32_t out);
 int xpngb_resize_coeffs(xpngb_ctx *ctx, int filter, uint32_t in, uint32_t out, uint32_t first, uint32_t count,
                         int32_t *xmin_n, int32_t *k);
 
+/* ---- Colour decode: torchvision's ColorJitter and RandomGrayscale per entry, byte-identical to their PIL path.
+ * Entry i is tensor(gray_i(jitter_i(orient(ops[i], window_i(resize_f(crop_i)))))): what xpngb_decode_resampled writes for it
+ * (sizes == NULL: what xpngb_decode_tensor / xpngb_decode_oriented write without a resize; filters and windows then must be
+ * NULL), with colors[i]'s steps applied to its 8-bit pixels before the tensor conversion (fmt == NULL: uint8 output).
+ *   jitter_i : the steps k = order[0], order[1], ... whose bit k of `on` is set, each mapping bytes to bytes as Pillow does
+ *              (every float / double operation rounded on its own):
+ *     L(p)        = (19595 R + 38470 G + 7471 B + 0x8000) >> 16, Pillow's L24 luma;
+ *     BRIGHTNESS, CONTRAST, SATURATION: Image.blend(d, p, f) per colour channel: a = (float)factor,
+ *                 t = (float)d + a * (float)(p - d), out = t <= 0 ? 0 : t >= 255 ? 255 : (int)t, with d = 0 (brightness),
+ *                 L(p) (saturation) or m = (int)((double)S / N + 0.5) (contrast), S the sum of L over the entry's N output
+ *                 pixels as they stand at that step (ImageStat's mean).  Alpha is unchanged;
+ *     HUE         : Pillow's rgb2hsv, H += (uint8_t)(int32_t)(factor * 255.0) mod 256, hsv2rgb (Convert.c).  On RGBA the
+ *                 alpha becomes 255: torchvision's adjust_hue converts through HSV, which has no alpha, and that quirk is kept.
+ *   gray_i   : gray == 1 sets R = G = B = L(p) after the jitter (RandomGrayscale(num_output_channels=3)).
+ * The steps are per pixel and contrast's mean does not depend on pixel order, so the op may come before or after them: the
+ * library applies them to the entry's pixels as written.  colors == NULL, or entries with on == 0 and gray == 0, give exactly
+ * what xpngb_decode_resampled / xpngb_decode_tensor / xpngb_decode_oriented give.  Every check of those calls runs before
+ * anything is launched, plus, naming the entry: an order that is not a permutation of 0..3, a bit of `on` above 3, gray other
+ * than 0 or 1, a brightness, contrast or saturation factor that is negative or not finite (also as a float), a hue factor
+ * outside [-0.5, 0.5] or NaN, and gray on an entry whose output keeps alpha (uint8 output or channels == 0 of an RGBA file:
+ * torchvision's RandomGrayscale refuses 4 channels).  Coloured tensor entries are first written as uint8 pixels into scratch
+ * (resized entries already are); one launch per chunk sums the luma of the entries with contrast on, and one applies the chain. */
+enum { XPNGB_CJ_BRIGHTNESS = 0, XPNGB_CJ_CONTRAST = 1, XPNGB_CJ_SATURATION = 2, XPNGB_CJ_HUE = 3 };   /* ColorJitter's fn_idx */
+typedef struct xpngb_color {
+    uint8_t  order[4];   /* the steps in the order applied: a permutation of 0..3, as ColorJitter.get_params' fn_idx */
+    uint32_t on;         /* bit k: step k applied (a None factor of get_params: bit clear) */
+    uint32_t gray;       /* 1: RandomGrayscale after the jitter */
+    double   factor[4];  /* brightness, contrast, saturation: finite, >= 0; hue: in [-0.5, 0.5] */
+} xpngb_color;
+int xpngb_decode_color(xpngb_ctx *ctx, const xpngb_tensor *fmt /* NULL: uint8 pixels */, const int *filters, const int *ops,
+                       xpngb_image *imgs, const xpngb_rect *rects, const xpngb_size *sizes /* NULL: no resize */,
+                       const xpngb_rect *windows, const xpngb_color *colors /* NULL: none */, uint32_t n,
+                       const void *files, uint64_t files_size, int files_on_device,
+                       const uint64_t *file_offsets, const uint64_t *file_sizes,
+                       void *out, uint64_t out_cap, int out_on_device);
+
 /* Device time of the kernels of the last encode/decode call on this context, in milliseconds
  * (CUDA events on the context's stream; excludes host<->device copies). */
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);

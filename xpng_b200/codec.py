@@ -38,6 +38,10 @@ class _Tensor(C.Structure):  # xpngb_tensor: the format of a tensor decode (see 
                 ("mean", C.c_float * 4), ("std", C.c_float * 4)]
 
 
+class _Color(C.Structure):  # xpngb_color: one entry's ColorJitter / RandomGrayscale (see color_params)
+    _fields_ = [("order", C.c_uint8 * 4), ("on", C.c_uint32), ("gray", C.c_uint32), ("factor", C.c_double * 4)]
+
+
 class _Xpng(C.Structure):  # xpng_t, xpng.h:10
     _fields_ = [("p", C.c_void_p), ("w", C.c_uint64), ("h", C.c_uint64), ("s", C.c_uint64), ("A", C.c_bool)]
 
@@ -86,6 +90,10 @@ def lib():
         L.xpngb_decode_resampled.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_Image),
                                              C.POINTER(_Rect), C.POINTER(_Size), C.POINTER(_Rect), u32, vp, u64, C.c_int, C.POINTER(u64),
                                              C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_decode_color.restype = C.c_int
+        L.xpngb_decode_color.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect),
+                                         C.POINTER(_Size), C.POINTER(_Rect), C.POINTER(_Color), u32, vp, u64, C.c_int, C.POINTER(u64),
+                                         C.POINTER(u64), vp, u64, C.c_int]
         L.xpngb_resize_ksize.restype = u32; L.xpngb_resize_ksize.argtypes = [C.c_int, u32, u32]
         L.xpngb_resize_coeffs.restype = C.c_int
         L.xpngb_resize_coeffs.argtypes = [vp, C.c_int, u32, u32, u32, u32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
@@ -251,6 +259,34 @@ def tensor_format(dtype, layout="chw", scale="div", mean=(0, 0, 0, 0), std=(1, 1
     return f
 
 
+def color_params(fn_idx, b, c, s, h, gray=False):
+    """One entry's xpngb_color from T.ColorJitter.get_params(...)'s tuple as returned: fn_idx (a tensor or sequence of the
+    step numbers 0 brightness, 1 contrast, 2 saturation, 3 hue, in the order applied) and the four factors, None for a
+    step that is not applied.  gray: RandomGrayscale after the jitter."""
+    col = _Color()
+    col.order[:] = [int(k) for k in fn_idx]
+    col.on = sum(1 << k for k, f in enumerate((b, c, s, h)) if f is not None)
+    col.gray = int(bool(gray))
+    col.factor[:] = [1.0 if b is None else float(b), 1.0 if c is None else float(c), 1.0 if s is None else float(s),
+                     0.0 if h is None else float(h)]
+    return col
+
+
+def color_array(colors, n):
+    """None, or one entry per file (color_params(...) or None for no colour) -> ctypes array of xpngb_color, or None."""
+    if colors is None:
+        return None
+    if len(colors) != n:
+        raise ValueError("one colour entry per file")
+    arr = (_Color * n)()
+    for i, c in enumerate(colors):
+        if c is None:
+            arr[i].order[:] = [0, 1, 2, 3]
+        else:
+            arr[i] = c
+    return arr
+
+
 def region_tiles(w, h, rect):
     """Tiles a region decode of rect = (x, y, w, h) inside a w x h coded image decodes, and their union (x, y, w, h):
     (0, None) when rect is empty or not inside the image.  Host only."""
@@ -376,6 +412,16 @@ class Codec:
                                         out_cap, int(out_dev)):
             raise RuntimeError("xpngb_decode_resampled: " + self._err())
 
+    def decode_color_raw(self, fmt, descs, filt_arr, ops_arr, rect_arr, size_arr, win_arr, color_arr, n, files_ptr, files_size, files_dev,
+                         offs, sizes, out_ptr, out_cap, out_dev):
+        """decode_resampled_raw (size_arr None: no resize, filt_arr and win_arr then None, as decode_tensor_raw /
+        decode_oriented_raw) with ColorJitter and RandomGrayscale color_arr[i] (see color_array(); None: none) applied to
+        entry i's pixels before they are written."""
+        if lib().xpngb_decode_color(self._h, None if fmt is None else C.byref(fmt), filt_arr, ops_arr, descs, rect_arr, size_arr, win_arr,
+                                    color_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev), offs, sizes, C.c_void_p(out_ptr),
+                                    out_cap, int(out_dev)):
+            raise RuntimeError("xpngb_decode_color: " + self._err())
+
     def resize_coeffs(self, filt, inn, out, first=0, count=None):
         """The device's weight tables of an inn -> out axis for output coordinates first .. first + count - 1: (xmin, n) as
         an (count, 2) int32 array and the (count, ksize) int32 weights, zero past each window."""
@@ -390,7 +436,7 @@ class Codec:
         return xn[:count], k[:count, :ksize]
 
     def decode_tensor(self, files, sizes=None, boxes=None, ops=None, dtype=None, layout="chw", scale="div", mean=None, std=None,
-                      drop_alpha=False, filters=None, windows=None):
+                      drop_alpha=False, filters=None, windows=None, colors=None):
         """list of .xpng byte strings -> one torch tensor on this codec's device, (N, C, H, W) for layout "chw" or (N, H, W, C)
         for "hwc": each whole image, or rectangle boxes[i] = (x, y, w, h) of it, resized to sizes[i] = (w, h) as decode_resized
         does (None: not resized), turned by ops[i] (None: no op), then scaled and normalised as torchvision does, bit for bit:
@@ -398,13 +444,14 @@ class Codec:
         float16 / bfloat16 are those results rounded by .to(dtype).  dtype: torch.float32 (default), float16, bfloat16 or
         uint8 (the bytes themselves, as F.pil_to_tensor).  mean / std None: 0 and 1 (no Normalize).  C is 3 + A, or 3 with
         drop_alpha.  filters and windows (only with sizes) as decode_resized: torchvision's Resize(256) + CenterCrop(224) of
-        each image is sizes[i], windows[i] = resize_center_crop(w, h, 256, 224).  Every entry must have the same output shape
-        (ValueError otherwise); ragged batches use decode_tensor_raw or decode_resampled_raw."""
+        each image is sizes[i], windows[i] = resize_center_crop(w, h, 256, 224).  colors: one color_params(...) or None per
+        entry, ColorJitter and RandomGrayscale applied before the conversion (sizes not needed).  Every entry must have the same
+        output shape (ValueError otherwise); ragged batches use decode_tensor_raw, decode_resampled_raw or decode_color_raw."""
         import torch
         n = len(files)
         if n == 0:
             raise ValueError("decode_tensor needs at least one file")
-        for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops), ("window", windows)):
+        for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops), ("window", windows), ("colour entry", colors)):
             if arg is not None and len(arg) != n:
                 raise ValueError(f"one {name} per file")
         if sizes is None and (filters is not None or windows is not None):
@@ -434,7 +481,10 @@ class Codec:
         # the library writes on its own stream: memory fresh from the caching allocator may still be in use by queued work
         torch.cuda.current_stream(dev).synchronize()
         oa = None if ops is None else op_codes(ops)
-        if fa is None and wa is None:
+        if colors is not None:
+            self.decode_color_raw(fmt, descs, fa, oa, ra, sa, wa, color_array(colors, n), n, fb.ctypes.data, off, 0, foffs, fsizes,
+                                  flat.data_ptr(), n * stride * DTYPE_BYTES[dname], 1)
+        elif fa is None and wa is None:
             self.decode_tensor_raw(fmt, descs, oa, ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes, flat.data_ptr(),
                                    n * stride * DTYPE_BYTES[dname], 1)
         else:
@@ -528,14 +578,14 @@ class Codec:
             self.decode_oriented_raw(descs, op_codes(ops), ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         return self._unpack(px, descs, [(r.w, r.h) for r in ra], ops)
 
-    def decode_resized(self, files, sizes, boxes=None, ops=None, filters=None, windows=None):
+    def decode_resized(self, files, sizes, boxes=None, ops=None, filters=None, windows=None, colors=None):
         """list of .xpng byte strings and one (w, h) output size per file -> list of (h, w, 3|4) uint8 arrays: each whole image,
         or rectangle boxes[i] = (x, y, w, h) of it, resampled as Pillow's Image.resize((w, h), filter) does, every channel on
         its own (alpha is not premultiplied).  filters: None (bilinear), one filter for all entries or one per entry, each a
         name ("bicubic", ...), a PIL.Image.Resampling value or a torchvision InterpolationMode.  windows: one (x, y, w, h) per
         entry in the resized image's coordinates, the part of it that is returned (None: all of it).  ops: one OPS name per
         entry, applied last; 'r90' and 'r270' entries come back as (w, h, 3|4).  An entry whose size equals its crop is the
-        crop itself."""
+        crop itself.  colors: one color_params(...) or None per entry, ColorJitter and RandomGrayscale applied to its pixels."""
         n = len(files)
         if len(sizes) != n:
             raise ValueError("one size per file")
@@ -545,13 +595,16 @@ class Codec:
             raise ValueError("one op per file")
         if windows is not None and len(windows) != n:
             raise ValueError("one window per file")
+        ca = color_array(colors, n)
         ra = None if boxes is None else rects(boxes)
         sa = _sizes(sizes)
         wa = None if windows is None else rects(windows)
         fa = filter_codes(filters, n)
         oa = None if ops is None else op_codes(ops)
         descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files, ra, sa, wa)
-        if fa is None and wa is None:
+        if ca is not None:
+            self.decode_color_raw(None, descs, fa, oa, ra, sa, wa, ca, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        elif fa is None and wa is None:
             self.decode_resized_raw(descs, oa, ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         else:
             self.decode_resampled_raw(None, descs, fa, oa, ra, sa, wa, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)

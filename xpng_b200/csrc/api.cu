@@ -33,6 +33,7 @@
 #include "region.cuh"
 #include "resize.cuh"
 #include "tensor.cuh"
+#include "color.cuh"
 
 using namespace xpb;
 
@@ -75,7 +76,8 @@ struct xpngb_ctx {
         region, crops,   // region decode: window of the selected tiles, crop descriptors
         orients,         // oriented decode: OrientDesc of the lane's chunk (odesc belongs to xpngb_transform / encode_oriented)
         rdescs, rtab, rtmp,   // resized decode: ResizeDesc of the lane's chunk, windows and weights, the first pass's rows
-        tdescs, tsrc;         // tensor decode: TensorDesc of the lane's chunk, the resized entries' pixels
+        tdescs, tsrc,         // tensor decode: TensorDesc of the lane's chunk, the resized (and coloured) entries' pixels
+        cdescs;               // colour decode: ColorDesc of the lane's chunk, then one 64-bit luma sum per descriptor
     PinBuf pin_a, pin_b, pin_o;   // pin_o: orientation descriptors (their upload may still be in flight when an encode reuses pin_a)
 };
 
@@ -395,7 +397,7 @@ static void lane_free(xpngb_ctx* ctx) {
                       &ctx->plane, &ctx->nlseq, &ctx->rowcnt, &ctx->rowbits, &ctx->rows, &ctx->edge, &ctx->errflag, &ctx->hdr,
                       &ctx->offs, &ctx->m2a, &ctx->m2b, &ctx->tclass, &ctx->tabs, &ctx->ccnt, &ctx->cbit, &ctx->resv, &ctx->oriented,
                       &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops, &ctx->orients,
-                      &ctx->rdescs, &ctx->rtab, &ctx->rtmp, &ctx->tdescs, &ctx->tsrc };
+                      &ctx->rdescs, &ctx->rtab, &ctx->rtmp, &ctx->tdescs, &ctx->tsrc, &ctx->cdescs };
     for (DevBuf* b : all) if (b->p) cudaFree(b->p);
     if (ctx->pin_a.p) cudaFreeHost(ctx->pin_a.p);
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
@@ -1066,9 +1068,13 @@ static uint64_t resize_side_max(uint32_t filter) { return filter == RF_LANCZOS ?
 // (sel[i].rs) also always goes through a window or its file, and is resampled and written through its op by one launch
 // of each resize kernel for the chunk.  fmt (only with sel): every entry goes through a window or its
 // file, a resized one is resampled without its op into the lane's tsrc scratch, and one k_to_tensor launch writes every
-// entry's tensor through its op.  Never waits for the device.
+// entry's tensor through its op.  colors (only with sel): a coloured entry's pixels are changed in place by one
+// k_color_mean and one k_color launch after the resize launches: at its uint8 output, or for a tensor entry in tsrc (a
+// resized one lands there anyway, any other is copied there by k_crop_rows), from which k_to_tensor reads it.  Never waits
+// for the device.
 static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
-                        const xpngb_tensor* fmt, uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
+                        const xpngb_tensor* fmt, const xpngb_color* colors, uint32_t n, const uint8_t* din, uint8_t* dpx,
+                        uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
@@ -1076,18 +1082,22 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     std::vector<OrientDesc> odescs;
     std::vector<ResizeDesc> rdescs;
     std::vector<TensorDesc> tdescs;
-    uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0, tctas = 0;
+    std::vector<ColorDesc> cdescs;
+    uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0, tctas = 0, cctas = 0, mctas = 0;
     bool any1 = false, any2 = false, any7 = false;
     for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
-    // resampled window of a tensor entry (16-byte aligned)
-    auto tsrc_bytes = [&](uint32_t i) -> uint64_t { return (sel[i].win.w * sel[i].win.h * DI[i].pxsz + 15) & ~15ull; };
+    auto colored = [&](uint32_t i) { return colors && (colors[i].on || colors[i].gray); };
+    // pixels entry i writes: its resampled window, or its rectangle
+    auto out_px = [&](uint32_t i) -> uint64_t { return sel[i].rs ? sel[i].win.w * sel[i].win.h : sel[i].rect.w * sel[i].rect.h; };
+    // uint8 pixels of a resized or coloured tensor entry (16-byte aligned)
+    auto tsrc_bytes = [&](uint32_t i) -> uint64_t { return (out_px(i) * DI[i].pxsz + 15) & ~15ull; };
     if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned, resized or tensor entry
         uint64_t need = 0, tab = 0, tmp = 0, tsz = 0;
         for (uint32_t i = 0; i < n; i++) {
             const bool rs = sel[i].rs;
             if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs || fmt)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
             if (rs) { tab += resize_tab_bytes(sel[i]); tmp += resize_tmp_bytes(sel[i], DI[i].pxsz); }
-            if (rs && fmt) tsz += tsrc_bytes(i);
+            if ((rs || colored(i)) && fmt) tsz += tsrc_bytes(i);
         }
         if (need) ENSURE(region, need);
         if (tab) ENSURE(rtab, tab);
@@ -1137,16 +1147,36 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         tdescs.push_back(d);
         return 0;
     };
+    // coloured entry i: its npx packed pixels at px, changed in place
+    auto color_desc = [&](uint32_t i, uint8_t* px, uint64_t npx) -> int {
+        const xpngb_color& c = colors[i];
+        ColorDesc d{};
+        d.px = (uint64_t)px; d.npx = npx; d.pxsz = DI[i].pxsz; d.on = c.on; d.gray = c.gray;
+        for (int k = 0; k < 3; k++) d.fac[k] = (float)c.factor[k];   // Pillow's ImagingBlend takes the factor as a float
+        d.hue = (uint8_t)(int32_t)(c.factor[XPNGB_CJ_HUE] * 255.0);   // np.array(h * 255).astype(np.uint8): truncate, then wrap
+        d.pre = 4;
+        for (uint32_t s = 0; s < 4; s++) { d.order[s] = c.order[s]; if (c.order[s] == XPNGB_CJ_CONTRAST) d.pre = s; }
+        d.first_cta = (uint32_t)cctas; d.mfirst_cta = (uint32_t)mctas;
+        const uint64_t ctas = (npx + CL_PX - 1) / CL_PX;
+        cctas += ctas;
+        if ((c.on >> XPNGB_CJ_CONTRAST) & 1) mctas += ctas;
+        if (cctas > 0x7FFFFFFFull) FAIL("too many pixels for one colour launch");
+        cdescs.push_back(d);
+        return 0;
+    };
     // entry i of a region call: its rectangle at src (rows `pitch` bytes apart) cropped, turned, resized or made a tensor
     uint64_t spos = 0;
     auto region_out = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out) -> int {
         const xpngb_rect& r = sel[i].rect;
         const uint32_t pxsz = DI[i].pxsz;
-        if (fmt && sel[i].rs) {   // resampled without the op; k_to_tensor applies it
+        if (fmt && (sel[i].rs || colored(i))) {   // uint8 pixels in tsrc, resampled or copied without the op; k_to_tensor applies it
             uint8_t* t = (uint8_t*)ctx->tsrc.p + spos;
             spos += tsrc_bytes(i);
-            if (resize_desc(i, src, pitch, t, OP_TL)) return 1;
-            return tensor_desc(i, (uint64_t)t, sel[i].win.w * pxsz, sel[i].win.w, sel[i].win.h, out);
+            const uint64_t w = sel[i].rs ? sel[i].win.w : r.w, h = sel[i].rs ? sel[i].win.h : r.h;
+            if (sel[i].rs) { if (resize_desc(i, src, pitch, t, OP_TL)) return 1; }
+            else crops.push_back(CropDesc{ src, (uint64_t)t, pitch, (uint32_t)(r.w * pxsz), (uint32_t)r.h });
+            if (colored(i) && color_desc(i, t, w * h)) return 1;
+            return tensor_desc(i, (uint64_t)t, w * pxsz, w, h, out);
         }
         if (fmt) return tensor_desc(i, src, pitch, r.w, r.h, out);
         if (sel[i].rs) return resize_desc(i, src, pitch, out, ops ? (uint32_t)ops[i] : (uint32_t)OP_TL);
@@ -1185,6 +1215,7 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             D.nrows = (uint32_t)(R.s.r1 - R.s.r0 + 1); D.ncols = (uint32_t)(R.s.c1 - R.s.c0 + 1);
         }
         D.tile0 = P.imgs[i].tile0; D.ntiles = P.imgs[i].ntiles;
+        if (!fmt && colored(i) && color_desc(i, out, out_px(i))) return 1;   // uint8 output: coloured where it is written
     }
     if (P.tiles.size() > (1u << 24) || P.seg_tile.size() > (1u << 28)) FAIL("too many tiles for one chunk (%zu)", P.tiles.size());
     const uint32_t ntiles = (uint32_t)P.tiles.size();
@@ -1193,7 +1224,8 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop, orientation, resize and tensor descriptors
     const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64, pin_orients = pin_crops + crops.size() * sizeof(CropDesc);
     const size_t pin_resize = pin_orients + odescs.size() * sizeof(OrientDesc), pin_tensor = pin_resize + rdescs.size() * sizeof(ResizeDesc);
-    if (ensure_pin(ctx, ctx->pin_b, pin_tensor + tdescs.size() * sizeof(TensorDesc))) return 1;
+    const size_t pin_color = pin_tensor + tdescs.size() * sizeof(TensorDesc);
+    if (ensure_pin(ctx, ctx->pin_b, pin_color + cdescs.size() * sizeof(ColorDesc))) return 1;
     memcpy(ctx->pin_b.p, DI.data(), n * sizeof(DecImage));
     CK(cudaMemcpyAsync(ctx->dimgs.p, ctx->pin_b.p, n * sizeof(DecImage), cudaMemcpyHostToDevice, ctx->stream));
     if (any7 && !sel) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
@@ -1224,6 +1256,13 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         ENSURE(tdescs, nb);
         memcpy((uint8_t*)ctx->pin_b.p + pin_tensor, tdescs.data(), nb);
         CK(cudaMemcpyAsync(ctx->tdescs.p, (uint8_t*)ctx->pin_b.p + pin_tensor, nb, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    const size_t csum = cdescs.size() * sizeof(ColorDesc);   // the luma sums follow the descriptors (8-byte aligned)
+    if (!cdescs.empty()) {
+        ENSURE(cdescs, csum + cdescs.size() * 8);
+        memcpy((uint8_t*)ctx->pin_b.p + pin_color, cdescs.data(), csum);
+        CK(cudaMemcpyAsync(ctx->cdescs.p, (uint8_t*)ctx->pin_b.p + pin_color, csum, cudaMemcpyHostToDevice, ctx->stream));
+        if (mctas) CK(cudaMemsetAsync((uint8_t*)ctx->cdescs.p + csum, 0, cdescs.size() * 8, ctx->stream));
     }
     CK(cudaMemsetAsync(ctx->errflag.p, 0, 4, ctx->stream));
     CK(cudaMemsetAsync(ctx->dtiles.p, 0, ntiles * sizeof(DecTile), ctx->stream));
@@ -1429,6 +1468,12 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         if (rh) LAUNCH(k_resize_h, (unsigned)rh, RH_X, 0, d_rd, nr);
         if (rv) LAUNCH(k_resize_v, (unsigned)rv, RV_X, 0, d_rd, nr, vfirst ? 2u : 3u);
     }
+    if (!cdescs.empty()) {   // the contrast means first, then every coloured entry's chain
+        const ColorDesc* d_cd = (const ColorDesc*)ctx->cdescs.p;
+        unsigned long long* d_sum = (unsigned long long*)((uint8_t*)ctx->cdescs.p + csum);
+        if (mctas) LAUNCH(k_color_mean, (unsigned)mctas, 256, 0, d_cd, (uint32_t)cdescs.size(), d_sum);
+        LAUNCH(k_color, (unsigned)cctas, 256, 0, d_cd, (uint32_t)cdescs.size(), (const unsigned long long*)d_sum);
+    }
     if (!tdescs.empty()) LAUNCH(k_to_tensor, (unsigned)tctas, 256, 0, (const TensorDesc*)ctx->tdescs.p, (uint32_t)tdescs.size(), *fmt);
     // the error flag travels to pinned memory behind the DecImage table
     CK(cudaMemcpyAsync((uint8_t*)ctx->pin_b.p + n * (sizeof(DecImage) + 8), d_err, 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1438,9 +1483,9 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
 // xpngb_decode (rects == nullptr), xpngb_decode_region and, with ops, xpngb_decode_oriented; with sizes
 // xpngb_decode_resized, with fmt xpngb_decode_tensor, with filters or windows (only with sizes) xpngb_decode_resampled.
 // An oriented, resized or tensor call always selects tiles per entry: without rects every entry's rectangle is its whole
-// image.
+// image.  With colors, xpngb_decode_color.
 static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, const xpngb_size* sizes,
-                       const int* filters, const xpngb_rect* windows, const xpngb_tensor* fmt, uint32_t n, const void* files,
+                       const int* filters, const xpngb_rect* windows, const xpngb_tensor* fmt, const xpngb_color* colors, uint32_t n, const void* files,
                        uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
                        uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
@@ -1459,6 +1504,21 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
         if (wr && (!wr->w || !wr->h || wr->x >= sizes[i].w || wr->w > sizes[i].w - wr->x || wr->y >= sizes[i].h || wr->h > sizes[i].h - wr->y))
             FAIL("entry %u: window (%llu, %llu) %llux%llu is empty or not inside the %ux%u resized image", i, (unsigned long long)wr->x,
                  (unsigned long long)wr->y, (unsigned long long)wr->w, (unsigned long long)wr->h, sizes[i].w, sizes[i].h);
+        if (colors) {
+            const xpngb_color& c = colors[i];
+            uint32_t seen = 0;
+            for (int k = 0; k < 4; k++) seen |= c.order[k] < 4 ? 1u << c.order[k] : 16u;
+            if (seen != 15u) FAIL("entry %u: colour order (%u, %u, %u, %u) is not a permutation of 0..3", i, c.order[0], c.order[1],
+                                  c.order[2], c.order[3]);
+            if (c.on & ~15u) FAIL("entry %u: colour steps 0x%x set a bit above 3", i, c.on);
+            if (c.gray > 1) FAIL("entry %u: gray %u is neither 0 nor 1", i, c.gray);
+            static const char* const step_name[3] = { "brightness", "contrast", "saturation" };
+            for (int k = 0; k < 3; k++)   // Pillow narrows the factor to a float: it must stay finite there too
+                if (!(c.factor[k] >= 0.0 && c.factor[k] <= 3.4028234663852886e38))
+                    FAIL("entry %u: %s factor %g is negative or not finite", i, step_name[k], c.factor[k]);
+            if (!(c.factor[XPNGB_CJ_HUE] >= -0.5 && c.factor[XPNGB_CJ_HUE] <= 0.5))
+                FAIL("entry %u: hue factor %g is not in [-0.5, 0.5]", i, c.factor[XPNGB_CJ_HUE]);
+        }
     }
     const uint8_t* din = (const uint8_t*)files;
     if (!files_on_device) { ENSURE(files, files_size); din = (const uint8_t*)ctx->files.p; }
@@ -1477,11 +1537,13 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     }
     // ---- every entry is checked before anything is decoded
     std::vector<DecImage> DI(n);
-    const bool use_sel = rects || ops || sizes || fmt;
+    const bool use_sel = rects || ops || sizes || fmt || colors;
     std::vector<RegionSel> sel(use_sel ? n : 0);
     for (uint32_t i = 0; i < n; i++) {
         if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr,
                          windows ? windows + i : nullptr, fmt, pixels_cap, DI[i])) return 1;
+        if (colors && colors[i].gray && imgs[i].A && (!fmt || fmt->channels == 0))
+            FAIL("entry %u: grayscale of an RGBA entry whose output keeps alpha (torchvision's RandomGrayscale refuses 4 channels)", i);
         if (use_sel) {
             RegionSel& R = sel[i];
             R.rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
@@ -1554,7 +1616,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             }
         }
         rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr,
-                          fmt, m, din, dpx,
+                          fmt, colors ? colors + i0 : nullptr, m, din, dpx,
                           (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
@@ -1589,7 +1651,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
 extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
                             const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
                             int pixels_on_device) {
-    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1598,7 +1660,7 @@ extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpng
                                    void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1607,7 +1669,7 @@ extern "C" int xpngb_decode_oriented(xpngb_ctx* ctx, const int* ops, xpngb_image
                                      const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!ops) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1616,7 +1678,7 @@ extern "C" int xpngb_decode_resized(xpngb_ctx* ctx, const int* ops, xpngb_image*
                                     const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!sizes) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1642,7 +1704,7 @@ extern "C" int xpngb_decode_tensor(xpngb_ctx* ctx, const xpngb_tensor* fmt, cons
     if (!ctx) return 1;
     ctx->err[0] = 0;
     if (tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, fmt, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, fmt, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
                        out_on_device);
 }
 
@@ -1654,8 +1716,20 @@ extern "C" int xpngb_decode_resampled(xpngb_ctx* ctx, const xpngb_tensor* fmt, c
     ctx->err[0] = 0;
     if (!sizes) FAIL("null argument (sizes)");
     if (fmt && tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, n, files, files_size, files_on_device, file_offsets, file_sizes,
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes,
                        out, out_cap, out_on_device);
+}
+
+extern "C" int xpngb_decode_color(xpngb_ctx* ctx, const xpngb_tensor* fmt, const int* filters, const int* ops, xpngb_image* imgs,
+                                  const xpngb_rect* rects, const xpngb_size* sizes, const xpngb_rect* windows, const xpngb_color* colors,
+                                  uint32_t n, const void* files, uint64_t files_size, int files_on_device, const uint64_t* file_offsets,
+                                  const uint64_t* file_sizes, void* out, uint64_t out_cap, int out_on_device) {
+    if (!ctx) return 1;
+    ctx->err[0] = 0;
+    if (!sizes && (filters || windows)) FAIL("null argument (sizes): filters and windows need sizes");
+    if (fmt && tensor_check(ctx, fmt)) return 1;
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, n, files, files_size, files_on_device, file_offsets,
+                       file_sizes, out, out_cap, out_on_device);
 }
 
 extern "C" uint32_t xpngb_resize_ksize(int filter, uint32_t in, uint32_t out) {
