@@ -244,6 +244,48 @@ int xpngb_decode_color(xpngb_ctx *ctx, const xpngb_tensor *fmt /* NULL: uint8 pi
                        const uint64_t *file_offsets, const uint64_t *file_sizes,
                        void *out, uint64_t out_cap, int out_on_device);
 
+/* ---- Blurred and solarized decode: Pillow's ImageFilter.GaussianBlur and ImageOps.solarize per entry, byte-identical to Pillow.
+ * Entry i is tensor(solarize_i(blur_i(gray_i(jitter_i(orient(ops[i], window_i(resize_f(crop_i)))))))): what xpngb_decode_color
+ * writes for it, with blurs[i] applied to its 8-bit pixels after the colour step and before the tensor conversion.  Both act
+ * on the entry's output image: the blur's x axis is the output's, and its edges are the output's edges.
+ *   blur_i     : img.filter(ImageFilter.GaussianBlur((radius[0], radius[1]))), Pillow's BoxBlur.c.  Per axis, with the radius
+ *                narrowed to float and every operation below in float:
+ *                  sigma2 = r * r / 3, L = (float)sqrt(sigma2 * 12 + 1), l = floor((L - 1) / 2),
+ *                  a = (2l + 1) * (l * (l + 1) - 3 * sigma2) / (6 * (sigma2 - (l + 1) * (l + 1))), fr = l + a,
+ *                  ri = (int)fr, ww = (uint32)(16777216.f / (fr * 2 + 1)), fw = (2^24 - (2 ri + 1) * ww) / 2 (uint32).
+ *                One pass along a line of one channel, edges clamped to the nearest pixel, in uint32:
+ *                  acc = sum of p[clamp(x + k)], k = -ri .. ri; bulk = acc * ww + (p[clamp(x - ri - 1)] + p[clamp(x + ri + 1)]) * fw;
+ *                  out = (bulk + 2^23) >> 24, a byte that the next pass reads.
+ *                Three passes along x with radius[0], then three along y with radius[1]; an axis whose float radius is 0 is
+ *                skipped.  Every channel is blurred on its own, alpha included (no premultiplication).
+ *   solarize_i : solarize == 1: every byte v < threshold is kept, every other becomes 255 - v (ImageOps.solarize(img,
+ *                threshold); 128 is its default).  All bytes of the output are treated: the call refuses it where alpha is kept.
+ * blurs == NULL, or entries with radius {0, 0} and solarize == 0, give exactly what xpngb_decode_color gives.  Every check of
+ * xpngb_decode_color runs before anything is launched, plus, naming the entry: a radius that is negative or not finite, a
+ * radius above XPNGB_BLUR_RADIUS_MAX as a float, solarize other than 0 or 1, a NaN threshold, and solarize on an entry whose
+ * output keeps alpha (uint8 output or channels == 0 of an RGBA file: ImageOps.solarize refuses RGBA).
+ * XPNGB_BLUR_RADIUS_MAX = 2^23 is the accumulator bound: up to it (2 ri + 1) * ww <= 2^24, so no uint32 above can wrap
+ * (acc * ww + far * fw + 2^23 <= 255 * 2^24 + 2^23); at the next float, 8388609, ri = 2^23, ww = 1 and fw wraps.  The box
+ * pass walks each line with a running sum, so its cost does not depend on the radius.  Blurred or solarized tensor entries
+ * are staged as uint8 pixels in scratch, as coloured ones are; tensor entries turned by r90 or r270 sit there un-turned and
+ * get the passes along y first with radius[0], then along x with radius[1], which equals blurring the turned image. */
+#define XPNGB_BLUR_RADIUS_MAX 8388608.0
+typedef struct xpngb_blur {
+    double   radius[2];   /* ImageFilter.GaussianBlur's (x, y) radius; {0, 0}: no blur */
+    uint32_t solarize;    /* 1: ImageOps.solarize after the blur */
+    double   threshold;   /* bytes v < threshold are kept, the others become 255 - v */
+} xpngb_blur;
+int xpngb_decode_blur(xpngb_ctx *ctx, const xpngb_tensor *fmt /* NULL: uint8 pixels */, const int *filters, const int *ops,
+                      xpngb_image *imgs, const xpngb_rect *rects, const xpngb_size *sizes /* NULL: no resize */,
+                      const xpngb_rect *windows, const xpngb_color *colors /* NULL: none */,
+                      const xpngb_blur *blurs /* NULL: none */, uint32_t n,
+                      const void *files, uint64_t files_size, int files_on_device,
+                      const uint64_t *file_offsets, const uint64_t *file_sizes,
+                      void *out, uint64_t out_cap, int out_on_device);
+/* Diagnostics: the host's box radius, ww and fw for one axis, as Pillow's _gaussian_blur_radius + ImagingHorizontalBoxBlur.
+ * Returns 1 (and sets nothing) for a radius the decode refuses: negative, not finite or above XPNGB_BLUR_RADIUS_MAX. */
+int xpngb_blur_box(double radius, int32_t *ri, uint32_t *ww, uint32_t *fw);
+
 /* Device time of the kernels of the last encode/decode call on this context, in milliseconds
  * (CUDA events on the context's stream; excludes host<->device copies). */
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);

@@ -42,6 +42,10 @@ class _Color(C.Structure):  # xpngb_color: one entry's ColorJitter / RandomGrays
     _fields_ = [("order", C.c_uint8 * 4), ("on", C.c_uint32), ("gray", C.c_uint32), ("factor", C.c_double * 4)]
 
 
+class _Blur(C.Structure):  # xpngb_blur: one entry's GaussianBlur / solarize (see blur_params)
+    _fields_ = [("radius", C.c_double * 2), ("solarize", C.c_uint32), ("threshold", C.c_double)]
+
+
 class _Xpng(C.Structure):  # xpng_t, xpng.h:10
     _fields_ = [("p", C.c_void_p), ("w", C.c_uint64), ("h", C.c_uint64), ("s", C.c_uint64), ("A", C.c_bool)]
 
@@ -94,6 +98,12 @@ def lib():
         L.xpngb_decode_color.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect),
                                          C.POINTER(_Size), C.POINTER(_Rect), C.POINTER(_Color), u32, vp, u64, C.c_int, C.POINTER(u64),
                                          C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_decode_blur.restype = C.c_int
+        L.xpngb_decode_blur.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect),
+                                        C.POINTER(_Size), C.POINTER(_Rect), C.POINTER(_Color), C.POINTER(_Blur), u32, vp, u64, C.c_int,
+                                        C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_blur_box.restype = C.c_int
+        L.xpngb_blur_box.argtypes = [C.c_double, C.POINTER(C.c_int32), C.POINTER(u32), C.POINTER(u32)]
         L.xpngb_resize_ksize.restype = u32; L.xpngb_resize_ksize.argtypes = [C.c_int, u32, u32]
         L.xpngb_resize_coeffs.restype = C.c_int
         L.xpngb_resize_coeffs.argtypes = [vp, C.c_int, u32, u32, u32, u32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
@@ -287,6 +297,38 @@ def color_array(colors, n):
     return arr
 
 
+def blur_params(radius=None, threshold=None):
+    """One entry's xpngb_blur: radius, a number or (x, y), is ImageFilter.GaussianBlur's (None: no blur); threshold is
+    ImageOps.solarize's after the blur (None: no solarize; 128 is ImageOps.solarize(img)'s default)."""
+    b = _Blur()
+    if radius is not None:
+        b.radius[:] = [float(radius)] * 2 if isinstance(radius, (int, float)) else [float(r) for r in radius]
+    if threshold is not None:
+        b.solarize, b.threshold = 1, float(threshold)
+    return b
+
+
+def blur_array(blurs, n):
+    """None, or one entry per file (blur_params(...) or None for neither step) -> ctypes array of xpngb_blur, or None."""
+    if blurs is None:
+        return None
+    if len(blurs) != n:
+        raise ValueError("one blur entry per file")
+    arr = (_Blur * n)()
+    for i, b in enumerate(blurs):
+        if b is not None:
+            arr[i] = b
+    return arr
+
+
+def blur_box(radius):
+    """The library's (ri, ww, fw) of one axis of GaussianBlur(radius), as Pillow computes them; None for a refused radius."""
+    ri, ww, fw = C.c_int32(), C.c_uint32(), C.c_uint32()
+    if lib().xpngb_blur_box(float(radius), C.byref(ri), C.byref(ww), C.byref(fw)):
+        return None
+    return ri.value, ww.value, fw.value
+
+
 def region_tiles(w, h, rect):
     """Tiles a region decode of rect = (x, y, w, h) inside a w x h coded image decodes, and their union (x, y, w, h):
     (0, None) when rect is empty or not inside the image.  Host only."""
@@ -422,6 +464,15 @@ class Codec:
                                     out_cap, int(out_dev)):
             raise RuntimeError("xpngb_decode_color: " + self._err())
 
+    def decode_blur_raw(self, fmt, descs, filt_arr, ops_arr, rect_arr, size_arr, win_arr, color_arr, blur_arr, n, files_ptr, files_size,
+                        files_dev, offs, sizes, out_ptr, out_cap, out_dev):
+        """decode_color_raw (color_arr None: no colour) with GaussianBlur and solarize blur_arr[i] (see blur_array(); None:
+        none) applied to entry i's pixels after its colour step."""
+        if lib().xpngb_decode_blur(self._h, None if fmt is None else C.byref(fmt), filt_arr, ops_arr, descs, rect_arr, size_arr, win_arr,
+                                   color_arr, blur_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev), offs, sizes,
+                                   C.c_void_p(out_ptr), out_cap, int(out_dev)):
+            raise RuntimeError("xpngb_decode_blur: " + self._err())
+
     def resize_coeffs(self, filt, inn, out, first=0, count=None):
         """The device's weight tables of an inn -> out axis for output coordinates first .. first + count - 1: (xmin, n) as
         an (count, 2) int32 array and the (count, ksize) int32 weights, zero past each window."""
@@ -436,7 +487,7 @@ class Codec:
         return xn[:count], k[:count, :ksize]
 
     def decode_tensor(self, files, sizes=None, boxes=None, ops=None, dtype=None, layout="chw", scale="div", mean=None, std=None,
-                      drop_alpha=False, filters=None, windows=None, colors=None):
+                      drop_alpha=False, filters=None, windows=None, colors=None, blurs=None):
         """list of .xpng byte strings -> one torch tensor on this codec's device, (N, C, H, W) for layout "chw" or (N, H, W, C)
         for "hwc": each whole image, or rectangle boxes[i] = (x, y, w, h) of it, resized to sizes[i] = (w, h) as decode_resized
         does (None: not resized), turned by ops[i] (None: no op), then scaled and normalised as torchvision does, bit for bit:
@@ -445,13 +496,16 @@ class Codec:
         uint8 (the bytes themselves, as F.pil_to_tensor).  mean / std None: 0 and 1 (no Normalize).  C is 3 + A, or 3 with
         drop_alpha.  filters and windows (only with sizes) as decode_resized: torchvision's Resize(256) + CenterCrop(224) of
         each image is sizes[i], windows[i] = resize_center_crop(w, h, 256, 224).  colors: one color_params(...) or None per
-        entry, ColorJitter and RandomGrayscale applied before the conversion (sizes not needed).  Every entry must have the same
-        output shape (ValueError otherwise); ragged batches use decode_tensor_raw, decode_resampled_raw or decode_color_raw."""
+        entry, ColorJitter and RandomGrayscale applied before the conversion (sizes not needed).  blurs: one blur_params(...) or
+        None per entry, GaussianBlur and solarize applied after the colour step (sizes not needed).  Every entry must have the
+        same output shape (ValueError otherwise); ragged batches use decode_tensor_raw, decode_resampled_raw, decode_color_raw
+        or decode_blur_raw."""
         import torch
         n = len(files)
         if n == 0:
             raise ValueError("decode_tensor needs at least one file")
-        for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops), ("window", windows), ("colour entry", colors)):
+        for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops), ("window", windows), ("colour entry", colors),
+                          ("blur entry", blurs)):
             if arg is not None and len(arg) != n:
                 raise ValueError(f"one {name} per file")
         if sizes is None and (filters is not None or windows is not None):
@@ -481,7 +535,10 @@ class Codec:
         # the library writes on its own stream: memory fresh from the caching allocator may still be in use by queued work
         torch.cuda.current_stream(dev).synchronize()
         oa = None if ops is None else op_codes(ops)
-        if colors is not None:
+        if blurs is not None:
+            self.decode_blur_raw(fmt, descs, fa, oa, ra, sa, wa, color_array(colors, n), blur_array(blurs, n), n, fb.ctypes.data, off, 0,
+                                 foffs, fsizes, flat.data_ptr(), n * stride * DTYPE_BYTES[dname], 1)
+        elif colors is not None:
             self.decode_color_raw(fmt, descs, fa, oa, ra, sa, wa, color_array(colors, n), n, fb.ctypes.data, off, 0, foffs, fsizes,
                                   flat.data_ptr(), n * stride * DTYPE_BYTES[dname], 1)
         elif fa is None and wa is None:
@@ -578,14 +635,15 @@ class Codec:
             self.decode_oriented_raw(descs, op_codes(ops), ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         return self._unpack(px, descs, [(r.w, r.h) for r in ra], ops)
 
-    def decode_resized(self, files, sizes, boxes=None, ops=None, filters=None, windows=None, colors=None):
+    def decode_resized(self, files, sizes, boxes=None, ops=None, filters=None, windows=None, colors=None, blurs=None):
         """list of .xpng byte strings and one (w, h) output size per file -> list of (h, w, 3|4) uint8 arrays: each whole image,
         or rectangle boxes[i] = (x, y, w, h) of it, resampled as Pillow's Image.resize((w, h), filter) does, every channel on
         its own (alpha is not premultiplied).  filters: None (bilinear), one filter for all entries or one per entry, each a
         name ("bicubic", ...), a PIL.Image.Resampling value or a torchvision InterpolationMode.  windows: one (x, y, w, h) per
         entry in the resized image's coordinates, the part of it that is returned (None: all of it).  ops: one OPS name per
         entry, applied last; 'r90' and 'r270' entries come back as (w, h, 3|4).  An entry whose size equals its crop is the
-        crop itself.  colors: one color_params(...) or None per entry, ColorJitter and RandomGrayscale applied to its pixels."""
+        crop itself.  colors: one color_params(...) or None per entry, ColorJitter and RandomGrayscale applied to its pixels.
+        blurs: one blur_params(...) or None per entry, GaussianBlur and solarize applied to its pixels after the colour step."""
         n = len(files)
         if len(sizes) != n:
             raise ValueError("one size per file")
@@ -596,13 +654,16 @@ class Codec:
         if windows is not None and len(windows) != n:
             raise ValueError("one window per file")
         ca = color_array(colors, n)
+        ba = blur_array(blurs, n)
         ra = None if boxes is None else rects(boxes)
         sa = _sizes(sizes)
         wa = None if windows is None else rects(windows)
         fa = filter_codes(filters, n)
         oa = None if ops is None else op_codes(ops)
         descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files, ra, sa, wa)
-        if ca is not None:
+        if ba is not None:
+            self.decode_blur_raw(None, descs, fa, oa, ra, sa, wa, ca, ba, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
+        elif ca is not None:
             self.decode_color_raw(None, descs, fa, oa, ra, sa, wa, ca, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         elif fa is None and wa is None:
             self.decode_resized_raw(descs, oa, ra, sa, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)

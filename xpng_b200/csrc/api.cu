@@ -34,6 +34,7 @@
 #include "resize.cuh"
 #include "tensor.cuh"
 #include "color.cuh"
+#include "blur.cuh"
 
 using namespace xpb;
 
@@ -77,7 +78,8 @@ struct xpngb_ctx {
         orients,         // oriented decode: OrientDesc of the lane's chunk (odesc belongs to xpngb_transform / encode_oriented)
         rdescs, rtab, rtmp,   // resized decode: ResizeDesc of the lane's chunk, windows and weights, the first pass's rows
         tdescs, tsrc,         // tensor decode: TensorDesc of the lane's chunk, the resized (and coloured) entries' pixels
-        cdescs;               // colour decode: ColorDesc of the lane's chunk, then one 64-bit luma sum per descriptor
+        cdescs,               // colour decode: ColorDesc of the lane's chunk, then one 64-bit luma sum per descriptor
+        bdescs, bscr;         // blurred decode: BlurPass of the lane's chunk, the second buffer of each entry's ping-pong
     PinBuf pin_a, pin_b, pin_o;   // pin_o: orientation descriptors (their upload may still be in flight when an encode reuses pin_a)
 };
 
@@ -397,7 +399,8 @@ static void lane_free(xpngb_ctx* ctx) {
                       &ctx->plane, &ctx->nlseq, &ctx->rowcnt, &ctx->rowbits, &ctx->rows, &ctx->edge, &ctx->errflag, &ctx->hdr,
                       &ctx->offs, &ctx->m2a, &ctx->m2b, &ctx->tclass, &ctx->tabs, &ctx->ccnt, &ctx->cbit, &ctx->resv, &ctx->oriented,
                       &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops, &ctx->orients,
-                      &ctx->rdescs, &ctx->rtab, &ctx->rtmp, &ctx->tdescs, &ctx->tsrc, &ctx->cdescs };
+                      &ctx->rdescs, &ctx->rtab, &ctx->rtmp, &ctx->tdescs, &ctx->tsrc, &ctx->cdescs,
+                      &ctx->bdescs, &ctx->bscr };
     for (DevBuf* b : all) if (b->p) cudaFree(b->p);
     if (ctx->pin_a.p) cudaFreeHost(ctx->pin_a.p);
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
@@ -1059,6 +1062,32 @@ static void resize_span(uint32_t filter, uint64_t in, uint64_t out, uint64_t o0,
 // 0.25) and lanczos 2^21 (room for N up to 0.375).
 static uint64_t resize_side_max(uint32_t filter) { return filter == RF_LANCZOS ? 1ull << 21 : filter == RF_BICUBIC ? 1ull << 22 : 1ull << 23; }
 
+// Pillow's box radius and weights of one axis of GaussianBlur(r), three passes: _gaussian_blur_radius and the head of
+// ImagingHorizontalBoxBlur (BoxBlur.c), operation for operation in float.  r is finite, 0 < r <= XPNGB_BLUR_RADIUS_MAX
+// (below it fr >= 0 and (2 ri + 1) * ww <= 2^24, so fw does not wrap; blur.cuh has the rest of the bound).
+struct BlurBox { int32_t ri; uint32_t ww, fw; };
+static BlurBox blur_box(float r) {
+    const float sigma2 = r * r / 3.f;
+    const float L = (float)sqrt((double)(sigma2 * 12.f + 1.f));
+    const float l = floorf((L - 1.f) / 2.f);
+    float a = (2.f * l + 1.f) * (l * (l + 1.f) - 3.f * sigma2);
+    a /= 6.f * (sigma2 - (l + 1.f) * (l + 1.f));
+    const float fr = l + a;
+    BlurBox b;
+    b.ri = (int32_t)fr;
+    b.ww = (uint32_t)(16777216.f / (fr * 2.f + 1.f));
+    b.fw = ((1u << 24) - (uint32_t)(b.ri * 2 + 1) * b.ww) / 2;
+    return b;
+}
+static bool blur_on(const xpngb_blur& b) { return (float)b.radius[0] != 0.f || (float)b.radius[1] != 0.f || b.solarize; }
+// ImageOps.solarize's `v < threshold` for bytes v is v < ceil(threshold), clamped to the bytes: 256 keeps them all
+static uint32_t solarize_t(double threshold) {
+    const double c = ceil(threshold);
+    return c <= 0.0 ? 0u : c >= 256.0 ? 256u : (uint32_t)c;
+}
+// the op turns the entry a quarter: its output's x axis is the staged pixels' y axis
+static bool quarter(const int* ops, uint32_t i) { return ops && (ops[i] == OP_R90 || ops[i] == OP_R270); }
+
 // Launch the decode of one chunk on lane `ctx`.  DI: the checked images of the chunk.  `lat`: warp-per-block chain
 // kernels (few blocks in the whole call) instead of the pair decoders.  sel == nullptr: every tile of every image, in
 // place.  Otherwise a region decode: only the tiles of sel[i].s, written in place when the rectangle is made of whole
@@ -1070,11 +1099,14 @@ static uint64_t resize_side_max(uint32_t filter) { return filter == RF_LANCZOS ?
 // file, a resized one is resampled without its op into the lane's tsrc scratch, and one k_to_tensor launch writes every
 // entry's tensor through its op.  colors (only with sel): a coloured entry's pixels are changed in place by one
 // k_color_mean and one k_color launch after the resize launches: at its uint8 output, or for a tensor entry in tsrc (a
-// resized one lands there anyway, any other is copied there by k_crop_rows), from which k_to_tensor reads it.  Never waits
+// resized one lands there anyway, any other is copied there by k_crop_rows), from which k_to_tensor reads it.  blurs (only
+// with sel): a blurred or solarized entry is staged as a coloured one is, then goes through its box passes after k_color,
+// ping-ponged between its pixels and the lane's bscr scratch, one k_blur launch per pass stage of the chunk; a tensor
+// entry's k_to_tensor reads whichever buffer its last pass wrote, a uint8 entry's passes end at its output.  Never waits
 // for the device.
 static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
-                        const xpngb_tensor* fmt, const xpngb_color* colors, uint32_t n, const uint8_t* din, uint8_t* dpx,
-                        uint32_t call_tiles) {
+                        const xpngb_tensor* fmt, const xpngb_color* colors, const xpngb_blur* blurs, uint32_t n, const uint8_t* din,
+                        uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
@@ -1083,26 +1115,31 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     std::vector<ResizeDesc> rdescs;
     std::vector<TensorDesc> tdescs;
     std::vector<ColorDesc> cdescs;
+    std::vector<BlurPass> bstage[BLUR_STAGES];   // the k-th pass of every blurred entry is in bstage[k]
     uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0, tctas = 0, cctas = 0, mctas = 0;
     bool any1 = false, any2 = false, any7 = false;
     for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
     auto colored = [&](uint32_t i) { return colors && (colors[i].on || colors[i].gray); };
+    auto blurred = [&](uint32_t i) { return blurs && blur_on(blurs[i]); };
+    auto staged = [&](uint32_t i) { return colored(i) || blurred(i); };   // needs its uint8 pixels to work on
     // pixels entry i writes: its resampled window, or its rectangle
     auto out_px = [&](uint32_t i) -> uint64_t { return sel[i].rs ? sel[i].win.w * sel[i].win.h : sel[i].rect.w * sel[i].rect.h; };
-    // uint8 pixels of a resized or coloured tensor entry (16-byte aligned)
+    // uint8 pixels of a resized or staged tensor entry, or of a blurred entry's scratch (16-byte aligned)
     auto tsrc_bytes = [&](uint32_t i) -> uint64_t { return (out_px(i) * DI[i].pxsz + 15) & ~15ull; };
     if (sel) {   // windows for the rectangles that are not made of whole tiles, and for every turned, resized or tensor entry
-        uint64_t need = 0, tab = 0, tmp = 0, tsz = 0;
+        uint64_t need = 0, tab = 0, tmp = 0, tsz = 0, bsz = 0;
         for (uint32_t i = 0; i < n; i++) {
             const bool rs = sel[i].rs;
             if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs || fmt)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
             if (rs) { tab += resize_tab_bytes(sel[i]); tmp += resize_tmp_bytes(sel[i], DI[i].pxsz); }
-            if ((rs || colored(i)) && fmt) tsz += tsrc_bytes(i);
+            if ((rs || staged(i)) && fmt) tsz += tsrc_bytes(i);
+            if (blurred(i)) bsz += tsrc_bytes(i);
         }
         if (need) ENSURE(region, need);
         if (tab) ENSURE(rtab, tab);
         if (tmp) ENSURE(rtmp, tmp);
         if (tsz) ENSURE(tsrc, tsz);
+        if (bsz) ENSURE(bscr, bsz);
     }
     // resampled entry i: the span of its crop at src (rows `pitch` bytes apart) resampled, and its window written into out
     // through its op, each pass reading the previous one's packed rows
@@ -1164,18 +1201,49 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         cdescs.push_back(d);
         return 0;
     };
+    // blurred entry i: its w x h packed pixels at px go through its passes, ping-ponged with its scratch; *res is where the
+    // last pass leaves them.  swap: the entry is staged un-turned and k_to_tensor turns it a quarter, so the passes of the
+    // output's x axis run along the staged columns, first.
+    uint64_t bpos = 0;
+    auto blur_desc = [&](uint32_t i, uint8_t* px, uint64_t w, uint64_t h, bool swap, uint8_t** res) -> int {
+        const xpngb_blur& b = blurs[i];
+        const uint32_t pxsz = DI[i].pxsz;
+        uint8_t* const buf[2] = { px, (uint8_t*)ctx->bscr.p + bpos };
+        bpos += tsrc_bytes(i);
+        uint32_t k = 0;
+        auto pass = [&](uint32_t vert, const BlurBox& bx) {
+            BlurPass& p = bstage[k].emplace_back();
+            p.src = (uint64_t)buf[k & 1]; p.dst = (uint64_t)buf[(k + 1) & 1]; p.pitch = w * pxsz;
+            p.w = (uint32_t)w; p.h = (uint32_t)h; p.pxsz = pxsz; p.vert = vert;
+            p.ri = (uint32_t)bx.ri; p.ww = bx.ww; p.fw = bx.fw; p.t = 256;
+            k++;
+        };
+        for (uint32_t a = 0; a < 2; a++) {   // output x, then output y
+            const float r = (float)b.radius[a];
+            if (r == 0.f) continue;
+            const BlurBox bx = blur_box(r);
+            for (int rep = 0; rep < 3; rep++) pass(a == 0 ? (swap ? 1u : 0u) : (swap ? 0u : 1u), bx);
+        }
+        const BlurBox id{ 0, 1u << 24, 0 };   // the identity pass: out = (p * 2^24 + 2^23) >> 24 = p
+        if (k == 0) pass(1, id);               // solarize alone
+        if (!fmt && (k & 1)) pass(1, id);      // a uint8 entry's result belongs at its output
+        if (b.solarize) bstage[k - 1].back().t = solarize_t(b.threshold);
+        *res = buf[k & 1];
+        return 0;
+    };
     // entry i of a region call: its rectangle at src (rows `pitch` bytes apart) cropped, turned, resized or made a tensor
     uint64_t spos = 0;
     auto region_out = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out) -> int {
         const xpngb_rect& r = sel[i].rect;
         const uint32_t pxsz = DI[i].pxsz;
-        if (fmt && (sel[i].rs || colored(i))) {   // uint8 pixels in tsrc, resampled or copied without the op; k_to_tensor applies it
+        if (fmt && (sel[i].rs || staged(i))) {   // uint8 pixels in tsrc, resampled or copied without the op; k_to_tensor applies it
             uint8_t* t = (uint8_t*)ctx->tsrc.p + spos;
             spos += tsrc_bytes(i);
             const uint64_t w = sel[i].rs ? sel[i].win.w : r.w, h = sel[i].rs ? sel[i].win.h : r.h;
             if (sel[i].rs) { if (resize_desc(i, src, pitch, t, OP_TL)) return 1; }
             else crops.push_back(CropDesc{ src, (uint64_t)t, pitch, (uint32_t)(r.w * pxsz), (uint32_t)r.h });
             if (colored(i) && color_desc(i, t, w * h)) return 1;
+            if (blurred(i) && blur_desc(i, t, w, h, quarter(ops, i), &t)) return 1;
             return tensor_desc(i, (uint64_t)t, w * pxsz, w, h, out);
         }
         if (fmt) return tensor_desc(i, src, pitch, r.w, r.h, out);
@@ -1216,6 +1284,25 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         }
         D.tile0 = P.imgs[i].tile0; D.ntiles = P.imgs[i].ntiles;
         if (!fmt && colored(i) && color_desc(i, out, out_px(i))) return 1;   // uint8 output: coloured where it is written
+        if (!fmt && blurred(i)) {   // and blurred there, in the output's orientation
+            uint64_t w = sel[i].rs ? sel[i].win.w : sel[i].rect.w, h = sel[i].rs ? sel[i].win.h : sel[i].rect.h;
+            if (quarter(ops, i)) { const uint64_t t = w; w = h; h = t; }
+            uint8_t* res;
+            if (blur_desc(i, out, w, h, false, &res)) return 1;
+        }
+    }
+    // blur passes stage by stage, each stage's CTAs numbered from 0
+    size_t bpasses = 0;
+    uint32_t nstage = 0;
+    uint64_t bctas[BLUR_STAGES] = {};
+    for (uint32_t k = 0; k < BLUR_STAGES; k++) {
+        for (BlurPass& p : bstage[k]) {
+            p.first_cta = (uint32_t)bctas[k];
+            bctas[k] += ((uint64_t)(p.vert ? p.w : p.h) * p.pxsz + BL_THREADS - 1) / BL_THREADS;
+            if (bctas[k] > 0x7FFFFFFFull) FAIL("too many pixels for one blur launch");
+        }
+        bpasses += bstage[k].size();
+        if (!bstage[k].empty()) nstage = k + 1;
     }
     if (P.tiles.size() > (1u << 24) || P.seg_tile.size() > (1u << 28)) FAIL("too many tiles for one chunk (%zu)", P.tiles.size());
     const uint32_t ntiles = (uint32_t)P.tiles.size();
@@ -1224,8 +1311,8 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop, orientation, resize and tensor descriptors
     const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64, pin_orients = pin_crops + crops.size() * sizeof(CropDesc);
     const size_t pin_resize = pin_orients + odescs.size() * sizeof(OrientDesc), pin_tensor = pin_resize + rdescs.size() * sizeof(ResizeDesc);
-    const size_t pin_color = pin_tensor + tdescs.size() * sizeof(TensorDesc);
-    if (ensure_pin(ctx, ctx->pin_b, pin_color + cdescs.size() * sizeof(ColorDesc))) return 1;
+    const size_t pin_color = pin_tensor + tdescs.size() * sizeof(TensorDesc), pin_blur = pin_color + cdescs.size() * sizeof(ColorDesc);
+    if (ensure_pin(ctx, ctx->pin_b, pin_blur + bpasses * sizeof(BlurPass))) return 1;
     memcpy(ctx->pin_b.p, DI.data(), n * sizeof(DecImage));
     CK(cudaMemcpyAsync(ctx->dimgs.p, ctx->pin_b.p, n * sizeof(DecImage), cudaMemcpyHostToDevice, ctx->stream));
     if (any7 && !sel) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
@@ -1263,6 +1350,15 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         memcpy((uint8_t*)ctx->pin_b.p + pin_color, cdescs.data(), csum);
         CK(cudaMemcpyAsync(ctx->cdescs.p, (uint8_t*)ctx->pin_b.p + pin_color, csum, cudaMemcpyHostToDevice, ctx->stream));
         if (mctas) CK(cudaMemsetAsync((uint8_t*)ctx->cdescs.p + csum, 0, cdescs.size() * 8, ctx->stream));
+    }
+    if (bpasses) {
+        ENSURE(bdescs, bpasses * sizeof(BlurPass));
+        size_t at = pin_blur;
+        for (uint32_t k = 0; k < nstage; k++) {
+            memcpy((uint8_t*)ctx->pin_b.p + at, bstage[k].data(), bstage[k].size() * sizeof(BlurPass));
+            at += bstage[k].size() * sizeof(BlurPass);
+        }
+        CK(cudaMemcpyAsync(ctx->bdescs.p, (uint8_t*)ctx->pin_b.p + pin_blur, bpasses * sizeof(BlurPass), cudaMemcpyHostToDevice, ctx->stream));
     }
     CK(cudaMemsetAsync(ctx->errflag.p, 0, 4, ctx->stream));
     CK(cudaMemsetAsync(ctx->dtiles.p, 0, ntiles * sizeof(DecTile), ctx->stream));
@@ -1474,6 +1570,8 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         if (mctas) LAUNCH(k_color_mean, (unsigned)mctas, 256, 0, d_cd, (uint32_t)cdescs.size(), d_sum);
         LAUNCH(k_color, (unsigned)cctas, 256, 0, d_cd, (uint32_t)cdescs.size(), (const unsigned long long*)d_sum);
     }
+    for (uint32_t k = 0, at = 0; k < nstage; at += (uint32_t)bstage[k].size(), k++)   // after the colour, pass stage by stage
+        LAUNCH(k_blur, (unsigned)bctas[k], BL_THREADS, 0, (const BlurPass*)ctx->bdescs.p + at, (uint32_t)bstage[k].size());
     if (!tdescs.empty()) LAUNCH(k_to_tensor, (unsigned)tctas, 256, 0, (const TensorDesc*)ctx->tdescs.p, (uint32_t)tdescs.size(), *fmt);
     // the error flag travels to pinned memory behind the DecImage table
     CK(cudaMemcpyAsync((uint8_t*)ctx->pin_b.p + n * (sizeof(DecImage) + 8), d_err, 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1485,7 +1583,8 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
 // An oriented, resized or tensor call always selects tiles per entry: without rects every entry's rectangle is its whole
 // image.  With colors, xpngb_decode_color.
 static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, const xpngb_size* sizes,
-                       const int* filters, const xpngb_rect* windows, const xpngb_tensor* fmt, const xpngb_color* colors, uint32_t n, const void* files,
+                       const int* filters, const xpngb_rect* windows, const xpngb_tensor* fmt, const xpngb_color* colors,
+                       const xpngb_blur* blurs, uint32_t n, const void* files,
                        uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
                        uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
@@ -1519,6 +1618,18 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             if (!(c.factor[XPNGB_CJ_HUE] >= -0.5 && c.factor[XPNGB_CJ_HUE] <= 0.5))
                 FAIL("entry %u: hue factor %g is not in [-0.5, 0.5]", i, c.factor[XPNGB_CJ_HUE]);
         }
+        if (blurs) {
+            const xpngb_blur& b = blurs[i];
+            for (int a = 0; a < 2; a++) {
+                if (!(b.radius[a] >= 0.0 && b.radius[a] <= 1.7976931348623157e308))
+                    FAIL("entry %u: blur radius %g is negative or not finite", i, b.radius[a]);
+                if ((float)b.radius[a] > (float)XPNGB_BLUR_RADIUS_MAX)   // Pillow narrows the radius to a float
+                    FAIL("entry %u: blur radius %.9g is above %.0f, where Pillow's uint32 box sums wrap", i, b.radius[a],
+                         XPNGB_BLUR_RADIUS_MAX);
+            }
+            if (b.solarize > 1) FAIL("entry %u: solarize %u is neither 0 nor 1", i, b.solarize);
+            if (b.threshold != b.threshold) FAIL("entry %u: solarize threshold is NaN", i);
+        }
     }
     const uint8_t* din = (const uint8_t*)files;
     if (!files_on_device) { ENSURE(files, files_size); din = (const uint8_t*)ctx->files.p; }
@@ -1537,13 +1648,15 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     }
     // ---- every entry is checked before anything is decoded
     std::vector<DecImage> DI(n);
-    const bool use_sel = rects || ops || sizes || fmt || colors;
+    const bool use_sel = rects || ops || sizes || fmt || colors || blurs;
     std::vector<RegionSel> sel(use_sel ? n : 0);
     for (uint32_t i = 0; i < n; i++) {
         if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr,
                          windows ? windows + i : nullptr, fmt, pixels_cap, DI[i])) return 1;
         if (colors && colors[i].gray && imgs[i].A && (!fmt || fmt->channels == 0))
             FAIL("entry %u: grayscale of an RGBA entry whose output keeps alpha (torchvision's RandomGrayscale refuses 4 channels)", i);
+        if (blurs && blurs[i].solarize && imgs[i].A && (!fmt || fmt->channels == 0))
+            FAIL("entry %u: solarize of an RGBA entry whose output keeps alpha (ImageOps.solarize refuses RGBA)", i);
         if (use_sel) {
             RegionSel& R = sel[i];
             R.rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
@@ -1616,7 +1729,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             }
         }
         rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr,
-                          fmt, colors ? colors + i0 : nullptr, m, din, dpx,
+                          fmt, colors ? colors + i0 : nullptr, blurs ? blurs + i0 : nullptr, m, din, dpx,
                           (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
@@ -1651,7 +1764,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
 extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
                             const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
                             int pixels_on_device) {
-    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1660,7 +1773,7 @@ extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpng
                                    void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1669,7 +1782,7 @@ extern "C" int xpngb_decode_oriented(xpngb_ctx* ctx, const int* ops, xpngb_image
                                      const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!ops) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1678,7 +1791,7 @@ extern "C" int xpngb_decode_resized(xpngb_ctx* ctx, const int* ops, xpngb_image*
                                     const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!sizes) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1704,7 +1817,7 @@ extern "C" int xpngb_decode_tensor(xpngb_ctx* ctx, const xpngb_tensor* fmt, cons
     if (!ctx) return 1;
     ctx->err[0] = 0;
     if (tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, fmt, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, fmt, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
                        out_on_device);
 }
 
@@ -1716,7 +1829,7 @@ extern "C" int xpngb_decode_resampled(xpngb_ctx* ctx, const xpngb_tensor* fmt, c
     ctx->err[0] = 0;
     if (!sizes) FAIL("null argument (sizes)");
     if (fmt && tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes,
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes,
                        out, out_cap, out_on_device);
 }
 
@@ -1728,8 +1841,27 @@ extern "C" int xpngb_decode_color(xpngb_ctx* ctx, const xpngb_tensor* fmt, const
     ctx->err[0] = 0;
     if (!sizes && (filters || windows)) FAIL("null argument (sizes): filters and windows need sizes");
     if (fmt && tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, n, files, files_size, files_on_device, file_offsets,
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, nullptr, n, files, files_size, files_on_device, file_offsets,
                        file_sizes, out, out_cap, out_on_device);
+}
+
+extern "C" int xpngb_decode_blur(xpngb_ctx* ctx, const xpngb_tensor* fmt, const int* filters, const int* ops, xpngb_image* imgs,
+                                 const xpngb_rect* rects, const xpngb_size* sizes, const xpngb_rect* windows, const xpngb_color* colors,
+                                 const xpngb_blur* blurs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
+                                 const uint64_t* file_offsets, const uint64_t* file_sizes, void* out, uint64_t out_cap, int out_on_device) {
+    if (!ctx) return 1;
+    ctx->err[0] = 0;
+    if (!sizes && (filters || windows)) FAIL("null argument (sizes): filters and windows need sizes");
+    if (fmt && tensor_check(ctx, fmt)) return 1;
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, blurs, n, files, files_size, files_on_device, file_offsets,
+                       file_sizes, out, out_cap, out_on_device);
+}
+
+extern "C" int xpngb_blur_box(double radius, int32_t* ri, uint32_t* ww, uint32_t* fw) {
+    if (!(radius >= 0.0 && radius <= 1.7976931348623157e308) || (float)radius > (float)XPNGB_BLUR_RADIUS_MAX) return 1;
+    const BlurBox b = blur_box((float)radius);
+    *ri = b.ri; *ww = b.ww; *fw = b.fw;
+    return 0;
 }
 
 extern "C" uint32_t xpngb_resize_ksize(int filter, uint32_t in, uint32_t out) {
