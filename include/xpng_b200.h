@@ -286,6 +286,60 @@ int xpngb_decode_blur(xpngb_ctx *ctx, const xpngb_tensor *fmt /* NULL: uint8 pix
  * Returns 1 (and sets nothing) for a radius the decode refuses: negative, not finite or above XPNGB_BLUR_RADIUS_MAX. */
 int xpngb_blur_box(double radius, int32_t *ri, uint32_t *ww, uint32_t *fw);
 
+/* ---- Auto-augmented decode: torchvision's AutoAugment, RandAugment and TrivialAugmentWide ops (_apply_op on the PIL path)
+ * per entry, byte-identical to Pillow.  Entry i is
+ *   tensor(solarize_i(blur_i(gray_i(jitter_i(augment_i(orient(ops[i], window_i(resize_f(crop_i)))))))))
+ * : what xpngb_decode_blur writes for it, with augs[i]'s program run on its 8-bit RGB image right after the op, where
+ * torchvision's ClassificationPresetTrain runs the policy (after RandomResizedCrop and the flip).  Every step acts on the
+ * output image: its axes, its size and its edges.  A program is up to XPNGB_AUG_STEPS_MAX steps, run in order; each step is
+ * one of the Pillow operations _apply_op ends in, with its parameters as Pillow receives them (xpng_b200.codec.augment_params
+ * builds them from (op_name, magnitude) as torchvision does):
+ *   AFFINE       img.transform(img.size, Image.AFFINE, data, resample, fillcolor=fill): ShearX/Y, TranslateX/Y and the
+ *                Rotate angles without a fast path.  data: the inverse matrix; arg: resample, NEAREST 0, BILINEAR 2 or
+ *                BICUBIC 3 (PIL numbering); fill: the RGB fill bytes of the pixels whose source is outside.  NEAREST follows
+ *                Pillow's three code paths (scale, 16.16 fixed point, running double sums), BILINEAR / BICUBIC its generic
+ *                transform with its filters, all in double with every operation rounded on its own.
+ *   TRANSPOSE    Image.rotate's fast paths: arg is XPNGB_OP_MVH (180), XPNGB_OP_R270 (ROTATE_90, square images only) or
+ *                XPNGB_OP_R90 (ROTATE_270, square only); any op code is accepted, a quarter turn only on a square output.
+ *   BRIGHTNESS, COLOR, CONTRAST   ImageEnhance.*(img).enhance(value): xpngb_decode_color's blends (value narrowed to float).
+ *   SHARPNESS    ImageEnhance.Sharpness(img).enhance(value): Image.blend(img.filter(SMOOTH), img, value); SMOOTH is
+ *                1 1 1 / 1 5 1 / 1 1 1 over 13, rounded, border rows and columns copied, images with a side below 3 copied.
+ *   POSTERIZE    ImageOps.posterize(img, arg): arg bits 0 .. 8 kept.
+ *   SOLARIZE     ImageOps.solarize(img, value): bytes v < value kept, others 255 - v.
+ *   AUTOCONTRAST, EQUALIZE, INVERT   ImageOps.autocontrast(img), ImageOps.equalize(img), ImageOps.invert(img): per RGB
+ *                channel, from the entry's histograms (a single-valued channel, or equalize's step 0, is left unchanged).
+ * augs == NULL, or entries with nsteps == 0, give exactly what xpngb_decode_blur gives.  An RGBA file written with
+ * channels == 3 is augmented as its RGB image (img.convert("RGB")).  Every check of xpngb_decode_blur runs before anything
+ * is launched, plus, naming the entry: nsteps above XPNGB_AUG_STEPS_MAX, an unknown kind, a resample other than 0, 2 or 3,
+ * a matrix coefficient that is not finite or is 2^64 or more in magnitude (Pillow's running sums could overflow), a
+ * TRANSPOSE arg that is not an op code or turns a non-square output a quarter, a negative or non-finite factor, posterize
+ * bits above 8, a NaN threshold, and any step on an entry whose output keeps alpha (uint8 output or channels == 0 of an RGBA
+ * file: Pillow's ImageOps refuse RGBA and torchvision documents these transforms for RGB).
+ * Warps read one buffer and write another: uint8 entries ping-pong between their output and the lane's scratch and end at
+ * their output; tensor entries are staged before the op as coloured ones are and map their warps through the op. */
+#define XPNGB_AUG_STEPS_MAX 8
+enum { XPNGB_AUG_AFFINE = 0, XPNGB_AUG_TRANSPOSE = 1, XPNGB_AUG_BRIGHTNESS = 2, XPNGB_AUG_COLOR = 3, XPNGB_AUG_CONTRAST = 4,
+       XPNGB_AUG_SHARPNESS = 5, XPNGB_AUG_POSTERIZE = 6, XPNGB_AUG_SOLARIZE = 7, XPNGB_AUG_AUTOCONTRAST = 8,
+       XPNGB_AUG_EQUALIZE = 9, XPNGB_AUG_INVERT = 10 };
+typedef struct xpngb_aug_step {
+    double   data[6];   /* AFFINE: the inverse matrix (x_src = data[0] x + data[1] y + data[2], y_src likewise, pixel centres) */
+    double   value;     /* BRIGHTNESS .. SHARPNESS: the factor; SOLARIZE: the threshold */
+    uint32_t kind;      /* XPNGB_AUG_* */
+    int32_t  arg;       /* AFFINE: resample; TRANSPOSE: XPNGB_OP_*; POSTERIZE: bits */
+    uint8_t  fill[4];   /* AFFINE: fill colour, RGB ([3] unused) */
+} xpngb_aug_step;
+typedef struct xpngb_augment {
+    uint32_t       nsteps;   /* 0: identity */
+    xpngb_aug_step step[XPNGB_AUG_STEPS_MAX];
+} xpngb_augment;
+int xpngb_decode_augment(xpngb_ctx *ctx, const xpngb_tensor *fmt /* NULL: uint8 pixels */, const int *filters, const int *ops,
+                         xpngb_image *imgs, const xpngb_rect *rects, const xpngb_size *sizes /* NULL: no resize */,
+                         const xpngb_rect *windows, const xpngb_color *colors /* NULL: none */, const xpngb_blur *blurs /* NULL: none */,
+                         const xpngb_augment *augs /* NULL: none */, uint32_t n,
+                         const void *files, uint64_t files_size, int files_on_device,
+                         const uint64_t *file_offsets, const uint64_t *file_sizes,
+                         void *out, uint64_t out_cap, int out_on_device);
+
 /* Device time of the kernels of the last encode/decode call on this context, in milliseconds
  * (CUDA events on the context's stream; excludes host<->device copies). */
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);

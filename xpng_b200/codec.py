@@ -5,6 +5,7 @@ Names and argument meaning follow the reference: `xpng_store(mode, pm, path)`, `
 here as exceptions carrying xpngb_last_error().
 """
 import ctypes as C
+import math
 import os
 
 import numpy as np
@@ -44,6 +45,17 @@ class _Color(C.Structure):  # xpngb_color: one entry's ColorJitter / RandomGrays
 
 class _Blur(C.Structure):  # xpngb_blur: one entry's GaussianBlur / solarize (see blur_params)
     _fields_ = [("radius", C.c_double * 2), ("solarize", C.c_uint32), ("threshold", C.c_double)]
+
+
+class _AugStep(C.Structure):  # xpngb_aug_step: one step of an entry's augment program (see augment_params)
+    _fields_ = [("data", C.c_double * 6), ("value", C.c_double), ("kind", C.c_uint32), ("arg", C.c_int32), ("fill", C.c_uint8 * 4)]
+
+
+AUG_STEPS_MAX = 8   # XPNGB_AUG_STEPS_MAX
+
+
+class _Augment(C.Structure):  # xpngb_augment: one entry's AutoAugment / RandAugment / TrivialAugmentWide ops
+    _fields_ = [("nsteps", C.c_uint32), ("step", _AugStep * AUG_STEPS_MAX)]
 
 
 class _Xpng(C.Structure):  # xpng_t, xpng.h:10
@@ -102,6 +114,10 @@ def lib():
         L.xpngb_decode_blur.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_Image), C.POINTER(_Rect),
                                         C.POINTER(_Size), C.POINTER(_Rect), C.POINTER(_Color), C.POINTER(_Blur), u32, vp, u64, C.c_int,
                                         C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
+        L.xpngb_decode_augment.restype = C.c_int
+        L.xpngb_decode_augment.argtypes = [vp, C.POINTER(_Tensor), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(_Image),
+                                           C.POINTER(_Rect), C.POINTER(_Size), C.POINTER(_Rect), C.POINTER(_Color), C.POINTER(_Blur),
+                                           C.POINTER(_Augment), u32, vp, u64, C.c_int, C.POINTER(u64), C.POINTER(u64), vp, u64, C.c_int]
         L.xpngb_blur_box.restype = C.c_int
         L.xpngb_blur_box.argtypes = [C.c_double, C.POINTER(C.c_int32), C.POINTER(u32), C.POINTER(u32)]
         L.xpngb_resize_ksize.restype = u32; L.xpngb_resize_ksize.argtypes = [C.c_int, u32, u32]
@@ -329,6 +345,182 @@ def blur_box(radius):
     return ri.value, ww.value, fw.value
 
 
+AUG_KINDS = {"affine": 0, "transpose": 1, "brightness": 2, "color": 3, "contrast": 4, "sharpness": 5, "posterize": 6,
+             "solarize": 7, "autocontrast": 8, "equalize": 9, "invert": 10}   # XPNGB_AUG_*
+AUG_RESAMPLE = {"nearest": 0, "bilinear": 2, "bicubic": 3}                   # PIL.Image.Resampling numbers
+
+
+def _inverse_affine(center, angle, translate, shear):
+    """torchvision's _get_inverse_affine_matrix at scale 1, operation for operation."""
+    rot, sx, sy = math.radians(angle), math.radians(shear[0]), math.radians(shear[1])
+    cx, cy = center
+    tx, ty = translate
+    a = math.cos(rot - sy) / math.cos(sy)
+    b = -math.cos(rot - sy) * math.tan(sx) / math.cos(sy) - math.sin(rot)
+    c = math.sin(rot - sy) / math.cos(sy)
+    d = -math.sin(rot - sy) * math.tan(sx) / math.cos(sy) + math.cos(rot)
+    m = [x / 1.0 for x in (d, -b, 0.0, -c, a, 0.0)]
+    m[2] += m[0] * (-cx - tx) + m[1] * (-cy - ty)
+    m[5] += m[3] * (-cx - tx) + m[4] * (-cy - ty)
+    m[2] += cx
+    m[5] += cy
+    return m
+
+
+def _rotate_matrix(angle, w, h):
+    """Image.rotate's matrix (no expand, centre (w / 2, h / 2)) for angle already reduced mod 360."""
+    angle = -math.radians(angle)
+    m = [round(math.cos(angle), 15), round(math.sin(angle), 15), 0.0, round(-math.sin(angle), 15), round(math.cos(angle), 15), 0.0]
+    cx, cy = w / 2, h / 2
+    m[2], m[5] = m[0] * (-cx - 0) + m[1] * (-cy - 0) + m[2], m[3] * (-cx - 0) + m[4] * (-cy - 0) + m[5]
+    m[2] += cx
+    m[5] += cy
+    return m
+
+
+def _resample_code(interpolation):
+    if isinstance(interpolation, int):
+        if interpolation not in AUG_RESAMPLE.values():
+            raise ValueError(f"unknown augment resample {interpolation!r}: PIL NEAREST 0, BILINEAR 2 or BICUBIC 3")
+        return int(interpolation)
+    name = getattr(interpolation, "value", interpolation)
+    if not isinstance(name, str) or name.lower() not in AUG_RESAMPLE:
+        raise ValueError(f"unknown augment interpolation {interpolation!r}: one of {sorted(AUG_RESAMPLE)}")
+    return AUG_RESAMPLE[name.lower()]
+
+
+def augment_params(steps, size, interpolation="nearest", fill=None):
+    """One entry's xpngb_augment: steps is a list of (op_name, magnitude) exactly as torchvision's
+    transforms.autoaugment._apply_op receives them, size the entry's output (w, h) at that point of the pipeline.  The
+    program is built as torchvision and Pillow build it in Python: _get_inverse_affine_matrix with torchvision's centres
+    (0, 0 for the shears, the image centre otherwise), Image.rotate's angle % 360, its copy / 180 / square 90 and 270
+    transposes and round(., 15), int(magnitude) for translate and posterize, 1 + magnitude factors and _parse_fill's int()."""
+    w, h = int(size[0]), int(size[1])
+    resample = _resample_code(interpolation)
+    if fill is None:
+        fill = 0
+    if isinstance(fill, (int, float)):
+        fill = (fill,) * 3
+    fill = tuple(fill) * 3 if len(fill) == 1 else tuple(fill)
+    if len(fill) != 3:
+        raise ValueError("fill: one value or one per RGB channel")
+    fill = tuple(int(v) for v in fill)
+    if any(not 0 <= v <= 255 for v in fill):
+        raise ValueError(f"fill {fill} is not a byte per channel")
+    aug = _Augment()
+
+    def add(kind, value=0.0, arg=0, data=None):
+        if aug.nsteps == AUG_STEPS_MAX:
+            raise ValueError(f"at most {AUG_STEPS_MAX} augment steps")
+        s = aug.step[aug.nsteps]
+        s.kind, s.value, s.arg = AUG_KINDS[kind], float(value), int(arg)
+        if data is not None:
+            s.data[:] = [float(v) for v in data]
+            s.fill[:] = list(fill) + [0]
+        aug.nsteps += 1
+
+    for name, m in steps:
+        if name == "ShearX":
+            add("affine", arg=resample, data=_inverse_affine([0, 0], 0.0, [0, 0], [math.degrees(math.atan(m)), 0.0]))
+        elif name == "ShearY":
+            add("affine", arg=resample, data=_inverse_affine([0, 0], 0.0, [0, 0], [0.0, math.degrees(math.atan(m))]))
+        elif name in ("TranslateX", "TranslateY"):
+            t = [int(m), 0] if name == "TranslateX" else [0, int(m)]
+            add("affine", arg=resample, data=_inverse_affine([w * 0.5, h * 0.5], 0.0, t, [0.0, 0.0]))
+        elif name == "Rotate":
+            a = m % 360.0
+            if a == 0:
+                continue
+            if a == 180:
+                add("transpose", arg=OPS["mvh"])
+            elif a in (90, 270) and w == h:   # Transpose.ROTATE_90 turns counter-clockwise: r270
+                add("transpose", arg=OPS["r270" if a == 90 else "r90"])
+            else:
+                add("affine", arg=resample, data=_rotate_matrix(a, w, h))
+        elif name in ("Brightness", "Color", "Contrast", "Sharpness"):
+            add(name.lower(), 1.0 + m)
+        elif name == "Posterize":
+            add("posterize", arg=int(m))
+        elif name == "Solarize":
+            add("solarize", m)
+        elif name in ("AutoContrast", "Equalize", "Invert"):
+            add(name.lower())
+        elif name != "Identity":
+            raise ValueError(f"unknown augment op {name!r}")
+    return aug
+
+
+def _replay_op(op_meta, name, magnitude_index, signed_draw):
+    magnitudes, signed = op_meta[name]
+    m = float(magnitudes[magnitude_index].item()) if magnitudes.ndim > 0 else 0.0
+    return name, (-m if signed and signed_draw() else m)
+
+
+def rand_augment_ops(ra, size):
+    """The (op_name, magnitude) list one forward of torchvision's RandAugment module ra passes to _apply_op on a w x h = size
+    image: its draws from torch's global RNG, in forward's order, with the module's own _augmentation_space."""
+    import torch
+    w, h = size
+    op_meta = ra._augmentation_space(ra.num_magnitude_bins, (h, w))
+    steps = []
+    for _ in range(ra.num_ops):
+        name = list(op_meta.keys())[int(torch.randint(len(op_meta), (1,)).item())]
+        steps.append(_replay_op(op_meta, name, ra.magnitude, lambda: torch.randint(2, (1,))))
+    return steps
+
+
+def trivial_augment_wide_ops(ta, size):
+    """The (op_name, magnitude) list of one forward of torchvision's TrivialAugmentWide module ta."""
+    import torch
+    op_meta = ta._augmentation_space(ta.num_magnitude_bins)
+    name = list(op_meta.keys())[int(torch.randint(len(op_meta), (1,)).item())]
+    magnitudes, _ = op_meta[name]
+    idx = torch.randint(len(magnitudes), (1,), dtype=torch.long) if magnitudes.ndim > 0 else None
+    return [_replay_op(op_meta, name, idx, lambda: torch.randint(2, (1,)))]
+
+
+def auto_augment_ops(aa, size):
+    """The (op_name, magnitude) list of one forward of torchvision's AutoAugment module aa (its own get_params and policies)."""
+    w, h = size
+    transform_id, probs, signs = aa.get_params(len(aa.policies))
+    op_meta = aa._augmentation_space(10, (h, w))
+    steps = []
+    for i, (name, p, magnitude_id) in enumerate(aa.policies[transform_id]):
+        if probs[i] <= p:
+            magnitudes, signed = op_meta[name]
+            m = float(magnitudes[magnitude_id].item()) if magnitude_id is not None else 0.0
+            steps.append((name, -m if signed and signs[i] == 0 else m))
+    return steps
+
+
+def rand_augment_steps(ra, size):
+    """The xpngb_augment of one forward of RandAugment module ra on a w x h = size image (rand_augment_ops' draws)."""
+    return augment_params(rand_augment_ops(ra, size), size, ra.interpolation, ra.fill)
+
+
+def trivial_augment_wide_steps(ta, size):
+    """The xpngb_augment of one forward of TrivialAugmentWide module ta on a w x h = size image."""
+    return augment_params(trivial_augment_wide_ops(ta, size), size, ta.interpolation, ta.fill)
+
+
+def auto_augment_steps(aa, size):
+    """The xpngb_augment of one forward of AutoAugment module aa on a w x h = size image."""
+    return augment_params(auto_augment_ops(aa, size), size, aa.interpolation, aa.fill)
+
+
+def augment_array(augs, n):
+    """None, or one entry per file (augment_params(...) or None for no step) -> ctypes array of xpngb_augment, or None."""
+    if augs is None:
+        return None
+    if len(augs) != n:
+        raise ValueError("one augment entry per file")
+    arr = (_Augment * n)()
+    for i, a in enumerate(augs):
+        if a is not None:
+            arr[i] = a
+    return arr
+
+
 def region_tiles(w, h, rect):
     """Tiles a region decode of rect = (x, y, w, h) inside a w x h coded image decodes, and their union (x, y, w, h):
     (0, None) when rect is empty or not inside the image.  Host only."""
@@ -473,6 +665,15 @@ class Codec:
                                    C.c_void_p(out_ptr), out_cap, int(out_dev)):
             raise RuntimeError("xpngb_decode_blur: " + self._err())
 
+    def decode_augment_raw(self, fmt, descs, filt_arr, ops_arr, rect_arr, size_arr, win_arr, color_arr, blur_arr, aug_arr, n, files_ptr,
+                           files_size, files_dev, offs, sizes, out_ptr, out_cap, out_dev):
+        """decode_blur_raw (blur_arr None: no blur) with the augment program aug_arr[i] (see augment_array(); None: none) run
+        on entry i's pixels right after its op, before its colour step."""
+        if lib().xpngb_decode_augment(self._h, None if fmt is None else C.byref(fmt), filt_arr, ops_arr, descs, rect_arr, size_arr,
+                                      win_arr, color_arr, blur_arr, aug_arr, n, C.c_void_p(files_ptr), files_size, int(files_dev), offs,
+                                      sizes, C.c_void_p(out_ptr), out_cap, int(out_dev)):
+            raise RuntimeError("xpngb_decode_augment: " + self._err())
+
     def resize_coeffs(self, filt, inn, out, first=0, count=None):
         """The device's weight tables of an inn -> out axis for output coordinates first .. first + count - 1: (xmin, n) as
         an (count, 2) int32 array and the (count, ksize) int32 weights, zero past each window."""
@@ -487,7 +688,7 @@ class Codec:
         return xn[:count], k[:count, :ksize]
 
     def decode_tensor(self, files, sizes=None, boxes=None, ops=None, dtype=None, layout="chw", scale="div", mean=None, std=None,
-                      drop_alpha=False, filters=None, windows=None, colors=None, blurs=None):
+                      drop_alpha=False, filters=None, windows=None, colors=None, blurs=None, augments=None):
         """list of .xpng byte strings -> one torch tensor on this codec's device, (N, C, H, W) for layout "chw" or (N, H, W, C)
         for "hwc": each whole image, or rectangle boxes[i] = (x, y, w, h) of it, resized to sizes[i] = (w, h) as decode_resized
         does (None: not resized), turned by ops[i] (None: no op), then scaled and normalised as torchvision does, bit for bit:
@@ -497,15 +698,17 @@ class Codec:
         drop_alpha.  filters and windows (only with sizes) as decode_resized: torchvision's Resize(256) + CenterCrop(224) of
         each image is sizes[i], windows[i] = resize_center_crop(w, h, 256, 224).  colors: one color_params(...) or None per
         entry, ColorJitter and RandomGrayscale applied before the conversion (sizes not needed).  blurs: one blur_params(...) or
-        None per entry, GaussianBlur and solarize applied after the colour step (sizes not needed).  Every entry must have the
-        same output shape (ValueError otherwise); ragged batches use decode_tensor_raw, decode_resampled_raw, decode_color_raw
-        or decode_blur_raw."""
+        None per entry, GaussianBlur and solarize applied after the colour step (sizes not needed).  augments: one
+        augment_params(...) (or rand_augment_steps / trivial_augment_wide_steps / auto_augment_steps) or None per entry, run
+        right after the op, before the colour step (sizes not needed).  Every entry must have the same output shape (ValueError
+        otherwise); ragged batches use decode_tensor_raw, decode_resampled_raw, decode_color_raw, decode_blur_raw or
+        decode_augment_raw."""
         import torch
         n = len(files)
         if n == 0:
             raise ValueError("decode_tensor needs at least one file")
         for name, arg in (("size", sizes), ("rectangle", boxes), ("op", ops), ("window", windows), ("colour entry", colors),
-                          ("blur entry", blurs)):
+                          ("blur entry", blurs), ("augment entry", augments)):
             if arg is not None and len(arg) != n:
                 raise ValueError(f"one {name} per file")
         if sizes is None and (filters is not None or windows is not None):
@@ -535,7 +738,10 @@ class Codec:
         # the library writes on its own stream: memory fresh from the caching allocator may still be in use by queued work
         torch.cuda.current_stream(dev).synchronize()
         oa = None if ops is None else op_codes(ops)
-        if blurs is not None:
+        if augments is not None:
+            self.decode_augment_raw(fmt, descs, fa, oa, ra, sa, wa, color_array(colors, n), blur_array(blurs, n), augment_array(augments, n),
+                                    n, fb.ctypes.data, off, 0, foffs, fsizes, flat.data_ptr(), n * stride * DTYPE_BYTES[dname], 1)
+        elif blurs is not None:
             self.decode_blur_raw(fmt, descs, fa, oa, ra, sa, wa, color_array(colors, n), blur_array(blurs, n), n, fb.ctypes.data, off, 0,
                                  foffs, fsizes, flat.data_ptr(), n * stride * DTYPE_BYTES[dname], 1)
         elif colors is not None:
@@ -635,7 +841,7 @@ class Codec:
             self.decode_oriented_raw(descs, op_codes(ops), ra, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         return self._unpack(px, descs, [(r.w, r.h) for r in ra], ops)
 
-    def decode_resized(self, files, sizes, boxes=None, ops=None, filters=None, windows=None, colors=None, blurs=None):
+    def decode_resized(self, files, sizes, boxes=None, ops=None, filters=None, windows=None, colors=None, blurs=None, augments=None):
         """list of .xpng byte strings and one (w, h) output size per file -> list of (h, w, 3|4) uint8 arrays: each whole image,
         or rectangle boxes[i] = (x, y, w, h) of it, resampled as Pillow's Image.resize((w, h), filter) does, every channel on
         its own (alpha is not premultiplied).  filters: None (bilinear), one filter for all entries or one per entry, each a
@@ -643,7 +849,8 @@ class Codec:
         entry in the resized image's coordinates, the part of it that is returned (None: all of it).  ops: one OPS name per
         entry, applied last; 'r90' and 'r270' entries come back as (w, h, 3|4).  An entry whose size equals its crop is the
         crop itself.  colors: one color_params(...) or None per entry, ColorJitter and RandomGrayscale applied to its pixels.
-        blurs: one blur_params(...) or None per entry, GaussianBlur and solarize applied to its pixels after the colour step."""
+        blurs: one blur_params(...) or None per entry, GaussianBlur and solarize applied to its pixels after the colour step.
+        augments: one augment_params(...) or None per entry, run on its pixels right after the op, before the colour step."""
         n = len(files)
         if len(sizes) != n:
             raise ValueError("one size per file")
@@ -655,13 +862,17 @@ class Codec:
             raise ValueError("one window per file")
         ca = color_array(colors, n)
         ba = blur_array(blurs, n)
+        aa = augment_array(augments, n)
         ra = None if boxes is None else rects(boxes)
         sa = _sizes(sizes)
         wa = None if windows is None else rects(windows)
         fa = filter_codes(filters, n)
         oa = None if ops is None else op_codes(ops)
         descs, foffs, fsizes, fb, off, px, poff = self._pack_files(files, ra, sa, wa)
-        if ba is not None:
+        if aa is not None:
+            self.decode_augment_raw(None, descs, fa, oa, ra, sa, wa, ca, ba, aa, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data,
+                                    poff, 0)
+        elif ba is not None:
             self.decode_blur_raw(None, descs, fa, oa, ra, sa, wa, ca, ba, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)
         elif ca is not None:
             self.decode_color_raw(None, descs, fa, oa, ra, sa, wa, ca, n, fb.ctypes.data, off, 0, foffs, fsizes, px.ctypes.data, poff, 0)

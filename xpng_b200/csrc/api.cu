@@ -35,6 +35,7 @@
 #include "tensor.cuh"
 #include "color.cuh"
 #include "blur.cuh"
+#include "augment.cuh"
 
 using namespace xpb;
 
@@ -79,7 +80,8 @@ struct xpngb_ctx {
         rdescs, rtab, rtmp,   // resized decode: ResizeDesc of the lane's chunk, windows and weights, the first pass's rows
         tdescs, tsrc,         // tensor decode: TensorDesc of the lane's chunk, the resized (and coloured) entries' pixels
         cdescs,               // colour decode: ColorDesc of the lane's chunk, then one 64-bit luma sum per descriptor
-        bdescs, bscr;         // blurred decode: BlurPass of the lane's chunk, the second buffer of each entry's ping-pong
+        bdescs, bscr,         // blurred decode: BlurPass of the lane's chunk, the second buffer of each entry's ping-pong
+        adescs;               // augmented decode: the chunk's AugPix, ColorDesc, luma sums, AugLut and histograms, stage by stage
     PinBuf pin_a, pin_b, pin_o;   // pin_o: orientation descriptors (their upload may still be in flight when an encode reuses pin_a)
 };
 
@@ -400,7 +402,7 @@ static void lane_free(xpngb_ctx* ctx) {
                       &ctx->offs, &ctx->m2a, &ctx->m2b, &ctx->tclass, &ctx->tabs, &ctx->ccnt, &ctx->cbit, &ctx->resv, &ctx->oriented,
                       &ctx->odesc, &ctx->pdw, &ctx->eord, &ctx->region, &ctx->crops, &ctx->orients,
                       &ctx->rdescs, &ctx->rtab, &ctx->rtmp, &ctx->tdescs, &ctx->tsrc, &ctx->cdescs,
-                      &ctx->bdescs, &ctx->bscr };
+                      &ctx->bdescs, &ctx->bscr, &ctx->adescs };
     for (DevBuf* b : all) if (b->p) cudaFree(b->p);
     if (ctx->pin_a.p) cudaFreeHost(ctx->pin_a.p);
     if (ctx->pin_b.p) cudaFreeHost(ctx->pin_b.p);
@@ -1088,6 +1090,19 @@ static uint32_t solarize_t(double threshold) {
 // the op turns the entry a quarter: its output's x axis is the staged pixels' y axis
 static bool quarter(const int* ops, uint32_t i) { return ops && (ops[i] == OP_R90 || ops[i] == OP_R270); }
 
+// C's (int) of a double as Pillow's x86-64 build computes it (cvttsd2si): INT_MIN for NaN and out of range
+static int32_t x86_int(double v) { return v > -2147483649.0 && v < 2147483648.0 ? (int32_t)v : INT32_MIN; }
+// Geometry.c's FIX: 16.16 fixed point, FLOOR(v * 65536.0 + 0.5)
+static int32_t pil_fix(double v) { const double t = v * 65536.0 + 0.5; return t < 0.0 ? x86_int(floor(t)) : x86_int(t); }
+// check_fixed at the four corners of a W x H output: affine_fixed's 16.16 arithmetic can hold every source coordinate
+static bool affine_fixed_ok(const double* a, double W, double H) {
+    const double cx[4] = { 0.0, W, 0.0, W }, cy[4] = { 0.0, H, H, 0.0 };
+    for (int k = 0; k < 4; k++)
+        if (!(fabs(cx[k] * a[0] + cy[k] * a[1] + a[2]) < 32768.0 && fabs(cx[k] * a[3] + cy[k] * a[4] + a[5]) < 32768.0)) return false;
+    return true;
+}
+constexpr uint32_t AUG_STAGES = XPNGB_AUG_STEPS_MAX + 1;   // a uint8 entry whose last step wrote its scratch gets one copy back
+
 // Launch the decode of one chunk on lane `ctx`.  DI: the checked images of the chunk.  `lat`: warp-per-block chain
 // kernels (few blocks in the whole call) instead of the pair decoders.  sel == nullptr: every tile of every image, in
 // place.  Otherwise a region decode: only the tiles of sel[i].s, written in place when the rectangle is made of whole
@@ -1105,8 +1120,8 @@ static bool quarter(const int* ops, uint32_t i) { return ops && (ops[i] == OP_R9
 // entry's k_to_tensor reads whichever buffer its last pass wrote, a uint8 entry's passes end at its output.  Never waits
 // for the device.
 static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
-                        const xpngb_tensor* fmt, const xpngb_color* colors, const xpngb_blur* blurs, uint32_t n, const uint8_t* din,
-                        uint8_t* dpx, uint32_t call_tiles) {
+                        const xpngb_tensor* fmt, const xpngb_color* colors, const xpngb_blur* blurs, const xpngb_augment* augs,
+                        uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
@@ -1116,12 +1131,18 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     std::vector<TensorDesc> tdescs;
     std::vector<ColorDesc> cdescs;
     std::vector<BlurPass> bstage[BLUR_STAGES];   // the k-th pass of every blurred entry is in bstage[k]
+    std::vector<AugPix> apix[AUG_STAGES];        // step k of every augmented entry, by kind: warps and SHARPNESS,
+    std::vector<ColorDesc> acol[AUG_STAGES];     // BRIGHTNESS, COLOR and CONTRAST,
+    std::vector<AugLut> alut[AUG_STAGES];        // and the LUT steps
+    uint64_t apctas[AUG_STAGES] = {}, acctas[AUG_STAGES] = {}, amctas[AUG_STAGES] = {}, alctas[AUG_STAGES] = {}, ahctas[AUG_STAGES] = {};
+    uint32_t anhist[AUG_STAGES] = {};
     uint64_t octas = 0, rcoef = 0, rh = 0, rv = 0, tctas = 0, cctas = 0, mctas = 0;
     bool any1 = false, any2 = false, any7 = false;
     for (uint32_t i = 0; i < n; i++) { any1 |= DI[i].mode == 1; any2 |= DI[i].mode == 2; any7 |= DI[i].mode == 7; }
     auto colored = [&](uint32_t i) { return colors && (colors[i].on || colors[i].gray); };
     auto blurred = [&](uint32_t i) { return blurs && blur_on(blurs[i]); };
-    auto staged = [&](uint32_t i) { return colored(i) || blurred(i); };   // needs its uint8 pixels to work on
+    auto augmented = [&](uint32_t i) { return augs && augs[i].nsteps; };
+    auto staged = [&](uint32_t i) { return colored(i) || blurred(i) || augmented(i); };   // needs its uint8 pixels to work on
     // pixels entry i writes: its resampled window, or its rectangle
     auto out_px = [&](uint32_t i) -> uint64_t { return sel[i].rs ? sel[i].win.w * sel[i].win.h : sel[i].rect.w * sel[i].rect.h; };
     // uint8 pixels of a resized or staged tensor entry, or of a blurred entry's scratch (16-byte aligned)
@@ -1133,7 +1154,7 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs || fmt)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
             if (rs) { tab += resize_tab_bytes(sel[i]); tmp += resize_tmp_bytes(sel[i], DI[i].pxsz); }
             if ((rs || staged(i)) && fmt) tsz += tsrc_bytes(i);
-            if (blurred(i)) bsz += tsrc_bytes(i);
+            if (blurred(i) || augmented(i)) bsz += tsrc_bytes(i);
         }
         if (need) ENSURE(region, need);
         if (tab) ENSURE(rtab, tab);
@@ -1204,12 +1225,10 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     // blurred entry i: its w x h packed pixels at px go through its passes, ping-ponged with its scratch; *res is where the
     // last pass leaves them.  swap: the entry is staged un-turned and k_to_tensor turns it a quarter, so the passes of the
     // output's x axis run along the staged columns, first.
-    uint64_t bpos = 0;
-    auto blur_desc = [&](uint32_t i, uint8_t* px, uint64_t w, uint64_t h, bool swap, uint8_t** res) -> int {
+    auto blur_desc = [&](uint32_t i, uint8_t* px, uint8_t* scr, uint64_t w, uint64_t h, bool swap, uint8_t** res) -> int {
         const xpngb_blur& b = blurs[i];
         const uint32_t pxsz = DI[i].pxsz;
-        uint8_t* const buf[2] = { px, (uint8_t*)ctx->bscr.p + bpos };
-        bpos += tsrc_bytes(i);
+        uint8_t* const buf[2] = { px, scr };
         uint32_t k = 0;
         auto pass = [&](uint32_t vert, const BlurBox& bx) {
             BlurPass& p = bstage[k].emplace_back();
@@ -1231,8 +1250,82 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         *res = buf[k & 1];
         return 0;
     };
+    // augmented entry i: its w x h staged pixels at px, turned by eop into the output image, go through its program; the
+    // warps and SHARPNESS ping-pong with its scratch scr, and *res is where the last step leaves the pixels (px for a uint8
+    // entry, whose eop is OP_TL: its pixels are staged as written)
+    auto aug_desc = [&](uint32_t i, uint8_t* px, uint8_t* scr, uint64_t w, uint64_t h, uint32_t eop, uint8_t** res) -> int {
+        const xpngb_augment& A = augs[i];
+        const uint32_t pxsz = DI[i].pxsz;
+        const uint64_t npx = w * h;
+        const bool q = eop == OP_R90 || eop == OP_R270;
+        const double W = (double)(q ? h : w), H = (double)(q ? w : h);
+        uint8_t *cur = px, *other = scr;
+        auto pix = [&](uint32_t k, uint32_t mode) -> AugPix& {
+            AugPix& d = apix[k].emplace_back();
+            d.src = (uint64_t)cur; d.dst = (uint64_t)other; d.w = (uint32_t)w; d.h = (uint32_t)h; d.pxsz = pxsz; d.eop = eop; d.mode = mode;
+            d.first_cta = (uint32_t)apctas[k];
+            apctas[k] += (npx + AP_THREADS - 1) / AP_THREADS;
+            uint8_t* t = cur; cur = other; other = t;
+            return d;
+        };
+        for (uint32_t k = 0; k < A.nsteps; k++) {
+            const xpngb_aug_step& s = A.step[k];
+            const double* a = s.data;
+            if (s.kind == XPNGB_AUG_AFFINE) {
+                const uint32_t mode = s.arg == 2 ? AP_BILINEAR : s.arg == 3 ? AP_BICUBIC
+                                      : a[1] != 0.0 || a[3] != 0.0 ? (affine_fixed_ok(a, W, H) ? AP_FIXED : AP_SEQ) : AP_SEQ;
+                AugPix& d = pix(k, mode);
+                memcpy(d.fill, s.fill, 4);
+                if (mode == AP_FIXED) {
+                    const double v[6] = { a[0], a[1], a[2] + a[0] * 0.5 + a[1] * 0.5, a[3], a[4], a[5] + a[3] * 0.5 + a[4] * 0.5 };
+                    for (int c = 0; c < 6; c++) d.fx[c] = pil_fix(v[c]);
+                } else if (mode == AP_SEQ && a[1] == 0.0 && a[3] == 0.0) {   // ImagingScaleAffine: x per column, y per row
+                    const double v[6] = { a[2] + a[0] * 0.5, 0.0, a[0], a[5] + a[4] * 0.5, a[4], 0.0 };
+                    memcpy(d.a, v, sizeof v);
+                } else if (mode == AP_SEQ) {   // ImagingTransformAffine's double path
+                    const double v[6] = { a[2] + a[1] * 0.5 + a[0] * 0.5, a[1], a[0], a[5] + a[4] * 0.5 + a[3] * 0.5, a[4], a[3] };
+                    memcpy(d.a, v, sizeof v);
+                } else memcpy(d.a, a, sizeof d.a);
+            } else if (s.kind == XPNGB_AUG_TRANSPOSE) {
+                pix(k, AP_TRANSPOSE).top = (uint32_t)s.arg;
+            } else if (s.kind == XPNGB_AUG_SHARPNESS) {
+                pix(k, AP_SHARP).fac = (float)s.value;
+            } else if (s.kind == XPNGB_AUG_BRIGHTNESS || s.kind == XPNGB_AUG_COLOR || s.kind == XPNGB_AUG_CONTRAST) {
+                const uint32_t step = s.kind == XPNGB_AUG_BRIGHTNESS ? XPNGB_CJ_BRIGHTNESS : s.kind == XPNGB_AUG_COLOR ? XPNGB_CJ_SATURATION
+                                                                                                                    : XPNGB_CJ_CONTRAST;
+                ColorDesc d{};   // colour decode with this one step on
+                d.px = (uint64_t)cur; d.npx = npx; d.pxsz = pxsz; d.on = 1u << step;
+                d.fac[step] = (float)s.value;
+                for (uint32_t c = 0; c < 4; c++) d.order[c] = (uint8_t)c;
+                d.pre = XPNGB_CJ_CONTRAST;
+                d.first_cta = (uint32_t)acctas[k]; d.mfirst_cta = (uint32_t)amctas[k];
+                const uint64_t ctas = (npx + CL_PX - 1) / CL_PX;
+                acctas[k] += ctas;
+                if (step == XPNGB_CJ_CONTRAST) amctas[k] += ctas;
+                acol[k].push_back(d);
+            } else {
+                AugLut& d = alut[k].emplace_back();
+                d.px = (uint64_t)cur; d.npx = npx; d.pxsz = pxsz; d.kind = s.kind; d.hist = 0;
+                d.first_cta = (uint32_t)alctas[k]; d.hfirst_cta = (uint32_t)ahctas[k];
+                alctas[k] += (npx + CL_PX - 1) / CL_PX;
+                const uint32_t t = solarize_t(s.value), keep = s.kind == XPNGB_AUG_POSTERIZE ? ~((1u << (8 - s.arg)) - 1) : 255u;
+                for (uint32_t v = 0; v < 256; v++) {
+                    const uint32_t o = s.kind == XPNGB_AUG_POSTERIZE ? v & keep : s.kind == XPNGB_AUG_SOLARIZE ? (v < t ? v : 255 - v) : 255 - v;
+                    d.lut[v] = d.lut[256 + v] = d.lut[512 + v] = (uint8_t)o;
+                }
+                if (s.kind == XPNGB_AUG_EQUALIZE || s.kind == XPNGB_AUG_AUTOCONTRAST) {   // from the histograms, on the device
+                    d.hist = 1 + anhist[k]++;   // the histogram's number + 1 until the layout is known
+                    ahctas[k] += (npx + AH_PX - 1) / AH_PX;
+                }
+            }
+            if (apctas[k] > 0x7FFFFFFFull || acctas[k] > 0x7FFFFFFFull || alctas[k] > 0x7FFFFFFFull) FAIL("too many pixels for one augment launch");
+        }
+        if (!fmt && cur != px) pix(A.nsteps, AP_TRANSPOSE).top = OP_TL;   // a uint8 entry's result belongs at its output
+        *res = cur;
+        return 0;
+    };
     // entry i of a region call: its rectangle at src (rows `pitch` bytes apart) cropped, turned, resized or made a tensor
-    uint64_t spos = 0;
+    uint64_t spos = 0, bpos = 0;
     auto region_out = [&](uint32_t i, uint64_t src, uint64_t pitch, uint8_t* out) -> int {
         const xpngb_rect& r = sel[i].rect;
         const uint32_t pxsz = DI[i].pxsz;
@@ -1242,8 +1335,15 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             const uint64_t w = sel[i].rs ? sel[i].win.w : r.w, h = sel[i].rs ? sel[i].win.h : r.h;
             if (sel[i].rs) { if (resize_desc(i, src, pitch, t, OP_TL)) return 1; }
             else crops.push_back(CropDesc{ src, (uint64_t)t, pitch, (uint32_t)(r.w * pxsz), (uint32_t)r.h });
+            uint8_t* scr = nullptr;
+            if (blurred(i) || augmented(i)) { scr = (uint8_t*)ctx->bscr.p + bpos; bpos += tsrc_bytes(i); }
+            if (augmented(i)) {   // the blur then ping-pongs between the buffer the program ended in and the other one
+                uint8_t* r;
+                if (aug_desc(i, t, scr, w, h, ops ? (uint32_t)ops[i] : (uint32_t)OP_TL, &r)) return 1;
+                if (r != t) { scr = t; t = r; }
+            }
             if (colored(i) && color_desc(i, t, w * h)) return 1;
-            if (blurred(i) && blur_desc(i, t, w, h, quarter(ops, i), &t)) return 1;
+            if (blurred(i) && blur_desc(i, t, scr, w, h, quarter(ops, i), &t)) return 1;
             return tensor_desc(i, (uint64_t)t, w * pxsz, w, h, out);
         }
         if (fmt) return tensor_desc(i, src, pitch, r.w, r.h, out);
@@ -1283,12 +1383,14 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             D.nrows = (uint32_t)(R.s.r1 - R.s.r0 + 1); D.ncols = (uint32_t)(R.s.c1 - R.s.c0 + 1);
         }
         D.tile0 = P.imgs[i].tile0; D.ntiles = P.imgs[i].ntiles;
-        if (!fmt && colored(i) && color_desc(i, out, out_px(i))) return 1;   // uint8 output: coloured where it is written
-        if (!fmt && blurred(i)) {   // and blurred there, in the output's orientation
+        if (!fmt && (augmented(i) || colored(i) || blurred(i))) {   // uint8 output: changed where it is written, as written
             uint64_t w = sel[i].rs ? sel[i].win.w : sel[i].rect.w, h = sel[i].rs ? sel[i].win.h : sel[i].rect.h;
             if (quarter(ops, i)) { const uint64_t t = w; w = h; h = t; }
-            uint8_t* res;
-            if (blur_desc(i, out, w, h, false, &res)) return 1;
+            uint8_t *scr = nullptr, *res;
+            if (blurred(i) || augmented(i)) { scr = (uint8_t*)ctx->bscr.p + bpos; bpos += tsrc_bytes(i); }
+            if (augmented(i) && aug_desc(i, out, scr, w, h, OP_TL, &res)) return 1;
+            if (colored(i) && color_desc(i, out, out_px(i))) return 1;
+            if (blurred(i) && blur_desc(i, out, scr, w, h, false, &res)) return 1;
         }
     }
     // blur passes stage by stage, each stage's CTAs numbered from 0
@@ -1304,6 +1406,27 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         bpasses += bstage[k].size();
         if (!bstage[k].empty()) nstage = k + 1;
     }
+    // augment stages in the lane's adescs: first every stage's AugPix, ColorDesc and AugLut (uploaded), then every stage's
+    // luma sums and histograms (zeroed)
+    struct AugAt { size_t pix, col, lut, sum, hist; };
+    AugAt aat[AUG_STAGES] = {};
+    size_t adesc_bytes = 0, azero_bytes = 0;
+    uint32_t anstage = 0;
+    for (uint32_t k = 0; k < AUG_STAGES; k++) {
+        aat[k].pix = adesc_bytes; adesc_bytes += apix[k].size() * sizeof(AugPix);
+        aat[k].col = adesc_bytes; adesc_bytes += acol[k].size() * sizeof(ColorDesc);
+        aat[k].lut = adesc_bytes; adesc_bytes += alut[k].size() * sizeof(AugLut);
+        aat[k].sum = azero_bytes; azero_bytes += acol[k].size() * 8;
+        aat[k].hist = azero_bytes; azero_bytes += (size_t)anhist[k] * 3 * 256 * 8;
+        if (!apix[k].empty() || !acol[k].empty() || !alut[k].empty()) anstage = k + 1;
+    }
+    adesc_bytes = (adesc_bytes + 15) & ~(size_t)15;
+    if (anstage) {
+        ENSURE(adescs, adesc_bytes + azero_bytes);
+        uint8_t* zero = (uint8_t*)ctx->adescs.p + adesc_bytes;
+        for (uint32_t k = 0; k < anstage; k++)
+            for (AugLut& d : alut[k]) if (d.hist) d.hist = (uint64_t)(zero + aat[k].hist + (d.hist - 1) * 3 * 256 * 8);
+    }
     if (P.tiles.size() > (1u << 24) || P.seg_tile.size() > (1u << 28)) FAIL("too many tiles for one chunk (%zu)", P.tiles.size());
     const uint32_t ntiles = (uint32_t)P.tiles.size();
     if (upload_plan(ctx, P)) return 1;
@@ -1312,7 +1435,8 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     const size_t pin_crops = n * (sizeof(DecImage) + 8) + 64, pin_orients = pin_crops + crops.size() * sizeof(CropDesc);
     const size_t pin_resize = pin_orients + odescs.size() * sizeof(OrientDesc), pin_tensor = pin_resize + rdescs.size() * sizeof(ResizeDesc);
     const size_t pin_color = pin_tensor + tdescs.size() * sizeof(TensorDesc), pin_blur = pin_color + cdescs.size() * sizeof(ColorDesc);
-    if (ensure_pin(ctx, ctx->pin_b, pin_blur + bpasses * sizeof(BlurPass))) return 1;
+    const size_t pin_aug = pin_blur + bpasses * sizeof(BlurPass);
+    if (ensure_pin(ctx, ctx->pin_b, pin_aug + (anstage ? adesc_bytes : 0))) return 1;
     memcpy(ctx->pin_b.p, DI.data(), n * sizeof(DecImage));
     CK(cudaMemcpyAsync(ctx->dimgs.p, ctx->pin_b.p, n * sizeof(DecImage), cudaMemcpyHostToDevice, ctx->stream));
     if (any7 && !sel) {   // where each stored image's file starts (k_load7), ~0 = not a stored image
@@ -1359,6 +1483,16 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             at += bstage[k].size() * sizeof(BlurPass);
         }
         CK(cudaMemcpyAsync(ctx->bdescs.p, (uint8_t*)ctx->pin_b.p + pin_blur, bpasses * sizeof(BlurPass), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (anstage) {
+        uint8_t* pa = (uint8_t*)ctx->pin_b.p + pin_aug;
+        for (uint32_t k = 0; k < anstage; k++) {
+            memcpy(pa + aat[k].pix, apix[k].data(), apix[k].size() * sizeof(AugPix));
+            memcpy(pa + aat[k].col, acol[k].data(), acol[k].size() * sizeof(ColorDesc));
+            memcpy(pa + aat[k].lut, alut[k].data(), alut[k].size() * sizeof(AugLut));
+        }
+        CK(cudaMemcpyAsync(ctx->adescs.p, pa, adesc_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        if (azero_bytes) CK(cudaMemsetAsync((uint8_t*)ctx->adescs.p + adesc_bytes, 0, azero_bytes, ctx->stream));
     }
     CK(cudaMemsetAsync(ctx->errflag.p, 0, 4, ctx->stream));
     CK(cudaMemsetAsync(ctx->dtiles.p, 0, ntiles * sizeof(DecTile), ctx->stream));
@@ -1564,6 +1698,24 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         if (rh) LAUNCH(k_resize_h, (unsigned)rh, RH_X, 0, d_rd, nr);
         if (rv) LAUNCH(k_resize_v, (unsigned)rv, RV_X, 0, d_rd, nr, vfirst ? 2u : 3u);
     }
+    for (uint32_t k = 0; k < anstage; k++) {   // augment step k of every entry that has one, before the colour
+        uint8_t* const ad = (uint8_t*)ctx->adescs.p;
+        if (!apix[k].empty()) LAUNCH(k_aug_pix, (unsigned)apctas[k], AP_THREADS, 0, (const AugPix*)(ad + aat[k].pix), (uint32_t)apix[k].size());
+        if (!acol[k].empty()) {
+            const ColorDesc* d_cd = (const ColorDesc*)(ad + aat[k].col);
+            unsigned long long* d_sum = (unsigned long long*)(ad + adesc_bytes + aat[k].sum);
+            if (amctas[k]) LAUNCH(k_color_mean, (unsigned)amctas[k], 256, 0, d_cd, (uint32_t)acol[k].size(), d_sum);
+            LAUNCH(k_color, (unsigned)acctas[k], 256, 0, d_cd, (uint32_t)acol[k].size(), (const unsigned long long*)d_sum);
+        }
+        if (!alut[k].empty()) {
+            AugLut* d_al = (AugLut*)(ad + aat[k].lut);
+            if (ahctas[k]) {
+                LAUNCH(k_aug_hist, (unsigned)ahctas[k], 256, 0, d_al, (uint32_t)alut[k].size());
+                LAUNCH(k_aug_lut_build, (unsigned)alut[k].size(), 256, 0, d_al);
+            }
+            LAUNCH(k_aug_lut, (unsigned)alctas[k], 256, 0, d_al, (uint32_t)alut[k].size());
+        }
+    }
     if (!cdescs.empty()) {   // the contrast means first, then every coloured entry's chain
         const ColorDesc* d_cd = (const ColorDesc*)ctx->cdescs.p;
         unsigned long long* d_sum = (unsigned long long*)((uint8_t*)ctx->cdescs.p + csum);
@@ -1584,7 +1736,7 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
 // image.  With colors, xpngb_decode_color.
 static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rects, const int* ops, const xpngb_size* sizes,
                        const int* filters, const xpngb_rect* windows, const xpngb_tensor* fmt, const xpngb_color* colors,
-                       const xpngb_blur* blurs, uint32_t n, const void* files,
+                       const xpngb_blur* blurs, const xpngb_augment* augs, uint32_t n, const void* files,
                        uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
                        uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
@@ -1630,6 +1782,28 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             if (b.solarize > 1) FAIL("entry %u: solarize %u is neither 0 nor 1", i, b.solarize);
             if (b.threshold != b.threshold) FAIL("entry %u: solarize threshold is NaN", i);
         }
+        if (augs) {
+            const xpngb_augment& A = augs[i];
+            if (A.nsteps > XPNGB_AUG_STEPS_MAX) FAIL("entry %u: %u augment steps, above %d", i, A.nsteps, XPNGB_AUG_STEPS_MAX);
+            for (uint32_t k = 0; k < A.nsteps; k++) {
+                const xpngb_aug_step& s = A.step[k];
+                if (s.kind > XPNGB_AUG_INVERT) FAIL("entry %u: augment step %u has unknown kind %u", i, k, s.kind);
+                if (s.kind == XPNGB_AUG_AFFINE) {
+                    if (s.arg != 0 && s.arg != 2 && s.arg != 3)
+                        FAIL("entry %u: augment step %u has unknown resample %d (NEAREST 0, BILINEAR 2, BICUBIC 3)", i, k, s.arg);
+                    for (int c = 0; c < 6; c++)   // below 2^64 no running sum or product of Pillow's can reach infinity
+                        if (!(fabs(s.data[c]) < 18446744073709551616.0))
+                            FAIL("entry %u: augment step %u matrix coefficient %g is not finite or not below 2^64", i, k, s.data[c]);
+                }
+                if (s.kind == XPNGB_AUG_TRANSPOSE && (s.arg < OP_R90 || s.arg > OP_TR))
+                    FAIL("entry %u: augment step %u transpose %d is not an op code", i, k, s.arg);
+                if (s.kind >= XPNGB_AUG_BRIGHTNESS && s.kind <= XPNGB_AUG_SHARPNESS && !(s.value >= 0.0 && s.value <= 3.4028234663852886e38))
+                    FAIL("entry %u: augment step %u factor %g is negative or not finite", i, k, s.value);   // Pillow narrows it to a float
+                if (s.kind == XPNGB_AUG_POSTERIZE && (s.arg < 0 || s.arg > 8))
+                    FAIL("entry %u: augment step %u posterize bits %d are not in 0..8", i, k, s.arg);
+                if (s.kind == XPNGB_AUG_SOLARIZE && s.value != s.value) FAIL("entry %u: augment step %u solarize threshold is NaN", i, k);
+            }
+        }
     }
     const uint8_t* din = (const uint8_t*)files;
     if (!files_on_device) { ENSURE(files, files_size); din = (const uint8_t*)ctx->files.p; }
@@ -1648,7 +1822,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     }
     // ---- every entry is checked before anything is decoded
     std::vector<DecImage> DI(n);
-    const bool use_sel = rects || ops || sizes || fmt || colors || blurs;
+    const bool use_sel = rects || ops || sizes || fmt || colors || blurs || augs;
     std::vector<RegionSel> sel(use_sel ? n : 0);
     for (uint32_t i = 0; i < n; i++) {
         if (decode_check(ctx, i, imgs[i], &hdr[2 * i], file_offsets[i], file_sizes[i], rects ? rects + i : nullptr, sizes ? sizes + i : nullptr,
@@ -1657,6 +1831,8 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             FAIL("entry %u: grayscale of an RGBA entry whose output keeps alpha (torchvision's RandomGrayscale refuses 4 channels)", i);
         if (blurs && blurs[i].solarize && imgs[i].A && (!fmt || fmt->channels == 0))
             FAIL("entry %u: solarize of an RGBA entry whose output keeps alpha (ImageOps.solarize refuses RGBA)", i);
+        if (augs && augs[i].nsteps && imgs[i].A && (!fmt || fmt->channels == 0))
+            FAIL("entry %u: augment of an RGBA entry whose output keeps alpha (Pillow's ImageOps refuse RGBA)", i);
         if (use_sel) {
             RegionSel& R = sel[i];
             R.rect = rects ? rects[i] : xpngb_rect{ 0, 0, imgs[i].w, imgs[i].h };
@@ -1677,6 +1853,13 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
                 R.rect = xpngb_rect{ R.crop.x + x0, R.crop.y + y0, x1 - x0, y1 - y0 };
             }
             region_select(imgs[i].w, imgs[i].h, R.rect, R.g, R.s, R.cover);
+            const uint64_t ow = sizes ? R.win.w : R.rect.w, oh = sizes ? R.win.h : R.rect.h;
+            for (uint32_t k = 0; augs && k < augs[i].nsteps; k++) {
+                const xpngb_aug_step& s = augs[i].step[k];
+                if (s.kind == XPNGB_AUG_TRANSPOSE && (s.arg == OP_R90 || s.arg == OP_R270) && ow != oh)
+                    FAIL("entry %u: augment step %u turns a %llux%llu output a quarter (Image.rotate does that for squares only)", i, k,
+                         (unsigned long long)ow, (unsigned long long)oh);
+            }
         }
     }
     uint8_t* dpx = (uint8_t*)pixels;
@@ -1729,7 +1912,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
             }
         }
         rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr,
-                          fmt, colors ? colors + i0 : nullptr, blurs ? blurs + i0 : nullptr, m, din, dpx,
+                          fmt, colors ? colors + i0 : nullptr, blurs ? blurs + i0 : nullptr, augs ? augs + i0 : nullptr, m, din, dpx,
                           (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
         if (!rc && !pixels_on_device) {
             uint64_t lo = ~0ull, hi = 0;
@@ -1764,7 +1947,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
 extern "C" int xpngb_decode(xpngb_ctx* ctx, xpngb_image* imgs, uint32_t n, const void* files, uint64_t files_size, int files_on_device,
                             const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap,
                             int pixels_on_device) {
-    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1773,7 +1956,7 @@ extern "C" int xpngb_decode_region(xpngb_ctx* ctx, xpngb_image* imgs, const xpng
                                    void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!rects) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1782,7 +1965,7 @@ extern "C" int xpngb_decode_oriented(xpngb_ctx* ctx, const int* ops, xpngb_image
                                      const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!ops) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1791,7 +1974,7 @@ extern "C" int xpngb_decode_resized(xpngb_ctx* ctx, const int* ops, xpngb_image*
                                     const uint64_t* file_sizes, void* pixels, uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
     if (!sizes) { ctx->err[0] = 0; FAIL("null argument"); }
-    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, pixels, pixels_cap,
                        pixels_on_device);
 }
 
@@ -1817,7 +2000,7 @@ extern "C" int xpngb_decode_tensor(xpngb_ctx* ctx, const xpngb_tensor* fmt, cons
     if (!ctx) return 1;
     ctx->err[0] = 0;
     if (tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, fmt, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
+    return decode_call(ctx, imgs, rects, ops, sizes, nullptr, nullptr, fmt, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes, out, out_cap,
                        out_on_device);
 }
 
@@ -1829,7 +2012,7 @@ extern "C" int xpngb_decode_resampled(xpngb_ctx* ctx, const xpngb_tensor* fmt, c
     ctx->err[0] = 0;
     if (!sizes) FAIL("null argument (sizes)");
     if (fmt && tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes,
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, nullptr, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets, file_sizes,
                        out, out_cap, out_on_device);
 }
 
@@ -1841,7 +2024,7 @@ extern "C" int xpngb_decode_color(xpngb_ctx* ctx, const xpngb_tensor* fmt, const
     ctx->err[0] = 0;
     if (!sizes && (filters || windows)) FAIL("null argument (sizes): filters and windows need sizes");
     if (fmt && tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, nullptr, n, files, files_size, files_on_device, file_offsets,
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, nullptr, nullptr, n, files, files_size, files_on_device, file_offsets,
                        file_sizes, out, out_cap, out_on_device);
 }
 
@@ -1853,8 +2036,21 @@ extern "C" int xpngb_decode_blur(xpngb_ctx* ctx, const xpngb_tensor* fmt, const 
     ctx->err[0] = 0;
     if (!sizes && (filters || windows)) FAIL("null argument (sizes): filters and windows need sizes");
     if (fmt && tensor_check(ctx, fmt)) return 1;
-    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, blurs, n, files, files_size, files_on_device, file_offsets,
-                       file_sizes, out, out_cap, out_on_device);
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, blurs, nullptr, n, files, files_size, files_on_device,
+                       file_offsets, file_sizes, out, out_cap, out_on_device);
+}
+
+extern "C" int xpngb_decode_augment(xpngb_ctx* ctx, const xpngb_tensor* fmt, const int* filters, const int* ops, xpngb_image* imgs,
+                                    const xpngb_rect* rects, const xpngb_size* sizes, const xpngb_rect* windows, const xpngb_color* colors,
+                                    const xpngb_blur* blurs, const xpngb_augment* augs, uint32_t n, const void* files, uint64_t files_size,
+                                    int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* out, uint64_t out_cap,
+                                    int out_on_device) {
+    if (!ctx) return 1;
+    ctx->err[0] = 0;
+    if (!sizes && (filters || windows)) FAIL("null argument (sizes): filters and windows need sizes");
+    if (fmt && tensor_check(ctx, fmt)) return 1;
+    return decode_call(ctx, imgs, rects, ops, sizes, filters, windows, fmt, colors, blurs, augs, n, files, files_size, files_on_device,
+                       file_offsets, file_sizes, out, out_cap, out_on_device);
 }
 
 extern "C" int xpngb_blur_box(double radius, int32_t* ri, uint32_t* ww, uint32_t* fw) {
