@@ -72,7 +72,12 @@ uint32_t xpngb_region_tiles(uint64_t w, uint64_t h, const xpngb_rect *r, xpngb_r
 
 /* xpngb_decode of rectangle rects[i] of file i only.  Crop i is written as rects[i].h packed rows of
  * rects[i].w * (3 + A) bytes at pixels + imgs[i].offset (a multiple of 16).  imgs[i] in/out exactly as for xpngb_decode
- * (w, h, A from xpngb_peek: the FULL image; mode out).  The same file may appear in several entries.
+ * (w, h, A from xpngb_peek: the FULL image; mode out).  The same file may appear in several entries.  Entries with
+ * equal (file_offsets[i], file_sizes[i]) share one decode, here and in every call below that takes rectangles, ops,
+ * sizes or a tensor format: the tiles of the bounding box of their rectangles' tiles are decoded once into a scratch
+ * window, and every entry of the group is cropped (turned, resized, ...) from there.  Equal bytes at different offsets
+ * are decoded once per offset.  The output bytes are those of decoding each entry on its own; xpngb_last_tiles counts
+ * the shared tiles once.
  * Every entry is checked before anything is decoded: an empty rectangle, one not inside its image, a crop past
  * pixels_cap or a misaligned offset fails the call (xpngb_last_error names the entry), as do the header checks of
  * xpngb_decode.  Corrupt data in a decoded tile fails the call as in a full decode.  Of the tiles a rectangle does not
@@ -345,6 +350,9 @@ int xpngb_decode_augment(xpngb_ctx *ctx, const xpngb_tensor *fmt /* NULL: uint8 
 float xpngb_last_kernel_ms(const xpngb_ctx *ctx);
 /* Number of kernel launches issued by the last call. */
 uint32_t xpngb_last_launches(const xpngb_ctx *ctx);
+/* Number of tiles the last decode call decoded, summed over its chunks.  Stored (level-7) files count 0.  Entries of one
+ * call that read the same file (equal offset and size) count the tiles of that file's shared window once. */
+uint64_t xpngb_last_tiles(const xpngb_ctx *ctx);
 /* Per-kernel timing: while on, every launch is bracketed by CUDA events and synchronised (so the call
  * gets slower); xpngb_profile_report writes "kernel_name total_ms launches\n" lines and returns the
  * length.  Turning profiling on or off clears the table. */

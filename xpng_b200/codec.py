@@ -125,6 +125,7 @@ def lib():
         L.xpngb_resize_coeffs.argtypes = [vp, C.c_int, u32, u32, u32, u32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.xpngb_last_kernel_ms.restype = C.c_float; L.xpngb_last_kernel_ms.argtypes = [vp]
         L.xpngb_last_launches.restype = u32; L.xpngb_last_launches.argtypes = [vp]
+        L.xpngb_last_tiles.restype = u64; L.xpngb_last_tiles.argtypes = [vp]
         L.xpngb_stream.restype = vp; L.xpngb_stream.argtypes = [vp]
         L.xpngb_profile.restype = None; L.xpngb_profile.argtypes = [vp, C.c_int]
         L.xpngb_profile_report.restype = u32; L.xpngb_profile_report.argtypes = [vp, C.c_char_p, u32]
@@ -566,6 +567,11 @@ class Codec:
         return int(lib().xpngb_last_launches(self._h))
 
     @property
+    def last_tiles(self):
+        """Tiles the last decode call decoded (stored files count 0; entries that share a file count its tiles once)."""
+        return int(lib().xpngb_last_tiles(self._h))
+
+    @property
     def stream(self):
         return lib().xpngb_stream(self._h)
 
@@ -757,6 +763,91 @@ class Codec:
         out = out.reshape(n, c, h, w) if layout == "chw" else out.reshape(n, h, w, c)
         return out.contiguous()
 
+    VIEW_KEYS = ("sizes", "boxes", "ops", "filters", "windows", "colors", "blurs", "augments")
+
+    def decode_views(self, files, views, dtype=None, layout="chw", scale="div", mean=None, std=None, drop_alpha=False):
+        """Every view of a multi-crop batch from one library call: a list of V tensors on this codec's device, view v of
+        shape (N, C, h_v, w_v) (or (N, h_v, w_v, C) for layout "hwc"), as decode_tensor(files, **views[v], dtype=dtype, ...)
+        returns it, bit for bit.  views: V dicts, each holding decode_tensor's per-entry arguments for one view of every
+        file (keys VIEW_KEYS: sizes, boxes, ops, filters, windows, colors, blurs, augments; a missing key is decode_tensor's
+        None).  Different views may have different shapes (DINO's 224 and 96); the entries of one view must share one
+        (ValueError naming the view otherwise).  Each file is packed and uploaded once, and the library decodes the tiles of
+        each file once for all its views: the bounding box of the tiles its views' rectangles touch."""
+        import torch
+        n, nv = len(files), len(views)
+        if n == 0 or nv == 0:
+            raise ValueError("decode_views needs at least one file and one view")
+        for v, d in enumerate(views):
+            bad = sorted(set(d) - set(self.VIEW_KEYS))
+            if bad:
+                raise ValueError(f"view {v}: unknown key {bad[0]!r} (one of {', '.join(self.VIEW_KEYS)})")
+            for k in ("sizes", "boxes", "ops", "windows", "colors", "blurs", "augments"):
+                if d.get(k) is not None and len(d[k]) != n:
+                    raise ValueError(f"view {v}: one {k[:-1] if k != 'boxes' else 'box'} per file")
+            if d.get("sizes") is None and (d.get("filters") is not None or d.get("windows") is not None):
+                raise ValueError(f"view {v}: filters and windows need sizes")
+        heads = []
+        for i, f in enumerate(files):
+            d = _Image()
+            if lib().xpngb_peek(np.frombuffer(f, dtype=np.uint8).ctypes.data, len(f), C.byref(d)):
+                raise ValueError(f"file {i}: not an .xpng header")
+            heads.append(d)
+        # entry v * n + i is view v of file i; a view without some argument gets the value that leaves its entries as
+        # decode_tensor leaves them without it (an output size equal to the crop is no resize)
+        any_of = {k: any(d.get(k) is not None for d in views) for k in self.VIEW_KEYS}
+        boxes, szs, wins, ops, filt, cols, bls, augs, shapes = [], [], [], [], [], [], [], [], []
+        for v, d in enumerate(views):
+            try:
+                fc = filter_codes(d.get("filters"), n)
+            except ValueError as e:
+                raise ValueError(f"view {v}: {e}") from None
+            shape = set()
+            for i in range(n):
+                b = d["boxes"][i] if d.get("boxes") is not None else (0, 0, heads[i].w, heads[i].h)
+                z = d["sizes"][i] if d.get("sizes") is not None else (b[2], b[3])
+                wn = d["windows"][i] if d.get("windows") is not None else (0, 0, z[0], z[1])
+                op = d["ops"][i] if d.get("ops") is not None else "tl"
+                boxes.append(b); szs.append(z); wins.append(wn); ops.append(op)
+                filt.append(FILTERS["bilinear"] if fc is None else fc[i])
+                cols.append(d["colors"][i] if d.get("colors") is not None else None)
+                bls.append(d["blurs"][i] if d.get("blurs") is not None else None)
+                augs.append(d["augments"][i] if d.get("augments") is not None else None)
+                w, h = int(wn[2]), int(wn[3])
+                shape.add((3 if drop_alpha else 3 + heads[i].A,) + ((w, h) if op in QUARTER_TURNS else (h, w)))
+            if len(shape) != 1:
+                raise ValueError(f"view {v}: entries have different output shapes {sorted(shape)}")
+            shapes.append(shape.pop())
+        m = n * nv
+        dname = _dtype_name(torch.float32 if dtype is None else dtype)
+        fmt = tensor_format(dname, layout, scale, (0, 0, 0, 0) if mean is None else mean, (1, 1, 1, 1) if std is None else std, drop_alpha)
+        ra = rects(boxes) if any_of["boxes"] else None
+        sa = _sizes(szs) if any_of["sizes"] else None
+        wa = rects(wins) if any_of["windows"] else None
+        descs, foffs, fsizes, fb, off, _, _ = self._pack_files(list(files) * nv, ra, sa)
+        eb = DTYPE_BYTES[dname]
+        bases, strides, at = [], [], 0
+        for c, h, w in shapes:
+            stride = _align16(c * h * w * eb) // eb   # entry offsets are multiples of 16 bytes
+            bases.append(at)
+            strides.append(stride)
+            at += n * stride
+        for v in range(nv):
+            for i in range(n):
+                descs[v * n + i].offset = (bases[v] + i * strides[v]) * eb
+        dev = torch.device("cuda", self.device)
+        flat = torch.empty(at, dtype=getattr(torch, dname), device=dev)
+        # the library writes on its own stream: memory fresh from the caching allocator may still be in use by queued work
+        torch.cuda.current_stream(dev).synchronize()
+        self.decode_augment_raw(fmt, descs, (C.c_int * m)(*filt) if any_of["filters"] else None, op_codes(ops) if any_of["ops"] else None,
+                                ra, sa, wa, color_array(cols, m) if any_of["colors"] else None,
+                                blur_array(bls, m) if any_of["blurs"] else None, augment_array(augs, m) if any_of["augments"] else None,
+                                m, fb.ctypes.data, off, 0, foffs, fsizes, flat.data_ptr(), at * eb, 1)
+        out = []
+        for v, (c, h, w) in enumerate(shapes):
+            t = flat[bases[v]: bases[v] + n * strides[v]].view(n, strides[v])[:, :c * h * w]
+            out.append((t.reshape(n, c, h, w) if layout == "chw" else t.reshape(n, h, w, c)).contiguous())
+        return out
+
     # ---------------------------------------------------------------- numpy convenience (host buffers)
     def encode(self, level, images):
         """list of (h,w,3|4) uint8 arrays -> list of .xpng byte strings."""
@@ -772,17 +863,23 @@ class Codec:
 
     def _pack_files(self, files, ra=None, sa=None, wa=None):
         """Files packed at 16-byte offsets and a host output buffer: one whole image, crop ra[i], size sa[i] or window wa[i]
-        per entry."""
+        per entry.  An object that appears in several entries is packed once: those entries share its offset, so the
+        library decodes it once for all of them."""
         n = len(files)
         descs = (_Image * n)()
         foffs, fsizes = (C.c_uint64 * n)(), (C.c_uint64 * n)()
         off = poff = 0
+        packed = {}   # id(file) -> offset
         for i, f in enumerate(files):
             b = np.frombuffer(f, dtype=np.uint8)
             if lib().xpngb_peek(b.ctypes.data, len(f), C.byref(descs[i])):
                 raise ValueError(f"file {i}: not an .xpng header")
-            foffs[i], fsizes[i] = off, len(f)
-            off = _align16(off + len(f))
+            if id(f) in packed:
+                foffs[i], fsizes[i] = packed[id(f)], len(f)
+            else:
+                packed[id(f)] = foffs[i] = off
+                fsizes[i] = len(f)
+                off = _align16(off + len(f))
             descs[i].offset = poff
             if wa is not None:
                 if 0 < wa[i].w <= 1 << 24 and 0 < wa[i].h <= 1 << 24:   # other windows are refused by the library, naming the entry
@@ -795,8 +892,8 @@ class Codec:
             elif ra[i].w <= descs[i].w and ra[i].h <= descs[i].h:     # other rectangles are refused by the library, naming the entry
                 poff = _align16(poff + ra[i].w * ra[i].h * (3 + descs[i].A))
         fb = np.zeros(off + 16, dtype=np.uint8)
-        for i, f in enumerate(files):
-            fb[foffs[i]: foffs[i] + len(f)] = np.frombuffer(f, dtype=np.uint8)
+        for f in {id(f): f for f in files}.values():
+            fb[packed[id(f)]: packed[id(f)] + len(f)] = np.frombuffer(f, dtype=np.uint8)
         px = np.empty(poff + 16, dtype=np.uint8)
         return descs, foffs, fsizes, fb, off, px, poff
 

@@ -13,6 +13,8 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
+#include <map>
 #include <vector>
 
 #include "../../include/xpng_b200.h"
@@ -62,6 +64,7 @@ struct xpngb_ctx {
     char err[512] = { 0 };
     float last_ms = 0.f;
     uint32_t launches = 0;
+    uint64_t decoded_tiles = 0;               // tiles the last decode call decoded, over all its chunks (xpngb_last_tiles)
     uint64_t max_chunk_px = 1ull << 30;       // XPNGB_CHUNK_MPIX: upper bound of a chunk (bounds the scratch of a lane)
     uint32_t pipe_lanes = 8;                  // XPNGB_PIPE_LANES: chunks in flight per call
     uint64_t pipe_min_px = 32ull << 20;       // XPNGB_PIPE_MIN_MPIX: no chunk smaller than this
@@ -486,6 +489,7 @@ extern "C" void xpngb_destroy(xpngb_ctx* ctx) {
 extern "C" const char* xpngb_last_error(const xpngb_ctx* ctx) { return ctx ? ctx->err : "no context"; }
 extern "C" float xpngb_last_kernel_ms(const xpngb_ctx* ctx) { return ctx ? ctx->last_ms : 0.f; }
 extern "C" uint32_t xpngb_last_launches(const xpngb_ctx* ctx) { return ctx ? ctx->launches : 0; }
+extern "C" uint64_t xpngb_last_tiles(const xpngb_ctx* ctx) { return ctx ? ctx->decoded_tiles : 0; }
 extern "C" void* xpngb_stream(const xpngb_ctx* ctx) { return ctx ? (void*)ctx->stream : nullptr; }
 
 extern "C" void xpngb_profile(xpngb_ctx* ctx, int on) { if (ctx) { ctx->profile = on == 3 ? 3 : (on ? (ctx->profile == 2 ? 2 : 1) : 0); ctx->prof.clear(); } }
@@ -516,7 +520,8 @@ extern "C" int xpngb_peek(const void* file, uint64_t size, xpngb_image* img) {
 
 // Cut n images into chunks of whole images: at most pipe_lanes chunks of roughly equal pixel count, none below
 // pipe_min_px (so small calls stay one chunk) and none above max_chunk_px (scratch bound).  Returns the chunk starts + n.
-static std::vector<uint32_t> cut_chunks(const xpngb_ctx* ctx, const xpngb_image* imgs, uint32_t n) {
+// first (may be null): a chunk may start at image i only where first[i] is set.
+static std::vector<uint32_t> cut_chunks(const xpngb_ctx* ctx, const xpngb_image* imgs, uint32_t n, const uint8_t* first = nullptr) {
     uint64_t total = 0;
     for (uint32_t i = 0; i < n; i++) total += imgs[i].w * imgs[i].h;
     uint64_t want = (total + ctx->pipe_lanes - 1) / ctx->pipe_lanes;
@@ -533,7 +538,7 @@ static std::vector<uint32_t> cut_chunks(const xpngb_ctx* ctx, const xpngb_image*
     for (uint32_t i = 0; i < n && c < k; i++) {
         px += imgs[i].w * imgs[i].h;
         typedef unsigned __int128 u128;   // w, h <= 2^24 each: the products exceed 64 bits for absurd batches only, but must not wrap
-        if ((u128)px * k >= (u128)c * total && i + 1 < n) {
+        if ((u128)px * k >= (u128)c * total && i + 1 < n && (!first || first[i + 1])) {
             cuts.push_back(i + 1);
             while (c < k && (u128)px * k >= (u128)c * total) c++;
         }
@@ -1023,7 +1028,12 @@ struct RegionSel {
 static bool whole_tiles(const RegionSel& R) {
     return R.rect.x == R.cover.x && R.rect.y == R.cover.y && R.rect.w == R.cover.w && R.rect.h == R.cover.h;
 }
-static uint64_t window_pitch(const RegionSel& R, uint32_t pxsz) { return (R.cover.w * pxsz + 15) & ~15ull; }   // keeps RGB rows word-aligned (tile_pitched)
+static uint64_t window_pitch(const xpngb_rect& cover, uint32_t pxsz) { return (cover.w * pxsz + 15) & ~15ull; }   // keeps RGB rows word-aligned (tile_pitched)
+static uint64_t window_pitch(const RegionSel& R, uint32_t pxsz) { return window_pitch(R.cover, pxsz); }
+// Position p of a call whose entries are ordered by file (group_entries).  n: entries decoded from one shared window, at
+// its first position (0 at the others); 1 for an entry decoded as on its own (the only entry of its file, or a stored
+// file).  s, cover (n > 1): the tile bounding box of the group's rectangles, and its pixels.
+struct Share { uint32_t n; TileSel s; xpngb_rect cover; };
 // Entry i of an oriented decode is written turned or mirrored.  TL and TR are copies in the reference: those entries are
 // decoded exactly as without an op.
 static bool turned(const int* ops, uint32_t i) { return ops && ops[i] != OP_TL && ops[i] != OP_TR; }
@@ -1117,11 +1127,13 @@ constexpr uint32_t AUG_STAGES = XPNGB_AUG_STEPS_MAX + 1;   // a uint8 entry whos
 // resized one lands there anyway, any other is copied there by k_crop_rows), from which k_to_tensor reads it.  blurs (only
 // with sel): a blurred or solarized entry is staged as a coloured one is, then goes through its box passes after k_color,
 // ping-ponged between its pixels and the lane's bscr scratch, one k_blur launch per pass stage of the chunk; a tensor
-// entry's k_to_tensor reads whichever buffer its last pass wrote, a uint8 entry's passes end at its output.  Never waits
-// for the device.
-static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const int* ops,
-                        const xpngb_tensor* fmt, const xpngb_color* colors, const xpngb_blur* blurs, const xpngb_augment* augs,
-                        uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
+// entry's k_to_tensor reads whichever buffer its last pass wrote, a uint8 entry's passes end at its output.  share (only
+// with sel, may be null): the entries of a group with share[i].n > 1 read one file; its first entry decodes the group's
+// tile bounding box into one window, and every entry of the group goes on from there as from its own window (the others
+// plan no tiles).  Never waits for the device.
+static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const DecImage* DI_in, const RegionSel* sel, const Share* share,
+                        const int* ops, const xpngb_tensor* fmt, const xpngb_color* colors, const xpngb_blur* blurs,
+                        const xpngb_augment* augs, uint32_t n, const uint8_t* din, uint8_t* dpx, uint32_t call_tiles) {
     ctx->cur = ctx->stream;
     Plan P;
     std::vector<DecImage> DI(DI_in, DI_in + n);
@@ -1143,6 +1155,7 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     auto blurred = [&](uint32_t i) { return blurs && blur_on(blurs[i]); };
     auto augmented = [&](uint32_t i) { return augs && augs[i].nsteps; };
     auto staged = [&](uint32_t i) { return colored(i) || blurred(i) || augmented(i); };   // needs its uint8 pixels to work on
+    auto shared = [&](uint32_t i) { return share && share[i].n != 1; };                  // goes on from its group's window
     // pixels entry i writes: its resampled window, or its rectangle
     auto out_px = [&](uint32_t i) -> uint64_t { return sel[i].rs ? sel[i].win.w * sel[i].win.h : sel[i].rect.w * sel[i].rect.h; };
     // uint8 pixels of a resized or staged tensor entry, or of a blurred entry's scratch (16-byte aligned)
@@ -1151,7 +1164,9 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
         uint64_t need = 0, tab = 0, tmp = 0, tsz = 0, bsz = 0;
         for (uint32_t i = 0; i < n; i++) {
             const bool rs = sel[i].rs;
-            if (DI[i].mode != 7 && (!whole_tiles(sel[i]) || turned(ops, i) || rs || fmt)) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
+            if (DI[i].mode == 7) { }
+            else if (shared(i)) { if (share[i].n) need += share[i].cover.h * window_pitch(share[i].cover, DI[i].pxsz); }
+            else if (!whole_tiles(sel[i]) || turned(ops, i) || rs || fmt) need += sel[i].cover.h * window_pitch(sel[i], DI[i].pxsz);
             if (rs) { tab += resize_tab_bytes(sel[i]); tmp += resize_tmp_bytes(sel[i], DI[i].pxsz); }
             if ((rs || staged(i)) && fmt) tsz += tsrc_bytes(i);
             if (blurred(i) || augmented(i)) bsz += tsrc_bytes(i);
@@ -1353,7 +1368,8 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             FAIL("too many pixels for one orientation launch");
         return 0;
     };
-    uint64_t wpos = 0;
+    uint64_t wpos = 0, gwin = 0, gpitch = 0;   // the window of the current group of a shared file, and its cover
+    xpngb_rect gcov{};
     for (uint32_t i = 0; i < n; i++) {
         DecImage& D = DI[i];
         uint8_t* out = dpx + imgs[i].offset;
@@ -1368,6 +1384,22 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
             P.imgs.push_back(I);
             const uint64_t src = (uint64_t)(din + D.file_off + 8 + (r.y * D.w + r.x) * D.pxsz);   // any byte alignment
             if (region_out(i, src, (uint64_t)D.w * D.pxsz, out)) return 1;
+        } else if (shared(i)) {   // never in place: the window holds every entry of the group
+            const RegionSel& R = sel[i];
+            const xpngb_rect& r = R.rect;
+            if (share[i].n) {
+                gcov = share[i].cover; gpitch = window_pitch(gcov, D.pxsz); gwin = (uint64_t)ctx->region.p + wpos;
+                const TileSel& s = share[i].s;
+                plan_image(P, R.g, s, gwin, gpitch, gcov.x, gcov.y, D.w, D.h, D.pxsz, D.mode, sfac, 0);
+                wpos += gcov.h * gpitch;
+                D.r0 = (uint32_t)s.r0; D.c0 = (uint32_t)s.c0; D.nrows = (uint32_t)(s.r1 - s.r0 + 1); D.ncols = (uint32_t)(s.c1 - s.c0 + 1);
+            } else {   // no tiles of its own: k_dec_tile_offsets walks no row of it
+                ImageDesc I{}; I.tile0 = (uint32_t)P.tiles.size(); I.mode = D.mode; I.w = D.w; I.h = D.h; I.pxsz = D.pxsz;
+                P.imgs.push_back(I);
+                D.r0 = 0; D.c0 = 0; D.nrows = 0; D.ncols = 0;
+            }
+            D.gcols = (uint32_t)R.g.nw;
+            if (region_out(i, gwin + (r.y - gcov.y) * gpitch + (r.x - gcov.x) * D.pxsz, gpitch, out)) return 1;
         } else {
             const RegionSel& R = sel[i];
             const xpngb_rect &r = R.rect, &c = R.cover;
@@ -1429,6 +1461,7 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     }
     if (P.tiles.size() > (1u << 24) || P.seg_tile.size() > (1u << 28)) FAIL("too many tiles for one chunk (%zu)", P.tiles.size());
     const uint32_t ntiles = (uint32_t)P.tiles.size();
+    ctx->root->decoded_tiles += ntiles;
     if (upload_plan(ctx, P)) return 1;
     ENSURE(dimgs, n * sizeof(DecImage)); ENSURE(dtiles, ntiles * sizeof(DecTile)); ENSURE(errflag, 4);
     // pinned staging: DecImage table, stored-file starts, error flag (64 bytes), crop, orientation, resize and tensor descriptors
@@ -1730,6 +1763,59 @@ static int decode_issue(xpngb_ctx* ctx, bool lat, const xpngb_image* imgs, const
     return 0;
 }
 
+// Entries with equal (file_offsets[i], file_sizes[i]) read one file.  When some file is read by several entries, ord gets
+// the entries group by group (ord[p]: the caller's index of position p; groups in the order of their first entry, entries
+// in the caller's order), first[p] marks where a group starts, and share[p] says how position p is decoded (Share).
+// Otherwise all three stay empty and the call runs in the caller's order, each entry on its own.
+static void group_entries(const xpngb_image* imgs, const RegionSel* sel, const uint64_t* file_offsets, const uint64_t* file_sizes,
+                          uint32_t n, std::vector<uint32_t>& ord, std::vector<uint8_t>& first, std::vector<Share>& share) {
+    std::map<std::pair<uint64_t, uint64_t>, uint32_t> key;
+    std::vector<uint32_t> gof(n), start;   // group of each entry; entries per group, then where each group starts
+    for (uint32_t i = 0; i < n; i++) {
+        const auto it = key.emplace(std::make_pair(file_offsets[i], file_sizes[i]), (uint32_t)start.size());
+        if (it.second) start.push_back(0);
+        gof[i] = it.first->second;
+        start[gof[i]]++;
+    }
+    if (start.size() == n) return;
+    const uint32_t ng = (uint32_t)start.size();
+    std::vector<uint32_t> cnt(start);
+    for (uint32_t g = 0, at = 0; g < ng; g++) { const uint32_t c = start[g]; start[g] = at; at += c; }
+    ord.resize(n); first.assign(n, 0); share.assign(n, Share{ 1, {}, {} });
+    std::vector<uint32_t> fill(start);
+    for (uint32_t i = 0; i < n; i++) ord[fill[gof[i]]++] = i;
+    for (uint32_t g = 0; g < ng; g++) {
+        const uint32_t p0 = start[g], i0 = ord[p0];
+        first[p0] = 1;
+        if (cnt[g] == 1 || imgs[i0].mode == 7) continue;   // stored rectangles are read straight out of the file
+        TileSel s = sel[i0].s;
+        for (uint32_t p = p0 + 1; p < p0 + cnt[g]; p++) {
+            const TileSel& t = sel[ord[p]].s;
+            if (t.r0 < s.r0) s.r0 = t.r0; if (t.r1 > s.r1) s.r1 = t.r1;
+            if (t.c0 < s.c0) s.c0 = t.c0; if (t.c1 > s.c1) s.c1 = t.c1;
+            share[p].n = 0;
+        }
+        const TileGrid& gr = sel[i0].g;
+        share[p0] = Share{ cnt[g], s, xpngb_rect{ gr.x_of(s.c0), gr.y_of(s.r0), gr.x_of(s.c1) + gr.w_of(s.c1) - gr.x_of(s.c0),
+                                                  gr.y_of(s.r1) + gr.h_of(s.r1) - gr.y_of(s.r0) } };
+    }
+}
+
+// The host copies of a call, [a, b) byte ranges each owned by one chunk: sorted by start, neighbouring ranges of one chunk
+// become one copy.  So a chunk's copy never spans bytes another chunk copies (its outputs, written back by another lane,
+// perhaps later), and a file read by several entries of one chunk crosses PCIe once.  Returns each chunk's copies.
+struct Span { uint64_t a, b; uint32_t chunk; };
+static std::vector<std::vector<std::pair<uint64_t, uint64_t>>> copy_runs(std::vector<Span>& s, uint32_t nchunks) {
+    std::sort(s.begin(), s.end(), [](const Span& x, const Span& y) { return x.a < y.a || (x.a == y.a && x.chunk < y.chunk); });
+    std::vector<std::vector<std::pair<uint64_t, uint64_t>>> runs(nchunks);
+    for (size_t k = 0; k < s.size(); k++) {
+        auto& r = runs[s[k].chunk];
+        if (k && s[k - 1].chunk == s[k].chunk && !r.empty()) { if (s[k].b > r.back().second) r.back().second = s[k].b; }
+        else r.emplace_back(s[k].a, s[k].b);
+    }
+    return runs;
+}
+
 // xpngb_decode (rects == nullptr), xpngb_decode_region and, with ops, xpngb_decode_oriented; with sizes
 // xpngb_decode_resized, with fmt xpngb_decode_tensor, with filters or windows (only with sizes) xpngb_decode_resampled.
 // An oriented, resized or tensor call always selects tiles per entry: without rects every entry's rectangle is its whole
@@ -1740,7 +1826,7 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
                        uint64_t files_size, int files_on_device, const uint64_t* file_offsets, const uint64_t* file_sizes, void* pixels,
                        uint64_t pixels_cap, int pixels_on_device) {
     if (!ctx) return 1;
-    ctx->err[0] = 0; ctx->launches = 0; ctx->last_ms = 0.f; ctx->cur = ctx->stream;
+    ctx->err[0] = 0; ctx->launches = 0; ctx->decoded_tiles = 0; ctx->last_ms = 0.f; ctx->cur = ctx->stream;
     if (!imgs || !files || !file_offsets || !file_sizes || !pixels) FAIL("null argument");
     if (n == 0) return 0;
     CK(cudaSetDevice(ctx->device));
@@ -1864,15 +1950,41 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     }
     uint8_t* dpx = (uint8_t*)pixels;
     if (!pixels_on_device) { ENSURE(pixels, pixels_cap); dpx = (uint8_t*)ctx->pixels.p; }
-    // chunks are cut by the pixels each entry decodes: the whole image, or the cover of its rectangle (stored: the rectangle)
+    // ---- entries that read the same file decode it once; the chunks then see them group by group, position p being
+    // the caller's entry at(p)
+    std::vector<uint32_t> ord;
+    std::vector<uint8_t> first;
+    std::vector<Share> share;
+    if (use_sel) group_entries(imgs, sel.data(), file_offsets, file_sizes, n, ord, first, share);
+    auto at = [&](uint32_t p) { return ord.empty() ? p : ord[p]; };
+    auto permuted = [&](auto* a, auto& v) -> decltype(a) {   // a in position order (a itself when nothing is reordered)
+        if (!a || ord.empty()) return a;
+        v.reserve(n);
+        for (uint32_t p = 0; p < n; p++) v.push_back(a[ord[p]]);
+        return v.data();
+    };
+    std::vector<xpngb_image> o_imgs; std::vector<DecImage> o_DI; std::vector<RegionSel> o_sel; std::vector<int> o_ops;
+    std::vector<xpngb_color> o_colors; std::vector<xpngb_blur> o_blurs; std::vector<xpngb_augment> o_augs;
+    const xpngb_image* p_imgs = permuted((const xpngb_image*)imgs, o_imgs);
+    const DecImage* p_DI = permuted((const DecImage*)DI.data(), o_DI);
+    const RegionSel* p_sel = use_sel ? permuted((const RegionSel*)sel.data(), o_sel) : nullptr;
+    const int* p_ops = permuted(ops, o_ops);
+    const xpngb_color* p_colors = permuted(colors, o_colors);
+    const xpngb_blur* p_blurs = permuted(blurs, o_blurs);
+    const xpngb_augment* p_augs = permuted(augs, o_augs);
+    // chunks are cut by the pixels each position decodes: the whole image, the cover of its rectangle (stored: the
+    // rectangle), or for a shared window its cover at the group's first position and nothing at the others
     std::vector<xpngb_image> dims(n);
     uint64_t tiles_est = 0; bool l2 = false;
-    for (uint32_t i = 0; i < n; i++) {
-        const uint32_t mode = imgs[i].mode;
-        const xpngb_rect* wh = !use_sel ? nullptr : (mode == 7 ? &sel[i].rect : &sel[i].cover);
-        dims[i].w = wh ? wh->w : imgs[i].w; dims[i].h = wh ? wh->h : imgs[i].h;
-        if (mode == 1 || mode == 2) tiles_est += use_sel ? (sel[i].s.r1 - sel[i].s.r0 + 1) * (sel[i].s.c1 - sel[i].s.c0 + 1)
-                                                         : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
+    for (uint32_t p = 0; p < n; p++) {
+        const uint32_t i = at(p), mode = imgs[i].mode;
+        const bool sh = !share.empty() && share[p].n != 1;
+        const xpngb_rect none{};
+        const xpngb_rect* wh = !use_sel ? nullptr : mode == 7 ? &sel[i].rect : !sh ? &sel[i].cover : share[p].n ? &share[p].cover : &none;
+        const TileSel& s = sh ? share[p].s : use_sel ? sel[i].s : TileSel{};
+        dims[p].w = wh ? wh->w : imgs[i].w; dims[p].h = wh ? wh->h : imgs[i].h;
+        if ((mode == 1 || mode == 2) && !(sh && !share[p].n))
+            tiles_est += use_sel ? (s.r1 - s.r0 + 1) * (s.c1 - s.c0 + 1) : (imgs[i].w * imgs[i].h + TILE_AREA - 1) / TILE_AREA;
         l2 |= mode == 2;
     }
     auto out_bytes = [&](uint32_t i) {
@@ -1881,8 +1993,16 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
     // level 2: above ~600 tiles the pair family wins, with the 16-symbol value streams warp-per-block while they all fit
     // (s16_lat_max_tiles); level 1: the warp-per-block family up to ~1300 tiles (measured at 125 / 250 / 500 frames, profiles/)
     const bool lat = l2 ? 17 * tiles_est <= (uint64_t)ctx->lat_max_blocks * 5 / 6 : 9 * tiles_est <= ctx->lat_max_blocks;
-    const std::vector<uint32_t> cuts = cut_chunks(ctx, dims.data(), n);
+    const std::vector<uint32_t> cuts = cut_chunks(ctx, dims.data(), n, first.empty() ? nullptr : first.data());
     const uint32_t nchunks = (uint32_t)cuts.size() - 1;
+    std::vector<Span> fspan, ospan;
+    for (uint32_t ci = 0; ci < nchunks; ci++)
+        for (uint32_t p = cuts[ci]; p < cuts[ci + 1]; p++) {
+            const uint32_t i = at(p);
+            if (!files_on_device) fspan.push_back(Span{ file_offsets[i], file_offsets[i] + file_sizes[i], ci });
+            if (!pixels_on_device) ospan.push_back(Span{ imgs[i].offset, imgs[i].offset + out_bytes(i), ci });
+        }
+    const auto uploads = copy_runs(fspan, nchunks), downloads = copy_runs(ospan, nchunks);
     CK(cudaEventRecord(ctx->ev0, ctx->stream));
     int rc = 0;
     std::vector<xpngb_ctx*> used(nchunks, nullptr);
@@ -1904,23 +2024,16 @@ static int decode_call(xpngb_ctx* ctx, xpngb_image* imgs, const xpngb_rect* rect
         used[ci] = lane; cn[ci] = cuts[ci + 1] - cuts[ci];
         const uint32_t i0 = cuts[ci], m = cn[ci];
         if (lane != ctx && cudaStreamWaitEvent(lane->stream, ctx->ev0, 0) != cudaSuccess) { snprintf(ctx->err, sizeof ctx->err, "cudaStreamWaitEvent failed"); rc = 1; break; }
-        if (!files_on_device) {
-            uint64_t lo = ~0ull, hi = 0;
-            for (uint32_t i = i0; i < i0 + m; i++) { if (file_offsets[i] < lo) lo = file_offsets[i]; if (file_offsets[i] + file_sizes[i] > hi) hi = file_offsets[i] + file_sizes[i]; }
-            if (cudaMemcpyAsync((uint8_t*)ctx->files.p + lo, (const uint8_t*)files + lo, hi - lo, cudaMemcpyHostToDevice, lane->stream) != cudaSuccess) {
-                snprintf(ctx->err, sizeof ctx->err, "host to device copy failed"); rc = 1; break;
-            }
-        }
-        rc = decode_issue(lane, lat, imgs + i0, DI.data() + i0, use_sel ? sel.data() + i0 : nullptr, ops ? ops + i0 : nullptr,
-                          fmt, colors ? colors + i0 : nullptr, blurs ? blurs + i0 : nullptr, augs ? augs + i0 : nullptr, m, din, dpx,
-                          (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
-        if (!rc && !pixels_on_device) {
-            uint64_t lo = ~0ull, hi = 0;
-            for (uint32_t i = i0; i < i0 + m; i++) {
-                const uint64_t a = imgs[i].offset, b = a + out_bytes(i);
-                if (a < lo) lo = a; if (b > hi) hi = b;
-            }
-            if (cudaMemcpyAsync((uint8_t*)pixels + lo, dpx + lo, hi - lo, cudaMemcpyDeviceToHost, lane->stream) != cudaSuccess) {
+        for (const auto& r : uploads[ci])
+            if (cudaMemcpyAsync((uint8_t*)ctx->files.p + r.first, (const uint8_t*)files + r.first, r.second - r.first, cudaMemcpyHostToDevice,
+                                lane->stream) != cudaSuccess) { snprintf(ctx->err, sizeof ctx->err, "host to device copy failed"); rc = 1; break; }
+        if (rc) break;
+        rc = decode_issue(lane, lat, p_imgs + i0, p_DI + i0, p_sel ? p_sel + i0 : nullptr, share.empty() ? nullptr : share.data() + i0,
+                          p_ops ? p_ops + i0 : nullptr, fmt, p_colors ? p_colors + i0 : nullptr, p_blurs ? p_blurs + i0 : nullptr,
+                          p_augs ? p_augs + i0 : nullptr, m, din, dpx, (uint32_t)(tiles_est > 0xFFFFFFFFull ? 0xFFFFFFFFu : tiles_est));
+        for (size_t k = 0; !rc && k < downloads[ci].size(); k++) {
+            const auto& r = downloads[ci][k];
+            if (cudaMemcpyAsync((uint8_t*)pixels + r.first, dpx + r.first, r.second - r.first, cudaMemcpyDeviceToHost, lane->stream) != cudaSuccess) {
                 snprintf(ctx->err, sizeof ctx->err, "device to host copy failed"); rc = 1;
             }
         }
