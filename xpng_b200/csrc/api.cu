@@ -561,6 +561,7 @@ __global__ void k_apply_scan(ImageDesc* imgs, const uint32_t* flags, uint32_t n)
 struct EncChunk {
     xpngb_ctx* lane = nullptr;
     xpngb_image* imgs = nullptr; uint32_t n = 0;
+    uint32_t first = 0; const uint32_t* index = nullptr;   // caller's index of imgs[i]: index[i], or first + i (error messages)
     uint64_t* out_offsets = nullptr; uint64_t* out_sizes = nullptr;
     std::vector<uint32_t> pxsz;
     uint64_t out_base = 0, out_end = 0;     // region of the device arena: [out_base, out_end) is this chunk's bound, files are packed from out_base
@@ -628,7 +629,8 @@ static int encode_issue(xpngb_ctx* ctx, int level, const uint8_t* dpix, uint8_t*
         if (m == 2 && any_rgba && !(flags[i] & SCAN_NOT_SINGLE)) m = 2 | 0x100;
         else if (m == 2 && pxsz[i] == 4) m = 1;
         if ((m == 1) && pxsz[i] == 4 && (imgs[i].w < 4 || imgs[i].h < 4))
-            FAIL("image %u: RGBA tiles thinner than 4 pixels are not encodable at level 1/2 (the reference crashes here)", i);
+            FAIL("image %u: RGBA tiles thinner than 4 pixels are not encodable at level 1/2 (the reference crashes here)",
+                 C.index ? C.index[i] : C.first + i);
         mode[i] = m; any1 |= m == 1; any2 |= m == 2;
     }
     if (any1 && any2) {
@@ -642,8 +644,10 @@ static int encode_issue(xpngb_ctx* ctx, int level, const uint8_t* dpix, uint8_t*
             if (idx.empty()) continue;
             std::vector<xpngb_image> sub(idx.size());
             std::vector<uint64_t> so(idx.size()), ss(idx.size());
-            for (size_t k = 0; k < idx.size(); k++) sub[k] = imgs[idx[k]];
+            std::vector<uint32_t> caller(idx.size());
+            for (size_t k = 0; k < idx.size(); k++) { sub[k] = imgs[idx[k]]; caller[k] = C.index ? C.index[idx[k]] : C.first + idx[k]; }
             EncChunk S; S.lane = ctx; S.imgs = sub.data(); S.n = (uint32_t)idx.size(); S.out_offsets = so.data(); S.out_sizes = ss.data();
+            S.index = caller.data();
             S.out_base = base; S.out_end = C.out_end;
             if (encode_issue(ctx, fam == 0 ? 1 : 2, dpix, dout, S) || encode_finish(ctx, S)) return 1;
             base = S.used_end;
@@ -831,7 +835,7 @@ extern "C" int xpngb_encode(xpngb_ctx* ctx, int level, xpngb_image* imgs, uint32
         xpngb_ctx* lane = lane_get(ctx, li);
         if (!lane) { snprintf(ctx->err, sizeof ctx->err, "cannot create pipeline lane %u", li); rc = 1; break; }
         EncChunk& C = chunks[ci];
-        C.lane = lane; C.imgs = imgs + cuts[ci]; C.n = cuts[ci + 1] - cuts[ci];
+        C.lane = lane; C.imgs = imgs + cuts[ci]; C.n = cuts[ci + 1] - cuts[ci]; C.first = cuts[ci];
         C.out_offsets = out_offsets + cuts[ci]; C.out_sizes = out_sizes + cuts[ci];
         C.out_base = region; region += xpngb_encode_bound(C.imgs, C.n); C.out_end = region;
         if (lane != ctx) { if (cudaStreamWaitEvent(lane->stream, ctx->ev0, 0) != cudaSuccess) { snprintf(ctx->err, sizeof ctx->err, "cudaStreamWaitEvent failed"); rc = 1; break; } }
