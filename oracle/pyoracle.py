@@ -54,6 +54,10 @@ def lib():
         L.xo_peek.argtypes = [C.c_void_p, u64, C.POINTER(u64), C.POINTER(u64), C.POINTER(C.c_int), C.POINTER(C.c_int)]
         L.xo_decode.restype = C.c_int
         L.xo_decode.argtypes = [C.c_void_p, u64, C.c_void_p]
+        L.xo_trace.restype = None
+        L.xo_trace.argtypes = [C.c_void_p, u64]
+        L.xo_trace_len.restype = u64
+        L.xo_trace_len.argtypes = []
         _lib = L
     return _lib
 
@@ -87,6 +91,28 @@ def encode(mode, px):
     if n == 0:
         raise ValueError("oracle: encode rejected the input")
     return out[:n].tobytes()
+
+
+# Decision log (xpng_oracle.h xo_trace): one record per size comparison of the encoder.
+DECISION = np.dtype([("kind", "<u4"), ("tile", "<u4"), ("stream", "<u4"), ("outcome", "<u4"), ("v", "<u8", (4,))])
+D_T1_TILE, D_FILE, D_T2_TILE, D_GREY_PLANE, D_GREY_PICK, D_V2_BLOCK, D_V2_TABLE, D_V1_BLOCK, D_V1_TABLE, D_PRED, D_STEAL = \
+    range(1, 12)
+
+
+def encode_traced(mode, px):
+    """encode() with the decision log on: (file bytes, structured array of DECISION records in decision order)."""
+    cap = 4096
+    while True:
+        buf = np.zeros(cap, dtype=DECISION)
+        lib().xo_trace(_ptr(buf), cap)
+        try:
+            data = encode(mode, px)
+            n = lib().xo_trace_len()
+        finally:
+            lib().xo_trace(None, 0)
+        if n <= cap:
+            return data, buf[:n].copy()
+        cap = int(n)
 
 
 def peek(data):

@@ -26,6 +26,22 @@ static inline void st32(uint8_t *p, uint32_t v) { memcpy(p, &v, 4); }
 static inline uint64_t ld64(const uint8_t *p) { uint64_t v; memcpy(&v, p, 8); return v; }
 static inline void st64(uint8_t *p, uint64_t v) { memcpy(p, &v, 8); }
 
+/* ------------------------------------------------------------------ decision log (xo_trace) */
+
+static __thread xo_decision_t *tr_buf;
+static __thread uint64_t tr_cap, tr_len;
+static __thread uint32_t tr_tile, tr_stream;
+
+void xo_trace(xo_decision_t *buf, uint64_t cap) { tr_buf = buf; tr_cap = buf ? cap : 0; tr_len = 0; tr_tile = tr_stream = 0; }
+uint64_t xo_trace_len(void) { return tr_len; }
+
+/* Records past the capacity are counted, not stored, so a caller can retry with a larger buffer. */
+static void tr_put(uint32_t kind, uint32_t outcome, uint64_t v0, uint64_t v1, uint64_t v2, uint64_t v3) {
+    if (!tr_buf) return;
+    if (tr_len < tr_cap) tr_buf[tr_len] = (xo_decision_t){ kind, tr_tile, tr_stream, outcome, { v0, v1, v2, v3 } };
+    tr_len++;
+}
+
 /* MSB-first bit writer over little-endian 32-bit words (ref: libxpng.c:8-11, :14-17). */
 typedef struct { uint64_t acc; uint32_t n; uint8_t *out; } bitw_t;
 static inline void bw_put(bitw_t *b, uint32_t c, uint32_t v) {
@@ -133,6 +149,7 @@ unsigned xo_select_predictor(const uint8_t *t, uint64_t w, uint64_t h, uint64_t 
     }
     unsigned m = 0;
     for (unsigned k = 1; k < 4; k++) if (cost[k] < cost[m]) m = k;
+    tr_put(XO_D_PRED, m, cost[0], cost[1], cost[2], cost[3]);
     return (unsigned)(pxsz & 4) | m;
 }
 
@@ -152,6 +169,11 @@ static void normalise_freqs(uint32_t *F, uint32_t *cum, unsigned N, uint64_t tot
             for (unsigned j = 0; j < N; j++) {
                 uint32_t wdt = cum[j + 1] - cum[j];
                 if (wdt > 1 && wdt < best) { best = wdt; donor = j; }
+            }
+            if (tr_buf) { /* how many symbols share the smallest width, and the last of them */
+                uint32_t ties = 0, last = 0;
+                for (unsigned j = 0; j < N; j++) if (cum[j + 1] - cum[j] == best) { ties++; last = j; }
+                tr_put(XO_D_STEAL, donor, i, best, ties, last);
             }
             if (donor < i) for (unsigned j = donor + 1; j <= i; j++) cum[j]--;
             else           for (unsigned j = i + 1; j <= donor; j++) cum[j]++;
@@ -220,6 +242,7 @@ uint64_t xo_block_v2_encode(uint32_t *F, unsigned nsym, const uint8_t *in, uint6
     st64(wp, x0); st64(wp + 8, x1); wp += 16; /* ref :394 */
 
     int sparse = (N + used * (unsigned)pb) < N * (unsigned)pb; /* ref :396-397 */
+    tr_put(XO_D_V2_TABLE, (uint32_t)sparse, N + used * (unsigned)pb, N * (unsigned)pb, used, N);
     st32(out + 4, (uint32_t)n | ((N - 2) << 24));
     st32(out + 8, (uint32_t)((wp - (out + 8)) / 4) | ((uint32_t)pb << 24)); /* ref :400 */
     bitw_t b = { 0, 0, wp };
@@ -228,6 +251,7 @@ uint64_t xo_block_v2_encode(uint32_t *F, unsigned nsym, const uint8_t *in, uint6
     st32(out, (uint32_t)csz | ((uint32_t)(3 + sparse) << 24));
 
     uint64_t rawbits = (uint64_t)nbit * n, rawsz = 8 + (rawbits / 32) * 4 + (rawbits % 32 ? 4 : 0);
+    tr_put(XO_D_V2_BLOCK, csz < rawsz, csz, rawsz, n, N);
     if (csz >= rawsz) { /* ref :417-424: plain nbit-wide symbols */
         out[7] = (uint8_t)nbit;
         bitw_t r = { 0, 0, out + 8 };
@@ -323,7 +347,10 @@ static uint64_t block_v1_encode(uint32_t *F, unsigned N, const uint8_t *in, uint
     }
     uint64_t payload = 16 + 4 * nw; /* states + words (ref :250: *_res - res before the header) */
     uint32_t tab_bits = (N - used) + used * ((uint32_t)pb + 1);
-    int sparse = tab_bits < N * (uint32_t)pb; if (!sparse) tab_bits = N * (uint32_t)pb;
+    int sparse = tab_bits < N * (uint32_t)pb;
+    tr_put(XO_D_V1_TABLE, (uint32_t)sparse, tab_bits, N * (uint32_t)pb, used, N);
+    if (!sparse) tab_bits = N * (uint32_t)pb;
+    tr_put(XO_D_V1_BLOCK, tab_bits + 8 * payload < (uint64_t)nbit * n, tab_bits + 8 * payload, (uint64_t)nbit * n, n, N);
 
     if (tab_bits + 8 * payload >= (uint64_t)nbit * n) { /* ref :250-254 raw symbols into sb */
         for (uint64_t k = 0; k < n; k++) bw_put(sb, nbit, in[k]);
@@ -431,10 +458,13 @@ uint64_t xo_encode_tile_m1(const uint8_t *tile, uint64_t w, uint64_t h, uint64_t
     uint64_t kw = xo_m1_front(tile, w, h, bpr, pxsz, pr, streams, lens, F, (uint32_t *)(out + 8));
     st32(out + 4, (uint32_t)(4 + 4 * kw));
     uint8_t *f = out + 8 + 4 * kw; const uint8_t *s = streams;
-    for (int c = 0; c < 9; c++) { f += xo_block_v2_encode(F + c * 16, 9, s, lens[c], f, 12); s += lens[c]; }
+    for (int c = 0; c < 9; c++) { tr_stream = (uint32_t)c; f += xo_block_v2_encode(F + c * 16, 9, s, lens[c], f, 12); s += lens[c]; }
+    tr_stream = 9;
     if (pxsz == 4) f += xo_block_v2_encode(F + 256, 256, s, lens[9], f, 15);
     free(streams);
     uint64_t raw = npx * (uint64_t)pxsz + 4, coded = (uint64_t)(f - out);
+    tr_stream = 0;
+    tr_put(XO_D_T1_TILE, coded < raw, coded, raw, pr, npx);
     if (coded < raw) { st32(out, (1u << 28) + (pr << 24) + (uint32_t)coded); return coded; }
     st32(out, (uint32_t)raw); /* ref :566-567 raw tile */
     for (uint64_t y = 0; y < h; y++) memcpy(out + 4 + y * w * pxsz, tile + y * bpr, w * pxsz);
@@ -511,10 +541,14 @@ static uint64_t encode_tile_grey(const uint8_t *t, uint64_t w, uint64_t h, uint6
     for (unsigned i = 0; i < 4; i++) {
         bits[i] = (uint8_t *)malloc(2 * npx + 4096); blk[i] = (uint8_t *)malloc(4 * npx + 4096);
         bitw_t b = { t[0], 8, bits[i] + 4 };
+        tr_stream = i;
         rsz[i] = block_v1_encode(F[i], 256, st + i * npx, n, blk[i], &b, 15);
         bw_end(&b); bsz[i] = (uint64_t)(b.out - bits[i]); st32(bits[i], (uint32_t)bsz[i]);
         if (bsz[i] + rsz[i] < bsz[best] + rsz[best]) best = i; /* ref :612 strict <, ties -> lowest */
     }
+    tr_stream = 0;
+    tr_put(XO_D_GREY_PICK, best, bsz[0] + rsz[0], bsz[1] + rsz[1], bsz[2] + rsz[2], bsz[3] + rsz[3]);
+    tr_put(XO_D_GREY_PLANE, bsz[best] + rsz[best] < npx, bsz[best] + rsz[best], npx, best, npx);
     uint64_t size;
     if (bsz[best] + rsz[best] >= npx) { /* ref :615-619 raw grey plane */
         size = npx + 4; st32(out, (uint32_t)size + (5u << 27));
@@ -555,10 +589,12 @@ uint64_t xo_encode_tile_m2(const uint8_t *t, uint64_t w, uint64_t h, uint64_t bp
     }
     uint8_t *bits = (uint8_t *)malloc(4 * npx + 65536), *blocks = (uint8_t *)malloc(6 * npx + 65536), *bp = blocks;
     bitw_t b = { ((uint32_t)t[0] << 16) | ((uint32_t)t[1] << 8) | t[2], 24, bits + 4 }; /* ref :659-660 */
-    for (int i = 0; i < 9; i++) bp += block_v1_encode(F[0] + i * 16, 9, cx[i], ncx[i], bp, &b, 14);
-    for (int i = 1; i < 9; i++) bp += block_v1_encode(F[i], M2_ALPHABET[i], sv[i], nsv[i], bp, &b, 14);
+    for (int i = 0; i < 9; i++) { tr_stream = (uint32_t)i; bp += block_v1_encode(F[0] + i * 16, 9, cx[i], ncx[i], bp, &b, 14); }
+    for (int i = 1; i < 9; i++) { tr_stream = 8 + (uint32_t)i; bp += block_v1_encode(F[i], M2_ALPHABET[i], sv[i], nsv[i], bp, &b, 14); }
     bw_end(&b);
     uint64_t bsz = (uint64_t)(b.out - bits), rsz = (uint64_t)(bp - blocks), size; st32(bits, (uint32_t)bsz);
+    tr_stream = 0;
+    tr_put(XO_D_T2_TILE, bsz + rsz < npx * 3, bsz + rsz, npx * 3, pr, npx);
     if (bsz + rsz >= npx * 3) { /* ref :675-677 raw tile */
         size = npx * 3 + 4; st32(out, (uint32_t)size);
         for (uint64_t y = 0; y < h; y++) memcpy(out + 4 + y * w * 3, t + y * bpr_, w * 3);
@@ -650,12 +686,15 @@ uint64_t xo_encode(int mode, const uint8_t *px_in, uint64_t w, uint64_t h, int A
         uint8_t *blob = (uint8_t *)malloc(8 * 700 * 700 + 65536); uint64_t total = 0; int overflow = 0;
         for (uint64_t i = 0; i < N; i++) {
             const uint8_t *tp = px + tl[i].y * bpr + tl[i].x * (uint64_t)pxsz;
+            tr_tile = (uint32_t)i; tr_stream = 0;
             uint64_t bs = mode == 1 ? xo_encode_tile_m1(tp, tl[i].w, tl[i].h, bpr, pxsz, blob)
                                     : xo_encode_tile_m2(tp, tl[i].w, tl[i].h, bpr, blob);
             if (!overflow && total + bs < s) memcpy(out + 8 + total, blob, bs); else overflow = 1;
             total += bs;
         }
         free(blob); free(tl);
+        tr_tile = (uint32_t)N; tr_stream = 0;
+        tr_put(XO_D_FILE, total < s, total, s, N, (uint64_t)mode);
         if (total >= s) { mode = 7; h0 = (uint32_t)(w - 1) | (7u << 24); goto stored; } /* ref :771-777 */
         st32(out, h0); st32(out + 4, h1); size = 8 + total;
         free(px); return size;

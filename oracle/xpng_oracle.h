@@ -63,6 +63,30 @@ int xo_peek(const uint8_t *file, uint64_t n, uint64_t *w, uint64_t *h, int *A, i
 /* .xpng file bytes -> pixels (libxpng.c:963-997).  px capacity w*h*(3+A).  Returns 0 on success. */
 int xo_decode(const uint8_t *file, uint64_t n, uint8_t *px);
 
+/* Decision log: every size comparison the encoder makes, in the order it makes them.  xo_trace(buf, cap) starts a log
+ * of this thread into buf (and empties it); xo_trace(NULL, 0) stops it.  xo_trace_len() is the number of decisions
+ * made since the start, which may exceed cap (only the first cap are stored).  Logging changes no output.
+ *
+ *   kind            outcome (1: first side won)        v[0] vs v[1]: the comparison   v[2], v[3]
+ *   XO_D_T1_TILE    coded (coded < raw)                coded, raw bytes               predictor, npx
+ *   XO_D_FILE       coded (total < s)                  sum of tile sizes, s           tiles, mode
+ *   XO_D_T2_TILE    coded (bsz + rsz < 3 npx)          bsz + rsz, 3 npx               predictor, npx
+ *   XO_D_GREY_PLANE coded (bsz + rsz < npx)            bsz + rsz of the pick, npx     pick, npx
+ *   XO_D_V2_BLOCK   rANS (csz < rawsz)                 csz, rawsz bytes               n, N
+ *   XO_D_V2_TABLE   sparse (N + used pb < N pb)        N + used pb, N pb bits         used, N
+ *   XO_D_V1_BLOCK   rANS (tab + 8 payload < nbit n)    tab + 8 payload, nbit n bits   n, N
+ *   XO_D_V1_TABLE   sparse (tab_sparse < N pb)         (N - used) + used (pb+1), N pb used, N
+ *   XO_D_PRED       the index picked                   v[0..3]: the four predictor costs
+ *   XO_D_GREY_PICK  the index picked                   v[0..3]: the four grey candidates' bsz + rsz
+ *   XO_D_STEAL      the donor                          starved symbol, smallest width >1  symbols of that width, last of them
+ * tile is the tile's index in the image (XO_D_FILE: the tile count); stream is the block's stream: level 1 contexts
+ * 0..8 and alpha 9, level 2 contexts 0..8 and values 9..16 (nl 1..8), grey candidates 0..3; 0 for tile-level kinds. */
+enum { XO_D_T1_TILE = 1, XO_D_FILE, XO_D_T2_TILE, XO_D_GREY_PLANE, XO_D_GREY_PICK, XO_D_V2_BLOCK, XO_D_V2_TABLE,
+       XO_D_V1_BLOCK, XO_D_V1_TABLE, XO_D_PRED, XO_D_STEAL };
+typedef struct xo_decision_t { uint32_t kind, tile, stream, outcome; uint64_t v[4]; } xo_decision_t;
+void xo_trace(xo_decision_t *buf, uint64_t cap);
+uint64_t xo_trace_len(void);
+
 /* Reversible YCoCg-R lifting, the side experiment of Tell_Me_Why/YCoCg-R.c:10-34 (NOT on the
  * .xpng path).  Co and Cg are 9-bit signed. */
 void xo_ycocg_r_fwd(int R, int G, int B, int *Y, int *Co, int *Cg);

@@ -88,12 +88,14 @@ def rans_features(tag, F, pb, n, nwords, out):
         out.add((tag, "dominant"))
 
 
-def walk_v2_block(f, q, end, tag, out):
+def walk_v2_block(f, q, end, tag, out, kinds=None):
     """One self-delimiting level-1 block at q (xo_block_v2_encode); returns (size, n)."""
     _need(q + 4 <= end, f"{tag}: block header past the tile")
     w0 = struct.unpack_from("<I", f, q)[0]
     typ, csz = w0 >> 24, w0 & 0xFFFFFF
     out.add((tag, f"type{typ}"))
+    if kinds is not None:
+        kinds.append(typ)
     _need(q + csz <= end, f"{tag}: block of {csz} bytes runs past the tile")
     if typ == 0:
         _need(csz == 4, f"{tag}: empty block of {csz} bytes")
@@ -120,12 +122,14 @@ def walk_v2_block(f, q, end, tag, out):
     return csz, n
 
 
-def walk_v1_block(f, q, end, N, pb, sb, tag, out):
+def walk_v1_block(f, q, end, N, pb, sb, tag, out, kinds=None):
     """One level-2 block at q (block_v1_encode); its table or raw symbols come next in the side stream sb."""
     _need(q + 4 <= end, f"{tag}: block header past the tile")
     w0 = struct.unpack_from("<I", f, q)[0]
     typ, size = w0 >> 24, w0 & 0xFFFFFF
     out.add((tag, f"type{typ}"))
+    if kinds is not None:
+        kinds.append(typ)
     _need(q + size <= end, f"{tag}: block of {size} bytes runs past the tile")
     if typ == 0:
         _need(size == 4, f"{tag}: empty block of {size} bytes")
@@ -148,7 +152,7 @@ def walk_v1_block(f, q, end, N, pb, sb, tag, out):
     return size, n
 
 
-def walk_tile_m1(f, p, size, npx, A, out):
+def walk_tile_m1(f, p, size, npx, A, out, kinds=None):
     m = f[p + 3]
     if m == 0:
         _need(size == 4 + npx * (3 + A), f"level-1 raw tile of {size} bytes for {npx} pixels")
@@ -161,10 +165,10 @@ def walk_tile_m1(f, p, size, npx, A, out):
     _need(bsz >= 4 + 4 * ((8 * (3 + A) + 31) // 32) and bsz % 4 == 0 and p + 4 + bsz <= end, f"level-1 tile: bsz {bsz}")
     q, nctx = p + 4 + bsz, 0
     for j in range(9):
-        csz, n = walk_v2_block(f, q, end, "v2ctx", out)
+        csz, n = walk_v2_block(f, q, end, "v2ctx", out, kinds)
         q, nctx = q + csz, nctx + n
     if A:
-        csz, n = walk_v2_block(f, q, end, "v2alpha", out)
+        csz, n = walk_v2_block(f, q, end, "v2alpha", out, kinds)
         q += csz
         _need(n == npx - 1 and nctx <= npx - 1, f"level-1 RGBA tile: alpha {n}, contexts {nctx}, npx {npx}")
     else:
@@ -172,7 +176,7 @@ def walk_tile_m1(f, p, size, npx, A, out):
     _need(q == end, f"level-1 tile: blocks end at {q - p}, tile at {size}")
 
 
-def walk_tile_m2(f, p, size, npx, out):
+def walk_tile_m2(f, p, size, npx, out, kinds=None):
     m = f[p + 3]
     end = p + size
     if m == 0:
@@ -196,24 +200,25 @@ def walk_tile_m2(f, p, size, npx, out):
     sb.skip(8 if grey else 24)   # the first pixel
     q = p + 4 + bsz
     if grey:
-        sz, n = walk_v1_block(f, q, end, 256, 15, sb, "v1grey", out)
+        sz, n = walk_v1_block(f, q, end, 256, 15, sb, "v1grey", out, kinds)
         q += sz
         _need(n == npx - 1, f"grey tile: {n} symbols, npx {npx}")
     else:
         nctx = 0
         for j in range(9):
-            sz, n = walk_v1_block(f, q, end, 9, 14, sb, "v1ctx", out)
+            sz, n = walk_v1_block(f, q, end, 9, 14, sb, "v1ctx", out, kinds)
             q, nctx = q + sz, nctx + n
         _need(nctx == npx - 1, f"level-2 tile: contexts hold {nctx} symbols, npx {npx}")
         for N in M2_ALPHABET[1:]:
-            sz, n = walk_v1_block(f, q, end, N, 14, sb, f"v1val{N}", out)
+            sz, n = walk_v1_block(f, q, end, N, 14, sb, f"v1val{N}", out, kinds)
             q += sz
     _need(4 * sb.words() == bsz - 4, f"level-2 tile: side stream uses {4 * sb.words()} bytes of {bsz - 4}")
     _need(q == end, f"level-2 tile: blocks end at {q - p}, tile at {size}")
 
 
-def walk(data, level=None):
-    """Feature set of one .xpng file; `level` is the level it was requested at (1, 2 or 7), if known."""
+def walk(data, level=None, tiles=None):
+    """Feature set of one .xpng file; `level` is the level it was requested at (1, 2 or 7), if known.  If `tiles` is a
+    list, one (tile mode byte, [block type of each block in file order]) per tile is appended to it."""
     f = bytes(data)
     _need(len(f) >= 11, "file shorter than a header and a pixel")
     w0, w1 = struct.unpack_from("<II", f, 0)
@@ -237,10 +242,13 @@ def walk(data, level=None):
         _need(p + 4 <= len(f), "tile header past the file")
         size = struct.unpack_from("<I", f, p)[0] & 0xFFFFFF
         _need(size >= 4 and p + size <= len(f), f"tile of {size} bytes past the file")
+        kinds = []
         if mode == 1:
-            walk_tile_m1(f, p, size, npx, A, out)
+            walk_tile_m1(f, p, size, npx, A, out, kinds)
         else:
-            walk_tile_m2(f, p, size, npx, out)
+            walk_tile_m2(f, p, size, npx, out, kinds)
+        if tiles is not None:
+            tiles.append((f[p + 3], kinds))
         p += size
     _need(p == len(f), f"tiles end at {p}, file at {len(f)}")
     return out
