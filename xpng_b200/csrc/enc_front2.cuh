@@ -2,9 +2,9 @@
 //
 // Same contract as front_segment<MODE, 3> of enc_front.cuh (same SegInfo / chunk / bit layout, so k_tile_scan,
 // k_compact and the assembly are unchanged), about a third of its instructions:
-//   stage    the tile rows that hold raster [r0 - w - 1, r1) are copied with coalesced 128-bit loads into shared
-//            memory as ONE packed byte run (rows back to back), so a pixel's L / U / UL neighbours sit at fixed byte
-//            distances (3, 3w, 3w + 3) whatever the tile's alignment in the image;
+//   stage    the tile rows that hold raster [r0 - w - 1, r1) are copied as aligned 16-byte vectors global -> shared by
+//            cp.async, then repacked in shared memory as ONE packed byte run (rows back to back), so a pixel's L / U / UL
+//            neighbours sit at fixed byte distances (3, 3w, 3w + 3) whatever the tile's alignment in the image;
 //   phase 1  a thread owns 16 consecutive pixels (48 bytes: three 128-bit shared loads, the row above through fourteen
 //            words and one funnel shift each); predictor, residual, zig-zag and bit length are computed on the three
 //            channels at once (byte- or 16-bit-lane arithmetic), everything stays in registers;
@@ -19,27 +19,36 @@
 
 namespace xpb {
 
-#ifndef F2_MINB1
-#define F2_MINB1 4
-#endif
-#ifndef F2_MINB2
-#define F2_MINB2 2
-#endif
+// CTAs per SM (64 registers) at both levels: the kernel waits on latency more than it issues, and at level 2 four CTAs with
+// the spills that 64 registers cost beat two CTAs at 128 registers without them (1000 1080p frames: 25.0 -> 22.1 ms)
+constexpr int F2_MINB = 4;
 constexpr int F2_PADPX = 672;                       // pixels staged before the segment's first (>= FRONT2_MAXW + 2, multiple of 16)
 static_assert(F2_PADPX >= (int)FRONT2_MAXW + 2 && F2_PADPX % 16 == 0, "staging pad");
 constexpr int F2_PIXB = (F2_PADPX + SEG) * 3;       // 14304 bytes
 static_assert(F2_PIXB >= SEG_BITS_BYTES, "the bit area reuses the staged pixels");
+
+// The stage copies the rows of a segment global -> shared by cp.async, all at once when they span at most F2_MAXROWS tile
+// rows (every segment of a tile at least 142 pixels wide), else row by row in each warp.
+constexpr int F2_MAXROWS = 32;
+constexpr int F2_RAWV = F2_PIXB / 16 + 2 * F2_MAXROWS;   // 16-byte slots: the packed run's, plus two per row (lead and tail)
+constexpr int F2_WARPV = F2_RAWV / (FRONT_THREADS / 32); // a warp's slice of them for the rows of narrower tiles
+static_assert(16 * F2_WARPV >= 3 * (SEG / (F2_MAXROWS - 2)) + 30, "a row of a narrow tile fits a warp's slice");
 
 struct Front2Shared {
     union {
         uint32_t pix[F2_PIXB / 4 + 8];              // packed RGB bytes of raster [r0 - F2_PADPX, r0 + SEG)
         uint32_t bits[SEG_BITS_BYTES / 4];          // phase 2 (the pixels are in registers by then): residual bits / value bytes
     };
-    uint8_t sym[SEG];                               // context chunks, concatenated
-    uint8_t cnt[9][FRONT_THREADS];                  // per-thread symbols per context
-    uint16_t pos[9][FRONT_THREADS];                 // per-thread write positions per context (then per value stream, mode 2)
-    uint32_t hist[9 * 16];
-    uint32_t hist2[576];                            // mode 2: value histograms (VAL_OFF)
+    union {
+        uint4 raw[F2_RAWV];                         // stage only: the aligned source vectors of each row, as cp.async lands them
+        struct {                                    // phases 1-3 (zeroed once the stage is done)
+            uint8_t sym[SEG];                       // context chunks, concatenated
+            uint8_t cnt[9][FRONT_THREADS];          // per-thread symbols per context
+            uint16_t pos[9][FRONT_THREADS];         // per-thread write positions per context (then per value stream, mode 2)
+            uint32_t hist[9 * 16];
+            uint32_t hist2[576];                    // mode 2: value histograms (VAL_OFF)
+        };
+    };
     ScanA wa[FRONT_THREADS / 32];
     Cnt9 wc[FRONT_THREADS / 32];
     uint8_t lastnl[FRONT_THREADS];
@@ -49,55 +58,40 @@ struct Front2Shared {
     uint32_t vbytes;
 };
 
-// 16 bytes at a 16-aligned address that may reach past `limit` (the end of the image): bytes past it read as zero.
-__device__ __forceinline__ uint4 f2_ld16(const uint8_t* a, const uint8_t* limit) {
-    if (a + 16 <= limit) return __ldg(reinterpret_cast<const uint4*>(a));
-    uint32_t w[4] = { 0, 0, 0, 0 };
-    for (int k = 0; k < 16; k++) if (a + k < limit) w[k >> 2] |= (uint32_t)__ldg(a + k) << (8 * (k & 3));
-    return make_uint4(w[0], w[1], w[2], w[3]);
+// 16 bytes global -> shared by cp.async (no register holds them); the bytes at and past `limit` (the end of the image)
+// are not read and land as zero.  `a` is 16-aligned and below `limit`.
+__device__ __forceinline__ void f2_cp16(uint4* dst, const uint8_t* a, const uint8_t* limit) {
+    const uint32_t n = a + 16 <= limit ? 16u : (uint32_t)(limit - a);
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;"
+                 :: "r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(a), "r"(n) : "memory");
 }
 
-// Copy nb bytes from global `src` (any alignment) to shared byte offset d of `pixb` (any alignment), one warp.
-// Whole destination words are written as words; the (at most two) words a row shares with its neighbours byte by byte.
-__device__ __forceinline__ void f2_copy_row(uint8_t* pixb, uint32_t d, const uint8_t* src, uint32_t nb, const uint8_t* limit, uint32_t lane) {
-    const uintptr_t sa = reinterpret_cast<uintptr_t>(src);
-    const uint8_t* a0 = reinterpret_cast<const uint8_t*>(sa & ~(uintptr_t)15);
-    const uint32_t lead = (uint32_t)(sa & 15u);                 // bytes of the first vector before the row
+// Write the nb bytes of a row to shared byte offset d of `pixb` (any alignment) from the row's aligned source vectors
+// src[0, nvec) that cp.async has put in shared memory (byte 0 of the row is byte `lead` of src[0]), one warp.  The carry
+// between lanes moves vectors that have already landed.  Whole destination words are written as words; the (at most two)
+// words a row shares with its neighbours byte by byte.
+__device__ __forceinline__ void f2_pack_row(uint8_t* pixb, uint32_t d, const uint4* src, uint32_t lead, uint32_t nb, uint32_t lane) {
     const uint32_t nvec = (lead + nb + 15u) >> 4;
     const int32_t e0 = (int32_t)d - (int32_t)lead;             // destination of byte 0 of vector 0 (may be negative)
     const uint32_t b = (uint32_t)e0 & 3u, sh = 8u * b;
     uint32_t carry = 0;                                         // last word of the vector before this round's first
-    // rounds of 32 vectors, four rounds per batch: all loads of a batch are issued before the first is used (a row of a
-    // 444-pixel tile is three rounds: one exposed memory latency per row instead of three)
-    for (uint32_t vb = 0; vb < nvec + 1; vb += 128) {
-        uint4 VV[4];
+    for (uint32_t v0 = 0; v0 < nvec + 1; v0 += 32) {
+        const uint32_t v = v0 + lane;
+        const uint4 V = v < nvec ? src[v] : make_uint4(0, 0, 0, 0);
+        uint32_t prev = __shfl_up_sync(0xffffffffu, V.w, 1);
+        if (lane == 0) prev = carry;
+        carry = __shfl_sync(0xffffffffu, V.w, 31);
+        if (v <= nvec) {
+            const uint32_t o[4] = { b ? __funnelshift_l(prev, V.x, sh) : V.x, b ? __funnelshift_l(V.x, V.y, sh) : V.y,
+                                    b ? __funnelshift_l(V.y, V.z, sh) : V.z, b ? __funnelshift_l(V.z, V.w, sh) : V.w };
+            const int32_t wb = e0 - (int32_t)b + 16 * (int32_t)v;   // byte offset of the first destination word of this vector
 #pragma unroll
-        for (int r = 0; r < 4; r++) {
-            const uint32_t v = vb + 32u * r + lane;
-            VV[r] = make_uint4(0, 0, 0, 0);
-            if (v < nvec) VV[r] = f2_ld16(a0 + 16ull * v, limit);
-        }
+            for (int i = 0; i < 4; i++) {
+                const int32_t p = wb + 4 * i;
+                if (p >= (int32_t)d && p + 4 <= (int32_t)(d + nb)) *reinterpret_cast<uint32_t*>(pixb + p) = o[i];
+                else if (p + 4 > (int32_t)d && p < (int32_t)(d + nb)) {
 #pragma unroll
-        for (int r = 0; r < 4; r++) {
-            const uint32_t v0 = vb + 32u * r;
-            if (v0 >= nvec + 1) break;                          // warp-uniform
-            const uint32_t v = v0 + lane;
-            const uint4 V = VV[r];
-            uint32_t prev = __shfl_up_sync(0xffffffffu, V.w, 1);
-            if (lane == 0) prev = carry;
-            carry = __shfl_sync(0xffffffffu, V.w, 31);
-            if (v <= nvec) {
-                const uint32_t o[4] = { b ? __funnelshift_l(prev, V.x, sh) : V.x, b ? __funnelshift_l(V.x, V.y, sh) : V.y,
-                                        b ? __funnelshift_l(V.y, V.z, sh) : V.z, b ? __funnelshift_l(V.z, V.w, sh) : V.w };
-                const int32_t wb = e0 - (int32_t)b + 16 * (int32_t)v;   // byte offset of the first destination word of this vector
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    const int32_t p = wb + 4 * i;
-                    if (p >= (int32_t)d && p + 4 <= (int32_t)(d + nb)) *reinterpret_cast<uint32_t*>(pixb + p) = o[i];
-                    else if (p + 4 > (int32_t)d && p < (int32_t)(d + nb)) {
-#pragma unroll
-                        for (int k = 0; k < 4; k++) if (p + k >= (int32_t)d && p + k < (int32_t)(d + nb)) pixb[p + k] = (uint8_t)(o[i] >> (8 * k));
-                    }
+                    for (int k = 0; k < 4; k++) if (p + k >= (int32_t)d && p + k < (int32_t)(d + nb)) pixb[p + k] = (uint8_t)(o[i] >> (8 * k));
                 }
             }
         }
@@ -124,17 +118,51 @@ __device__ __forceinline__ void front2_segment(const FrontArgs& A, Front2Shared&
         const uint8_t* base = A.px + t.src_off;
         // end of the image: the tile's last row may be the image's last row, whose final vector must not read past it
         const uint8_t* limit = base + (uint64_t)(t.h - 1) * t.bpr + (uint64_t)w * 3 + ((uint64_t)t.bpr - (uint64_t)t.x0 * 3 - (uint64_t)w * 3);
-        for (uint32_t y = ys + wid; y <= ye; y += FRONT_THREADS / 32) {
+        // row y: source bytes [src, src + nb) go to packed-run bytes [d, d + nb)
+        auto row = [&](uint32_t y, uint32_t& d, uint32_t& nb) {
             const uint32_t xa = y == ys ? ps - ys * w : 0u, xb = y == ye ? r1 - ye * w : w;
-            const uint32_t d = (y * w + xa + F2_PADPX - r0) * 3u;
-            f2_copy_row(pixb, d, base + (uint64_t)y * t.bpr + (uint64_t)xa * 3, (xb - xa) * 3u, limit, lane);
+            d = (y * w + xa + F2_PADPX - r0) * 3u; nb = (xb - xa) * 3u;
+            return base + (uint64_t)y * t.bpr + (uint64_t)xa * 3;
+        };
+        if (ye - ys < (uint32_t)F2_MAXROWS) {
+            // every load of the segment in flight at once: row y's aligned vectors go to raw slots from (d >> 4) + 2 (y - ys) on
+            // (two slots per row more than the packed run: the lead and the tail vector)
+            for (uint32_t y = ys + wid; y <= ye; y += FRONT_THREADS / 32) {
+                uint32_t d, nb;
+                const uint8_t* src = row(y, d, nb);
+                const uint8_t* a0 = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(src) & ~(uintptr_t)15);
+                const uint32_t nvec = ((uint32_t)(reinterpret_cast<uintptr_t>(src) & 15u) + nb + 15u) >> 4;
+                uint4* dst = S.raw + (d >> 4) + 2 * (y - ys);
+                for (uint32_t v = lane; v < nvec; v += 32) f2_cp16(dst + v, a0 + 16ull * v, limit);
+            }
+            asm volatile("cp.async.wait_all;" ::: "memory");
+            __syncthreads();
+            for (uint32_t y = ys + wid; y <= ye; y += FRONT_THREADS / 32) {
+                uint32_t d, nb;
+                const uint8_t* src = row(y, d, nb);
+                f2_pack_row(pixb, d, S.raw + (d >> 4) + 2 * (y - ys), (uint32_t)(reinterpret_cast<uintptr_t>(src) & 15u), nb, lane);
+            }
+        } else {
+            // narrow tile (w <= SEG / (F2_MAXROWS - 2)): each warp stages its rows one at a time through its own slice of raw[]
+            uint4* dst = S.raw + wid * F2_WARPV;
+            for (uint32_t y = ys + wid; y <= ye; y += FRONT_THREADS / 32) {
+                uint32_t d, nb;
+                const uint8_t* src = row(y, d, nb);
+                const uint8_t* a0 = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(src) & ~(uintptr_t)15);
+                const uint32_t lead = (uint32_t)(reinterpret_cast<uintptr_t>(src) & 15u), nvec = (lead + nb + 15u) >> 4;
+                for (uint32_t v = lane; v < nvec; v += 32) f2_cp16(dst + v, a0 + 16ull * v, limit);
+                asm volatile("cp.async.wait_all;" ::: "memory");
+                __syncwarp();
+                f2_pack_row(pixb, d, dst, lead, nb, lane);
+                __syncwarp();                                   // the slice is free for the warp's next row
+            }
         }
     }
+    __syncthreads();                                            // the packed run is complete, raw[] is free
     if (tid < 144) S.hist[tid] = 0;
     if (MODE == 2) for (uint32_t k = tid; k < 576; k += FRONT_THREADS) S.hist2[k] = 0;
 #pragma unroll
     for (int c = 0; c < 9; c++) S.cnt[c][tid] = 0;
-    __syncthreads();
 
     // ---------------- phase 1: 16 consecutive pixels per thread, all in registers
     uint32_t fld[16];             // mode 1: residual bit field; mode 2: zig-zagged residual bytes u0 | u1 << 8 | u2 << 16
@@ -333,7 +361,7 @@ __device__ __forceinline__ void front2_segment(const FrontArgs& A, Front2Shared&
 }
 
 template <int MODE>
-__global__ void __launch_bounds__(FRONT_THREADS, MODE == 1 ? F2_MINB1 : F2_MINB2) k_front2(FrontArgs A) {
+__global__ void __launch_bounds__(FRONT_THREADS, F2_MINB) k_front2(FrontArgs A) {
     __shared__ __align__(16) Front2Shared S;
     const uint32_t gseg = blockIdx.x, tile = A.seg_tile[gseg];
     const TileDesc t = A.tiles[tile];
